@@ -300,10 +300,17 @@ def load_traffic():
     return None
 
 
+def dump_outputs(dirname, outputs):
+    """Write each array as <dirname>/<name>.npy in float64 (exact here: integers below 2**53, 32-bit generator words)."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed passes per leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=10_000_000, help="rows of the whole-genome .mut (default: configs[1])")
@@ -312,7 +319,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config3", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs: device-resident leg only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed device-resident pass returned (rank 0's pair) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this project's timed pass computed; --impl reference runs the reference CLI")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -388,6 +401,7 @@ def main():
             h.ingest_colate_in(slot, img, sites.chr_names)               # records -> genome arrays on the GPU
 
     acc = {}
+    last = {}                           # what the last pass returned to its caller (--dump-outputs)
 
     def one_pass():
         s1 = h.stage1(api.mt_seed(SEED), fetch=False)                    # block histograms stay on the device
@@ -401,6 +415,8 @@ def main():
         t2 = time.perf_counter()
         acc.setdefault("bootstrap_wall_ms", []).append((t1 - t0) * 1e3)
         acc.setdefault("em_wall_ms", []).append((t2 - t1) * 1e3)
+        last.update(num_blocks=[s1.num_blocks], n_used=[s1.n_used], mt_state=s1.mt_state, block_weights=w,
+                    rates=rates, em_iterations=iters, log_likelihood=ll)
         return s1, rates, iters
 
     # pipelined form: the EM of the previous pass is still running (EM stream) while this pass is uploaded and taken
@@ -472,6 +488,8 @@ def main():
     launches0 = h.launch_count()
     ms_res, (s1, rates, iters) = timed(one_pass, args.steps)
     launches = h.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"epochs": ep, **last})
     t_stage = {k: float(np.mean(v)) for k, v in acc.items() if k.endswith("_ms")}
     rates_soa = rates.copy()
     # the same device-resident passes with the EM of pass i under stage i of pass i+1 (not the headline `value`: its stage-i
@@ -500,8 +518,8 @@ def main():
 
         for _ in range(2):
             e2e_pass()
-        ms_e2e_serial, (s1f, rates_f, iters_f) = timed(e2e_pass, max(3, args.steps // 2))
-        ms_e2e_serial /= max(3, args.steps // 2)
+        ms_e2e_serial, (s1f, rates_f, iters_f) = timed(e2e_pass, args.steps)
+        ms_e2e_serial /= args.steps
         if not (np.array_equal(rates_f, rates_soa) and s1f.n_used == s1.n_used):
             raise SystemExit("bench.py: the pass from the file bytes and the pass from the parsed arrays disagree")
         for _ in range(2):
