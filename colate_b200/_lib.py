@@ -65,6 +65,7 @@ SIGNATURES = {
     "colate_stage3_em": (C.c_int, [VP, C.c_int, C.c_int, VP, VP, VP, C.c_int, VP, VP, VP]),
     "colate_stage3_em_begin": (C.c_int, [VP, C.c_int, C.c_int, VP, VP, C.c_int]),
     "colate_stage3_em_end": (C.c_int, [VP, VP, VP, VP]),
+    "colate_stage3_em_grids": (C.c_int, [VP, C.c_int, i32, C.c_int, i32, i64, f64, f64, f64, C.c_int, f64, i32, f64]),
     "colate_set_age_bins": (C.c_int, [VP, VP]),
     "colate_estep": (C.c_int, [VP, C.c_int, C.c_int, VP, VP, C.c_int, VP, VP, VP, VP]),
     "colate_libm_exact": (C.c_int, []),

@@ -394,6 +394,25 @@ class Handle:
         check(lib().colate_stage3_em_end(self._h, ptr(rates), ptr(iters), ptr(ll)))
         return rates, iters, ll
 
+    def stage3_em_grids(self, grid_of, grids, counts, max_iter=100000):
+        """EM of R replicates on mixed epoch grids (colate_stage3_em_grids): grids = [(epochs, rates_init)], replicate r runs on
+        grids[grid_of[r]] with counts[r] ([R][2][185]).  Returns (rates[R][E_max] zero-padded, iters[R], ll[R]); row r equals
+        stage3_em(1, *grids[grid_of[r]], counts[r:r+1]) bit for bit."""
+        go = np.ascontiguousarray(grid_of, dtype=np.int32)
+        R = go.shape[0]
+        eps = [np.ascontiguousarray(e, dtype=np.float64) for e, _ in grids]
+        ris = [np.ascontiguousarray(r, dtype=np.float64) for _, r in grids]
+        gE = np.array([e.shape[0] for e in eps], dtype=np.int32)
+        assert all(r.shape == e.shape for e, r in zip(eps, ris))
+        goff = np.concatenate([[0], np.cumsum(gE)[:-1]]).astype(np.int64)
+        cn = np.ascontiguousarray(counts, dtype=np.float64)
+        assert cn.shape == (R, 2, NBINS)
+        E_max = int(gE.max())
+        rates = np.zeros((R, E_max)); iters = np.zeros(R, dtype=np.int32); ll = np.zeros(R)
+        check(lib().colate_stage3_em_grids(self._h, R, go, len(eps), gE, goff, np.concatenate(eps), np.concatenate(ris),
+                                           cn.reshape(-1), max_iter, rates.reshape(-1), iters, ll))
+        return rates, iters, ll
+
     def estep(self, shared: bool, epochs, rates, t):
         ep = np.ascontiguousarray(epochs, dtype=np.float64)
         r = np.ascontiguousarray(rates, dtype=np.float64)

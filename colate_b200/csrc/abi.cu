@@ -151,7 +151,7 @@ void colate_destroy(colate_handle* h)
                     &h->chr_used, &h->chr_blocks, &h->chr_block_base, &h->misc, &h->u_hdr, &h->u_eb2, &h->u_ews, &h->u_ewn, &h->u_cnt,
                     &h->u_blk, &h->blk_rank_start, &h->out_f, &h->out_n, &h->thrA, &h->lut, &h->d_scratch, &h->d_prof, &h->libm_tab, &h->ing_text, &h->ing_tile_cnt, &h->ing_tile_off, &h->ing_nl, &h->ing_status, &h->ing_fb,
                     &h->windows, &h->rng_stream, &h->mt_tail, &h->poly, &h->thr10, &h->d_counts, &h->d_blockstats, &h->d_weights, &h->d_epochs,
-                    &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo};
+                    &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo};
   for (DevBuf* b : bufs) b->release();
   for (auto& g : h->genomes) {
     DevBuf* gb[] = {&g.bp, &g.aaf, &g.daf, &g.alleles, &g.chr_first, &g.chr_end, &g.mask_bits, &g.j_aaf, &g.j_daf, &g.j_prevbp, &g.j_flag, &g.pile};
@@ -679,6 +679,93 @@ int colate_stage3_em_end(colate_handle* h, double* rates, int32_t* iters, double
   CK(cudaStreamSynchronize(s));
   for (int r = 0; r < R; r++)
     if (it_host[r] < 0) return fail(COLATE_ERR_CUDA, "EM kernel: the cluster handshake timed out (replicate " + std::to_string(r) + ")");
+  return 0;
+}
+
+// ---- mixed epoch grids: one k_em_cta_grids launch for every replicate whose grid fits it --------------------------------
+int colate_stage3_em_grids(colate_handle* h, int R, const int32_t* grid_of, int n_grids, const int32_t* grid_E, const int64_t* grid_off,
+                           const double* epochs, const double* rates_init, const double* counts, int max_iter, double* rates, int32_t* iters,
+                           double* final_ll)
+{
+  if (!h || R <= 0 || n_grids <= 0 || !grid_of || !grid_E || !grid_off || !epochs || !rates_init || !counts || max_iter < 0 || !rates ||
+      !iters || !final_ll)
+    return fail(COLATE_ERR_ARG, "colate_stage3_em_grids: bad arguments");
+  int E_max = 0;
+  for (int g = 0; g < n_grids; g++) {
+    if (grid_E[g] < 2 || grid_E[g] > 1024 || grid_off[g] < 0) return fail(COLATE_ERR_ARG, "colate_stage3_em_grids: bad grid " + std::to_string(g));
+    E_max = std::max(E_max, (int)grid_E[g]);
+  }
+  for (int r = 0; r < R; r++)
+    if (grid_of[r] < 0 || grid_of[r] >= n_grids) return fail(COLATE_ERR_ARG, "colate_stage3_em_grids: grid_of[" + std::to_string(r) + "] out of range");
+  if (h->em_inflight) return fail(COLATE_ERR_STATE, "colate_stage3_em_grids: an EM is in flight (colate_stage3_em_begin): call colate_stage3_em_end first");
+  CK(cudaSetDevice(h->device));
+  int rc = ensure_tables(h);
+  if (rc) return rc;
+  constexpr int C2 = 2 * NBINS;
+  std::vector<int> cap(n_grids, 0), fits(n_grids, 0);
+  size_t smem = 0;
+  int64_t ep_len = 0;
+  for (int g = 0; g < n_grids; g++) {
+    size_t sm = 0;
+    fits[g] = em_cta_fits(h, grid_E[g], epochs + grid_off[g], &cap[g], &sm) ? 1 : 0;
+    if (fits[g]) { smem = std::max(smem, sm); ep_len = std::max(ep_len, grid_off[g] + grid_E[g]); }
+  }
+  memset(rates, 0, (size_t)R * E_max * 8);
+  auto put = [&](int r, const double* row, int E, int32_t it, double l) {
+    memcpy(rates + (size_t)r * E_max, row, (size_t)E * 8);
+    iters[r] = it;
+    final_ll[r] = l;
+  };
+  // grids the throughput kernel does not fit (shared memory or thread bound): colate_stage3_em on each of them alone
+  for (int g = 0; g < n_grids; g++) {
+    if (fits[g]) continue;
+    std::vector<int> reps;
+    for (int r = 0; r < R; r++) if (grid_of[r] == g) reps.push_back(r);
+    if (reps.empty()) continue;
+    const int n = (int)reps.size(), E = grid_E[g];
+    std::vector<double> cn((size_t)n * C2), rt((size_t)n * E), l2(n);
+    std::vector<int32_t> it(n);
+    for (int k = 0; k < n; k++) memcpy(cn.data() + (size_t)k * C2, counts + (size_t)reps[k] * C2, C2 * 8);
+    if ((rc = colate_stage3_em(h, n, E, epochs + grid_off[g], rates_init + grid_off[g], cn.data(), max_iter, rt.data(), it.data(), l2.data())))
+      return rc;
+    for (int k = 0; k < n; k++) put(reps[k], rt.data() + (size_t)k * E, E, it[k], l2[k]);
+  }
+  std::vector<int> reps;
+  for (int r = 0; r < R; r++) if (fits[grid_of[r]]) reps.push_back(r);
+  h->counts_R = 0;   // d_counts no longer holds the last colate_stage2_bootstrap's counts
+  if (reps.empty()) return 0;
+  const int n = (int)reps.size();
+  cudaStream_t s = h->stream;
+  std::vector<int32_t> tab((size_t)n + 4 * (size_t)n_grids, 0);   // grid_of of the launch's replicates, then int4 {E, offset, n_pairs_cap, 0}
+  std::vector<double> cn((size_t)n * C2);
+  for (int k = 0; k < n; k++) {
+    tab[k] = grid_of[reps[k]];
+    memcpy(cn.data() + (size_t)k * C2, counts + (size_t)reps[k] * C2, C2 * 8);
+  }
+  const size_t info0 = ((size_t)n + 3) & ~(size_t)3;   // int4-aligned
+  tab.resize(info0 + 4 * (size_t)n_grids, 0);
+  for (int g = 0; g < n_grids; g++)
+    if (fits[g]) { tab[info0 + 4 * g] = grid_E[g]; tab[info0 + 4 * g + 1] = (int32_t)grid_off[g]; tab[info0 + 4 * g + 2] = cap[g]; }
+  CK(h->d_gr_tab.ensure(tab.size() * 4));
+  CK(h->d_epochs.ensure((size_t)ep_len * 8));
+  CK(h->d_rates.ensure((size_t)ep_len * 8));
+  CK(h->d_counts.ensure((size_t)n * C2 * 8));
+  CK(h->d_gr_rates.ensure((size_t)n * E_max * 8));
+  CK(h->d_iters.ensure((size_t)n * 4));
+  CK(h->d_ll.ensure((size_t)n * 8));
+  CK(cudaMemcpyAsync(h->d_gr_tab.p, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(h->d_epochs.p, epochs, (size_t)ep_len * 8, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(h->d_rates.p, rates_init, (size_t)ep_len * 8, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(h->d_counts.p, cn.data(), (size_t)n * C2 * 8, cudaMemcpyHostToDevice, s));
+  const int32_t* d_tab = h->d_gr_tab.as<int32_t>();
+  if ((rc = run_em_grids(h, n, d_tab, d_tab + info0, E_max, smem, max_iter, s))) return rc;
+  std::vector<double> rt((size_t)n * E_max), l2(n);
+  std::vector<int32_t> it(n);
+  CK(cudaMemcpyAsync(rt.data(), h->d_gr_rates.p, (size_t)n * E_max * 8, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(it.data(), h->d_iters.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(l2.data(), h->d_ll.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  for (int k = 0; k < n; k++) put(reps[k], rt.data() + (size_t)k * E_max, E_max, it[k], l2[k]);
   return 0;
 }
 

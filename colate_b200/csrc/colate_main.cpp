@@ -39,7 +39,7 @@ const char* kValueOpts[] = {"mode", "anc", "mut", "target_bcf", "reference_bcf",
                             "anc_genome", "mask", "mask_cutoff", "chr", "bins", "lineage_bin", "outgroup_tmrca", "years_per_gen",
                             "coal", "seed", "num_bootstraps", "filters", "groups", "poplabels", "map", "input", "output",
                             // additions of this build
-                            "num_bootstrap", "device", "devices"};
+                            "num_bootstrap", "device", "devices", "pairs"};
 
 void help()
 {
@@ -47,6 +47,12 @@ void help()
                "         [--chr <file>] [--target_mask <prefix>] [--reference_mask <prefix>] [--target_age <years>]\n"
                "         [--reference_age <years>] [--years_per_gen <float>] [--coal <file>] [--seed <int>]\n"
                "         [--num_bootstraps <int>] [--device <int> | --devices <i,j,...>] [--host_parse] -o <output prefix>\n"
+               "  Colate --mode mut --mut <prefix> --pairs <file> --seed <int> (--bins x,y,step | --coal <file>) [--chr <file>]\n"
+               "         [--years_per_gen <float>] [--num_bootstraps <int>] [--devices <i,j,...>] [--host_parse]\n"
+               "    a cohort in one job: every non-blank line of <file> not starting with '#' is one run\n"
+               "      <target_tmp> <reference_tmp> <output_prefix> [target_age=<years>] [reference_age=<years>]\n"
+               "      [target_mask=<prefix>] [reference_mask=<prefix>]\n"
+               "    with the shared flags; each line's .coal / .bin equal those of the single-pair run with the same flags\n"
             << std::endl;
 }
 
@@ -488,6 +494,382 @@ int run_mut(const Options& options)
   return 0;
 }
 
+// ---- --pairs: a cohort of target / reference runs in one job ------------------------------------------------------------
+// Every line is the run `Colate --mode mut --target_tmp T --reference_tmp R -o OUT [--target_age ..] ...` with the shared
+// flags, and its .coal / .bin are those of that run.  The .mut text is parsed once per device, every genome (a .colate.in
+// file under one mask) is decoded once into a slot of its own, all pairs consume prefixes of the one --seed generator
+// stream (colate_set_stream_cache), and the EM of all pairs' replicates runs on their mixed epoch grids in one launch
+// (colate_stage3_em_grids).
+struct PairLine {
+  int line = 0;
+  std::string tmp[2], out, age[2], mask[2];
+  bool has_age[2] = {false, false};
+  int genome[2] = {-1, -1};   // index into the job's genome list
+  bool cached = false;        // <out>.colate_mat exists: the reference's stale-cache path
+  // results
+  std::string err;
+  int num_blocks = 0, E = 0, ep_null = 0, grid = -1;
+  int64_t n_used = 0;
+  double age_gen = 0.0;
+  std::vector<double> epochs, rates_init, counts, rates, ll;
+  std::vector<int32_t> iters;
+};
+
+struct GenomeKey { std::string tmp, mask; bool operator<(const GenomeKey& o) const { return tmp != o.tmp ? tmp < o.tmp : mask < o.mask; } };
+
+// The pairs file, checked completely before any device is touched.  false: the message (naming the line) is on stderr.
+bool read_pairs_file(const std::string& path, std::vector<PairLine>& pl, std::vector<GenomeKey>& genomes)
+{
+  std::ifstream is(path);
+  if (is.fail()) { std::cerr << "Error: cannot open the pairs file " << path << std::endl; return false; }
+  std::map<GenomeKey, int> gidx;
+  std::map<std::string, int> out_line;
+  std::string text;
+  int ln = 0;
+  auto bad = [&](const std::string& what) { std::cerr << "Error in pairs file " << path << ", line " << ln << ": " << what << std::endl; return false; };
+  while (std::getline(is, text)) {
+    ln++;
+    std::stringstream ss(text);
+    std::vector<std::string> f;
+    std::string tok;
+    while (ss >> tok) f.push_back(tok);
+    if (f.empty() || f[0][0] == '#') continue;
+    if (f.size() < 3) return bad("expected <target_tmp> <reference_tmp> <output_prefix> [key=value ...], found " + std::to_string(f.size()) + " field(s)");
+    PairLine p;
+    p.line = ln;
+    p.tmp[0] = f[0]; p.tmp[1] = f[1]; p.out = f[2];
+    std::set<std::string> seen;
+    for (size_t k = 3; k < f.size(); k++) {
+      const size_t eq = f[k].find('=');
+      if (eq == std::string::npos || eq == 0 || eq + 1 == f[k].size()) return bad("'" + f[k] + "' is not of the form key=value");
+      const std::string key = f[k].substr(0, eq), val = f[k].substr(eq + 1);
+      if (!seen.insert(key).second) return bad("'" + key + "' is given twice");
+      if (key == "target_age") { p.age[0] = val; p.has_age[0] = true; }
+      else if (key == "reference_age") { p.age[1] = val; p.has_age[1] = true; }
+      else if (key == "target_mask") p.mask[0] = val;
+      else if (key == "reference_mask") p.mask[1] = val;
+      else return bad("unknown key '" + key + "' (known: target_age, reference_age, target_mask, reference_mask)");
+    }
+    auto dup = out_line.find(p.out);
+    if (dup != out_line.end()) return bad("output prefix " + p.out + " is already used on line " + std::to_string(dup->second));
+    out_line[p.out] = ln;
+    for (int g = 0; g < 2; g++) {
+      FILE* fp = fopen(p.tmp[g].c_str(), "rb");
+      if (!fp) return bad("cannot read " + p.tmp[g]);
+      fclose(fp);
+      const GenomeKey key{p.tmp[g], p.mask[g]};
+      auto it = gidx.find(key);
+      if (it == gidx.end()) {
+        if ((int)genomes.size() == COLATE_MAX_GENOMES)
+          return bad("more than " + std::to_string(COLATE_MAX_GENOMES) + " distinct genomes ((.colate.in, mask) combinations) in one job");
+        it = gidx.emplace(key, (int)genomes.size()).first;
+        genomes.push_back(key);
+      }
+      p.genome[g] = it->second;
+    }
+    p.cached = file_exists(p.out + ".colate_mat");
+    pl.push_back(p);
+  }
+  if (pl.empty()) { std::cerr << "Error: the pairs file " << path << " lists no pair" << std::endl; return false; }
+  return true;
+}
+
+int run_cohort(const Options& options)
+{
+  const std::string pairs_path = options.get("pairs");
+  for (const char* k : {"target_tmp", "reference_tmp", "output", "target_age", "reference_age", "target_mask", "reference_mask", "target_bcf",
+                        "reference_bcf", "target_bam", "reference_bam", "device"})
+    if (options.count(k)) {
+      std::cerr << "Error: --" << (strcmp(k, "output") ? k : "output/-o") << " cannot be combined with --pairs (give it per line of the pairs file"
+                << (strcmp(k, "device") ? "" : "; use --devices") << ")" << std::endl;
+      return 1;
+    }
+  if (!options.count("mut")) { std::cerr << "Error: --pairs needs --mut" << std::endl; return 1; }
+  if (!options.count("seed")) { std::cerr << "Error: --pairs needs --seed (all pairs share the generator stream of that seed)" << std::endl; return 1; }
+  if (!options.count("bins") && !options.count("coal")) { std::cerr << "Error: --bins or --coal is required." << std::endl; return 1; }
+  std::vector<PairLine> pl;
+  std::vector<GenomeKey> genomes;
+  if (!read_pairs_file(pairs_path, pl, genomes)) return 1;
+
+  const int seed = atoi(options.get("seed").c_str());
+  int R = 1;
+  if (options.count("num_bootstraps")) R = atoi(options.get("num_bootstraps").c_str());
+  else if (options.count("num_bootstrap")) R = atoi(options.get("num_bootstrap").c_str());
+  if (R < 0) R = 0;
+  const bool has_ypg = options.count("years_per_gen");
+  const float ypg_flag = has_ypg ? strtof(options.get("years_per_gen").c_str(), nullptr) : 0.0f;
+  std::vector<int> dev_ids;
+  {
+    std::stringstream ss(options.count("devices") ? options.get("devices") : "0");
+    std::string tok;
+    while (std::getline(ss, tok, ',')) if (!tok.empty()) dev_ids.push_back(atoi(tok.c_str()));
+    if (dev_ids.empty()) dev_ids.push_back(0);
+  }
+  const int G = (int)dev_ids.size();
+  std::cerr << "Cohort: " << pl.size() << " pairs, " << genomes.size() << " genomes, " << G << " device(s)" << std::endl;
+
+  // file lists, coal.cpp:3290-3316
+  std::vector<std::string> name_chr, f_mut;
+  if (options.count("chr")) {
+    std::ifstream is(options.get("chr"));
+    if (is.fail()) std::cerr << "Error while opening file " << options.get("chr") << std::endl;
+    std::string line;
+    while (std::getline(is, line)) { name_chr.push_back(line); f_mut.push_back(options.get("mut") + "_chr" + line + ".mut"); }
+  } else {
+    name_chr.push_back("");
+    f_mut.push_back(options.get("mut"));
+  }
+  const int n_chr = (int)name_chr.size();
+  {
+    std::set<std::string> uniq(name_chr.begin(), name_chr.end());
+    if ((int)uniq.size() != n_chr) { std::cerr << "Duplicate chromosome names in --chr" << std::endl; return 1; }
+  }
+  auto mask_file = [&](const std::string& prefix, int c) { return options.count("chr") ? prefix + "_chr" + name_chr[c] + ".fa" : prefix; };
+  std::vector<const char*> names;
+  for (auto& s : name_chr) names.push_back(s.c_str());
+  bool any_live = false, any_mask = false;
+  for (auto& p : pl)
+    if (!p.cached) { any_live = true; any_mask = any_mask || !p.mask[0].empty() || !p.mask[1].empty(); }
+  // the .mut text, read once for all devices: parsed on the GPU, or by the host reader (zlib) if a file only exists as .gz
+  std::vector<std::vector<char>> texts(n_chr);
+  bool all_plain = !options.count("host_parse");
+  struct SitesHost { std::vector<int64_t> off; std::vector<int32_t> pos; std::vector<float> ab, ae; std::vector<uint32_t> meta; } sh;
+  if (any_live) {
+    for (int c = 0; c < n_chr && all_plain; c++) {
+      FILE* f = fopen(f_mut[c].c_str(), "rb");
+      if (!f) { all_plain = false; break; }
+      fseek(f, 0, SEEK_END);
+      const long sz = ftell(f);
+      fseek(f, 0, SEEK_SET);
+      texts[c].resize((size_t)std::max(sz, 0L));
+      if (sz > 0 && fread(texts[c].data(), 1, (size_t)sz, f) != (size_t)sz) all_plain = false;
+      fclose(f);
+    }
+    if (!all_plain) {
+      sh.off.assign(n_chr + 1, 0);
+      for (int c = 0; c < n_chr; c++) {
+        const int64_t n = colate_read_mut(f_mut[c].c_str(), 0, nullptr, nullptr, nullptr, nullptr);
+        if (n < 0) { std::cerr << colate_last_error() << std::endl; return 1; }
+        const size_t o = sh.pos.size();
+        sh.pos.resize(o + n); sh.ab.resize(o + n); sh.ae.resize(o + n); sh.meta.resize(o + n);
+        if (colate_read_mut(f_mut[c].c_str(), n, sh.pos.data() + o, sh.ab.data() + o, sh.ae.data() + o, sh.meta.data() + o) < 0) {
+          std::cerr << colate_last_error() << std::endl;
+          return 1;
+        }
+        sh.off[c + 1] = (int64_t)sh.pos.size();
+      }
+    }
+  }
+  // the epoch grid of an age, coal.cpp:3503-3646
+  auto grid_of_age = [&](PairLine& p, double ypg) -> bool {
+    p.epochs.assign(4096, 0.0);
+    p.rates_init.assign(4096, 1.0 / 20000.0);
+    p.ep_null = 0;
+    if (options.count("coal")) p.E = colate_epochs_from_coal_file(options.get("coal").c_str(), p.age_gen, p.epochs.data(), p.rates_init.data(), 4096);
+    else p.E = colate_epochs_from_bins(options.get("bins").c_str(), p.age_gen, ypg, p.epochs.data(), 4096, &p.ep_null);
+    if (p.E < 0) { p.err = std::string(options.count("coal") ? "--coal" : "--bins") + ": " + colate_last_error(); return false; }
+    p.epochs.resize(p.E);
+    p.rates_init.resize(p.E);
+    return true;
+  };
+  uint32_t mt0[COLATE_MT_WORDS];
+  colate_mt_seed((uint32_t)seed, mt0);
+  constexpr int C2 = 2 * COLATE_NUM_AGE_BINS;
+  constexpr int kEmBatch = 2048;   // replicates per EM launch
+  std::vector<std::string> dev_err(G);
+
+  // one host thread per device; pairs are dealt round-robin in file order
+  auto work = [&](int g) {
+    std::vector<PairLine*> mine;
+    for (size_t k = g; k < pl.size(); k += G) mine.push_back(&pl[k]);
+    if (mine.empty()) return;
+    colate_handle* h = nullptr;
+    auto dev_fail = [&](const std::string& what) {
+      dev_err[g] = "device " + std::to_string(dev_ids[g]) + ": " + what + ": " + colate_last_error();
+      for (PairLine* p : mine) if (p->err.empty()) p->err = dev_err[g];
+    };
+    if (colate_create(dev_ids[g], &h)) { dev_fail("colate_create"); return; }
+    struct Destroy { colate_handle* h; ~Destroy() { colate_destroy(h); } } destroy{h};
+    bool live = false, masked = false;
+    for (PairLine* p : mine) if (!p->cached) { live = true; masked = masked || !p->mask[0].empty() || !p->mask[1].empty(); }
+    if (live) {
+      // sites (coal.cpp:2148-2176), then every genome this device needs, decoded into its own slot and masked there
+      std::vector<int64_t> site_off(n_chr + 1, 0);
+      std::vector<int32_t> pos;
+      if (all_plain) {
+        int64_t bytes = 0;
+        for (auto& t : texts) bytes += (int64_t)t.size();
+        if (colate_ingest_begin(h, n_chr, bytes / 20 + n_chr)) { dev_fail("colate_ingest_begin"); return; }
+        for (int c = 0; c < n_chr; c++) {
+          const int64_t n = colate_ingest_mut_text(h, texts[c].data(), (int64_t)texts[c].size(), 0);
+          if (n < 0) { dev_fail("colate_ingest_mut_text"); return; }
+          site_off[c + 1] = site_off[c] + n;
+        }
+        if (colate_ingest_end(h)) { dev_fail("colate_ingest_end"); return; }
+        if (masked) {
+          pos.resize((size_t)site_off[n_chr]);
+          if (colate_ingest_fetch(h, 0, site_off[n_chr], pos.data(), nullptr, nullptr, nullptr)) { dev_fail("colate_ingest_fetch"); return; }
+        }
+      } else {
+        site_off = sh.off;
+        if (colate_set_sites(h, n_chr, sh.off.data(), sh.pos.data(), sh.ab.data(), sh.ae.data(), sh.meta.data(), 0)) { dev_fail("colate_set_sites"); return; }
+        pos = sh.pos;
+      }
+      std::map<int, int> slot_of;     // genome -> slot on this device
+      std::map<int, std::string> genome_err;
+      for (PairLine* p : mine) {
+        if (p->cached) continue;
+        for (int k = 0; k < 2; k++) {
+          const int gi = p->genome[k];
+          if (slot_of.count(gi)) continue;
+          const int slot = (int)slot_of.size();
+          slot_of[gi] = slot;
+          std::vector<char> image;
+          FILE* f = fopen(genomes[gi].tmp.c_str(), "rb");
+          if (!f) { genome_err[gi] = "cannot read " + genomes[gi].tmp; continue; }
+          fseek(f, 0, SEEK_END);
+          const long sz = ftell(f);
+          fseek(f, 0, SEEK_SET);
+          image.resize((size_t)std::max(sz, 0L));
+          const bool short_read = sz > 0 && fread(image.data(), 1, (size_t)sz, f) != (size_t)sz;
+          fclose(f);
+          if (short_read) { genome_err[gi] = "short read on " + genomes[gi].tmp; continue; }
+          if (colate_ingest_colate_in(h, slot, image.data(), (int64_t)image.size(), n_chr, names.data(), 0) < 0) {
+            genome_err[gi] = genomes[gi].tmp + ": " + colate_last_error();
+            continue;
+          }
+          if (genomes[gi].mask.empty()) continue;
+          std::vector<uint32_t> bits(((size_t)site_off[n_chr] + 31) / 32 + 1, 0);
+          bool ok = true;
+          for (int c = 0; c < n_chr && ok; c++)
+            ok = !colate_mask_bits_from_fasta(mask_file(genomes[gi].mask, c).c_str(), site_off[c + 1] - site_off[c], pos.data() + site_off[c], site_off[c],
+                                              bits.data());
+          if (ok) ok = !colate_set_mask(h, slot, bits.data(), 0);
+          if (!ok) genome_err[gi] = "mask " + genomes[gi].mask + ": " + colate_last_error();
+        }
+      }
+      // stages i-ii per pair (coal.cpp:3317-3451) and its epoch grid
+      if (colate_set_stream_cache(h, 1)) { dev_fail("colate_set_stream_cache"); return; }
+      for (PairLine* p : mine) {
+        if (p->cached) continue;
+        for (int k = 0; k < 2 && p->err.empty(); k++)
+          if (genome_err.count(p->genome[k])) p->err = genome_err[p->genome[k]];
+        if (!p->err.empty()) continue;
+        double ypg = 28.0;
+        p->age_gen = colate_age_generations(p->has_age[0] ? p->age[0].c_str() : nullptr, p->has_age[1] ? p->age[1].c_str() : nullptr, has_ypg, ypg_flag, &ypg);
+        uint32_t mt[COLATE_MT_WORDS];
+        if (colate_stage1(h, slot_of[p->genome[0]], slot_of[p->genome[1]], mt0, &p->num_blocks, nullptr, nullptr, &p->n_used, mt)) {
+          p->err = std::string("stage i: ") + colate_last_error();
+          continue;
+        }
+        if (R > 0) {
+          std::vector<int32_t> w((size_t)R * p->num_blocks);
+          colate_draw_block_weights(mt, R, p->num_blocks, w.data());
+          p->counts.assign((size_t)R * C2, 0.0);
+          if (colate_stage2_bootstrap(h, R, p->num_blocks, w.data(), nullptr, p->age_gen, p->counts.data())) {
+            p->err = std::string("stage ii: ") + colate_last_error();
+            continue;
+          }
+        }
+        grid_of_age(*p, ypg);
+      }
+      colate_set_stream_cache(h, 0);
+      // stage iii: every replicate of every pair on its own grid, kEmBatch replicates per launch (coal.cpp:3675-3827)
+      if (R > 0) {
+        std::vector<PairLine*> run;
+        for (PairLine* p : mine) if (!p->cached && p->err.empty()) run.push_back(p);
+        for (size_t b0 = 0; b0 < run.size();) {
+          size_t b1 = b0;
+          while (b1 < run.size() && (int)(b1 - b0 + 1) * R <= std::max(kEmBatch, R)) b1++;
+          std::map<std::vector<double>, int> gidx;   // grids (epochs then initial rates) of this launch
+          std::vector<int32_t> grid_E, grid_of;
+          std::vector<int64_t> grid_off;
+          std::vector<double> ep, init, cn;
+          for (size_t k = b0; k < b1; k++) {
+            PairLine* p = run[k];
+            std::vector<double> key(p->epochs);
+            key.insert(key.end(), p->rates_init.begin(), p->rates_init.end());
+            auto it = gidx.find(key);
+            if (it == gidx.end()) {
+              it = gidx.emplace(key, (int)grid_E.size()).first;
+              grid_E.push_back(p->E);
+              grid_off.push_back((int64_t)ep.size());
+              ep.insert(ep.end(), p->epochs.begin(), p->epochs.end());
+              init.insert(init.end(), p->rates_init.begin(), p->rates_init.end());
+            }
+            for (int r = 0; r < R; r++) grid_of.push_back(it->second);
+            cn.insert(cn.end(), p->counts.begin(), p->counts.end());
+          }
+          const int n = (int)grid_of.size();
+          const int E_max = *std::max_element(grid_E.begin(), grid_E.end());
+          std::vector<double> rt((size_t)n * E_max), l2(n);
+          std::vector<int32_t> itv(n);
+          const bool ok = !colate_stage3_em_grids(h, n, grid_of.data(), (int)grid_E.size(), grid_E.data(), grid_off.data(), ep.data(), init.data(),
+                                                  cn.data(), 100000, rt.data(), itv.data(), l2.data());
+          for (size_t k = b0; k < b1; k++) {
+            PairLine* p = run[k];
+            if (!ok) { p->err = std::string("EM: ") + colate_last_error(); continue; }
+            const size_t r0 = (k - b0) * R;
+            p->rates.assign((size_t)R * p->E, 0.0);
+            for (int r = 0; r < R; r++) memcpy(p->rates.data() + (size_t)r * p->E, rt.data() + (r0 + r) * E_max, (size_t)p->E * 8);
+            p->iters.assign(itv.begin() + r0, itv.begin() + r0 + R);
+            p->ll.assign(l2.begin() + r0, l2.begin() + r0 + R);
+          }
+          b0 = b1;
+        }
+      }
+    }
+    // pairs with <out>.colate_mat: stages i-ii are skipped and the EM runs on the age grid read back from that file
+    // (coal.cpp:3169-3170, 3471-3499), in a launch of their own
+    for (PairLine* p : mine) {
+      if (!p->cached || !p->err.empty()) continue;
+      double ypg = 28.0;
+      p->age_gen = colate_age_generations(p->has_age[0] ? p->age[0].c_str() : nullptr, p->has_age[1] ? p->age[1].c_str() : nullptr, has_ypg, ypg_flag, &ypg);
+      double cached_age_bin[COLATE_NUM_AGE_BINS];
+      p->counts.assign((size_t)std::max(R, 1) * C2, 0.0);
+      std::ifstream is(p->out + ".colate_mat");
+      for (int b = 0; b < COLATE_NUM_AGE_BINS; b++) is >> cached_age_bin[b];
+      for (int i = 0; i < R; i++)
+        for (int k = 0; k < C2; k++) is >> p->counts[(size_t)i * C2 + k];
+      if (!grid_of_age(*p, ypg) || R == 0) continue;
+      p->rates.assign((size_t)R * p->E, 0.0);
+      p->iters.assign(R, 0);
+      p->ll.assign(R, 0.0);
+      if (colate_set_age_bins(h, cached_age_bin) ||
+          colate_stage3_em(h, R, p->E, p->epochs.data(), p->rates_init.data(), p->counts.data(), 100000, p->rates.data(), p->iters.data(), p->ll.data()))
+        p->err = std::string("EM: ") + colate_last_error();
+      if (colate_set_age_bins(h, nullptr)) { dev_fail("colate_set_age_bins"); return; }
+    }
+  };
+  {
+    std::vector<std::thread> th;
+    for (int g = 1; g < G; g++) th.emplace_back(work, g);
+    work(0);
+    for (auto& t : th) t.join();
+  }
+  for (auto& e : dev_err) if (!e.empty()) std::cerr << e << std::endl;
+  // outputs in file order; a failed pair writes nothing
+  int n_failed = 0;
+  for (auto& p : pl) {
+    if (p.err.empty() && (colate_write_coal((p.out + ".coal").c_str(), R, p.E, p.epochs.data(), p.rates.data(), p.age_gen > 0.0, p.ep_null) ||
+                          colate_write_bin((p.out + ".bin").c_str(), R, p.E, p.epochs.data(), p.rates.data(), p.iters.data())))
+      p.err = std::string("writing the output: ") + colate_last_error();
+    if (!p.err.empty()) {
+      n_failed++;
+      std::cerr << "pair on line " << p.line << " (" << p.out << ") FAILED: " << p.err << std::endl;
+      continue;
+    }
+    std::cerr << "pair on line " << p.line << " (" << p.out << "): ";
+    if (p.cached) std::cerr << "from " << p.out << ".colate_mat";
+    else std::cerr << "blocks " << p.num_blocks << ", used rows " << p.n_used;
+    std::cerr << ", iterations";
+    for (int32_t it : p.iters) std::cerr << " " << it;
+    std::cerr << std::endl;
+  }
+  if (n_failed) std::cerr << n_failed << " of " << pl.size() << " pairs failed" << std::endl;
+  return n_failed ? 1 : 0;
+}
+
 // --mode make_tmp with --target_table (make_tmp(), coal.cpp:2923-3069 -> maketmp_table, 2682-2808): host-only
 int run_make_tmp(const Options& options)
 {
@@ -564,7 +946,7 @@ int main(int argc, char* argv[])
   }
   const std::string mode = options.get("mode");
   int rc = 0;
-  if (mode == "mut") rc = run_mut(options);
+  if (mode == "mut") rc = options.count("pairs") ? run_cohort(options) : run_mut(options);
   else if (mode == "make_tmp") rc = run_make_tmp(options);
   else {
     std::cout << "####### error #######" << std::endl;

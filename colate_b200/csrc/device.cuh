@@ -106,6 +106,7 @@ struct colate_handle {
   bool em_inflight = false;
   int em_R = 0, em_E = 0;
   std::vector<double> em_host_in;   // epochs + initial rates of the EM in flight (the async copies read the handle's copy)
+  colate::DevBuf d_gr_tab, d_gr_rates;   // colate_stage3_em_grids: grid_of + grid table, rates [R][E_max]
   colate::DevBuf d_em_scratch;      // the EM kernels' global scratch (apart from d_scratch: stage i of the next pair may use that)
   int em_kernel = -1, em_csize = 0;   // last EM launch: 0 k_em, 1 k_em_split, 2 k_em_cta; CTAs per replicate
   int64_t launches = 0;
@@ -152,6 +153,11 @@ int mt_window_after(colate_handle* h, uint32_t* window_after);
 // kernels_em.cu
 int run_bootstrap(colate_handle* h, int R, int num_blocks, const double* block_stats_dev, double age);
 int run_em(colate_handle* h, int R, int E, int max_iter, const double* epochs_host, cudaStream_t stream);
+bool em_cta_fits(const colate_handle* h, int E, const double* epochs_host, int* n_pairs_cap, size_t* smem);
+// k_em_cta_grids on R replicates: d_epochs / d_rates hold the packed grids and initial rates, d_counts the counts;
+// grid_info_dev = int4 {E, offset, n_pairs_cap, 0} per grid; results -> d_gr_rates [R][E_out], d_iters, d_ll
+int run_em_grids(colate_handle* h, int R, const int32_t* grid_of_dev, const int* grid_info_dev, int E_out, size_t smem, int max_iter,
+                 cudaStream_t stream);
 int run_estep(colate_handle* h, int shared, int E, int n_t);
 int run_libm(colate_handle* h, int which, int n, const double* x_host, double* y_host);
 }  // namespace colate

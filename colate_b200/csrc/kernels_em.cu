@@ -946,13 +946,24 @@ __host__ __device__ inline int emc_block(int type, int et, int E)
   return type ? (n + 1) & ~1 : n | 1;
 }
 
-__global__ void __launch_bounds__(EMC_THREADS, 1)
-k_em_cta(int E, int n_pairs_cap, const double* __restrict__ epochs, const double* __restrict__ rates_init,
-         const double* __restrict__ age_bin_g, const double* __restrict__ counts, int max_iter,
-         const uint64_t* __restrict__ exp_tab_g, const uint64_t* __restrict__ log_tab_g,
-         double* __restrict__ rates_out, int32_t* __restrict__ iters_out, double* __restrict__ ll_out, long long* prof_g)
+// The body of k_em_cta and of k_em_cta_grids.  kGrids: every CTA reads its own epoch grid -- grid_of[rep] indexes
+// grid_info = {E, offset into the packed epochs / rates_init, n_pairs_cap} -- and writes its row of rates_out with stride
+// E_out (zeros past its E).  Everything that depends on E (the shared-memory carve-up, emc_block, the task table, wz) is
+// derived from the CTA's own E below, so a replicate's arithmetic is that of a uniform launch on its grid.
+template <bool kGrids>
+__device__ __forceinline__ void em_cta_body(int E, int n_pairs_cap, const double* __restrict__ epochs, const double* __restrict__ rates_init,
+                                            const double* __restrict__ age_bin_g, const double* __restrict__ counts, int max_iter,
+                                            const uint64_t* __restrict__ exp_tab_g, const uint64_t* __restrict__ log_tab_g,
+                                            double* __restrict__ rates_out, int32_t* __restrict__ iters_out, double* __restrict__ ll_out,
+                                            long long* prof_g, const int32_t* __restrict__ grid_of, const int4* __restrict__ grid_info,
+                                            int E_out)
 {
   const int rep = blockIdx.x;
+  if (kGrids) {
+    const int4 g = grid_info[grid_of[rep]];
+    E = g.x; n_pairs_cap = g.z;
+    epochs += g.y; rates_init += g.y;
+  }
   extern __shared__ double sm[];
   double* ep = sm;                  // [E]
   double* rate = ep + E;            // [E]
@@ -1268,8 +1279,34 @@ k_em_cta(int E, int n_pairs_cap, const double* __restrict__ epochs, const double
   // (the clock is read when the thread ARRIVES at a barrier: a thread without work in a phase shows the phase's length
   // in the NEXT slot; thread 639 has no work in heads / P3 / P4)
   if (prof && (tid == 0 || tid == 639)) for (int i = 0; i < 8; i++) prof[(tid ? 8 : 0) + i] = tp[i];
-  for (int e = tid; e < E; e += blockDim.x) rates_out[(size_t)rep * E + e] = rate[e];
+  if (kGrids) {
+    for (int e = tid; e < E_out; e += blockDim.x) rates_out[(size_t)rep * E_out + e] = e < E ? rate[e] : 0.0;
+  } else {
+    for (int e = tid; e < E; e += blockDim.x) rates_out[(size_t)rep * E + e] = rate[e];
+  }
   if (tid == 0) { iters_out[rep] = iter; ll_out[rep] = ll_s; }
+}
+
+__global__ void __launch_bounds__(EMC_THREADS, 1)
+k_em_cta(int E, int n_pairs_cap, const double* __restrict__ epochs, const double* __restrict__ rates_init,
+         const double* __restrict__ age_bin_g, const double* __restrict__ counts, int max_iter,
+         const uint64_t* __restrict__ exp_tab_g, const uint64_t* __restrict__ log_tab_g,
+         double* __restrict__ rates_out, int32_t* __restrict__ iters_out, double* __restrict__ ll_out, long long* prof_g)
+{
+  em_cta_body<false>(E, n_pairs_cap, epochs, rates_init, age_bin_g, counts, max_iter, exp_tab_g, log_tab_g, rates_out, iters_out, ll_out,
+                     prof_g, nullptr, nullptr, 0);
+}
+
+// k_em_cta over mixed epoch grids (cohorts: every pair's age moves its grid).  Launched with the shared memory of the
+// largest grid; no profiling counters.
+__global__ void __launch_bounds__(EMC_THREADS, 1)
+k_em_cta_grids(const int32_t* __restrict__ grid_of, const int4* __restrict__ grid_info, const double* __restrict__ epochs,
+               const double* __restrict__ rates_init, const double* __restrict__ age_bin_g, const double* __restrict__ counts, int max_iter,
+               const uint64_t* __restrict__ exp_tab_g, const uint64_t* __restrict__ log_tab_g, int E_out,
+               double* __restrict__ rates_out, int32_t* __restrict__ iters_out, double* __restrict__ ll_out)
+{
+  em_cta_body<true>(0, 0, epochs, rates_init, age_bin_g, counts, max_iter, exp_tab_g, log_tab_g, rates_out, iters_out, ll_out,
+                    nullptr, grid_of, grid_info, E_out);
 }
 
 // E-step probe: one thread per age, plain stores
@@ -1334,6 +1371,23 @@ int run_bootstrap(colate_handle* h, int R, int num_blocks, const double* block_s
   return 0;
 }
 
+// k_em_cta's compact-store size and shared memory for the grid epochs_host[E] under the handle's age grid; true if the
+// kernel fits (shared memory, and the threads of its first phase)
+bool em_cta_fits(const colate_handle* h, int E, const double* epochs_host, int* n_pairs_cap, size_t* smem)
+{
+  const double* ab = h->h_agebin;
+  int cap = 0;
+  for (int b = 0; b < NBINS; b++) {
+    int k = E;
+    for (int e = 0; e < E; e++) if (ab[b] < epochs_host[e]) { k = e; break; }
+    cap += emc_block(0, k - 1, E) + emc_block(1, k - 1, E);
+  }
+  *n_pairs_cap = cap;
+  *smem = sizeof(double) * ((size_t)11 * E + 4 + 192 + 6 * EMC_NT + 2 * (size_t)cap) + 512 * 8 + EMC_NT * (sizeof(EmcTask) + 4) + 192 * 16 +
+          (size_t)cap * 2 + 32;
+  return *smem <= 225 * 1024 && ((E + 31) & ~31) + NBINS <= EMC_THREADS;
+}
+
 int run_em(colate_handle* h, int R, int E, int max_iter, const double* epochs_host, cudaStream_t stream)
 {
   int rc = ensure_libm_tables(h);
@@ -1367,15 +1421,7 @@ int run_em(colate_handle* h, int R, int E, int max_iter, const double* epochs_ho
   int n_pairs_cap = 0;
   const char* force = getenv("COLATE_EM_KERNEL");   // "cta", "task" (k_em), "split": tests and tuning
   if ((!split && csize == 1 && !(force && !strcmp(force, "task"))) || (force && !strcmp(force, "cta"))) {
-    const double* ab = h->h_agebin;
-    for (int b = 0; b < NBINS; b++) {
-      int k = E;
-      for (int e = 0; e < E; e++) if (ab[b] < epochs_host[e]) { k = e; break; }
-      n_pairs_cap += emc_block(0, k - 1, E) + emc_block(1, k - 1, E);
-    }
-    smem_cta = sizeof(double) * ((size_t)11 * E + 4 + 192 + 6 * EMC_NT + 2 * (size_t)n_pairs_cap) + 512 * 8 + EMC_NT * (sizeof(EmcTask) + 4) + 192 * 16 +
-               (size_t)n_pairs_cap * 2 + 32;
-    cta = smem_cta <= 225 * 1024 && ((E + 31) & ~31) + NBINS <= EMC_THREADS;
+    cta = em_cta_fits(h, E, epochs_host, &n_pairs_cap, &smem_cta);
     if (cta) { split = false; csize = 1; }
   }
   const size_t smem = cta ? smem_cta : split ? smem_split : sizeof(double) * ((size_t)10 * E + 1 + 2 * EM_STAGE_DOUBLES) + 512 * 8;
@@ -1439,6 +1485,23 @@ int run_em(colate_handle* h, int R, int E, int max_iter, const double* epochs_ho
                 r, q[0], q[1], q[6], q[7], q[3], q[4], q[5], csize);
     }
   }
+  return 0;
+}
+
+int run_em_grids(colate_handle* h, int R, const int32_t* grid_of_dev, const int* grid_info_dev, int E_out, size_t smem, int max_iter,
+                 cudaStream_t stream)
+{
+  int rc = ensure_libm_tables(h);
+  if (rc) return rc;
+  CK(cudaFuncSetAttribute(k_em_cta_grids, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const uint64_t* tabs = h->libm_tab.as<uint64_t>();
+  k_em_cta_grids<<<R, EMC_THREADS, smem, stream>>>(grid_of_dev, (const int4*)grid_info_dev, h->d_epochs.as<double>(), h->d_rates.as<double>(),
+                                                   h->d_agebin.as<double>(), h->d_counts.as<double>(), max_iter, tabs, tabs + 256, E_out,
+                                                   h->d_gr_rates.as<double>(), h->d_iters.as<int32_t>(), h->d_ll.as<double>());
+  h->launches += 1;
+  h->em_kernel = 2;
+  h->em_csize = 1;
+  CK(cudaGetLastError());
   return 0;
 }
 

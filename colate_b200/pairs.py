@@ -72,6 +72,65 @@ def all_pairs(handle: api.Handle, n_genomes: int, seed: int, bins: str = "3,7,0.
                 ll=ll, num_blocks=nb, n_used=nu, counts=counts, seconds=dict(stage12=t1 - t0, em=t2 - t1))
 
 
+def cohort(handle: api.Handle, pairs, seed: int, bins: str | None = None, coal: str | None = None, num_bootstraps: int = 1,
+           years_per_gen=None, max_iter: int = 100000, em_batch: int = 2048):
+    """A cohort: pairs = [(target_slot, reference_slot, target_age, reference_age)], ages in years as the CLI takes them (str,
+    number or None), genomes (and their masks) already in the handle's slots.  Per pair: stage i from the --seed state (the
+    generator stream is shared, colate_set_stream_cache), `num_bootstraps` block weights drawn from the pair's post-stage-i state,
+    stage ii at the pair's age and the pair's epoch grid (--bins, or --coal with its initial rates).  Then the EM of all
+    P x num_bootstraps replicates on their mixed grids (Handle.stage3_em_grids, em_batch replicates per call).
+    Every pair's result is what `api.mut()` returns for that pair alone.  Returns dict(pairs=[per-pair dict(epochs, ep_null,
+    is_ancient, rates[R][E], iters[R], ll[R], num_blocks, n_used, counts[R][2][185])], seconds=dict(stage12, em))."""
+    if (bins is None) == (coal is None):
+        raise ValueError("give exactly one of bins and coal")
+    R = int(num_bootstraps)
+    if R < 1:
+        raise ValueError("num_bootstraps must be >= 1")
+    txt = lambda a: None if a is None else str(a)
+    t0 = time.perf_counter()
+    mt0 = api.mt_seed(seed)
+    out, grids, grid_key = [], [], {}
+    handle.set_stream_cache(True)       # every pair reseeds with the same --seed: one generator stream serves them all
+    try:
+        for t_slot, r_slot, t_age, r_age in pairs:
+            age, ypg = api.ages(txt(t_age), txt(r_age), years_per_gen)
+            s1 = handle.stage1(mt0, target_slot=int(t_slot), reference_slot=int(r_slot), fetch=False)
+            w = api.draw_block_weights(s1.mt_state, R, s1.num_blocks)
+            counts = handle.stage2_bootstrap_dev(w, None, s1.num_blocks, age, fetch=True)
+            if coal is not None:
+                epochs, init = api.epochs_from_coal_file(coal, age)
+                ep_null = 0
+            else:
+                epochs, ep_null = api.epochs_from_bins(bins, age, ypg)
+                init = np.full(epochs.shape[0], 1.0 / 20000.0)
+            key = (epochs.tobytes(), init.tobytes())
+            if key not in grid_key:
+                grid_key[key] = len(grids)
+                grids.append((epochs, init))
+            out.append(dict(epochs=epochs, ep_null=ep_null, is_ancient=age > 0.0, num_blocks=s1.num_blocks, n_used=s1.n_used,
+                            counts=counts, grid=grid_key[key]))
+    finally:
+        handle.set_stream_cache(False)
+    t1 = time.perf_counter()
+    P = len(out)
+    grid_of = np.repeat(np.array([p["grid"] for p in out], dtype=np.int32), R)
+    counts = np.concatenate([p["counts"] for p in out]) if P else np.zeros((0, 2, api.NBINS))
+    E_max = max((g[0].shape[0] for g in grids), default=0)
+    rates, iters, ll = np.zeros((P * R, E_max)), np.zeros(P * R, dtype=np.int32), np.zeros(P * R)
+    for b0 in range(0, P * R, em_batch):
+        b1 = min(P * R, b0 + em_batch)
+        used = sorted(set(grid_of[b0:b1].tolist()))            # the grids of this batch only: the launch is sized to its largest
+        remap = {g: k for k, g in enumerate(used)}
+        r_, i_, l_ = handle.stage3_em_grids([remap[g] for g in grid_of[b0:b1]], [grids[g] for g in used], counts[b0:b1], max_iter)
+        rates[b0:b1, :r_.shape[1]], iters[b0:b1], ll[b0:b1] = r_, i_, l_
+    t2 = time.perf_counter()
+    for p, res in enumerate(out):
+        E = res["epochs"].shape[0]
+        res.update(rates=rates[p * R:(p + 1) * R, :E].copy(), iters=iters[p * R:(p + 1) * R].copy(), ll=ll[p * R:(p + 1) * R].copy())
+        del res["grid"]
+    return dict(pairs=out, seconds=dict(stage12=t1 - t0, em=t2 - t1))
+
+
 def all_pairs_sharded(handle, n_genomes: int, seed: int, bins: str = "3,7,0.1", pairs=None, device="cuda", **kw):
     """`all_pairs` across the ranks of the default torch.distributed process group (NCCL on GPUs, gloo in the CPU
     tests).  Pair p of the list goes to rank p mod world; each rank runs its pairs exactly as `all_pairs` does (its own

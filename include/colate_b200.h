@@ -181,6 +181,17 @@ int colate_stage3_em(colate_handle* h, int R, int E, const double* epochs, const
 int colate_stage3_em_begin(colate_handle* h, int R, int E, const double* epochs, const double* rates_init, int max_iter);
 int colate_stage3_em_end(colate_handle* h, double* rates, int32_t* iters, double* final_ll);
 
+/* The EM of R replicates that do not share one epoch grid (a cohort: every pair's age moves its grid, coal.cpp:3553-3630).
+ * Grid g has grid_E[g] epochs at epochs[grid_off[g] ..] with initial rates at rates_init[grid_off[g] ..]; replicate r runs on
+ * grid grid_of[r] with counts[r][2][185] (host).  Outputs (host): rates[R][E_max] (E_max = max grid_E; entries past the row's own E
+ * are 0), iters[R], final_ll[R].  Row r equals colate_stage3_em(h, 1, grid_E[g], epochs + grid_off[g], rates_init + grid_off[g],
+ * counts[r], ...) bit for bit: the replicates of every grid the throughput kernel fits run in ONE launch, each CTA on its own grid;
+ * a grid it does not fit (shared memory or threads) runs through colate_stage3_em alone.  The EM uses the age grid of
+ * colate_set_age_bins() for all rows.  Afterwards no device-resident counts remain for colate_stage3_em(counts = NULL). */
+int colate_stage3_em_grids(colate_handle* h, int R, const int32_t* grid_of, int n_grids, const int32_t* grid_E, const int64_t* grid_off,
+                           const double* epochs, const double* rates_init, const double* counts, int max_iter, double* rates,
+                           int32_t* iters, double* final_ll);
+
 /* The age grid colate_stage3_em() evaluates (the point ages t = age_bin[b], coal.cpp:3708, 3721).  Default: colate_age_bins().
  * mut() started from a <out>.colate_mat cache reads the grid back from that file's first line, i.e. rounded to six
  * significant digits (coal.cpp:3481-3483), and runs the EM on THOSE ages: the host passes them here.  NULL restores the
