@@ -109,6 +109,8 @@ TEST_HOOKS = {
     "colate_test_colate_in_runs": (C.c_int64, [VP, C.c_int64, C.c_int, C.POINTER(C.c_char_p), C.c_int, i64, i64, i64]),
     "colate_test_libm": (C.c_int, [VP, C.c_int, C.c_int, f64, f64]),
     "colate_test_log1p_wide": (C.c_int, [C.c_int, f64, f64, i32]),
+    "colate_test_em_prims": (C.c_int, [VP, C.c_int, C.c_int, f64, VP, f64, i32]),
+    "colate_test_last_em": (C.c_int, [VP, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "colate_test_bin_fast": (C.c_int, [VP, C.c_int, f64, i32, i32]),
     "colate_test_bin_sweep": (C.c_int, [VP, C.c_uint32, C.c_uint32, _p(dtype=np.uint64, flags="C_CONTIGUOUS")]),
     "colate_test_mt_stream": (C.c_int, [VP, u32, C.c_int64, C.c_int64, C.c_int, u32]),

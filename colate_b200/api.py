@@ -429,6 +429,26 @@ class Handle:
         check(lib().colate_test_libm(self._h, {"exp": 0, "log": 1, "log1p": 2}[which], x.shape[0], x, y))
         return y
 
+    EM_PRIMS = ("exp_main", "log1p_k0", "log1p_wide", "div_midrange", "lse", "lse_wide", "lme")
+
+    def em_prims(self, which: str, a, b=None):
+        """Test hook: one straight-line piece of the EM folds on the device, element by element -> (y, ok).  ok: the piece's
+        validity predicate (exp_is_main, log1p_is_k0, log1p_wide_ok; always 1 for div_midrange), or for lse / lse_wide / lme
+        whether the straight-line path was taken.  b: second operand of div_midrange / lse / lse_wide / lme."""
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        bb = None if b is None else np.ascontiguousarray(b, dtype=np.float64)
+        assert bb is None or bb.shape == a.shape
+        y, ok = np.zeros_like(a), np.zeros(a.shape[0], dtype=np.int32)
+        check(lib().colate_test_em_prims(self._h, self.EM_PRIMS.index(which), a.shape[0], a, ptr(bb), y, ok))
+        return y, ok
+
+    def last_em(self):
+        """Test hook: (kernel, CTAs per replicate) of the last EM launch; kernel is "task" (k_em), "split" (k_em_split),
+        "cta" (k_em_cta / k_em_cta_grids) or None."""
+        k, c = C.c_int(0), C.c_int(0)
+        check(lib().colate_test_last_em(self._h, C.byref(k), C.byref(c)))
+        return {0: "task", 1: "split", 2: "cta"}.get(k.value), c.value
+
     def bin_fast(self, ages):
         """Test hook: k_sample's table-free age-bin index (-1 = sample flagged for the exact table) and the exact one."""
         a = np.ascontiguousarray(ages, dtype=np.float64)

@@ -823,6 +823,26 @@ int colate_test_libm(colate_handle* h, int which, int n, const double* x, double
   return run_libm(h, which, n, x, y);
 }
 
+// test hook: the straight-line fold pieces of the EM kernels on the device (which: see k_test_em_prims); b may be NULL
+// for the one-operand pieces
+int colate_test_em_prims(colate_handle* h, int which, int n, const double* a, const double* b, double* y, int32_t* ok)
+{
+  if (!h || which < 0 || which > 6 || n <= 0 || !a || !y || !ok || (which >= 3 && !b))
+    return fail(COLATE_ERR_ARG, "colate_test_em_prims: bad arguments");
+  CK(cudaSetDevice(h->device));
+  return run_test_em_prims(h, which, n, a, b, y, ok);
+}
+
+// test hook: the kernel of the handle's last EM launch (0 k_em, 1 k_em_split, 2 k_em_cta / k_em_cta_grids, -1 none yet) and
+// its CTAs per replicate
+int colate_test_last_em(colate_handle* h, int* kernel, int* csize)
+{
+  if (!h || !kernel || !csize) return fail(COLATE_ERR_ARG, "colate_test_last_em: bad arguments");
+  *kernel = h->em_kernel;
+  *csize = h->em_csize;
+  return 0;
+}
+
 // test hooks: k_sample's table-free age-bin index (fast[i] = -1 where the kernel would consult the exact
 // table) next to the exact index, on given ages / swept over all floats with bit patterns in [lo, hi)
 int colate_test_bin_fast(colate_handle* h, int n, const double* ages, int32_t* fast, int32_t* exact)

@@ -160,4 +160,5 @@ int run_em_grids(colate_handle* h, int R, const int32_t* grid_of_dev, const int*
                  cudaStream_t stream);
 int run_estep(colate_handle* h, int shared, int E, int n_t);
 int run_libm(colate_handle* h, int which, int n, const double* x_host, double* y_host);
+int run_test_em_prims(colate_handle* h, int which, int n, const double* a_host, const double* b_host, double* y_host, int32_t* ok_host);
 }  // namespace colate

@@ -100,6 +100,8 @@ int64_t colate_test_colate_in_runs(const char* buf, int64_t sz, int n_chr, const
                                    int64_t* runs4, int64_t* chr_first, int64_t* chr_end);
 int colate_test_libm(colate_handle* h, int which, int n, const double* x, double* y);
 int colate_test_log1p_wide(int n, const double* x, double* y, int32_t* ok);
+int colate_test_em_prims(colate_handle* h, int which, int n, const double* a, const double* b, double* y, int32_t* ok);
+int colate_test_last_em(colate_handle* h, int* kernel, int* csize);
 int colate_test_bin_fast(colate_handle* h, int n, const double* ages, int32_t* fast, int32_t* exact);
 int colate_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, uint64_t* out3);
 int colate_test_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words,

@@ -482,9 +482,12 @@ k_em(int E, const double* __restrict__ epochs, const double* __restrict__ rates_
       cluster.sync();
       if (tid == 0) { prev_s = ll_s; ll_s = ll_new; }
     } else {
-      // single CTA: chunks of TJ rows of M are staged through shared memory (double-buffered), thread = column
+      // single CTA: chunks of TJ rows of M are staged through shared memory (double-buffered), thread = column.
+      // 2E + 1 columns can outnumber the threads (E >= 208): thread tid also owns columns tid + EM_THREADS, ..., whose
+      // running sums live in their final places (tn / td are contiguous; column 2E is ll_new), summed in the same task order
       double acc = 0.0;
       int buf = 0;
+      for (int col = tid + EM_THREADS; col <= 2 * E; col += EM_THREADS) (col < 2 * E ? tn[col] : ll_new) = 0.0;
       for (int i = tid; i < min(TJ, n_task) * RS; i += blockDim.x) stage[i] = __ldcg(M + i);
       __syncthreads();
       for (int j0 = 0; j0 < n_task; j0 += TJ) {
@@ -498,6 +501,13 @@ k_em(int E, const double* __restrict__ epochs, const double* __restrict__ rates_
           const double* col = stage + (size_t)buf * EM_STAGE_DOUBLES + tid;
           for (int j = 0; j < nj; j++) acc += col[(size_t)j * RS];
         }
+        for (int c2 = tid + EM_THREADS; c2 <= 2 * E; c2 += EM_THREADS) {
+          const double* col = stage + (size_t)buf * EM_STAGE_DOUBLES + c2;
+          double& a2 = c2 < 2 * E ? tn[c2] : ll_new;
+          double s = a2;
+          for (int j = 0; j < nj; j++) s += col[(size_t)j * RS];
+          a2 = s;
+        }
         double* dst = stage + (size_t)(buf ^ 1) * EM_STAGE_DOUBLES;
 #pragma unroll
         for (int u = 0; u < 9; u++) { const int i = tid + u * EM_THREADS; if (i < nn * RS) dst[i] = pre[u]; }
@@ -507,6 +517,7 @@ k_em(int E, const double* __restrict__ epochs, const double* __restrict__ rates_
       if (tid < E) tn[tid] = acc;
       else if (tid < 2 * E) td[tid - E] = acc;
       else if (tid == 2 * E) { prev_s = ll_s; ll_s = acc; }
+      if (2 * E >= EM_THREADS && tid == 2 * E % EM_THREADS) { prev_s = ll_s; ll_s = ll_new; }
     }
     __syncthreads();
     if (prof) { t1 = clock64(); tp[4] += t1 - t0; t0 = t1; }
@@ -1351,6 +1362,36 @@ __global__ void k_libm(int which, int n, const double* __restrict__ x, const uin
     y[i] = which == 0 ? glm::exp(x[i], T) : which == 1 ? glm::log(x[i], T) : glm::log1p(x[i]);
 }
 
+// test hook: the straight-line pieces of the EM folds, element by element.  which = 0 exp_main, 1 log1p_k0, 2 log1p_wide,
+// 3 div_midrange(a, b), 4 lse(a, b), 5 lse_wide(a, b), 6 lme(a, b); ok[i] = the piece's validity predicate (0..2), 1 (3), or
+// whether the fold step took its straight-line path (4..6: the predicates inside lse / lse_wide / lme)
+__global__ void k_test_em_prims(int which, int n, const double* __restrict__ a, const double* __restrict__ b,
+                                const uint64_t* __restrict__ exp_tab_g, const uint64_t* __restrict__ log_tab_g, double* __restrict__ y,
+                                int32_t* __restrict__ ok)
+{
+  glm::Tables T{exp_tab_g, log_tab_g};
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const double x = a[i], x2 = b[i];
+    double r = 0.0;
+    bool k = true;
+    if (which == 0) { r = glm::exp_main(x, T); k = glm::exp_is_main(x); }
+    else if (which == 1) { r = glm::log1p_k0(x); k = glm::log1p_is_k0(x); }
+    else if (which == 2) { r = glm::log1p_wide(x); k = glm::log1p_wide_ok(x); }
+    else if (which == 3) r = glm::div_midrange(x, x2);
+    else if (which == 4 || which == 5) {
+      const double d = -fabs(x - x2), e = glm::exp_main(d, T);
+      r = which == 4 ? lse(x, x2, T) : lse_wide(x, x2, T);
+      k = !bad(x) & !bad(x2) & glm::exp_is_main(d) & (which == 4 ? glm::log1p_is_k0(e) : glm::log1p_wide_ok(e));
+    } else {
+      const double d = x2 - x, e = -glm::exp_main(d, T);
+      r = lme(x, x2, T);
+      k = !bad(x) & !bad(x2) & !(x < x2) & glm::exp_is_main(d) & glm::log1p_is_k0(e);
+    }
+    y[i] = r;
+    ok[i] = k ? 1 : 0;
+  }
+}
+
 // ---- launchers -------------------------------------------------------------------------------
 int ensure_libm_tables(colate_handle* h)
 {
@@ -1398,9 +1439,9 @@ int run_em(colate_handle* h, int R, int E, int max_iter, const double* epochs_ho
     const int sms = h->sm_count;
     while (csize < 8 && R * csize * 2 <= sms) csize *= 2;
     if (csize == 8 && R * 16 * 2 <= sms) csize = 16;   // non-portable cluster size: one GPC (16-20 SMs) per replicate
-    // up to 4 replicates: one GPC each (20.5 ms for 1001 iterations at E = 43); up to 9: clusters of 8, one CTA per SM
-    // (23 ms); from 10 on one CTA per replicate (k_em_cta: 31 ms for any count up to the number of SMs, against 59 ms
-    // for 30 replicates on clusters of 8 at two CTAs per SM; profiles/r02_em_throughput.md)
+    // up to SMs/32 replicates (4 on 148 SMs): one GPC each (20.5 ms for 1001 iterations at E = 43); up to SMs/8 (18):
+    // clusters of 8, one CTA per SM (23 ms); beyond that one CTA per replicate (k_em_cta: 31 ms for any count up to the
+    // number of SMs, against 59 ms for 30 replicates on clusters of 8 at two CTAs per SM; profiles/r02_em_throughput.md)
     if (csize < 8) csize = 1;
   }
   if (csize != 1 && csize != 2 && csize != 4 && csize != 8 && csize != 16) csize = 1;
@@ -1509,7 +1550,8 @@ int run_estep(colate_handle* h, int shared, int E, int n_t)
 {
   int rc = ensure_libm_tables(h);
   if (rc) return rc;
-  const size_t smem = sizeof(double) * (6 * E + 1);
+  const size_t smem = sizeof(double) * (6 * E + 1);   // above the default 48 KB from E = 1024 on
+  CK(cudaFuncSetAttribute(k_estep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   double* base = h->d_tmp.as<double>();  // [t: n_t][num: n_t*E][denom: n_t*E][logl: n_t]
   const uint64_t* tabs = h->libm_tab.as<uint64_t>();
   k_estep<<<1, 256, smem, h->stream>>>(shared, E, h->d_epochs.as<double>(), h->d_rates.as<double>(), n_t, base, tabs, tabs + 256,
@@ -1528,6 +1570,25 @@ int run_libm(colate_handle* h, int which, int n, const double* x_host, double* y
   CK(cudaMemcpyAsync(d, x_host, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
   k_libm<<<296, 256, 0, h->stream>>>(which, n, d, tabs, tabs + 256, d + n);
   CK(cudaMemcpyAsync(y_host, d + n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+int run_test_em_prims(colate_handle* h, int which, int n, const double* a_host, const double* b_host, double* y_host, int32_t* ok_host)
+{
+  int rc = ensure_libm_tables(h);
+  if (rc) return rc;
+  CK(h->d_tmp.ensure((size_t)n * 28));
+  double* d = h->d_tmp.as<double>();   // [a: n][b: n][y: n][ok: n int32]
+  int32_t* dok = (int32_t*)(d + 3 * (size_t)n);
+  const uint64_t* tabs = h->libm_tab.as<uint64_t>();
+  CK(cudaMemcpyAsync(d, a_host, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
+  if (b_host) CK(cudaMemcpyAsync(d + n, b_host, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
+  else CK(cudaMemsetAsync(d + n, 0, (size_t)n * 8, h->stream));
+  k_test_em_prims<<<296, 256, 0, h->stream>>>(which, n, d, d + n, tabs, tabs + 256, d + 2 * (size_t)n, dok);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(y_host, d + 2 * (size_t)n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(ok_host, dok, (size_t)n * 4, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return 0;
 }

@@ -611,6 +611,9 @@ int oracle_epochs_from_coal_line(const char* line, double age, double* epochs, i
  * ---------------------------------------------------------------------------------- */
 static int bad(double x) { return isinf(x) || isnan(x); }
 
+/* the largest epoch grid the C ABI accepts (colate_stage3_em, colate_estep) */
+#define ORACLE_MAX_E 1024
+
 /* coal_EM::logsumexp, coal_EM.cpp:5-31 */
 static double lse(double a, double b)
 {
@@ -761,8 +764,8 @@ double oracle_em_notshared(int E, const double* ep, const double* rate, const do
 /* convenience for E-step parity tests: builds A/B like the coal_EM ctor, then one call */
 double oracle_estep(int shared, int E, const double* ep, const double* rate, double t, double* num, double* denom)
 {
-  double A[512], B[512], Lam[512];
-  if (E > 512) return NAN;
+  double A[ORACLE_MAX_E], B[ORACLE_MAX_E], Lam[ORACLE_MAX_E];
+  if (E > ORACLE_MAX_E) return NAN;
   oracle_get_AB(E, ep, rate, A, B, Lam);
   return shared ? oracle_em_shared(E, ep, rate, A, B, Lam, t, num, denom)
                 : oracle_em_notshared(E, ep, rate, A, B, Lam, t, num, denom);
@@ -774,8 +777,9 @@ double oracle_estep(int shared, int E, const double* ep, const double* rate, dou
 int oracle_em_run(int E, const double* ep, const double* rates_init, const double* age_bin,
                   const double* counts, int max_iter, double* rates_out, double* final_ll)
 {
-  double rate[512], num[512], denom[512], tn[512], td[512], A[512], B[512], Lam[512];
-  if (E > 512) return -1;
+  double rate[ORACLE_MAX_E], num[ORACLE_MAX_E], denom[ORACLE_MAX_E], tn[ORACLE_MAX_E], td[ORACLE_MAX_E], A[ORACLE_MAX_E], B[ORACLE_MAX_E],
+      Lam[ORACLE_MAX_E];
+  if (E > ORACLE_MAX_E) return -1;
   const double* S = counts; const double* N = counts + NBINS;
   for (int e = 0; e < E; e++) { rate[e] = rates_init[e]; tn[e] = 0; td[e] = 0; num[e] = 0; denom[e] = 0; }
   double ll = log(0.0), prev;
