@@ -127,6 +127,26 @@ def mask_bits_from_seq(seqs, site_off, pos) -> np.ndarray:
     return np.ascontiguousarray(by).view("<u4").astype(np.uint32).reshape(-1)
 
 
+def bam_scan(path: str, chr_names, window_bytes: int = 0) -> dict:
+    """Host-only walk of a BAM file (no GPU): per --chr entry the record count, the first / last position and the index of the
+    header contig it matched (colate_bam_scan).  Raises ColateError for the files colate_pileup_bam refuses."""
+    n = len(chr_names)
+    names = (C.c_char_p * n)(*[s.encode() for s in chr_names])
+    cnt = np.zeros(n, np.int64); first = np.zeros(n, np.int32); last = np.zeros(n, np.int32); rid = np.zeros(n, np.int32)
+    check(lib().colate_bam_scan(str(path).encode(), n, names, window_bytes, cnt, first, last, rid))
+    return {"n_records": cnt, "first_pos": first, "last_pos": last, "ref_id": rid}
+
+
+def read_fasta(path: str) -> np.ndarray:
+    """fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz."""
+    p = C.POINTER(C.c_uint8)()
+    n = check(lib().colate_read_fasta(str(path).encode(), C.byref(p)))
+    try:
+        return np.ctypeslib.as_array(p, shape=(n,)).copy() if n else np.zeros(0, np.uint8)
+    finally:
+        lib().colate_free(C.cast(p, C.c_void_p))
+
+
 @dataclass
 class Stage1Result:
     num_blocks: int
@@ -214,6 +234,27 @@ class Handle:
         out = np.zeros((self.n_site, 4), dtype=np.int32) if fetch else None
         check(lib().colate_pileup_end(self._h, slot, ptr(out) if fetch else None))
         return out
+
+    def pileup_from_bam(self, slot, path, chr_names, ref_genomes, filters=(20, 30, 10), chunk_bytes=0, fetch=False):
+        """The same pileup straight from a BAM file (colate_pileup_bam): chr_names = the site set's --chr list (header contig <name> or
+        chr<name>), ref_genomes[c] = uint8 / bytes sequence of contig c (upper-cased on the device as fasta::Read does).  BGZF is
+        inflated on the host, the records are decoded and counted on the device in chunks of at most chunk_bytes record bytes (0:
+        64 MiB).  Makes `slot` a pileup genome; fetch=True returns counts[n_site][4]."""
+        n = len(chr_names)
+        names = (C.c_char_p * n)(*[s.encode() for s in chr_names])
+        refs = [np.ascontiguousarray(np.frombuffer(g, np.uint8) if isinstance(g, (bytes, bytearray)) else g, dtype=np.uint8) for g in ref_genomes]
+        seqs = (C.c_void_p * n)(*[r.ctypes.data if r.shape[0] else None for r in refs])
+        lens = np.array([r.shape[0] for r in refs], dtype=np.int64)
+        out = np.zeros((self.n_site, 4), dtype=np.int32) if fetch else None
+        check(lib().colate_pileup_bam(self._h, slot, str(path).encode(), n, names, seqs, lens, *filters, chunk_bytes, ptr(out) if fetch else None))
+        return out
+
+    def last_bam_timing(self) -> dict:
+        """Phases of the last pileup_from_bam (colate_last_bam_timing; copy / decode / pileup need set_option("bam_timing", 1))."""
+        t = np.zeros(10)
+        check(lib().colate_last_bam_timing(self._h, t))
+        keys = ("index_s", "inflate_s", "walk_s", "h2d_ms", "decode_ms", "pileup_ms", "total_s", "threads", "inflated_bytes", "records")
+        return dict(zip(keys, t.tolist()))
 
     def set_mask(self, slot, pass_bits):
         if pass_bits is None:

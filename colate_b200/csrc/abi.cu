@@ -151,7 +151,7 @@ void colate_destroy(colate_handle* h)
                     &h->chr_used, &h->chr_blocks, &h->chr_block_base, &h->misc, &h->u_hdr, &h->u_eb2, &h->u_ews, &h->u_ewn, &h->u_cnt,
                     &h->u_blk, &h->blk_rank_start, &h->out_f, &h->out_n, &h->thrA, &h->lut, &h->d_scratch, &h->d_prof, &h->libm_tab, &h->ing_text, &h->ing_tile_cnt, &h->ing_tile_off, &h->ing_nl, &h->ing_status, &h->ing_fb,
                     &h->windows, &h->rng_stream, &h->mt_tail, &h->poly, &h->thr10, &h->d_counts, &h->d_blockstats, &h->d_weights, &h->d_epochs,
-                    &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo};
+                    &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo, &h->bam_buf, &h->bam_ref, &h->bam_state};
   for (DevBuf* b : bufs) b->release();
   for (auto& g : h->genomes) {
     DevBuf* gb[] = {&g.bp, &g.aaf, &g.daf, &g.alleles, &g.chr_first, &g.chr_end, &g.mask_bits, &g.j_aaf, &g.j_daf, &g.j_prevbp, &g.j_flag, &g.pile};
@@ -330,7 +330,7 @@ int colate_pileup_reads(colate_handle* h, int slot, int chr_index, int64_t n_rea
   CK(cudaMemcpyAsync(d + o_ref, ref_seq, ref_len, cudaMemcpyHostToDevice, s));
   int rc = run_pileup_reads(h, slot, chr_index, n_reads, (const int32_t*)(d + o_pos), (const uint8_t*)(d + o_mq), (const int32_t*)(d + o_len),
                             (const int64_t*)(d + o_off), (const uint8_t*)(d + o_seq), (const uint8_t*)(d + o_q), (const uint8_t*)(d + o_ref), ref_len,
-                            max_len, mapq_th, len_th, mismatch_th, (uint8_t*)(d + o_pass));
+                            max_len, mapq_th, len_th, mismatch_th, (uint8_t*)(d + o_pass), true, 0, -1);
   if (rc) return rc;
   CK(cudaStreamSynchronize(s));      // the caller's buffers and the staging buffer are free again
   return 0;
@@ -547,6 +547,8 @@ int colate_set_option(colate_handle* h, const char* key, int64_t value)
   // async_uploads = 1: colate_set_sites / colate_set_genome / colate_set_mask queue their copies and return; the
   // caller keeps the (pinned) host buffers unchanged until the next colate_stage1_flags() has returned
   if (!strcmp(key, "async_uploads")) { h->opt_async_uploads = value != 0; return 0; }
+  // bam_timing = 1: colate_pileup_bam times its copies, decode and pileup per chunk (colate_last_bam_timing) and waits for each
+  if (!strcmp(key, "bam_timing")) { h->opt_bam_timing = value != 0; return 0; }
   // front_end: which of mut()'s input branches the handle reproduces (coal.cpp:3175-3319).  0 = tmp/tmp (parse_tmptmp: pseudo-
   // genotype weights, no normalisation).  1 = the bcf / bam front-ends fed from pre-decoded per-row counts (SURVEY.md 8f N3):
   // raw count weights (coal.cpp:2005-2039, 1164-1197) and both count vectors of stage ii divided by 1e3 (coal.cpp:3453-3463).

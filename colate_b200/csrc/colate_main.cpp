@@ -53,6 +53,13 @@ void help()
                "      <target_tmp> <reference_tmp> <output_prefix> [target_age=<years>] [reference_age=<years>]\n"
                "      [target_mask=<prefix>] [reference_mask=<prefix>]\n"
                "    with the shared flags; each line's .coal / .bin equal those of the single-pair run with the same flags\n"
+               "  Colate --mode mut --mut <prefix> --target_bam <t.bam> --reference_bam <r.bam> --ref_genome <prefix> (--bins x,y,step | --coal <file>)\n"
+               "         [--chr <file>] [--target_mask <prefix>] [--reference_mask <prefix>] [--target_age <years>] [--reference_age <years>]\n"
+               "         [--years_per_gen <float>] [--seed <int>] [--num_bootstraps <int>] [--filters mapq,length,mismatches] [--device <int>]\n"
+               "         -o <output prefix>     (also writes <output prefix>.colate_mat; one device; no --strandfilter)\n"
+               "  Colate --mode make_tmp --mut <prefix> --target_bam <t.bam> --ref_genome <prefix> [--chr <file>] [--target_mask <prefix>]\n"
+               "         [--filters mapq,length,mismatches] [--device <int>] -o <output prefix>     (writes <output prefix>.colate.in)\n"
+               "  Colate --mode make_tmp --mut <prefix> --target_table <file> --ref_genome <prefix> [--chr <file>] [--target_mask <prefix>] -o <output prefix>\n"
             << std::endl;
 }
 
@@ -152,6 +159,60 @@ bool all_ok(const std::vector<Dev>& devs)
   return ok;
 }
 
+// --filters mapq,length,mismatches (coal.cpp:3096: default "20,30,10")
+bool parse_filters(const Options& o, int f[3])
+{
+  f[0] = 20; f[1] = 30; f[2] = 10;
+  if (!o.count("filters")) return true;
+  std::stringstream ss(o.get("filters"));
+  std::string tok;
+  int k = 0;
+  while (std::getline(ss, tok, ',')) {
+    if (k == 3 || tok.empty()) return false;
+    char* end = nullptr;
+    f[k++] = (int)strtol(tok.c_str(), &end, 10);
+    if (*end) return false;
+  }
+  return k == 3;
+}
+
+// --ref_genome (fasta::Read, data.cpp:213-237): <prefix>_chr<name>.fa per --chr entry, or the file itself without --chr
+struct RefGenome {
+  std::vector<uint8_t*> seq;
+  std::vector<int64_t> len;
+  ~RefGenome() { for (uint8_t* p : seq) colate_free(p); }
+  bool read(const Options& o, const std::vector<std::string>& name_chr)
+  {
+    for (auto& nm : name_chr) {
+      const std::string f = o.count("chr") ? o.get("ref_genome") + "_chr" + nm + ".fa" : o.get("ref_genome");
+      uint8_t* p = nullptr;
+      const int64_t n = colate_read_fasta(f.c_str(), &p);
+      if (n < 0) { std::cerr << colate_last_error() << std::endl; return false; }
+      seq.push_back(p);
+      len.push_back(n);
+    }
+    return true;
+  }
+};
+
+// BAM inputs (--target_bam / --reference_bam): what this build does not restate is refused before any device is touched
+bool bam_args_ok(const Options& o, bool need_both)
+{
+  auto bad = [](const std::string& what) { std::cerr << "Error: " << what << std::endl; return false; };
+  if (o.count("strandfilter")) return bad("--strandfilter is not supported with BAM inputs (its read filter is not restated)");
+  for (const char* k : {"target_tmp", "reference_tmp", "target_bcf", "reference_bcf", "target_table"})
+    if (o.count(k)) return bad(std::string("--") + k + " cannot be mixed with BAM inputs");
+  if (need_both && !(o.count("target_bam") && o.count("reference_bam")))
+    return bad("--mode mut with BAM inputs needs both --target_bam and --reference_bam (bam/tmp and bam/bcf mixes are not supported)");
+  if (o.count("pairs")) return bad("--pairs cannot be combined with BAM inputs");
+  const std::string dev = o.count("devices") ? o.get("devices") : "";
+  if (dev.find(',') != std::string::npos) return bad("BAM inputs run on one device (--device <i>)");
+  if (!o.count("ref_genome")) return bad("BAM inputs need --ref_genome");
+  int f[3];
+  if (!parse_filters(o, f)) return bad("--filters takes three integers: mapq,length,mismatches");
+  return true;
+}
+
 int run_mut(const Options& options)
 {
   if (!options.count("mut") || !options.count("output")) {  // coal.cpp:3077-3086
@@ -163,6 +224,8 @@ int run_mut(const Options& options)
     std::cout << "Calculate coalescence rates for sample." << std::endl;
     exit(0);
   }
+  const bool bam = options.count("target_bam") || options.count("reference_bam");
+  if (bam && !bam_args_ok(options, true)) return 1;
   std::cerr << "---------------------------------------------------------" << std::endl;
   std::cerr << "Calculating coalescence rates for (ancient) samples.." << std::endl;
 
@@ -225,8 +288,9 @@ int run_mut(const Options& options)
       for (int k = 0; k < 2 * COLATE_NUM_AGE_BINS; k++) is >> counts[(size_t)i * 2 * COLATE_NUM_AGE_BINS + k];
     from_cache = true;
   } else {
-    if (!(options.count("target_tmp") && options.count("reference_tmp"))) {
-      std::cerr << "This build reads --target_tmp/--reference_tmp (.colate.in) inputs only; bcf/bam front-ends are out of scope." << std::endl;
+    if (!bam && !(options.count("target_tmp") && options.count("reference_tmp"))) {
+      std::cerr << "This build reads --target_tmp/--reference_tmp (.colate.in) or --target_bam/--reference_bam inputs; the bcf front-ends "
+                   "are out of scope." << std::endl;
       return 1;
     }
     // file lists, coal.cpp:3290-3316
@@ -272,9 +336,13 @@ int run_mut(const Options& options)
     // stream, and every device receives the records and ranges of its own chromosomes.
     std::vector<const char*> names;
     for (auto& s : name_chr) names.push_back(s.c_str());
-    const std::string files[2] = {options.get("target_tmp"), options.get("reference_tmp")};
+    const std::string files[2] = {options.get(bam ? "target_bam" : "target_tmp"), options.get(bam ? "reference_bam" : "reference_tmp")};
     struct GenomeHost { int64_t n = 0; std::vector<char> image; std::vector<int32_t> rc, bp, aaf, daf; std::vector<uint16_t> al; std::vector<int64_t> first, end; } gh[2];
-    for (int g = 0; g < 2; g++) {
+    RefGenome refg;
+    int filters[3];
+    parse_filters(options, filters);
+    if (bam && !refg.read(options, name_chr)) return 1;
+    for (int g = 0; g < 2 && !bam; g++) {
       FILE* f = fopen(files[g].c_str(), "rb");
       if (!f) { std::cerr << "Failed to open " << files[g] << std::endl; continue; }  // the reference only warns (coal.cpp:2093-2098)
       fseek(f, 0, SEEK_END);
@@ -354,8 +422,17 @@ int run_mut(const Options& options)
         }
         d.pos.assign(sh.pos.begin() + s0, sh.pos.begin() + sh.off[d.c_hi]);
       }
+      // BAM genomes: the pileup of each file at the rows (parse_onebambam's bam_parser, coal.cpp:1799-2069) and the bam
+      // front-end's raw count weights and 1e3 normalisation
+      if (bam && colate_set_option(d.h, "front_end", 1)) { d.fail("colate_set_option"); return; }
       for (int g = 0; g < 2; g++) {
-        if (G == 1) {
+        if (bam) {
+          if (colate_pileup_bam(d.h, g, files[g].c_str(), n_chr, names.data(), (const uint8_t* const*)refg.seq.data(), refg.len.data(), filters[0],
+                                filters[1], filters[2], 0, nullptr)) {
+            d.fail(files[g]);
+            return;
+          }
+        } else if (G == 1) {
           if (colate_ingest_colate_in(d.h, g, gh[g].image.data(), (int64_t)gh[g].image.size(), n_chr, names.data(), 0) < 0) {
             d.fail("colate_ingest_colate_in");
             return;
@@ -467,7 +544,9 @@ int run_mut(const Options& options)
       } else {
         std::vector<int32_t> w((size_t)n * num_blocks);
         for (int k = 0; k < n; k++) memcpy(w.data() + (size_t)k * num_blocks, weights.data() + (size_t)mine[k] * num_blocks, (size_t)num_blocks * 4);
-        if (colate_stage2_bootstrap(d.h, n, num_blocks, w.data(), block_stats.data(), age, nullptr)) { d.fail("colate_stage2_bootstrap"); return; }
+        if (colate_stage2_bootstrap(d.h, n, num_blocks, w.data(), block_stats.data(), age, bam ? cn.data() : nullptr)) { d.fail("colate_stage2_bootstrap"); return; }
+        for (int k = 0; k < n && bam; k++)
+          memcpy(counts.data() + (size_t)mine[k] * 2 * COLATE_NUM_AGE_BINS, cn.data() + (size_t)k * 2 * COLATE_NUM_AGE_BINS, 2 * COLATE_NUM_AGE_BINS * 8);
       }
       if (colate_stage3_em(d.h, n, E, epochs.data(), rates_init.data(), cn_in, 100000, rt.data(), it.data(), l2.data())) { d.fail("colate_stage3_em"); return; }
       for (int k = 0; k < n; k++) {
@@ -478,6 +557,11 @@ int run_mut(const Options& options)
     });
     if (!all_ok(devs)) return 1;
     for (int i = 0; i < R; i++) std::cerr << "Bootstrap " << i + 1 << ": Total iterations " << iters[i] << std::endl;
+  }
+  if (bam && !from_cache) {   // every front-end but tmp/tmp keeps its bootstrap counts (coal.cpp:3336-3343, 3453-3465)
+    double age_bin[COLATE_NUM_AGE_BINS];
+    colate_age_bins(age_bin);
+    if (colate_write_colate_mat((out + ".colate_mat").c_str(), R, age_bin, counts.data())) return die("write .colate_mat");
   }
   // .coal first: for ancient samples it zeroes rates[0..ep_null] (coal.cpp:3832-3834); the fp64 side
   // output then holds exactly the values the text was printed from
@@ -870,6 +954,79 @@ int run_cohort(const Options& options)
   return n_failed ? 1 : 0;
 }
 
+// --mode make_tmp --target_bam (maketmp_bam, coal.cpp:2527-2680): the pileup of the BAM file at the .mut rows comes from the
+// device (colate_pileup_bam), the .colate.in is written on the host from it (colate_maketmp_pileup)
+int run_make_tmp_bam(const Options& options)
+{
+  std::cerr << options.get("target_bam") << ".." << std::endl;
+  if (!bam_args_ok(options, false)) return 1;
+  std::vector<std::string> name_chr, f_mut, f_mask;
+  if (options.count("chr")) {
+    std::ifstream is(options.get("chr"));
+    if (is.fail()) std::cerr << "Error while opening file " << options.get("chr") << std::endl;
+    std::string line;
+    while (std::getline(is, line)) {
+      name_chr.push_back(line);
+      f_mut.push_back(options.get("mut") + "_chr" + line + ".mut");
+      if (options.count("target_mask")) f_mask.push_back(options.get("target_mask") + "_chr" + line + ".fa");
+    }
+  } else {
+    name_chr.push_back("");
+    f_mut.push_back(options.get("mut"));
+    if (options.count("target_mask")) f_mask.push_back(options.get("target_mask"));
+  }
+  const int n_chr = (int)name_chr.size();
+  {
+    std::set<std::string> uniq(name_chr.begin(), name_chr.end());
+    if ((int)uniq.size() != n_chr) { std::cerr << "Duplicate chromosome names in --chr" << std::endl; return 1; }
+  }
+  int filters[3];
+  parse_filters(options, filters);
+  std::vector<int64_t> off(n_chr + 1, 0);
+  std::vector<int32_t> pos;
+  std::vector<float> ab, ae;
+  std::vector<uint32_t> meta;
+  for (int c = 0; c < n_chr; c++) {
+    std::cerr << "parsing CHR: " << c + 1 << " / " << n_chr << std::endl;
+    const int64_t n = colate_read_mut(f_mut[c].c_str(), 0, nullptr, nullptr, nullptr, nullptr);
+    if (n < 0) { std::cerr << colate_last_error() << std::endl; return 1; }
+    const size_t o = pos.size();
+    pos.resize(o + n); ab.resize(o + n); ae.resize(o + n); meta.resize(o + n);
+    if (colate_read_mut(f_mut[c].c_str(), n, pos.data() + o, ab.data() + o, ae.data() + o, meta.data() + o) < 0) {
+      std::cerr << colate_last_error() << std::endl;
+      return 1;
+    }
+    off[c + 1] = (int64_t)pos.size();
+  }
+  RefGenome refg;
+  if (!refg.read(options, name_chr)) return 1;
+  colate_handle* h = nullptr;
+  if (colate_create(options.count("device") ? atoi(options.get("device").c_str()) : 0, &h)) return die("colate_create");
+  struct Destroy { colate_handle* h; ~Destroy() { colate_destroy(h); } } destroy{h};
+  std::vector<const char*> names, muts, masks;
+  for (int c = 0; c < n_chr; c++) {
+    names.push_back(name_chr[c].c_str());
+    muts.push_back(f_mut[c].c_str());
+    if (!f_mask.empty()) masks.push_back(f_mask[c].c_str());
+  }
+  std::vector<int32_t> counts((size_t)off[n_chr] * 4 + 4);
+  if (colate_set_sites(h, n_chr, off.data(), pos.data(), ab.data(), ae.data(), meta.data(), 0)) return die("colate_set_sites");
+  if (colate_pileup_bam(h, 0, options.get("target_bam").c_str(), n_chr, names.data(), (const uint8_t* const*)refg.seq.data(), refg.len.data(),
+                        filters[0], filters[1], filters[2], 0, counts.data()))
+    return die(options.get("target_bam"));
+  const std::string out = options.get("output") + ".colate.in";
+  if (colate_maketmp_pileup(n_chr, names.data(), muts.data(), counts.data(), off[n_chr], masks.empty() ? nullptr : masks.data(), out.c_str()) < 0) {
+    std::cerr << colate_last_error() << std::endl;
+    return 1;
+  }
+  rusage usage;
+  getrusage(RUSAGE_SELF, &usage);
+  std::cerr << "CPU Time spent: " << usage.ru_utime.tv_sec << "." << std::setfill('0') << std::setw(6) << usage.ru_utime.tv_usec
+            << "s; Max Memory usage: " << usage.ru_maxrss / 1000.0 << "Mb." << std::endl;
+  std::cerr << "---------------------------------------------------------" << std::endl << std::endl;
+  return 0;
+}
+
 // --mode make_tmp with --target_table (make_tmp(), coal.cpp:2923-3069 -> maketmp_table, 2682-2808): host-only
 int run_make_tmp(const Options& options)
 {
@@ -882,10 +1039,11 @@ int run_make_tmp(const Options& options)
   }
   std::cerr << "---------------------------------------------------------" << std::endl;
   std::cerr << "Calculating Colate tmp input file for ";
-  if (options.count("target_bcf") || options.count("target_bam")) {
-    std::cerr << std::endl << "This build writes .colate.in files from a --target_table only; bcf / bam inputs need htslib and are out of scope." << std::endl;
+  if (options.count("target_bcf")) {
+    std::cerr << std::endl << "This build writes .colate.in files from a --target_table or a --target_bam; bcf inputs are out of scope." << std::endl;
     return 1;
   }
+  if (options.count("target_bam")) return run_make_tmp_bam(options);
   if (!options.count("target_table")) { std::cerr << std::endl; return 0; }   // the reference does nothing without an input either
   if (!options.count("ref_genome")) { std::cerr << std::endl << "Option 'ref_genome' has no value" << std::endl; return 1; }   // cxxopts throws in the reference
   std::cerr << options.get("target_table") << ".." << std::endl;
@@ -951,8 +1109,8 @@ int main(int argc, char* argv[])
   else {
     std::cout << "####### error #######" << std::endl;
     std::cout << "Invalid or missing mode." << std::endl;
-    std::cout << "This build implements --mode mut (tmp/tmp inputs) and --mode make_tmp from a --target_table. The reference's other "
-                 "modes (preprocess_mut, make_tmp from bcf / bam, calc_depth, print_tmp, CondCoalRates) are out of scope." << std::endl;
+    std::cout << "This build implements --mode mut (tmp/tmp or bam/bam inputs) and --mode make_tmp from a --target_table or a --target_bam. "
+                 "The reference's other modes (preprocess_mut, make_tmp from bcf, calc_depth, print_tmp, CondCoalRates) are out of scope." << std::endl;
   }
   if (options.count("help")) help();
   return rc;

@@ -124,6 +124,10 @@ struct colate_handle {
   std::vector<cudaEvent_t> ing_evs;               // one per chromosome text in flight on the copy stream
   void* ing_bounce[2] = {nullptr, nullptr};       // pinned staging for pageable callers
   cudaEvent_t ing_bounce_ev[2] = {nullptr, nullptr};
+  // colate_pileup_bam (kernels_bam.cu): one window's bytes and decoded columns, the current contig's reference, the order state
+  colate::DevBuf bam_buf, bam_ref, bam_state;
+  bool opt_bam_timing = false;
+  double bam_timing[10] = {};
 };
 
 namespace colate {
@@ -142,7 +146,7 @@ int run_replay(colate_handle* h);
 int run_pack_row_counts(colate_handle* h, int slot, const int32_t* aaf_dev, const int32_t* daf_dev);
 int run_pileup_reads(colate_handle* h, int slot, int chr, int64_t n_reads, const int32_t* pos, const uint8_t* mapq, const int32_t* len,
                      const int64_t* off, const uint8_t* seq, const uint8_t* qual, const uint8_t* ref, int64_t ref_len, int max_len,
-                     int mapq_th, int len_th, int mismatch_th, uint8_t* pass_scratch);
+                     int mapq_th, int len_th, int mismatch_th, uint8_t* pass_scratch, bool starts_contig, int64_t row_lo, int64_t row_hi);
 int run_test_bin_fast(colate_handle* h, int n, const double* a_host, int32_t* fast_host, int32_t* exact_host);
 int run_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, uint64_t* out3_host);
 // kernels_mt.cu

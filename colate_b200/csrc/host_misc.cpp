@@ -652,6 +652,22 @@ static bool read_fasta_seq(const std::string& path, std::vector<char>& seq)
   return true;
 }
 
+extern "C" int64_t colate_read_fasta(const char* path, uint8_t** seq_out)
+{
+  using colate::fail;
+  if (!path || !seq_out) return fail(COLATE_ERR_ARG, "colate_read_fasta: bad arguments");
+  *seq_out = nullptr;
+  std::vector<char> seq;
+  if (!read_fasta_seq(path, seq)) return fail(COLATE_ERR_IO, std::string("Error while opening file ") + path + ".");
+  uint8_t* p = (uint8_t*)malloc(seq.size() + 1);
+  if (!p) return fail(COLATE_ERR_ARG, "colate_read_fasta: out of host memory");
+  memcpy(p, seq.data(), seq.size());
+  *seq_out = p;
+  return (int64_t)seq.size();
+}
+
+extern "C" void colate_free(void* p) { free(p); }
+
 // maketmp_table (coal.cpp:2682-2808): a .colate.in record stream for a haploid target given as a whitespace-separated
 // table of (chromosome, position, allele) triples in --chr order.  For every row of the .mut files that is not
 // flipped, maps to one branch and has single-letter allele codes (no age condition here), passes the optional mask

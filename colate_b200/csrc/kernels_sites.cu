@@ -215,9 +215,11 @@ __device__ __forceinline__ int nt16_code(uint8_t c)
   for (int i = 0; i < 16; i++) k = (c == (uint8_t)t[i]) ? i : k;
   return k;
 }
-__device__ __forceinline__ int read_base_quality(int64_t k, int64_t i, int l, int64_t o, const uint8_t* __restrict__ seq, const uint8_t* __restrict__ qual)
+// k_quirk: index of the contig's first record in the arrays (0), or -1 when they do not start the contig (a later BAM chunk)
+__device__ __forceinline__ int read_base_quality(int64_t k, int64_t k_quirk, int64_t i, int l, int64_t o, const uint8_t* __restrict__ seq,
+                                                 const uint8_t* __restrict__ qual)
 {
-  if (k != 0) return qual[o + i];
+  if (k != k_quirk) return qual[o + i];
   const int64_t nb = ((int64_t)l + 1) >> 1;
   if (i >= nb) return qual[o + i - nb];
   const int hi = nt16_code(seq[o + 2 * i]), lo = 2 * i + 1 < l ? nt16_code(seq[o + 2 * i + 1]) : 0;
@@ -225,7 +227,8 @@ __device__ __forceinline__ int read_base_quality(int64_t k, int64_t i, int l, in
 }
 __global__ void k_read_filter(int64_t n_reads, const int32_t* __restrict__ pos, const uint8_t* __restrict__ mapq, const int32_t* __restrict__ len,
                               const int64_t* __restrict__ off, const uint8_t* __restrict__ seq, const uint8_t* __restrict__ qual,
-                              const uint8_t* __restrict__ ref, int64_t ref_len, int mapq_th, int len_th, int mismatch_th, uint8_t* __restrict__ pass)
+                              const uint8_t* __restrict__ ref, int64_t ref_len, int mapq_th, int len_th, int mismatch_th, int64_t k_quirk,
+                              uint8_t* __restrict__ pass)
 {
   const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= n_reads) return;
@@ -236,7 +239,7 @@ __global__ void k_read_filter(int64_t n_reads, const int32_t* __restrict__ pos, 
     int total = 0, matching = 0;
     for (int i = 3; i < l - 3; i++) {
       if (p + i >= ref_len) break;
-      if (read_base_quality(k, i, l, o, seq, qual) >= 30) { total++; matching += ref[p + i] == seq[o + i]; }
+      if (read_base_quality(k, k_quirk, i, l, o, seq, qual) >= 30) { total++; matching += ref[p + i] == seq[o + i]; }
     }
     ok = total > 0 && total - matching <= mismatch_th;
   }
@@ -245,7 +248,8 @@ __global__ void k_read_filter(int64_t n_reads, const int32_t* __restrict__ pos, 
 
 __global__ void k_pileup_rows(int64_t row0, int64_t n_rows, const int32_t* __restrict__ site_pos, int64_t n_reads, const int32_t* __restrict__ pos,
                               const int32_t* __restrict__ len, const int64_t* __restrict__ off, const uint8_t* __restrict__ seq,
-                              const uint8_t* __restrict__ qual, const uint8_t* __restrict__ pass, int max_len, int4* __restrict__ pile)
+                              const uint8_t* __restrict__ qual, const uint8_t* __restrict__ pass, int max_len, int64_t k_quirk,
+                              int4* __restrict__ pile)
 {
   const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (m >= n_rows) return;
@@ -257,7 +261,7 @@ __global__ void k_pileup_rows(int64_t row0, int64_t n_rows, const int32_t* __res
     if (!pass[k]) continue;
     const int64_t i = p - pos[k];
     if (i < 3 || i >= (int64_t)len[k] - 3) continue;
-    if (read_base_quality(k, i, len[k], off[k], seq, qual) < 30) continue;
+    if (read_base_quality(k, k_quirk, i, len[k], off[k], seq, qual) < 30) continue;
     const uint8_t b = seq[off[k] + i];
     c.x += b == 'A'; c.y += b == 'C'; c.z += b == 'G'; c.w += b == 'T';
   }
@@ -1400,18 +1404,24 @@ int run_pack_row_counts(colate_handle* h, int slot, const int32_t* aaf_dev, cons
   return 0;
 }
 
-// pileup of one contig's decoded reads at the rows of chromosome chr (device pointers throughout)
+// pileup of one contig's decoded reads at the rows of chromosome chr (device pointers throughout).  starts_contig: reads[0] is the
+// contig's first record (the assign_contig quirk applies to it); only rows [row_lo, row_hi) of the contig are searched (rows the
+// reads cannot cover are left as they are; row_hi < 0: all rows).
 int run_pileup_reads(colate_handle* h, int slot, int chr, int64_t n_reads, const int32_t* pos, const uint8_t* mapq, const int32_t* len,
                      const int64_t* off, const uint8_t* seq, const uint8_t* qual, const uint8_t* ref, int64_t ref_len, int max_len,
-                     int mapq_th, int len_th, int mismatch_th, uint8_t* pass_scratch)
+                     int mapq_th, int len_th, int mismatch_th, uint8_t* pass_scratch, bool starts_contig, int64_t row_lo, int64_t row_hi)
 {
   GenomeDev& g = h->genomes[slot];
-  const int64_t row0 = h->h_site_off[chr], n_rows = h->h_site_off[chr + 1] - row0;
+  const int64_t n_chr_rows = h->h_site_off[chr + 1] - h->h_site_off[chr];
+  if (row_hi < 0) { row_lo = 0; row_hi = n_chr_rows; }
+  const int64_t row0 = h->h_site_off[chr] + row_lo, n_rows = row_hi - row_lo;
   if (n_reads <= 0 || n_rows <= 0) return 0;
+  const int64_t k_quirk = starts_contig ? 0 : -1;
   cudaStream_t s = h->stream;
-  k_read_filter<<<grid_for(n_reads, 256), 256, 0, s>>>(n_reads, pos, mapq, len, off, seq, qual, ref, ref_len, mapq_th, len_th, mismatch_th, pass_scratch);
+  k_read_filter<<<grid_for(n_reads, 256), 256, 0, s>>>(n_reads, pos, mapq, len, off, seq, qual, ref, ref_len, mapq_th, len_th, mismatch_th, k_quirk,
+                                                       pass_scratch);
   k_pileup_rows<<<grid_for(n_rows, 128), 128, 0, s>>>(row0, n_rows, h->pos.as<int32_t>(), n_reads, pos, len, off, seq, qual, pass_scratch, max_len,
-                                                     g.pile.as<int4>());
+                                                     k_quirk, g.pile.as<int4>());
   h->launches += 2;
   CK(cudaGetLastError());
   return 0;

@@ -322,3 +322,130 @@ def write_dataset(dirname: str, sites: Sites, genomes: dict, masks: dict | None 
         for c, nm in enumerate(sites.chr_names):
             write_mask(os.path.join(dirname, f"{mname}_chr{nm}.fa"), per_chr[c])
     return dirname
+
+
+# ---- BAM files (SAM/BAM format specification 4.1-4.2): BGZF blocks around the binary records, written with zlib ----------------
+NT16 = b"=ACMGRSVTWYHKDBN"
+_NT16_CODE = np.full(256, 15, dtype=np.uint8)
+_NT16_CODE[np.frombuffer(NT16, np.uint8)] = np.arange(16, dtype=np.uint8)
+CIGAR_OPS = "MIDNSHP=X"
+
+
+def bam_record(tid, pos0, mapq, flag, seq, qual, name=b"r", cigar=None, aux=b"", next_tid=-1, next_pos=-1, tlen=0) -> bytes:
+    """One BAM record (block_size included).  seq: letters of seq_nt16_str (others become N); qual: phred bytes (len(seq) of them);
+    cigar: [(length, op letter)] (default: one <len>M op, none for an empty sequence); aux: raw aux bytes."""
+    import struct
+    seq = bytes(seq)
+    l = len(seq)
+    if cigar is None:
+        cigar = [(l, "M")] if l else []
+    nm = bytes(name) + b"\0"
+    codes = _NT16_CODE[np.frombuffer(seq, np.uint8)] if l else np.zeros(0, np.uint8)
+    if l & 1:
+        codes = np.concatenate([codes, np.zeros(1, np.uint8)])
+    packed = (codes[0::2] << 4 | codes[1::2]).astype(np.uint8).tobytes()
+    q = bytes(bytearray(qual))
+    assert len(q) == l and len(nm) <= 255
+    cig = b"".join(struct.pack("<I", n << 4 | CIGAR_OPS.index(op)) for n, op in cigar)
+    core = struct.pack("<iiBBHHHiiii", tid, pos0, len(nm), mapq, 4680, len(cigar), flag, l, next_tid, next_pos, tlen)
+    body = core + nm + cig + packed + q + bytes(aux)
+    return struct.pack("<i", len(body)) + body
+
+
+def bam_header(contig_names, contig_lens=None, text=b"") -> bytes:
+    import struct
+    lens = contig_lens if contig_lens is not None else [1 << 29] * len(contig_names)
+    out = [b"BAM\1", struct.pack("<i", len(text)), bytes(text), struct.pack("<i", len(contig_names))]
+    for nm, L in zip(contig_names, lens):
+        b = nm.encode() + b"\0"
+        out += [struct.pack("<i", len(b)), b, struct.pack("<i", int(L))]
+    return b"".join(out)
+
+
+def bgzf_block(data: bytes, level=6) -> bytes:
+    """One BGZF block: a gzip member with the 'BC' extra subfield holding the block size - 1."""
+    import struct
+    import zlib
+    c = zlib.compressobj(level, zlib.DEFLATED, -15)
+    body = c.compress(data) + c.flush()
+    hdr = struct.pack("<BBBBIBBH", 31, 139, 8, 4, 0, 0, 255, 6) + b"BC" + struct.pack("<HH", 2, 18 + len(body) + 8 - 1)
+    return hdr + body + struct.pack("<II", zlib.crc32(data) & 0xFFFFFFFF, len(data))
+
+
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+
+
+def bgzf_compress(data: bytes, block_size=65280, empty_blocks=(), eof=True, level=6, threads=1) -> bytes:
+    """`data` cut into BGZF blocks of block_size inflated bytes (1..65536; records straddle blocks wherever the cut falls),
+    an empty block inserted before block k for every k in empty_blocks, the EOF block at the end if eof."""
+    assert 1 <= block_size <= 65536
+    pieces = [data[i:i + block_size] for i in range(0, len(data), block_size)]
+    if threads > 1:
+        from concurrent.futures import ThreadPoolExecutor
+        with ThreadPoolExecutor(threads) as ex:
+            blocks = list(ex.map(lambda p: bgzf_block(p, level), pieces, chunksize=256))
+    else:
+        blocks = [bgzf_block(p, level) for p in pieces]
+    empty = bgzf_block(b"", level)
+    out = []
+    for k, b in enumerate(blocks):
+        out += [empty] * sum(1 for e in empty_blocks if e == k)
+        out.append(b)
+    out += [empty] * sum(1 for e in empty_blocks if e >= len(blocks))
+    if eof:
+        out.append(BGZF_EOF)
+    return b"".join(out)
+
+
+def write_bam(path, contig_names, reads, contig_lens=None, text=b"", block_size=65280, empty_blocks=(), eof=True, level=6, threads=1):
+    """A BAM file: header (contig_names, optional lengths and SAM text) and `reads`, each either a record from bam_record() or the
+    tuple of its arguments (tid, pos0, mapq, flag, seq, qual[, name, cigar, aux]); records are written in the order given."""
+    recs = [r if isinstance(r, (bytes, bytearray)) else bam_record(*r) for r in reads]
+    data = bam_header(contig_names, contig_lens, text) + b"".join(recs)
+    with open(path, "wb") as f:
+        f.write(bgzf_compress(data, block_size, empty_blocks, eof, level, threads))
+
+
+def bam_records_np(tid, pos0, mapq, lens, seq, qual, flag=None):
+    """Many records at once (benchmarks): arrays tid/pos0/mapq/lens [n], seq letters and qual phred bytes concatenated in read order;
+    name "r", one <len>M CIGAR op, no aux.  Returns the records as one uint8 array."""
+    n = len(pos0)
+    lens = np.asarray(lens, np.int64)
+    nb = (lens + 1) // 2
+    size = 36 + 2 + 4 + nb + lens                    # block_size field + core + name + cigar + packed + qual
+    off = np.zeros(n + 1, np.int64)
+    np.cumsum(size, out=off[1:])
+    buf = np.zeros(int(off[-1]), np.uint8)
+    o = off[:-1]
+
+    def put(at, v, nbytes):
+        v = np.asarray(v, np.int64) & ((1 << (8 * nbytes)) - 1)
+        for b in range(nbytes):
+            buf[at + b] = (v >> (8 * b)) & 0xFF
+    put(o, size - 4, 4)
+    put(o + 4, tid, 4)
+    put(o + 8, pos0, 4)
+    buf[o + 12] = 2
+    buf[o + 13] = np.asarray(mapq, np.uint8)
+    put(o + 14, 4680, 2)
+    put(o + 16, 1, 2)
+    put(o + 18, 0 if flag is None else flag, 2)
+    put(o + 20, lens, 4)
+    put(o + 24, -1, 4)
+    put(o + 28, -1, 4)
+    buf[o + 36] = ord("r")
+    put(o + 38, lens << 4, 4)
+    # packed sequence: read r's byte j = code(2j) << 4 | code(2j + 1)
+    codes = _NT16_CODE[np.frombuffer(bytes(seq), np.uint8) if not isinstance(seq, np.ndarray) else seq]
+    sstart = np.zeros(n + 1, np.int64)
+    np.cumsum(lens, out=sstart[1:])
+    rid = np.repeat(np.arange(n), nb)
+    j = np.arange(int(nb.sum())) - np.repeat(np.cumsum(nb) - nb, nb)
+    hi_i = sstart[rid] + 2 * j
+    lo_i = hi_i + 1
+    lo_ok = 2 * j + 1 < lens[rid]
+    packed = (codes[hi_i] << 4) | np.where(lo_ok, codes[np.minimum(lo_i, len(codes) - 1)], 0)
+    buf[np.repeat(o + 42, nb) + j] = packed.astype(np.uint8)
+    qi = np.arange(int(lens.sum())) - np.repeat(sstart[:-1], lens)
+    buf[np.repeat(o + 42 + nb, lens) + qi] = np.asarray(qual, np.uint8)
+    return buf

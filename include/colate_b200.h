@@ -116,6 +116,28 @@ int colate_pileup_reads(colate_handle* h, int slot, int chr_index, int64_t n_rea
                         int mapq_th, int len_th, int mismatch_th);
 int colate_pileup_end(colate_handle* h, int slot, int32_t* counts_out);
 
+/* The same pileup straight from a BAM file: replaces colate_pileup_begin / _reads / _end for `slot` and leaves it a pileup genome
+ * (counts_out, optional: counts[n_site][4]).  What htslib's sam_read1 and bam_parser::read_entry / assign_contig do for the bam
+ * front-ends (include/vcf/htslib.cpp:379-437, 490-573) is done here: BGZF blocks are inflated in parallel on the host (CRC32 and
+ * ISIZE checked), the header's contigs are matched to the --chr list (`<name>` or `chr<name>`, htslib.cpp:388), the records are
+ * decoded on the device (pos, mapq, l_seq, packed sequence, qualities; read name, CIGAR, flag and aux data are not looked at)
+ * and counted by the same kernels as colate_pileup_reads, in chunks of at most chunk_bytes record bytes (0: 64 MiB) while the
+ * host inflates the next one.  The assign_contig quirk applies to the first record of every contig.
+ *   chr_names[n_chr]: the site set's --chr list; ref_seqs[c] / ref_lens[c]: contig c of --ref_genome (host memory; upper-cased
+ *   on the device as fasta::Read does, data.cpp:213-237); mapq_th, len_th, mismatch_th: --filters.
+ * Refused: COLATE_ERR_IO for a file that is not BGZF (plain gzip included), truncated blocks, CRC / ISIZE mismatches, a wrong
+ * magic, a header or record that runs past the data, a listed contig absent from the header or present under both spellings,
+ * listed contigs whose records are not contiguous or not in --chr order (message: file and byte offset); COLATE_ERR_ORDER for
+ * descending positions within a contig ("BAM file not sorted by position.", htslib.cpp:411-414, checked on the device across
+ * chunks) or a record of a listed contig with a negative position (checked on the host before anything is launched).
+ * Records of unlisted contigs and unmapped records without a contig (refID -1) are skipped.  A missing EOF block is accepted. */
+int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_chr, const char* const* chr_names, const uint8_t* const* ref_seqs,
+                      const int64_t* ref_lens, int mapq_th, int len_th, int mismatch_th, int64_t chunk_bytes, int32_t* counts_out);
+/* Phases of the last colate_pileup_bam: [0] BGZF index s, [1] inflate s (wall, summed over windows), [2] record walk s, [3] host-to-device
+ * copies ms, [4] device decode ms, [5] filter + pileup ms ([3]-[5] only with colate_set_option(h, "bam_timing", 1)), [6] whole call s,
+ * [7] inflate threads, [8] inflated bytes, [9] records of listed contigs. */
+int colate_last_bam_timing(colate_handle* h, double* out10);
+
 /* P/N mask of genome `slot` evaluated at the site positions (fasta::Read,
  * include/src/data.cpp:213-237; test at coal.cpp:2169-2174): bit m of pass_bits = row m is
  * NOT rejected by the mask (positions at or beyond the mask end pass).  NULL clears it. */
@@ -293,6 +315,15 @@ int64_t colate_read_mut(const char* path, int64_t cap, int32_t* pos, float* age_
 /* .colate.in (coal.cpp:2505-2514).  rec_chrom[k] = index of the record's name in chr_names. */
 int64_t colate_read_colate_in(const char* path, int n_chr, const char* const* chr_names, int64_t cap,
                               int32_t* rec_chrom, int32_t* bp, int32_t* aaf, int32_t* daf, uint16_t* alleles);
+/* BAM file, host only (no GPU): per --chr entry the number of records, the first and the last record's position and the index of
+ * the header contig it matched, with every check of colate_pileup_bam but the order of positions.  window_bytes: inflated bytes per
+ * window (0: 64 MiB).  0 or a negative status. */
+int colate_bam_scan(const char* path, int n_chr, const char* const* chr_names, int64_t window_bytes, int64_t* n_records, int32_t* first_pos,
+                    int32_t* last_pos, int32_t* ref_id);
+/* fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz.  *seq_out: malloc'd,
+ * release with colate_free.  Returns the length or < 0. */
+int64_t colate_read_fasta(const char* path, uint8_t** seq_out);
+void colate_free(void* p);
 /* fasta mask (data.cpp:213-237) evaluated at positions -> pass bits for rows [row0, row0+n). */
 int colate_mask_bits_from_fasta(const char* path, int64_t n, const int32_t* pos, int64_t row0, uint32_t* pass_bits);
 /* make_tmp from a table (maketmp_table, coal.cpp:2682-2808; README.md:86-127): writes the .colate.in record stream of a
