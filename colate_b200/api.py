@@ -137,6 +137,16 @@ def bam_scan(path: str, chr_names, window_bytes: int = 0) -> dict:
     return {"n_records": cnt, "first_pos": first, "last_pos": last, "ref_id": rid}
 
 
+def bcf_scan(path: str, window_bytes: int = 0) -> dict:
+    """Host-only walk of a BCF file (no GPU): the record count, the first / last POS (0-based), the records' contig, the header's
+    sample count and the dictionary index of GT (colate_bcf_scan).  Raises ColateError for the files colate_rows_from_bcf refuses
+    on the host."""
+    v = [np.zeros(1, t) for t in (np.int64, np.int32, np.int32, np.int32, np.int32, np.int32)]
+    check(lib().colate_bcf_scan(str(path).encode(), window_bytes, *[ptr(x) for x in v]))
+    keys = ("n_records", "first_pos", "last_pos", "contig", "n_sample", "gt_key")
+    return {k: int(x[0]) for k, x in zip(keys, v)}
+
+
 def read_fasta(path: str) -> np.ndarray:
     """fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz."""
     p = C.POINTER(C.c_uint8)()
@@ -254,6 +264,47 @@ class Handle:
         t = np.zeros(10)
         check(lib().colate_last_bam_timing(self._h, t))
         keys = ("index_s", "inflate_s", "walk_s", "h2d_ms", "decode_ms", "pileup_ms", "total_s", "threads", "inflated_bytes", "records")
+        return dict(zip(keys, t.tolist()))
+
+    def rows_from_bcf(self, slot, paths, role, ref_genomes=None, chunk_bytes=0, fetch=False):
+        """The row counts of genome `slot` straight from BCF files (colate_rows_from_bcf): paths[c] = the file of chromosome c of the
+        site set (the reference's <prefix>_chr<c>.bcf), role "target" / "reference" (or 0 / 1), ref_genomes[c] = uint8 / bytes
+        sequence of contig c of --ref_genome or None.  BGZF is inflated on the host, the records are decoded and resolved on the
+        device.  Makes `slot` a row-count genome (use with front_end = 1); fetch=True returns (aaf, daf) per row."""
+        role = {"target": 0, "reference": 1}.get(role, role)
+        n = len(paths)
+        names = (C.c_char_p * n)(*[str(c).encode() for c in range(n)])
+        files = (C.c_char_p * n)(*[str(p).encode() for p in paths])
+        seqs = lens = None
+        if ref_genomes is not None:
+            refs = [np.ascontiguousarray(np.frombuffer(g, np.uint8) if isinstance(g, (bytes, bytearray)) else g, dtype=np.uint8) for g in ref_genomes]
+            seqs = (C.c_void_p * n)(*[r.ctypes.data if r.shape[0] else None for r in refs])
+            lens = np.array([r.shape[0] for r in refs], dtype=np.int64)
+        aaf = np.zeros(self.n_site, np.int32) if fetch else None
+        daf = np.zeros(self.n_site, np.int32) if fetch else None
+        check(lib().colate_rows_from_bcf(self._h, slot, role, n, names, files, C.cast(seqs, C.c_void_p) if seqs is not None else None,
+                                         ptr(lens) if lens is not None else None, chunk_bytes, ptr(aaf) if fetch else None,
+                                         ptr(daf) if fetch else None))
+        return (aaf, daf) if fetch else None
+
+    def decode_bcf(self, path, chunk_bytes=0) -> dict:
+        """One BCF file's records as the device reduces them (colate_decode_bcf + colate_bcf_records): pos (1-based), a0 / a1 (first
+        two alleles: 0 empty or absent, the letter, 0xff longer), alt_sum (sum of the GT allele indices), biallelic, and n_hap."""
+        n = np.zeros(1, np.int64)
+        nh = np.zeros(1, np.int32)
+        check(lib().colate_decode_bcf(self._h, str(path).encode(), chunk_bytes, ptr(n), ptr(nh)))
+        k = int(n[0])
+        out = {"pos": np.zeros(k, np.int32), "a0": np.zeros(k, np.uint8), "a1": np.zeros(k, np.uint8), "alt_sum": np.zeros(k, np.int32),
+               "biallelic": np.zeros(k, np.uint8)}
+        check(lib().colate_bcf_records(self._h, 0, k, *[ptr(out[x]) for x in ("pos", "a0", "a1", "alt_sum", "biallelic")]))
+        out["n_hap"] = int(nh[0])
+        return out
+
+    def last_bcf_timing(self) -> dict:
+        """Phases of the last rows_from_bcf / decode_bcf (colate_last_bcf_timing; copy / decode / rows need set_option("bcf_timing", 1))."""
+        t = np.zeros(10)
+        check(lib().colate_last_bcf_timing(self._h, t))
+        keys = ("index_s", "inflate_s", "walk_s", "h2d_ms", "decode_ms", "rows_ms", "total_s", "threads", "inflated_bytes", "records")
         return dict(zip(keys, t.tolist()))
 
     def set_mask(self, slot, pass_bits):

@@ -151,7 +151,8 @@ void colate_destroy(colate_handle* h)
                     &h->chr_used, &h->chr_blocks, &h->chr_block_base, &h->misc, &h->u_hdr, &h->u_eb2, &h->u_ews, &h->u_ewn, &h->u_cnt,
                     &h->u_blk, &h->blk_rank_start, &h->out_f, &h->out_n, &h->thrA, &h->lut, &h->d_scratch, &h->d_prof, &h->libm_tab, &h->ing_text, &h->ing_tile_cnt, &h->ing_tile_off, &h->ing_nl, &h->ing_status, &h->ing_fb,
                     &h->windows, &h->rng_stream, &h->mt_tail, &h->poly, &h->thr10, &h->d_counts, &h->d_blockstats, &h->d_weights, &h->d_epochs,
-                    &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo, &h->bam_buf, &h->bam_ref, &h->bam_state};
+                    &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo, &h->bam_buf, &h->bam_ref, &h->bam_state,
+                    &h->bcf_buf, &h->bcf_cols, &h->bcf_ref, &h->bcf_state};
   for (DevBuf* b : bufs) b->release();
   for (auto& g : h->genomes) {
     DevBuf* gb[] = {&g.bp, &g.aaf, &g.daf, &g.alleles, &g.chr_first, &g.chr_end, &g.mask_bits, &g.j_aaf, &g.j_daf, &g.j_prevbp, &g.j_flag, &g.pile};
@@ -549,6 +550,8 @@ int colate_set_option(colate_handle* h, const char* key, int64_t value)
   if (!strcmp(key, "async_uploads")) { h->opt_async_uploads = value != 0; return 0; }
   // bam_timing = 1: colate_pileup_bam times its copies, decode and pileup per chunk (colate_last_bam_timing) and waits for each
   if (!strcmp(key, "bam_timing")) { h->opt_bam_timing = value != 0; return 0; }
+  // bcf_timing = 1: colate_rows_from_bcf / colate_decode_bcf time their copies, decode and row kernels (colate_last_bcf_timing)
+  if (!strcmp(key, "bcf_timing")) { h->opt_bcf_timing = value != 0; return 0; }
   // front_end: which of mut()'s input branches the handle reproduces (coal.cpp:3175-3319).  0 = tmp/tmp (parse_tmptmp: pseudo-
   // genotype weights, no normalisation).  1 = the bcf / bam front-ends fed from pre-decoded per-row counts (SURVEY.md 8f N3):
   // raw count weights (coal.cpp:2005-2039, 1164-1197) and both count vectors of stage ii divided by 1e3 (coal.cpp:3453-3463).

@@ -36,6 +36,24 @@ struct DevBuf {
   template <class T> T* as() const { return (T*)p; }
 };
 
+// growable pinned host buffer (the BGZF readers' windows)
+struct Pinned {
+  void* p = nullptr;
+  size_t cap = 0;
+  cudaError_t ensure(size_t bytes)
+  {
+    if (bytes <= cap) return cudaSuccess;
+    if (p) cudaFreeHost(p);
+    p = nullptr;
+    cap = 0;
+    const size_t want = bytes + bytes / 4 + 4096;
+    cudaError_t e = cudaMallocHost(&p, want);
+    if (e == cudaSuccess) cap = want;
+    return e;
+  }
+  ~Pinned() { if (p) cudaFreeHost(p); }
+};
+
 // one .colate.in file on the device, plus its join onto the site axis
 struct GenomeDev {
   bool set = false, joined = false, has_mask = false;
@@ -128,6 +146,13 @@ struct colate_handle {
   colate::DevBuf bam_buf, bam_ref, bam_state;
   bool opt_bam_timing = false;
   double bam_timing[10] = {};
+  // colate_rows_from_bcf / colate_decode_bcf (kernels_bcf.cu): one window's bytes and record offsets, the decoded columns of one
+  // file (12 B per record, resident), the current chromosome's reference genome, the decode state (GT length, first error)
+  colate::DevBuf bcf_buf, bcf_cols, bcf_ref, bcf_state;
+  int64_t bcf_n_rec = 0;       // records of the last decoded file in bcf_cols
+  int32_t bcf_n_hap = 0;
+  bool opt_bcf_timing = false;
+  double bcf_timing[10] = {};
 };
 
 namespace colate {

@@ -62,23 +62,6 @@ __global__ void k_upper(int64_t n, uint8_t* __restrict__ s)
 inline int grid_for(int64_t n, int threads) { return (int)((n + threads - 1) / threads); }
 inline size_t up(size_t x) { return (x + 255) & ~(size_t)255; }
 
-struct Pinned {
-  void* p = nullptr;
-  size_t cap = 0;
-  cudaError_t ensure(size_t bytes)
-  {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFreeHost(p);
-    p = nullptr;
-    cap = 0;
-    const size_t want = bytes + bytes / 4 + 4096;
-    cudaError_t e = cudaMallocHost(&p, want);
-    if (e == cudaSuccess) cap = want;
-    return e;
-  }
-  ~Pinned() { if (p) cudaFreeHost(p); }
-};
-
 int bam_threads()
 {
   if (const char* e = getenv("COLATE_BAM_THREADS")) return std::max(1, atoi(e));

@@ -449,3 +449,133 @@ def bam_records_np(tid, pos0, mapq, lens, seq, qual, flag=None):
     qi = np.arange(int(lens.sum())) - np.repeat(sstart[:-1], lens)
     buf[np.repeat(o + 42 + nb, lens) + qi] = np.asarray(qual, np.uint8)
     return buf
+
+
+# ---- BCF files (VCF specification v4.3, 6.3 "BCF2"): BGZF blocks around the header text and the binary records ------------------
+BCF_INT8, BCF_INT16, BCF_INT32, BCF_FLOAT, BCF_CHAR = 1, 2, 3, 5, 7
+_BCF_FMT = {BCF_INT8: "b", BCF_INT16: "h", BCF_INT32: "i", BCF_FLOAT: "f"}
+GT_MISSING = {BCF_INT8: -128, BCF_INT16: -32768, BCF_INT32: -2 ** 31}
+GT_VECTOR_END = {BCF_INT8: -127, BCF_INT16: -32767, BCF_INT32: -2 ** 31 + 1}
+
+
+def _bcf_int_type(values):
+    lo, hi = (min(values), max(values)) if len(values) else (0, 0)
+    return BCF_INT8 if -120 <= lo and hi <= 127 else BCF_INT16 if -32760 <= lo and hi <= 32767 else BCF_INT32
+
+
+def bcf_descr(t, n) -> bytes:
+    """Typed-value descriptor: size << 4 | type, sizes from 15 up as the overflow form (15 << 4 | type, then a typed integer)."""
+    return bytes([n << 4 | t]) if n < 15 else bytes([0xF0 | t]) + bcf_typed_ints([n])
+
+
+def bcf_typed_ints(values, t=None) -> bytes:
+    import struct
+    t = t or _bcf_int_type(values)
+    return bcf_descr(t, len(values)) + struct.pack("<%d%s" % (len(values), _BCF_FMT[t]), *values)
+
+
+def bcf_typed_floats(values) -> bytes:
+    import struct
+    return bcf_descr(BCF_FLOAT, len(values)) + struct.pack("<%df" % len(values), *values)
+
+
+def bcf_typed_str(s) -> bytes:
+    return bcf_descr(BCF_CHAR, len(s)) + bytes(s)
+
+
+BCF_FLAG = b"\x00"      # an INFO flag: type 0, size 0
+
+
+def bcf_header(n_sample, ids=(("FORMAT", "GT"),), idx=None, contigs=("1",), minor=2, extra=b"") -> bytes:
+    """Magic, l_text and header text.  ids: (kind, ID) pairs (FILTER / INFO / FORMAT) in order of appearance; PASS is implicit.
+    idx: None (no IDX=, as a hand-written header) or {ID: number} (IDX= on every line, as bcftools writes; PASS gets 0)."""
+    import struct
+    lines = [b"##fileformat=VCFv4.3"]
+    ix = (lambda i: b",IDX=%d" % idx[i]) if idx is not None else (lambda i: b"")
+    lines.append(b'##FILTER=<ID=PASS,Description="All filters passed"' + (b",IDX=0" if idx is not None else b"") + b">")
+    for kind, i in ids:
+        typ = b"String" if i == "GT" else b"Integer"
+        lines.append(b'##%s=<ID=%s,Number=1,Type=%s,Description="a \\"quoted\\", IDX=99 text"%s>' % (kind.encode(), i.encode(), typ, ix(i)))
+    for k, c in enumerate(contigs):
+        lines.append(b"##contig=<ID=%s,length=1000000000%s>" % (c.encode(), b",IDX=%d" % k if idx is not None else b""))
+    lines.append(bytes(extra) if extra else b"##source=colate_b200.synth")
+    cols = b"#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO"
+    if n_sample:
+        cols += b"\tFORMAT" + b"".join(b"\ts%d" % s for s in range(n_sample))
+    text = b"\n".join(lines + [cols]) + b"\n\0"
+    return b"BCF\2" + bytes([minor]) + struct.pack("<I", len(text)) + text
+
+
+def bcf_gt_values(gt, phased=False, t=BCF_INT8):
+    """Allele indices [n_sample][ploidy] (-1: missing '.', None: vector end) -> the typed GT values ((a + 1) << 1 | phased)."""
+    out = []
+    for s in gt:
+        for j, a in enumerate(s):
+            if a is None:
+                out.append(GT_VECTOR_END[t])
+            else:
+                ph = int(phased[j] if isinstance(phased, (list, tuple)) else phased) if j > 0 else 0
+                out.append((int(a) + 1) << 1 | ph)
+    return out
+
+
+def bcf_record(chrom, pos0, alleles, gt, gt_key, phased=False, gt_type=BCF_INT8, rid=b".", qual=None, filters=(), info=(),
+               fmt_before=(), fmt_after=(), gt_raw=None, n_sample=None) -> bytes:
+    """One BCF record (l_shared and l_indiv included).  gt: allele indices [n_sample][ploidy] (bcf_gt_values); gt_raw: the typed GT
+    values themselves instead (per sample a list); gt_key=None writes no GT.  info: (key, typed value bytes) pairs; filters: dictionary
+    indices; fmt_before / fmt_after: FORMAT fields (key, type, values per sample) around GT."""
+    import struct
+    ns = len(gt) if n_sample is None else n_sample
+    shared = [struct.pack("<ii", chrom, pos0), struct.pack("<i", max(1, len(alleles[0]) if alleles else 1)),
+              struct.pack("<I", 0x7F800001) if qual is None else struct.pack("<f", qual)]
+    fmts = list(fmt_before)
+    if gt_key is not None:
+        vals = gt_raw if gt_raw is not None else [bcf_gt_values([s], phased, gt_type) for s in gt]
+        fmts.append((gt_key, gt_type, vals))
+    fmts += list(fmt_after)
+    shared.append(struct.pack("<II", len(alleles) << 16 | len(info), len(fmts) << 24 | ns))
+    shared.append(bcf_typed_str(rid))
+    shared += [bcf_typed_str(a) for a in alleles]
+    shared.append(bcf_typed_ints(list(filters), BCF_INT8) if filters else bytes([BCF_INT8]))
+    for key, val in info:
+        shared += [bcf_typed_ints([key]), bytes(val)]
+    indiv = []
+    for key, t, vals in fmts:
+        size = max(len(v) for v in vals) if vals else 0
+        indiv += [bcf_typed_ints([key]), bcf_descr(t, size)]
+        for v in vals:
+            v = list(v) + [0] * (size - len(v)) if t != BCF_CHAR else bytes(v).ljust(size, b"\0")
+            indiv.append(bytes(v) if t == BCF_CHAR else struct.pack("<%d%s" % (size, _BCF_FMT[t]), *v))
+    s, i = b"".join(shared), b"".join(indiv)
+    return struct.pack("<II", len(s), len(i)) + s + i
+
+
+def write_bcf(path, header, records, block_size=65280, empty_blocks=(), eof=True, level=6, threads=1):
+    """A BCF file: `header` (bcf_header) and the records (bytes or a uint8 array) in the order given, BGZF-compressed."""
+    data = bytes(header) + (records.tobytes() if isinstance(records, np.ndarray) else b"".join(records))
+    with open(path, "wb") as f:
+        f.write(bgzf_compress(data, block_size, empty_blocks, eof, level, threads))
+
+
+def bcf_records_np(pos0, a0, a1, gt_values, gt_key, ploidy=2, chrom=0) -> np.ndarray:
+    """Many records at once (benchmarks): pos0 [n], a0 / a1 [n] one-letter alleles (uint8), gt_values [n][n_hap] the typed int8 GT
+    values; ID '.', FILTER PASS, no INFO, GT the only FORMAT field.  Returns the records as one uint8 array."""
+    gt_values = np.asarray(gt_values, np.int8)
+    n, n_hap = gt_values.shape
+    assert n_hap % ploidy == 0 and ploidy < 15 and gt_key < 120
+    ns = n_hap // ploidy
+    l_shared, l_indiv = 24 + 2 + 2 + 2 + 2, 2 + 1 + n_hap
+    size = 8 + l_shared + l_indiv
+    buf = np.zeros((n, size), np.uint8)
+    head = np.array([l_shared, l_indiv, chrom, 0, 1, 0x7F800001, 2 << 16, 1 << 24 | ns], np.uint32).view(np.uint8)
+    buf[:, :32] = head
+    buf[:, 12:16] = np.asarray(pos0, np.int32).view(np.uint8).reshape(n, 4)
+    buf[:, 32:34] = [0x17, ord(".")]
+    buf[:, 34] = 0x17
+    buf[:, 35] = a0
+    buf[:, 36] = 0x17
+    buf[:, 37] = a1
+    buf[:, 38:40] = [0x11, 0x00]                     # FILTER: PASS
+    buf[:, 40:43] = [0x11, gt_key, ploidy << 4 | BCF_INT8]
+    buf[:, 43:] = gt_values.view(np.uint8)
+    return buf.reshape(-1)

@@ -138,6 +138,44 @@ int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_ch
  * [7] inflate threads, [8] inflated bytes, [9] records of listed contigs. */
 int colate_last_bam_timing(colate_handle* h, double* out10);
 
+/* The row counts of genome `slot` straight from BCF files: replaces colate_set_row_counts for that slot (use with front_end = 1).
+ * What htslib and parse_vcfvcf's decoder half do for the bcf/bcf front-end (coal.cpp:997-1137) is done here: per --chr entry c
+ * the file bcf_paths[c] (the reference's <prefix>_chr<c>.bcf) is inflated on the host (BGZF, CRC32 and ISIZE checked) in windows
+ * of about chunk_bytes inflated bytes (0: 64 MiB) while the device decodes the previous one: every record is reduced to its
+ * position, the codes of its first two alleles, the sum of its GT allele indices and whether all of them are <= 1.  Those 12 bytes
+ * per record stay on the device for the file; then one thread per .mut row of the chromosome finds the first record at or after
+ * the row's position and applies the rules of `role`:
+ *   role 1 (reference, COLATE_BCF_REFERENCE): the record's two alleles are the row's, in either order (flipped: DAF = N - sum),
+ *     and it is biallelic; without a record there, DAF = N if ref_seqs shows the derived allele; DAF = 0 makes the row unusable;
+ *   role 0 (target, COLATE_BCF_TARGET): as the reference, or the record reports one allele (second allele empty or absent) that is
+ *     one of the row's and its allele sum is 0 (DAF = N when that allele is the derived one); without a record there, ref_seqs
+ *     gives DAF = N for the derived base and 0 for the ancestral base, any other base makes the row unusable.
+ * N = samples x GT length.  Only rows with meta bit 0 set and ancestral != derived are resolved (coal.cpp:966-995).  The cursors of
+ * the reference need no state here: rows and records ascend, so its record for a row is that lower bound, and the target cursor
+ * moving only for rows the reference kept changes nothing; k_pileup_join / k_ok then keep a row iff both slots are usable.
+ *   chr_names: the site set's --chr list (messages); ref_seqs / ref_lens: contig c of --ref_genome (host memory, read upper-cased
+ *   as fasta::Read leaves it), or ref_seqs = NULL for no --ref_genome; aaf_out / daf_out (optional, host): the counts per row.
+ * Refused, with the file and the (inflated) byte offset: COLATE_ERR_IO for a file that is not BGZF (plain gzip, uncompressed BCF,
+ * text VCF), a truncated block, a CRC or ISIZE mismatch, a wrong magic (BCF\2\1 or BCF\2\2), a header or record that runs past the
+ * data, a header without ##FORMAT=<ID=GT, records on more than one contig, a record whose sample count is not the header's, a
+ * file without records (all on the host, before the file's records are launched); a record without GT, with a missing ('.') or
+ * vector-end GT value, whose GT length differs from the file's first record's or whose typed fields run past it (on the device:
+ * the first such record of the file is reported).  COLATE_ERR_ORDER for a POS below the previous record's (equal ones are fine). */
+#define COLATE_BCF_TARGET 0
+#define COLATE_BCF_REFERENCE 1
+int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const char* const* chr_names, const char* const* bcf_paths,
+                         const uint8_t* const* ref_seqs, const int64_t* ref_lens, int64_t chunk_bytes, int32_t* aaf_out, int32_t* daf_out);
+/* Decode only: one BCF file's records reduced on the device as colate_rows_from_bcf does (same checks), kept on the device;
+ * colate_bcf_records copies records [r0, r0 + n) out in the arrays colate_maketmp_records takes (position 1-based, allele codes,
+ * allele sum, biallelic flag).  *n_hap = samples x GT length. */
+int colate_decode_bcf(colate_handle* h, const char* bcf_path, int64_t chunk_bytes, int64_t* n_records, int32_t* n_hap);
+int colate_bcf_records(colate_handle* h, int64_t r0, int64_t n, int32_t* rec_pos, uint8_t* rec_a0, uint8_t* rec_a1, int32_t* rec_alt_sum,
+                       uint8_t* rec_biallelic);
+/* Phases of the last colate_rows_from_bcf / colate_decode_bcf, summed over its files: [0] BGZF index s, [1] inflate s, [2] record
+ * walk s, [3] host-to-device copies ms, [4] k_bcf_decode ms, [5] k_bcf_rows ms ([3]-[5] only with colate_set_option(h, "bcf_timing",
+ * 1)), [6] whole call s, [7] inflate threads, [8] inflated bytes, [9] records. */
+int colate_last_bcf_timing(colate_handle* h, double* out10);
+
 /* P/N mask of genome `slot` evaluated at the site positions (fasta::Read,
  * include/src/data.cpp:213-237; test at coal.cpp:2169-2174): bit m of pass_bits = row m is
  * NOT rejected by the mask (positions at or beyond the mask end pass).  NULL clears it. */
@@ -320,6 +358,11 @@ int64_t colate_read_colate_in(const char* path, int n_chr, const char* const* ch
  * window (0: 64 MiB).  0 or a negative status. */
 int colate_bam_scan(const char* path, int n_chr, const char* const* chr_names, int64_t window_bytes, int64_t* n_records, int32_t* first_pos,
                     int32_t* last_pos, int32_t* ref_id);
+/* BCF file, host only (no GPU): the record count, the first and last POS (0-based), the records' contig (CHROM), the header's sample
+ * count and the dictionary index of GT, with every host check of colate_rows_from_bcf.  window_bytes: inflated bytes per window
+ * (0: 64 MiB).  0 or a negative status. */
+int colate_bcf_scan(const char* path, int64_t window_bytes, int64_t* n_records, int32_t* first_pos, int32_t* last_pos, int32_t* contig,
+                    int32_t* n_sample, int32_t* gt_key);
 /* fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz.  *seq_out: malloc'd,
  * release with colate_free.  Returns the length or < 0. */
 int64_t colate_read_fasta(const char* path, uint8_t** seq_out);
