@@ -65,6 +65,7 @@ SIGNATURES = {
     "colate_bcf_records": (C.c_int, [VP, C.c_int64, C.c_int64, VP, VP, VP, VP, VP]),
     "colate_last_bcf_timing": (C.c_int, [VP, f64]),
     "colate_bcf_scan": (C.c_int, [C.c_char_p, C.c_int64, VP, VP, VP, VP, VP, VP]),
+    "colate_vcf_scan": (C.c_int, [C.c_char_p, C.c_int64, VP, VP, VP, VP, C.c_char_p, C.c_int64]),
     "colate_read_fasta": (C.c_int64, [C.c_char_p, C.POINTER(C.POINTER(C.c_uint8))]),
     "colate_free": (None, [VP]),
     "colate_set_mask": (C.c_int, [VP, C.c_int, VP, C.c_int]),
@@ -121,6 +122,7 @@ TEST_HOOKS = {
     "colate_test_log1p_wide": (C.c_int, [C.c_int, f64, f64, i32]),
     "colate_test_em_prims": (C.c_int, [VP, C.c_int, C.c_int, f64, VP, f64, i32]),
     "colate_test_last_em": (C.c_int, [VP, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "colate_test_last_vcf_paths": (C.c_int, [VP, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "colate_test_bin_fast": (C.c_int, [VP, C.c_int, f64, i32, i32]),
     "colate_test_bin_sweep": (C.c_int, [VP, C.c_uint32, C.c_uint32, _p(dtype=np.uint64, flags="C_CONTIGUOUS")]),
     "colate_test_mt_stream": (C.c_int, [VP, u32, C.c_int64, C.c_int64, C.c_int, u32]),

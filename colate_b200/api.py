@@ -147,6 +147,18 @@ def bcf_scan(path: str, window_bytes: int = 0) -> dict:
     return {k: int(x[0]) for k, x in zip(keys, v)}
 
 
+def vcf_scan(path: str, window_bytes: int = 0) -> dict:
+    """Host-only walk of a bgzipped text VCF (no GPU): the record count, the first / last POS (0-based, as htslib's bcf1_t.pos), the
+    header's sample count and the records' CHROM (colate_vcf_scan).  Raises ColateError for the files colate_rows_from_bcf refuses
+    on the host, and for a BCF file (bcf_scan reads it)."""
+    v = [np.zeros(1, t) for t in (np.int64, np.int32, np.int32, np.int32)]
+    chrom = C.create_string_buffer(1 << 16)
+    check(lib().colate_vcf_scan(str(path).encode(), window_bytes, *[ptr(x) for x in v], chrom, len(chrom)))
+    out = {k: int(x[0]) for k, x in zip(("n_records", "first_pos", "last_pos", "n_sample"), v)}
+    out["chrom"] = chrom.value.decode(errors="surrogateescape")
+    return out
+
+
 def read_fasta(path: str) -> np.ndarray:
     """fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz."""
     p = C.POINTER(C.c_uint8)()
@@ -267,8 +279,8 @@ class Handle:
         return dict(zip(keys, t.tolist()))
 
     def rows_from_bcf(self, slot, paths, role, ref_genomes=None, chunk_bytes=0, fetch=False):
-        """The row counts of genome `slot` straight from BCF files (colate_rows_from_bcf): paths[c] = the file of chromosome c of the
-        site set (the reference's <prefix>_chr<c>.bcf), role "target" / "reference" (or 0 / 1), ref_genomes[c] = uint8 / bytes
+        """The row counts of genome `slot` straight from BCF or bgzipped text VCF files (colate_rows_from_bcf): paths[c] = the file
+        of chromosome c of the site set (the reference's <prefix>_chr<c>.bcf, either format, as htslib reads it), role "target" / "reference" (or 0 / 1), ref_genomes[c] = uint8 / bytes
         sequence of contig c of --ref_genome or None.  BGZF is inflated on the host, the records are decoded and resolved on the
         device.  Makes `slot` a row-count genome (use with front_end = 1); fetch=True returns (aaf, daf) per row."""
         role = {"target": 0, "reference": 1}.get(role, role)
@@ -288,7 +300,7 @@ class Handle:
         return (aaf, daf) if fetch else None
 
     def decode_bcf(self, path, chunk_bytes=0) -> dict:
-        """One BCF file's records as the device reduces them (colate_decode_bcf + colate_bcf_records): pos (1-based), a0 / a1 (first
+        """One BCF or bgzipped text VCF file's records as the device reduces them (colate_decode_bcf + colate_bcf_records): pos (1-based), a0 / a1 (first
         two alleles: 0 empty or absent, the letter, 0xff longer), alt_sum (sum of the GT allele indices), biallelic, and n_hap."""
         n = np.zeros(1, np.int64)
         nh = np.zeros(1, np.int32)
@@ -533,6 +545,13 @@ class Handle:
         y, ok = np.zeros_like(a), np.zeros(a.shape[0], dtype=np.int32)
         check(lib().colate_test_em_prims(self._h, self.EM_PRIMS.index(which), a.shape[0], a, ptr(bb), y, ok))
         return y, ok
+
+    def last_vcf_paths(self):
+        """Test hook: (lines on k_vcf_decode's fast path only, lines with a general-path step) of the last decode_bcf /
+        rows_from_bcf file; counted only with set_option("vcf_paths", 1), else (0, 0), as after a BCF file."""
+        f, g = C.c_int64(0), C.c_int64(0)
+        check(lib().colate_test_last_vcf_paths(self._h, C.byref(f), C.byref(g)))
+        return f.value, g.value
 
     def last_em(self):
         """Test hook: (kernel, CTAs per replicate) of the last EM launch; kernel is "task" (k_em), "split" (k_em_split),

@@ -552,6 +552,8 @@ int colate_set_option(colate_handle* h, const char* key, int64_t value)
   if (!strcmp(key, "bam_timing")) { h->opt_bam_timing = value != 0; return 0; }
   // bcf_timing = 1: colate_rows_from_bcf / colate_decode_bcf time their copies, decode and row kernels (colate_last_bcf_timing)
   if (!strcmp(key, "bcf_timing")) { h->opt_bcf_timing = value != 0; return 0; }
+  // vcf_paths = 1 (test hook): k_vcf_decode counts the lines it decodes on its fast and general paths (colate_test_last_vcf_paths)
+  if (!strcmp(key, "vcf_paths")) { h->opt_vcf_paths = value != 0; return 0; }
   // front_end: which of mut()'s input branches the handle reproduces (coal.cpp:3175-3319).  0 = tmp/tmp (parse_tmptmp: pseudo-
   // genotype weights, no normalisation).  1 = the bcf / bam front-ends fed from pre-decoded per-row counts (SURVEY.md 8f N3):
   // raw count weights (coal.cpp:2005-2039, 1164-1197) and both count vectors of stage ii divided by 1e3 (coal.cpp:3453-3463).

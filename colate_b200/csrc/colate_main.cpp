@@ -60,7 +60,8 @@ void help()
                "  Colate --mode mut --mut <prefix> --chr <file> --target_bcf <prefix> --reference_bcf <prefix> [--ref_genome <prefix>]\n"
                "         (--bins x,y,step | --coal <file>) [--target_mask <prefix>] [--reference_mask <prefix>] [--target_age <years>]\n"
                "         [--reference_age <years>] [--years_per_gen <float>] [--seed <int>] [--num_bootstraps <int>] [--device <int>]\n"
-               "         -o <output prefix>     (reads <prefix>_chr<c>.bcf per --chr entry; also writes <output prefix>.colate_mat; one device)\n"
+               "         -o <output prefix>     (reads <prefix>_chr<c>.bcf per --chr entry, BCF or bgzipped VCF as for htslib;\n"
+               "                                 also writes <output prefix>.colate_mat; one device)\n"
                "  Colate --mode make_tmp --mut <prefix> --chr <file> --target_bcf <prefix> --ref_genome <prefix> [--target_mask <prefix>]\n"
                "         [--device <int>] -o <output prefix>     (writes <output prefix>.colate.in)\n"
                "  Colate --mode make_tmp --mut <prefix> --target_bam <t.bam> --ref_genome <prefix> [--chr <file>] [--target_mask <prefix>]\n"

@@ -151,6 +151,8 @@ struct colate_handle {
   colate::DevBuf bcf_buf, bcf_cols, bcf_ref, bcf_state;
   int64_t bcf_n_rec = 0;       // records of the last decoded file in bcf_cols
   int32_t bcf_n_hap = 0;
+  int64_t vcf_paths[2] = {};   // lines of the last decoded text VCF on k_vcf_decode's fast path only / with a general step
+  bool opt_vcf_paths = false;  // (counted only with the vcf_paths test option: the count is an atomic per line)
   bool opt_bcf_timing = false;
   double bcf_timing[10] = {};
 };

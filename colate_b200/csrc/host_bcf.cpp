@@ -40,6 +40,7 @@ std::string field(const std::string& body, const std::string& key)
   }
   return "";
 }
+}  // namespace
 
 // Header text -> sample count and GT's dictionary index (-1: no ##FORMAT=<ID=GT line).  The dictionary holds the FILTER, INFO
 // and FORMAT IDs (one entry per ID, shared by the three kinds): PASS is 0, the others are numbered in order of first appearance
@@ -80,11 +81,15 @@ void header_text(const char* text, size_t n, int* n_sample, int* gt_key)
     if (is_format && id == "GT") *gt_key = (int)k;
   }
 }
-}  // namespace
 
 int BcfReader::open(const std::string& path, int threads)
 {
   if (int rc = open_bgzf(path, "BCF", threads)) return rc;
+  return read_header();
+}
+
+int BcfReader::read_header()
+{
   if (int rc = need_header_bytes(5, 0)) return rc;
   if (memcmp(carry_.data(), "BCF\2", 4) != 0 || (carry_[4] != 1 && carry_[4] != 2))
     return err("not a BCF file (magic BCF\\2\\1 or BCF\\2\\2 missing)", 0, false);

@@ -1,4 +1,5 @@
-// BGZF blocks on the host (SAM/BAM format specification 4.1), for the BAM (host_bam.cpp) and BCF (host_bcf.cpp) readers.
+// BGZF blocks on the host (SAM/BAM format specification 4.1), for the BAM (host_bam.cpp), BCF (host_bcf.cpp) and text VCF
+// (host_vcf.cpp) readers.
 #include "bgzf.h"
 
 #include <fcntl.h>
@@ -89,10 +90,11 @@ int BgzfFile::open_bgzf(const std::string& path, const char* format, int threads
 }
 
 // raw deflate of blocks [b0, b1) into dst (block b at dst + uoff(b) - uoff(b0)), n_threads threads; CRC32 and ISIZE checked
-int BgzfFile::inflate_blocks(size_t b0, size_t b1, uint8_t* dst)
+int BgzfFile::inflate_blocks(size_t b0, size_t b1, uint8_t* dst, bool scan_newlines)
 {
   if (b1 <= b0) return 0;
   const double t0 = now_s();
+  if (scan_newlines && block_nl_.size() < b1 - b0) block_nl_.resize(b1 - b0);
   std::atomic<size_t> next{b0};
   std::mutex mu;
   size_t bad = SIZE_MAX;
@@ -118,6 +120,10 @@ int BgzfFile::inflate_blocks(size_t b0, size_t b1, uint8_t* dst)
       if (what) {
         std::lock_guard<std::mutex> g(mu);
         if (b < bad) { bad = b; bad_what = what; }
+      } else if (scan_newlines) {
+        std::vector<uint32_t>& nl = block_nl_[b - b0];
+        nl.clear();
+        for (const uint8_t* q = out; (q = (const uint8_t*)memchr(q, '\n', out + k.isize - q)); q++) nl.push_back((uint32_t)(q - out));
       }
     }
     inflateEnd(&s);
@@ -134,13 +140,39 @@ int BgzfFile::inflate_blocks(size_t b0, size_t b1, uint8_t* dst)
 
 int BgzfFile::need_header_bytes(size_t n, size_t at)
 {
+  const uint8_t* p;
+  size_t got;
+  if (int rc = peek(n, &p, &got)) return rc;
+  return got >= n ? 0 : err(format_ + " header runs past the end of the data", at, false);
+}
+
+int BgzfFile::peek(size_t n, const uint8_t** p, size_t* got)
+{
   while (carry_.size() < n && next_block_ < blocks_.size()) {
     const size_t o = carry_.size();
     carry_.resize(o + blocks_[next_block_].isize);
     if (int rc = inflate_blocks(next_block_, next_block_ + 1, carry_.data() + o)) return rc;
     next_block_++;
   }
-  return carry_.size() >= n ? 0 : err(format_ + " header runs past the end of the data", at, false);
+  *p = carry_.data();
+  *got = std::min(n, carry_.size());
+  return 0;
+}
+
+void BgzfFile::adopt(BgzfFile& o)
+{
+  std::swap(path_, o.path_);
+  std::swap(format_, o.format_);
+  std::swap(carry_, o.carry_);
+  std::swap(carry_uoff_, o.carry_uoff_);
+  std::swap(fd_, o.fd_);
+  std::swap(map_, o.map_);
+  std::swap(size_, o.size_);
+  std::swap(blocks_, o.blocks_);
+  std::swap(next_block_, o.next_block_);
+  std::swap(index_s, o.index_s);
+  std::swap(inflate_s, o.inflate_s);
+  std::swap(n_threads, o.n_threads);
 }
 
 void BgzfFile::drop_header(size_t o)
@@ -164,7 +196,14 @@ int BgzfFile::fill_window(uint8_t* buf, size_t target, size_t* n_out, uint64_t* 
   size_t n = carry_.size();
   if (b1 < blocks_.size()) do n += blocks_[b1++].isize; while (b1 < blocks_.size() && n < target);
   if (!carry_.empty()) memcpy(buf, carry_.data(), carry_.size());
-  if (int rc = inflate_blocks(next_block_, b1, buf + carry_.size())) return rc;
+  if (int rc = inflate_blocks(next_block_, b1, buf + carry_.size(), record_newlines)) return rc;
+  if (record_newlines) {
+    newlines.clear();
+    for (size_t b = next_block_; b < b1; b++) {
+      const int64_t base = (int64_t)(carry_.size() + (blocks_[b].uoff - blocks_[next_block_].uoff));
+      for (uint32_t x : block_nl_[b - next_block_]) newlines.push_back(base + x);
+    }
+  }
   next_block_ = b1;
   *n_out = n;
   *ustart = carry_uoff_;

@@ -3,15 +3,16 @@
 // k_bcf_decode reduces every record to 12 bytes (position, the codes of its first two alleles, the GT allele sum, the biallelic
 // flag), which stay resident for the whole file while the raw bytes stream through; k_bcf_rows<role> gives every .mut row of
 // the chromosome its (AAF, DAF) straight in the slot's row-count columns.  Window n+1 is inflated on the host while window n
-// is on the device.
+// is on the device.  Bgzipped text VCF (host_vcf.cpp) takes the same path with k_vcf_decode in place of k_bcf_decode: the
+// format is detected from the file's first inflated bytes (open_genotypes), as htslib's bcf_open does.
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
 #include <cstring>
 #include <thread>
 
-#include "bcf_reader.h"
 #include "device.cuh"
+#include "vcf_reader.h"
 
 using namespace colate;
 
@@ -203,6 +204,218 @@ __global__ void k_bcf_decode(int64_t n, const uint8_t* __restrict__ raw, const i
   cols[k] = o;
 }
 
+// ---- text VCF ------------------------------------------------------------------------------------------------------------
+// k_vcf_decode reduces a VCF line to the BcfCol that k_bcf_decode makes from the BCF of the same record, with the semantics of
+// htslib's vcf_parse:
+//   pos = the text POS (the host checked it: a plain decimal);
+//   a0  = REF coded as k_bcf_decode codes allele 0 (0 empty, the letter, 0xff longer);
+//   a1  = the first ALT allele (up to ',' or the tab) coded so; an ALT of exactly "." is n_allele = 1, so a1 = 0;
+//   GT  = the subfield of each sample column at GT's index among FORMAT's ':'-separated keys (GT need not be first);
+//         its syntax is allele([/|]allele)*, an allele is decimal digits or '.';
+//   alt_sum = the sum of the allele indices mod 2^32, biallelic = every index <= 1.
+// Refused, as the BCF path refuses what htslib would hand it: '.' in a GT (bcf_gt_missing); samples of one line with different
+// ploidies (htslib pads the shorter ones with vector-end); a line whose n_hap = samples x ploidy is not the file's first line's;
+// no FORMAT column, no GT key in FORMAT, or a sample column that stops before GT's subfield (no GT value).  Refused as new cases:
+// fewer than 8 fixed fields, a sample-column count other than the header's, a GT off the syntax, an allele index over 2^29.
+// Kinds (the BCF numbers where the meaning is the same); when a line has several, the first in this order is reported:
+// fewer than 8 fields, no FORMAT or no GT key in it, the sample count, a sample without GT, syntax, missing, ploidy, n_hap.
+enum : unsigned { kVcfNoGT = 1, kVcfMissing = 2, kVcfHapCount = 3, kVcfFixed = 4, kVcfSyntax = 5, kVcfSamples = 6, kVcfPloidy = 7 };
+constexpr uint64_t kVcfMaxAllele = 1u << 29;
+
+// 4-bit mask of the bytes of w equal to c4's (c4: the byte repeated)
+__device__ __forceinline__ unsigned byte_bits(uint32_t w, uint32_t c4)
+{
+  const uint32_t m = (__vcmpeq4(w, c4) >> 7) & 0x01010101u;
+  return (m | m >> 7 | m >> 14 | m >> 21) & 15u;
+}
+// 16-bit mask of the tabs in the 16 bytes at c (16-aligned) that lie in [lo, hi)
+__device__ __forceinline__ unsigned tab_mask(const uint8_t* raw, int64_t c, int64_t lo, int64_t hi)
+{
+  if (c >= hi || c + 16 <= lo) return 0;
+  const uint4 x = *(const uint4*)(raw + c);
+  unsigned m = byte_bits(x.x, 0x09090909u) | byte_bits(x.y, 0x09090909u) << 4 | byte_bits(x.z, 0x09090909u) << 8 | byte_bits(x.w, 0x09090909u) << 12;
+  const int j0 = lo > c ? (int)(lo - c) : 0, j1 = hi - c < 16 ? (int)(hi - c) : 16;
+  return m & (((1u << j1) - 1u) & ~((1u << j0) - 1u));
+}
+__device__ __forceinline__ int warp_excl_sum(int x, int lane)
+{
+  int s = x;
+  for (int d = 1; d < 32; d <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, s, d);
+    if (lane >= d) s += y;
+  }
+  return s - x;
+}
+// 4 bytes at any address (the window buffer is padded past its end)
+__device__ __forceinline__ uint32_t ld4_any(const uint8_t* p)
+{
+  const uint32_t* q = (const uint32_t*)((uintptr_t)p & ~(uintptr_t)3);
+  return __funnelshift_r(q[0], q[1], ((uint32_t)(uintptr_t)p & 3u) * 8u);
+}
+// Fast path: a sample column at p whose GT is d|d or d/d followed by a tab, ':' or the line's end (GT first in FORMAT).  The
+// two digits go into sum / mx4 byte-wise.
+__device__ __forceinline__ bool gt_fast(const uint8_t* raw, int64_t p, int64_t e, uint32_t& sum, uint32_t& mx4)
+{
+  if (p + 3 > e) return false;
+  const uint32_t w = ld4_any(raw + p);
+  const uint32_t d = __vsub4(w, 0x30303030u) & 0x00ff00ffu;                          // the digits, as byte lanes 0 and 2
+  const bool digits = (__vcmpleu4(__vsub4(w, 0x30303030u), 0x09090909u) & 0x00ff00ffu) == 0x00ff00ffu;
+  const bool sep = ((__vcmpeq4(w, 0x7c7c7c7cu) | __vcmpeq4(w, 0x2f2f2f2fu)) & 0x0000ff00u) != 0;
+  const bool term = p + 3 == e || ((__vcmpeq4(w, 0x09090909u) | __vcmpeq4(w, 0x3a3a3a3au)) & 0xff000000u) != 0;
+  sum = __dp4a(d, 0x01010101u, sum);
+  mx4 = __vmaxu4(mx4, d);
+  return digits && sep && term;
+}
+// General path: one sample column at p (up to the next tab or e), GT at subfield gt_idx.  flags |= 1 << kind.
+__device__ __forceinline__ void gt_general(const uint8_t* raw, int64_t p, int64_t e, int gt_idx, uint32_t& sum, uint32_t& mx, int& pmin,
+                                           int& pmax, unsigned& flags)
+{
+  for (int i = 0; i < gt_idx; i++) {
+    while (p < e && raw[p] != ':' && raw[p] != '\t') p++;
+    if (p >= e || raw[p] == '\t') { flags |= 1u << kVcfNoGT; return; }
+    p++;
+  }
+  int ploidy = 0;
+  for (;;) {
+    uint32_t c = p < e ? raw[p] : '\t';
+    if (c == '.') {
+      flags |= 1u << kVcfMissing;
+      p++;
+    } else if (c - '0' <= 9u) {
+      uint64_t v = 0;
+      do {
+        v = v * 10 + (c - '0');
+        if (v > kVcfMaxAllele) { flags |= 1u << kVcfSyntax; return; }
+        p++;
+        c = p < e ? raw[p] : '\t';
+      } while (c - '0' <= 9u);
+      sum += (uint32_t)v;
+      mx = max(mx, (uint32_t)v);
+    } else {
+      flags |= 1u << kVcfSyntax;
+      return;
+    }
+    ploidy++;
+    c = p < e ? raw[p] : '\t';
+    if (c == '/' || c == '|') { p++; continue; }
+    if (c == ':' || c == '\t') break;
+    flags |= 1u << kVcfSyntax;
+    return;
+  }
+  pmin = min(pmin, ploidy);
+  pmax = max(pmax, ploidy);
+}
+
+// warp = line k0 + warp of the window: [rec_off[k], rec_off[k + 1] or text_end), its newline dropped.  Pass 1 finds the tabs
+// that end the first nine columns (INFO may be tens of KB: 512 bytes a step, a tab ballot and a warp prefix sum); lane 0 codes
+// REF / ALT and finds GT in FORMAT.  Pass 2 walks the sample columns 512 bytes a step: a step whose sample columns all start
+// with a single-digit diploid GT (and GT is FORMAT's first key) is summed byte-wise (gt_fast), any other step parses each
+// sample on the lane holding the tab before it (gt_general).  Both give the same bits.  paths (the vcf_paths test option,
+// else null): [0] / [1] count the lines decoded on the fast path only / with a general step.
+__global__ void __launch_bounds__(256) k_vcf_decode(int64_t k0, int64_t k1, int64_t n_win, const uint8_t* __restrict__ raw,
+                                                    const int64_t* __restrict__ rec_off, int64_t text_end, uint64_t ustart, int n_sample,
+                                                    BcfCol* __restrict__ cols, int32_t* __restrict__ nhap_state,
+                                                    unsigned long long* __restrict__ err, unsigned long long* __restrict__ paths)
+{
+  __shared__ int64_t tabs_s[8][10];
+  const int lane = threadIdx.x & 31;
+  const int64_t k = k0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  if (k >= k1) return;
+  int64_t* tp = tabs_s[threadIdx.x >> 5];
+  const int64_t b = rec_off[k];
+  int64_t e = k + 1 < n_win ? rec_off[k + 1] : text_end;
+  if (e > b && raw[e - 1] == '\n') e--;
+  // pass 1: tp[1..9] = the tabs that end columns 1..9
+  int ntab = 0;
+  for (int64_t c0 = b & ~(int64_t)15; c0 < e && ntab < 9; c0 += 512) {
+    const int64_t c = c0 + 16 * lane;
+    unsigned m = tab_mask(raw, c, b, e);
+    const int cnt = __popc(m);
+    int g = ntab + warp_excl_sum(cnt, lane);
+    for (; m && g < 9; m &= m - 1) tp[++g] = c + __ffs(m) - 1;
+    ntab += __reduce_add_sync(0xffffffffu, cnt);
+  }
+  __syncwarp();
+  ntab = min(ntab, 9);
+  unsigned flags = 0;
+  int gt_idx = -1;
+  uint32_t code0 = 0, code1 = 0;
+  int32_t pos = 0;
+  if (ntab < 7) flags |= 1u << kVcfFixed;
+  else if (lane == 0) {
+    for (int64_t q = tp[1] + 1; q < tp[2]; q++) pos = pos * 10 + (raw[q] - '0');
+    const int64_t r0 = tp[3] + 1, rl = tp[4] - r0, al0 = tp[4] + 1, al = tp[5] - al0;
+    code0 = rl == 0 ? 0u : rl == 1 ? raw[r0] : 0xffu;
+    if (al == 0 || raw[al0] == ',' || (al == 1 && raw[al0] == '.')) code1 = 0;
+    else code1 = al == 1 || raw[al0 + 1] == ',' ? raw[al0] : 0xffu;
+    if (ntab >= 8) {                                        // FORMAT: [tp[8] + 1, tp[9] or e)
+      const int64_t f1 = ntab >= 9 ? tp[9] : e;
+      int key = 0;
+      for (int64_t q = tp[8] + 1; q <= f1 && gt_idx < 0;) {
+        int64_t qe = q;
+        while (qe < f1 && raw[qe] != ':') qe++;
+        if (qe - q == 2 && raw[q] == 'G' && raw[q + 1] == 'T') gt_idx = key;
+        key++;
+        q = qe + 1;
+      }
+    }
+  }
+  gt_idx = __shfl_sync(0xffffffffu, gt_idx, 0);
+  // pass 2: the sample columns, each starting after a tab from tp[9] on
+  int n_col = 0;
+  uint32_t sum = 0, mx = 0;
+  int pmin = 1 << 30, pmax = 0;
+  bool all_fast = true;
+  if (ntab == 9 && gt_idx >= 0) {
+    const int64_t s0 = tp[9];
+    for (int64_t c0 = s0 & ~(int64_t)15; c0 < e; c0 += 512) {
+      const int64_t c = c0 + 16 * lane;
+      const unsigned m = tab_mask(raw, c, s0, e);
+      n_col += __reduce_add_sync(0xffffffffu, __popc(m));
+      uint32_t fsum = 0, fmx4 = 0;
+      bool fast = gt_idx == 0;
+      for (unsigned mm = m; mm && fast; mm &= mm - 1) fast = gt_fast(raw, c + __ffs(mm), e, fsum, fmx4);
+      if (__all_sync(0xffffffffu, fast)) {
+        sum += fsum;
+        mx = max(mx, max(fmx4 & 0xffu, fmx4 >> 16));
+        if (m) pmin = min(pmin, 2), pmax = max(pmax, 2);
+      } else {
+        all_fast = false;
+        for (unsigned mm = m; mm; mm &= mm - 1) gt_general(raw, c + __ffs(mm), e, gt_idx, sum, mx, pmin, pmax, flags);
+      }
+    }
+  }
+  sum = __reduce_add_sync(0xffffffffu, sum);
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  pmin = __reduce_min_sync(0xffffffffu, pmin);
+  pmax = __reduce_max_sync(0xffffffffu, pmax);
+  flags = __reduce_or_sync(0xffffffffu, flags);
+  if (lane != 0) return;
+  const int64_t n_hap = (int64_t)n_col * pmax;
+  unsigned kind = 0;
+  if (flags >> kVcfFixed & 1u) kind = kVcfFixed;
+  else if (ntab == 7 || gt_idx < 0) kind = kVcfNoGT;
+  else if (n_col != n_sample) kind = kVcfSamples;
+  else if (flags >> kVcfNoGT & 1u) kind = kVcfNoGT;
+  else if (flags >> kVcfSyntax & 1u) kind = kVcfSyntax;
+  else if (flags >> kVcfMissing & 1u) kind = kVcfMissing;
+  else if (pmin != pmax) kind = kVcfPloidy;
+  else {
+    const int32_t old = atomicCAS(nhap_state, -1, (int32_t)n_hap);
+    if (old != -1 && old != (int32_t)n_hap) kind = kVcfHapCount;
+  }
+  if (kind) atomicMin(err, (unsigned long long)(ustart + b) << 3 | kind);
+  if (paths) atomicAdd(paths + (all_fast ? 0 : 1), 1ull);
+  BcfCol o;
+  o.pos = pos;
+  o.alt_sum = (int32_t)sum;
+  o.a0 = (uint8_t)code0;
+  o.a1 = (uint8_t)code1;
+  o.biallelic = mx <= 1u;
+  o.pad = 0;
+  cols[k - k0] = o;
+}
+
 __device__ __forceinline__ bool letter(uint32_t x) { return x != 0u && x != 0xffu; }
 
 // thread = .mut row of the chromosome: the record at the row is the first one at or after its position (both cursors of
@@ -270,14 +483,17 @@ int ensure_cols(colate_handle* h, int64_t n, int64_t keep)
   return 0;
 }
 
-// one BCF file -> h->bcf_cols (h->bcf_n_rec records of h->bcf_n_hap haplotypes).  t[]: timing accumulators as colate_last_bcf_timing
+// one BCF or bgzipped text VCF file -> h->bcf_cols (h->bcf_n_rec records of h->bcf_n_hap haplotypes).  t[]: timing accumulators as colate_last_bcf_timing
 int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t)
 {
-  BcfReader rd;
-  if (int rc = rd.open(path, bcf_threads())) return rc;
+  std::unique_ptr<GenotypeReader> rdp;
+  if (int rc = open_genotypes(path, bcf_threads(), &rdp)) return rc;
+  GenotypeReader& rd = *rdp;
+  const int gt_key = rd.text ? -1 : static_cast<BcfReader&>(rd).gt_key;
   cudaStream_t s = h->stream;
-  CK(h->bcf_state.ensure(16));
+  CK(h->bcf_state.ensure(32));
   CK(cudaMemsetAsync(h->bcf_state.p, 0xff, 16, s));          // GT length -1, no error (~0)
+  CK(cudaMemsetAsync(h->bcf_state.as<char>() + 16, 0, 16, s));   // text VCF, vcf_paths option: lines on the fast / the general path
   const size_t target = chunk_bytes > 0 ? (size_t)chunk_bytes : (size_t)64 << 20;
   Pinned raw[2], offs[2];
   cudaEvent_t done[2];
@@ -307,7 +523,7 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     memcpy(offs[b].p, w.rec_off.data(), (size_t)n * 8);
     if (int rc = ensure_cols(h, n_rec + n, n_rec)) return rc;
     const size_t o_off = up(w.n_bytes), total = o_off + (size_t)n * 8;
-    CK(h->bcf_buf.ensure(total));   // (a reallocation waits for the device: cudaFree synchronises)
+    CK(h->bcf_buf.ensure(total + 16));   // (a reallocation waits for the device: cudaFree synchronises; k_vcf_decode reads past the end)
     char* d = h->bcf_buf.as<char>();
     if (tev[0]) CK(cudaEventRecord(tev[0], s));
     CK(cudaMemcpyAsync(d, raw[b].p, w.n_bytes, cudaMemcpyHostToDevice, s));
@@ -316,9 +532,15 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     // the file's first record alone first: its GT length is the one every later record must have
     for (int64_t k0 = 0; k0 < n;) {
       const int64_t k1 = n_rec == 0 && k0 == 0 ? 1 : n;
-      k_bcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k1 - k0, (const uint8_t*)d, (const int64_t*)(d + o_off) + k0, w.ustart, rd.gt_key,
-                                                                 h->bcf_cols.as<BcfCol>() + n_rec + k0, h->bcf_state.as<int32_t>(),
-                                                                 (unsigned long long*)(h->bcf_state.as<char>() + 8));
+      if (rd.text)
+        k_vcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k0, k1, n, (const uint8_t*)d, (const int64_t*)(d + o_off), w.text_end, w.ustart,
+                                                                   rd.n_sample, h->bcf_cols.as<BcfCol>() + n_rec + k0, h->bcf_state.as<int32_t>(),
+                                                                   (unsigned long long*)(h->bcf_state.as<char>() + 8),
+                                                                   h->opt_vcf_paths ? (unsigned long long*)(h->bcf_state.as<char>() + 16) : nullptr);
+      else
+        k_bcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k1 - k0, (const uint8_t*)d, (const int64_t*)(d + o_off) + k0, w.ustart, gt_key,
+                                                                   h->bcf_cols.as<BcfCol>() + n_rec + k0, h->bcf_state.as<int32_t>(),
+                                                                   (unsigned long long*)(h->bcf_state.as<char>() + 8));
       h->launches += 1;
       CK(cudaGetLastError());
       k0 = k1;
@@ -337,9 +559,11 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     pending[b] = true;
   }
   CK(cudaStreamSynchronize(s));
-  if (n_rec == 0) return rd.err("BCF file without records (the reference reads a first record unconditionally)", 0, false);
-  struct { int32_t nhap, pad; unsigned long long err; } st;
-  CK(cudaMemcpy(&st, h->bcf_state.p, 16, cudaMemcpyDeviceToHost));
+  if (n_rec == 0) return rd.err(std::string(rd.text ? "VCF" : "BCF") + " file without records (the reference reads a first record unconditionally)", 0, false);
+  struct { int32_t nhap, pad; unsigned long long err, paths[2]; } st;
+  CK(cudaMemcpy(&st, h->bcf_state.p, 32, cudaMemcpyDeviceToHost));
+  h->vcf_paths[0] = rd.text ? (int64_t)st.paths[0] : 0;
+  h->vcf_paths[1] = rd.text ? (int64_t)st.paths[1] : 0;
   t[0] += rd.index_s;
   t[1] += rd.inflate_s;
   t[2] += rd.walk_s;
@@ -350,7 +574,12 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     static const char* what[] = {"", "BCF record without a GT field", "BCF record with a missing or vector-end genotype (or an allele index below 0)",
                                  "BCF record whose GT length differs from the file's first record's", "BCF record whose typed fields run past its l_shared / l_indiv",
                                  "BCF record whose GT is not an integer vector"};
-    return rd.err(what[st.err & 7], st.err >> 3, false);
+    static const char* what_vcf[] = {"", "VCF line without a GT value (no FORMAT column, no GT key in FORMAT, or a sample column that stops before GT)",
+                                     "VCF line with a missing allele ('.') in a GT", "VCF line whose samples x ploidy differs from the file's first line's",
+                                     "VCF line with fewer than 8 fixed fields", "VCF line with a GT that is not allele([/|]allele)* (allele: digits up to 2^29)",
+                                     "VCF line whose sample-column count differs from the header's",
+                                     "VCF line whose samples have different ploidies"};
+    return rd.err((rd.text ? what_vcf : what)[st.err & 7], st.err >> 3, false);
   }
   h->bcf_n_rec = n_rec;
   h->bcf_n_hap = st.nhap;
@@ -460,6 +689,14 @@ int colate_bcf_records(colate_handle* h, int64_t r0, int64_t n, int32_t* rec_pos
     if (rec_alt_sum) rec_alt_sum[k] = c[k].alt_sum;
     if (rec_biallelic) rec_biallelic[k] = c[k].biallelic;
   }
+  return 0;
+}
+
+int colate_test_last_vcf_paths(colate_handle* h, int64_t* fast, int64_t* general)
+{
+  if (!h || !fast || !general) return fail(COLATE_ERR_ARG, "colate_test_last_vcf_paths: bad arguments");
+  *fast = h->vcf_paths[0];
+  *general = h->vcf_paths[1];
   return 0;
 }
 

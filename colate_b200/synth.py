@@ -579,3 +579,90 @@ def bcf_records_np(pos0, a0, a1, gt_values, gt_key, ploidy=2, chrom=0) -> np.nda
     buf[:, 40:43] = [0x11, gt_key, ploidy << 4 | BCF_INT8]
     buf[:, 43:] = gt_values.view(np.uint8)
     return buf.reshape(-1)
+
+
+# ---- bgzipped text VCF (VCF specification v4.3, section 1): what htslib's bcf_open reads in place of BCF ------------------------
+def vcf_header(n_sample, ids=(("FORMAT", "GT"),), contigs=("1",), extra=(), fileformat=b"##fileformat=VCFv4.3") -> bytes:
+    """The ## lines and the #CHROM line.  ids: (kind, ID) pairs as bcf_header; contigs: ##contig lines; extra: more ## lines."""
+    lines = [fileformat, b'##FILTER=<ID=PASS,Description="All filters passed">']
+    for kind, i in ids:
+        typ = b"String" if i == "GT" else b"Integer"
+        lines.append(b'##%s=<ID=%s,Number=1,Type=%s,Description="a \\"quoted\\" text">' % (kind.encode(), i.encode(), typ))
+    lines += [b"##contig=<ID=%s,length=1000000000>" % c.encode() for c in contigs]
+    lines += [bytes(x) for x in extra] or [b"##source=colate_b200.synth"]
+    cols = b"#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO"
+    if n_sample:
+        cols += b"\tFORMAT" + b"".join(b"\ts%d" % s for s in range(n_sample))
+    return b"\n".join(lines + [cols]) + b"\n"
+
+
+def vcf_gt_text(alleles, phased=False) -> bytes:
+    """One sample's GT: allele indices (-1 or None: '.') joined by '|' (phased) or '/'; phased may be a list per separator."""
+    out = b""
+    for j, a in enumerate(alleles):
+        if j:
+            ph = phased[j - 1] if isinstance(phased, (list, tuple)) else phased
+            out += b"|" if ph else b"/"
+        out += b"." if a is None or a < 0 else b"%d" % a
+    return out
+
+
+def vcf_line(chrom, pos0, alleles, gt, phased=False, rid=b".", qual=b".", filt=b"PASS", info=b".", fmt_before=(), fmt_after=(),
+             gt_text=None, keep=None, fmt=None, newline=True) -> bytes:
+    """One record line.  alleles: REF then the ALT alleles (ALT '.' when there are none); gt: allele indices [n_sample][ploidy]
+    (-1: '.'), or gt_text: the GT strings themselves; fmt_before / fmt_after: (key, [value per sample]) FORMAT fields around GT;
+    keep: per sample, the number of leading subfields written (trailing ones dropped); fmt: the FORMAT column itself (b"" drops
+    FORMAT and the samples)."""
+    keys = [k for k, _ in fmt_before] + ["GT"] + [k for k, _ in fmt_after]
+    fmt = b":".join(k.encode() for k in keys) if fmt is None else fmt
+    gts = gt_text if gt_text is not None else [vcf_gt_text(s, phased) for s in gt]
+    cols = [chrom.encode() if isinstance(chrom, str) else bytes(chrom), b"%d" % (pos0 + 1), bytes(rid), bytes(alleles[0]),
+            b",".join(bytes(a) for a in alleles[1:]) or b".", bytes(qual), bytes(filt), bytes(info)]
+    if fmt != b"":
+        cols.append(fmt)
+        for s, g in enumerate(gts):
+            sub = [bytes(v[s]) for _, v in fmt_before] + [bytes(g)] + [bytes(v[s]) for _, v in fmt_after]
+            cols.append(b":".join(sub[:keep[s]] if keep is not None else sub))
+    return b"\t".join(cols) + (b"\n" if newline else b"")
+
+
+def write_vcf(path, header, lines, block_size=65280, empty_blocks=(), eof=True, level=6, threads=1):
+    """A bgzipped VCF: `header` (vcf_header) and the lines (bytes or a uint8 array) in the order given, in BGZF blocks."""
+    data = bytes(header) + (lines.tobytes() if isinstance(lines, np.ndarray) else b"".join(lines))
+    with open(path, "wb") as f:
+        f.write(bgzf_compress(data, block_size, empty_blocks, eof, level, threads))
+
+
+def vcf_lines_np(pos0, a0, a1, alleles, phased=None, chrom=b"1") -> np.ndarray:
+    """Many diploid lines at once (benchmarks): pos0 [n], a0 / a1 [n] one-letter alleles (uint8), alleles [n][2 n_sample] single-digit
+    allele indices, phased [n][n_sample] (None: unphased); ID '.', QUAL '.', FILTER PASS, INFO '.', FORMAT GT.  The lines as one
+    uint8 array."""
+    alleles = np.asarray(alleles, np.uint8)
+    n, n_hap = alleles.shape
+    ns = n_hap // 2
+    if n == 0:
+        return np.zeros(0, np.uint8)
+    pos_txt = np.char.mod(b"%d", np.asarray(pos0, np.int64) + 1).astype(bytes)
+    W = pos_txt.dtype.itemsize
+    head = np.frombuffer(bytes(chrom) + b"\t", np.uint8)
+    rest = np.frombuffer(b"\t.\tPASS\t.\tGT", np.uint8)
+    # one row per line with POS left-aligned in W columns; the padding is dropped at the end
+    cols = head.size + W + 3 + 3 + rest.size + 4 * ns + 1
+    buf = np.empty((n, cols), np.uint8)
+    buf[:, :head.size] = head
+    buf[:, head.size:head.size + W] = pos_txt.view(np.uint8).reshape(n, W)
+    q = head.size + W
+    buf[:, q:q + 3] = np.frombuffer(b"\t.\t", np.uint8)
+    buf[:, q + 3] = a0
+    buf[:, q + 4] = 9
+    buf[:, q + 5] = a1
+    buf[:, q + 6:q + 6 + rest.size] = rest
+    smp = buf[:, q + 6 + rest.size:cols - 1].reshape(n, ns, 4)
+    smp[:, :, 0] = 9
+    smp[:, :, 1] = alleles[:, 0::2] + 48
+    smp[:, :, 2] = ord("/") if phased is None else np.where(np.asarray(phased, bool), ord("|"), ord("/"))
+    smp[:, :, 3] = alleles[:, 1::2] + 48
+    buf[:, -1] = 10
+    keep = np.ones((n, cols), bool)
+    keep[:, head.size:head.size + W] = buf[:, head.size:head.size + W] != 0
+    return buf[keep]

@@ -155,17 +155,24 @@ int colate_last_bam_timing(colate_handle* h, double* out10);
  * moving only for rows the reference kept changes nothing; k_pileup_join / k_ok then keep a row iff both slots are usable.
  *   chr_names: the site set's --chr list (messages); ref_seqs / ref_lens: contig c of --ref_genome (host memory, read upper-cased
  *   as fasta::Read leaves it), or ref_seqs = NULL for no --ref_genome; aaf_out / daf_out (optional, host): the counts per row.
- * Refused, with the file and the (inflated) byte offset: COLATE_ERR_IO for a file that is not BGZF (plain gzip, uncompressed BCF,
- * text VCF), a truncated block, a CRC or ISIZE mismatch, a wrong magic (BCF\2\1 or BCF\2\2), a header or record that runs past the
- * data, a header without ##FORMAT=<ID=GT, records on more than one contig, a record whose sample count is not the header's, a
- * file without records (all on the host, before the file's records are launched); a record without GT, with a missing ('.') or
- * vector-end GT value, whose GT length differs from the file's first record's or whose typed fields run past it (on the device:
- * the first such record of the file is reported).  COLATE_ERR_ORDER for a POS below the previous record's (equal ones are fine). */
+ * Each file is BCF or bgzipped text VCF, told apart by its first inflated bytes as htslib's bcf_open does (BCF\2\1 / BCF\2\2 or
+ * ##fileformat=VCF); a VCF line decodes to the record the BCF of the same record gives (k_vcf_decode, DESIGN.md section 6h).
+ * Refused, with the file and the (inflated) byte offset: COLATE_ERR_IO for a file that is not BGZF (plain gzip, uncompressed BCF
+ * or VCF), a truncated block, a CRC or ISIZE mismatch, a wrong magic (BCF\2\1 or BCF\2\2, or ##fileformat=VCF), a header or record
+ * that runs past the data, a header without ##FORMAT=<ID=GT, records on more than one contig, a record whose sample count is not
+ * the header's, a file without records (all on the host, before the file's records are launched); a record without GT, with a
+ * missing ('.') or vector-end GT value, whose GT length differs from the file's first record's or whose typed fields run past it
+ * (on the device: the first such record of the file is reported).  COLATE_ERR_ORDER for a POS below the previous record's (equal
+ * ones are fine).  Text VCF, on the host: a header without a #CHROM line, a #CHROM line whose first eight columns are not CHROM POS
+ * ID REF ALT QUAL FILTER INFO or that has no sample column, an empty line, a line ending in \r\n, a POS that is not a plain decimal
+ * in [0, 2^31 - 2]; on the device: fewer than 8 fixed fields, a sample-column count other than the header's, no FORMAT column or no
+ * GT key in FORMAT, a sample column that stops before its GT, a GT that is not allele([/|]allele)* with alleles of digits up to
+ * 2^29, a '.' allele, samples of one line with different ploidies, samples x ploidy other than the first line's. */
 #define COLATE_BCF_TARGET 0
 #define COLATE_BCF_REFERENCE 1
 int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const char* const* chr_names, const char* const* bcf_paths,
                          const uint8_t* const* ref_seqs, const int64_t* ref_lens, int64_t chunk_bytes, int32_t* aaf_out, int32_t* daf_out);
-/* Decode only: one BCF file's records reduced on the device as colate_rows_from_bcf does (same checks), kept on the device;
+/* Decode only: one BCF or bgzipped text VCF file's records reduced on the device as colate_rows_from_bcf does (same checks), kept on the device;
  * colate_bcf_records copies records [r0, r0 + n) out in the arrays colate_maketmp_records takes (position 1-based, allele codes,
  * allele sum, biallelic flag).  *n_hap = samples x GT length. */
 int colate_decode_bcf(colate_handle* h, const char* bcf_path, int64_t chunk_bytes, int64_t* n_records, int32_t* n_hap);
@@ -363,6 +370,11 @@ int colate_bam_scan(const char* path, int n_chr, const char* const* chr_names, i
  * (0: 64 MiB).  0 or a negative status. */
 int colate_bcf_scan(const char* path, int64_t window_bytes, int64_t* n_records, int32_t* first_pos, int32_t* last_pos, int32_t* contig,
                     int32_t* n_sample, int32_t* gt_key);
+/* Bgzipped text VCF file, host only (no GPU): the record count, the first and last POS (0-based, as htslib's bcf1_t.pos), the header's
+ * sample count and the records' CHROM (NUL-terminated, cut to chrom_cap - 1 bytes), with every host check of colate_rows_from_bcf
+ * on such a file.  A BCF file is refused (colate_bcf_scan reads it).  0 or a negative status. */
+int colate_vcf_scan(const char* path, int64_t window_bytes, int64_t* n_records, int32_t* first_pos, int32_t* last_pos, int32_t* n_sample,
+                    char* chrom, int64_t chrom_cap);
 /* fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz.  *seq_out: malloc'd,
  * release with colate_free.  Returns the length or < 0. */
 int64_t colate_read_fasta(const char* path, uint8_t** seq_out);
