@@ -57,7 +57,7 @@ SIGNATURES = {
     "colate_pileup_begin": (C.c_int, [VP, C.c_int]),
     "colate_pileup_reads": (C.c_int, [VP, C.c_int, C.c_int, C.c_int64, VP, VP, VP, VP, VP, VP, VP, C.c_int64, C.c_int, C.c_int, C.c_int]),
     "colate_pileup_end": (C.c_int, [VP, C.c_int, VP]),
-    "colate_pileup_bam": (C.c_int, [VP, C.c_int, C.c_char_p, C.c_int, C.POINTER(C.c_char_p), C.POINTER(VP), i64, C.c_int, C.c_int, C.c_int, C.c_int64, VP]),
+    "colate_pileup_bam": (C.c_int, [VP, C.c_int, C.c_char_p, C.c_int, C.POINTER(C.c_char_p), C.POINTER(VP), VP, C.c_int, C.c_int, C.c_int, C.c_int64, VP]),
     "colate_last_bam_timing": (C.c_int, [VP, f64]),
     "colate_bam_scan": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_char_p), C.c_int64, i64, i32, i32, i32]),
     "colate_rows_from_bcf": (C.c_int, [VP, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), VP, VP, C.c_int64, VP, VP]),
@@ -106,6 +106,16 @@ SIGNATURES = {
     "colate_maketmp_table": (C.c_int64, [C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.c_char_p, C.POINTER(C.c_char_p), C.c_int, C.c_char_p]),
     "colate_maketmp_records": (C.c_int64, [C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), VP, VP, VP, VP, VP, VP, VP, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.c_char_p]),
     "colate_maketmp_pileup": (C.c_int64, [C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), VP, C.c_int64, C.POINTER(C.c_char_p), C.c_char_p]),
+    "colate_set_ref_genome": (C.c_int, [VP, C.c_int, C.POINTER(VP), VP]),
+    "colate_maketmp_word": (C.c_uint32, [C.c_int, C.c_int, C.c_char_p]),
+    "colate_read_mut_words": (C.c_int64, [C.c_char_p, C.c_int64, VP]),
+    "colate_set_maketmp_words": (C.c_int, [VP, VP, C.c_int]),
+    "colate_fetch_maketmp_words": (C.c_int, [VP, C.c_int64, C.c_int64, VP]),
+    "colate_maketmp_mask_bits": (C.c_int, [C.c_char_p, C.c_int64, VP, C.c_int64, VP]),
+    "colate_maketmp_write_pileup": (C.c_int64, [VP, C.c_int, C.c_int, C.POINTER(C.c_char_p), VP, C.c_char_p]),
+    "colate_maketmp_write_bcf": (C.c_int64, [VP, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), VP, C.c_int64, C.c_char_p]),
+    "colate_last_maketmp_timing": (C.c_int, [VP, f64]),
+    "colate_upload_counts": (C.c_int, [VP, i64]),
     "colate_write_colate_mat": (C.c_int, [C.c_char_p, C.c_int, f64, f64]),
     "colate_write_coal": (C.c_int, [C.c_char_p, C.c_int, C.c_int, f64, f64, C.c_int, C.c_int]),
     "colate_write_bin": (C.c_int, [C.c_char_p, C.c_int, C.c_int, f64, f64, i32]),

@@ -169,6 +169,27 @@ def read_fasta(path: str) -> np.ndarray:
         lib().colate_free(C.cast(p, C.c_void_p))
 
 
+def maketmp_word(flipped: int, n_branch: int, mutation_type: bytes) -> int:
+    """The make_tmp row word of a .mut row (colate_maketmp_word): bit 0 vcf filter, bit 1 bam filter, bit 2 one-letter derived string,
+    byte 1 ancestral letter, byte 2 first derived letter."""
+    return int(lib().colate_maketmp_word(flipped, n_branch, mutation_type))
+
+
+def read_mut_words(path: str) -> np.ndarray:
+    """The make_tmp row words of a .mut[.gz] file on the host (colate_read_mut_words), row for row as read_mut."""
+    n = check(lib().colate_read_mut_words(str(path).encode(), 0, None))
+    w = np.zeros(n, np.uint32)
+    check(lib().colate_read_mut_words(str(path).encode(), n, ptr(w)))
+    return w
+
+
+def maketmp_mask_bits(path: str, pos: np.ndarray, row0: int, bits: np.ndarray):
+    """The make_tmp mask rule at the site positions -> pass bits of rows [row0, row0+len(pos)) (colate_maketmp_mask_bits): rows at or
+    beyond the mask's end are dropped, unlike mask_bits_from_fasta."""
+    pos = np.ascontiguousarray(pos, dtype=np.int32)
+    check(lib().colate_maketmp_mask_bits(str(path).encode(), pos.shape[0], ptr(pos), row0, ptr(bits)))
+
+
 @dataclass
 class Stage1Result:
     num_blocks: int
@@ -259,17 +280,66 @@ class Handle:
 
     def pileup_from_bam(self, slot, path, chr_names, ref_genomes, filters=(20, 30, 10), chunk_bytes=0, fetch=False):
         """The same pileup straight from a BAM file (colate_pileup_bam): chr_names = the site set's --chr list (header contig <name> or
-        chr<name>), ref_genomes[c] = uint8 / bytes sequence of contig c (upper-cased on the device as fasta::Read does).  BGZF is
+        chr<name>), ref_genomes[c] = uint8 / bytes sequence of contig c (upper-cased on the device as fasta::Read does), or None for
+        the genome of set_ref_genome.  BGZF is
         inflated on the host, the records are decoded and counted on the device in chunks of at most chunk_bytes record bytes (0:
         64 MiB).  Makes `slot` a pileup genome; fetch=True returns counts[n_site][4]."""
         n = len(chr_names)
         names = (C.c_char_p * n)(*[s.encode() for s in chr_names])
+        seqs = lens = None                       # ref_genomes None: the resident genome of set_ref_genome
+        if ref_genomes is not None:
+            refs = [np.ascontiguousarray(np.frombuffer(g, np.uint8) if isinstance(g, (bytes, bytearray)) else g, dtype=np.uint8) for g in ref_genomes]
+            seqs = (C.c_void_p * n)(*[r.ctypes.data if r.shape[0] else None for r in refs])
+            lens = np.array([r.shape[0] for r in refs], dtype=np.int64)
+        out = np.zeros((self.n_site, 4), dtype=np.int32) if fetch else None
+        check(lib().colate_pileup_bam(self._h, slot, str(path).encode(), n, names, seqs, ptr(lens), *filters, chunk_bytes, ptr(out) if fetch else None))
+        return out
+
+    # ---- make_tmp for many targets (DESIGN.md section 6i)
+    def set_ref_genome(self, ref_genomes):
+        """Upload --ref_genome once (colate_set_ref_genome): ref_genomes[c] = uint8 / bytes contig per --chr entry.  pileup_from_bam
+        with ref_genomes=None and maketmp_write_bcf read it on the device."""
+        n = len(ref_genomes)
         refs = [np.ascontiguousarray(np.frombuffer(g, np.uint8) if isinstance(g, (bytes, bytearray)) else g, dtype=np.uint8) for g in ref_genomes]
         seqs = (C.c_void_p * n)(*[r.ctypes.data if r.shape[0] else None for r in refs])
         lens = np.array([r.shape[0] for r in refs], dtype=np.int64)
-        out = np.zeros((self.n_site, 4), dtype=np.int32) if fetch else None
-        check(lib().colate_pileup_bam(self._h, slot, str(path).encode(), n, names, seqs, lens, *filters, chunk_bytes, ptr(out) if fetch else None))
-        return out
+        check(lib().colate_set_ref_genome(self._h, n, seqs, ptr(lens)))
+
+    def set_maketmp_words(self, words):
+        """make_tmp row words for sites given with set_sites (read_mut_words); ingest_mut* builds them itself."""
+        w = np.ascontiguousarray(words, dtype=np.uint32)
+        assert w.shape == (self.n_site,)
+        check(lib().colate_set_maketmp_words(self._h, ptr(w), 0))
+
+    def maketmp_words(self, row0=0, n_rows=None):
+        n = self.n_site - row0 if n_rows is None else n_rows
+        w = np.zeros(n, np.uint32)
+        check(lib().colate_fetch_maketmp_words(self._h, row0, n, ptr(w)))
+        return w
+
+    def maketmp_write_pileup(self, slot, chr_names, out_file, mask_bits=None) -> int:
+        """The .colate.in of pileup slot `slot` written on the device (colate_maketmp_write_pileup); returns the records written."""
+        names = (C.c_char_p * len(chr_names))(*[s.encode() for s in chr_names])
+        mb = None if mask_bits is None else np.ascontiguousarray(mask_bits, dtype=np.uint32)
+        return check(lib().colate_maketmp_write_pileup(self._h, slot, len(chr_names), names, ptr(mb), str(out_file).encode()))
+
+    def maketmp_write_bcf(self, paths, chr_names, out_file, mask_bits=None, chunk_bytes=0) -> int:
+        """The .colate.in of one BCF / VCF target (paths[c] per --chr entry) written on the device (colate_maketmp_write_bcf)."""
+        n = len(paths)
+        names = (C.c_char_p * n)(*[s.encode() for s in chr_names])
+        files = (C.c_char_p * n)(*[str(p).encode() for p in paths])
+        mb = None if mask_bits is None else np.ascontiguousarray(mask_bits, dtype=np.uint32)
+        return check(lib().colate_maketmp_write_bcf(self._h, n, names, files, ptr(mb), chunk_bytes, str(out_file).encode()))
+
+    def last_maketmp_timing(self) -> dict:
+        t = np.zeros(4)
+        check(lib().colate_last_maketmp_timing(self._h, t))
+        return dict(zip(("kernel_ms", "d2h_ms", "write_s", "records"), t.tolist()))
+
+    def upload_counts(self) -> dict:
+        c = np.zeros(4, np.int64)
+        check(lib().colate_upload_counts(self._h, c))
+        return dict(zip(("mut_texts_parsed", "mut_rows_parsed", "ref_uploads", "ref_h2d_bytes"), c.tolist()))
 
     def last_bam_timing(self) -> dict:
         """Phases of the last pileup_from_bam (colate_last_bam_timing; copy / decode / pileup need set_option("bam_timing", 1))."""

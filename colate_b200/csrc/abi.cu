@@ -152,7 +152,8 @@ void colate_destroy(colate_handle* h)
                     &h->u_blk, &h->blk_rank_start, &h->out_f, &h->out_n, &h->thrA, &h->lut, &h->d_scratch, &h->d_prof, &h->libm_tab, &h->ing_text, &h->ing_tile_cnt, &h->ing_tile_off, &h->ing_nl, &h->ing_status, &h->ing_fb,
                     &h->windows, &h->rng_stream, &h->mt_tail, &h->poly, &h->thr10, &h->d_counts, &h->d_blockstats, &h->d_weights, &h->d_epochs,
                     &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo, &h->bam_buf, &h->bam_ref, &h->bam_state,
-                    &h->bcf_buf, &h->bcf_cols, &h->bcf_ref, &h->bcf_state};
+                    &h->bcf_buf, &h->bcf_cols, &h->bcf_ref, &h->bcf_state, &h->mkt, &h->refg, &h->mk_ad, &h->mk_emit, &h->mk_blk, &h->mk_acc,
+                    &h->mk_name, &h->mk_out, &h->mk_mask};
   for (DevBuf* b : bufs) b->release();
   for (auto& g : h->genomes) {
     DevBuf* gb[] = {&g.bp, &g.aaf, &g.daf, &g.alleles, &g.chr_first, &g.chr_end, &g.mask_bits, &g.j_aaf, &g.j_daf, &g.j_prevbp, &g.j_flag, &g.pile};
@@ -195,6 +196,7 @@ int colate_set_sites(colate_handle* h, int n_chr, const int64_t* site_off, const
   if (n >= (int64_t(1) << 31)) return fail(COLATE_ERR_ARG, "more than 2^31 rows per handle");
   CK(h->site_off.ensure((n_chr + 1) * 8)); CK(h->pos.ensure(n * 4 + 4)); CK(h->ab.ensure(n * 4 + 4));
   CK(h->ae.ensure(n * 4 + 4)); CK(h->meta.ensure(n * 4 + 4));
+  h->mkt_valid = false;   // colate_set_maketmp_words gives these rows their make_tmp words
   h->h_site_off = off;   // (the async copy below reads the handle's copy, not the local)
   CK(cudaMemcpyAsync(h->site_off.p, h->h_site_off.data(), (n_chr + 1) * 8, cudaMemcpyHostToDevice, h->stream));
   int rc;
@@ -244,6 +246,7 @@ int colate_set_pileup(colate_handle* h, int slot, const int32_t* counts, int loc
   if ((rc = copy_in(g.pile.p, counts, (size_t)h->n_site * 16, location, h->stream))) return rc;
   g.n_rec = 0;
   g.pileup = true;
+  g.acgt = true;
   g.set = true;
   g.joined = false;
   h->flags_done = false;
@@ -272,6 +275,7 @@ int colate_set_row_counts(colate_handle* h, int slot, const int32_t* aaf, const 
   if (rc) return rc;
   g.n_rec = 0;
   g.pileup = true;
+  g.acgt = false;
   g.set = true;
   g.joined = false;
   h->flags_done = false;
@@ -346,6 +350,7 @@ int colate_pileup_end(colate_handle* h, int slot, int32_t* counts_out)
   if (counts_out) CK(cudaMemcpyAsync(counts_out, g.pile.p, (size_t)h->n_site * 16, cudaMemcpyDeviceToHost, h->stream));
   g.n_rec = 0;
   g.pileup = true;
+  g.acgt = true;
   g.set = true;
   g.joined = false;
   h->flags_done = false;

@@ -39,7 +39,7 @@ const char* kValueOpts[] = {"mode", "anc", "mut", "target_bcf", "reference_bcf",
                             "anc_genome", "mask", "mask_cutoff", "chr", "bins", "lineage_bin", "outgroup_tmrca", "years_per_gen",
                             "coal", "seed", "num_bootstraps", "filters", "groups", "poplabels", "map", "input", "output",
                             // additions of this build
-                            "num_bootstrap", "device", "devices", "pairs"};
+                            "num_bootstrap", "device", "devices", "pairs", "targets"};
 
 void help()
 {
@@ -67,6 +67,12 @@ void help()
                "  Colate --mode make_tmp --mut <prefix> --target_bam <t.bam> --ref_genome <prefix> [--chr <file>] [--target_mask <prefix>]\n"
                "         [--filters mapq,length,mismatches] [--device <int>] -o <output prefix>     (writes <output prefix>.colate.in)\n"
                "  Colate --mode make_tmp --mut <prefix> --target_table <file> --ref_genome <prefix> [--chr <file>] [--target_mask <prefix>] -o <output prefix>\n"
+               "  Colate --mode make_tmp --mut <prefix> --ref_genome <prefix> --targets <file> [--chr <file>] [--filters mapq,length,mismatches]\n"
+               "         [--device <int>]\n"
+               "    many targets in one job: every non-blank line of <file> not starting with '#' is one target\n"
+               "      (target_bam=<t.bam> | target_bcf=<prefix>) <output_prefix> [target_mask=<prefix>]\n"
+               "    with the shared flags; each line's <output_prefix>.colate.in equals that of the single-target run (target_bcf needs --chr;\n"
+               "    a failing line writes no file, the others complete, the exit status is 1)\n"
             << std::endl;
 }
 
@@ -1130,9 +1136,262 @@ int run_make_tmp_bcf(const Options& options)
   return 0;
 }
 
+// ---- --targets: make_tmp for many BAM / BCF / VCF targets in one job --------------------------------------------------------
+// Every line is the run `Colate --mode make_tmp --target_bam B | --target_bcf P [--target_mask M] -o OUT` with the shared flags, and
+// its OUT.colate.in is that run's, byte for byte.  The .mut text is parsed once (on the GPU), --ref_genome is read and uploaded
+// once, every distinct mask becomes per-row bits once; per target what remains is the BGZF inflation of its own file, its device
+// decode (and pileup), and the device writer (colate_maketmp_write_pileup / _bcf).
+struct TargetLine {
+  int line = 0;
+  bool bam = false;
+  std::string input, out, mask;
+  int mask_id = -1;
+  int64_t records = -1;
+  std::string err;
+};
+
+// The targets file, checked completely before any device is touched.  false: the message (naming the line) is on stderr.
+bool read_targets_file(const std::string& path, const std::vector<std::string>& name_chr, bool has_chr, std::vector<TargetLine>& tl)
+{
+  std::ifstream is(path);
+  if (is.fail()) { std::cerr << "Error: cannot open the targets file " << path << std::endl; return false; }
+  std::map<std::string, int> out_line;
+  std::string text;
+  int ln = 0;
+  auto bad = [&](const std::string& what) { std::cerr << "Error in targets file " << path << ", line " << ln << ": " << what << std::endl; return false; };
+  while (std::getline(is, text)) {
+    ln++;
+    std::stringstream ss(text);
+    std::vector<std::string> f;
+    std::string tok;
+    while (ss >> tok) f.push_back(tok);
+    if (f.empty() || f[0][0] == '#') continue;
+    if (f.size() < 2 || f.size() > 3)
+      return bad("expected (target_bam=<file> | target_bcf=<prefix>) <output_prefix> [target_mask=<prefix>], found " + std::to_string(f.size()) + " field(s)");
+    TargetLine t;
+    t.line = ln;
+    std::set<std::string> seen;
+    int n_out = 0;
+    for (auto& x : f) {
+      const size_t eq = x.find('=');
+      if (eq == std::string::npos) { t.out = x; n_out++; continue; }
+      if (eq == 0 || eq + 1 == x.size()) return bad("'" + x + "' is not of the form key=value");
+      const std::string key = x.substr(0, eq), val = x.substr(eq + 1);
+      if (!seen.insert(key).second) return bad("'" + key + "' is given twice");
+      if (key == "target_table") return bad("target_table= is not supported with --targets (the table variant of make_tmp runs on the host alone: use --target_table)");
+      if (key == "target_bam" || key == "target_bcf") {
+        if (!t.input.empty()) return bad("give exactly one of target_bam= and target_bcf=");
+        t.bam = key == "target_bam";
+        t.input = val;
+      } else if (key == "target_mask") t.mask = val;
+      else return bad("unknown key '" + key + "' (known: target_bam, target_bcf, target_mask)");
+    }
+    if (t.input.empty()) return bad("give exactly one of target_bam= and target_bcf=");
+    if (n_out != 1) return bad("expected one output prefix, found " + std::to_string(n_out));
+    auto dup = out_line.find(t.out);
+    if (dup != out_line.end()) return bad("output prefix " + t.out + " is already used on line " + std::to_string(dup->second));
+    out_line[t.out] = ln;
+    if (t.bam) {
+      FILE* fp = fopen(t.input.c_str(), "rb");
+      if (!fp) return bad("cannot read " + t.input);
+      fclose(fp);
+    } else {
+      if (!has_chr) return bad("target_bcf needs --chr (one <prefix>_chr<c>.bcf file per chromosome)");
+      for (auto& nm : name_chr) {
+        const std::string fbcf = t.input + "_chr" + nm + ".bcf";
+        FILE* fp = fopen(fbcf.c_str(), "rb");
+        if (!fp) return bad("cannot read " + fbcf);
+        fclose(fp);
+      }
+    }
+    tl.push_back(t);
+  }
+  if (tl.empty()) { std::cerr << "Error: the targets file " << path << " lists no target" << std::endl; return false; }
+  return true;
+}
+
+int run_make_tmp_batch(const Options& options)
+{
+  auto bad = [](const std::string& what) { std::cerr << "Error: " << what << std::endl; return 1; };
+  for (const char* k : {"target_bam", "target_bcf", "target_table", "target_mask", "output"})
+    if (options.count(k))
+      return bad(std::string("--") + (strcmp(k, "output") ? k : "output/-o") + " cannot be combined with --targets (give it per line of the targets file)");
+  if (options.count("strandfilter")) return bad("--strandfilter is not supported with BAM inputs (its read filter is not restated)");
+  if (!options.count("mut")) return bad("--targets needs --mut");
+  if (!options.count("ref_genome")) return bad("--targets needs --ref_genome");
+  int filters[3];
+  if (!parse_filters(options, filters)) return bad("--filters takes three integers: mapq,length,mismatches");
+  const std::string dev = options.count("devices") ? options.get("devices") : "";
+  if (dev.find(',') != std::string::npos) return bad("--targets runs on one device (--device <i>): inflating the targets on the host bounds the job");
+  const bool has_chr = options.count("chr");
+  std::vector<std::string> name_chr, f_mut;
+  if (has_chr) {
+    std::ifstream is(options.get("chr"));
+    if (is.fail()) return bad("cannot open " + options.get("chr"));
+    std::string line;
+    while (std::getline(is, line)) { name_chr.push_back(line); f_mut.push_back(options.get("mut") + "_chr" + line + ".mut"); }
+    if (name_chr.empty()) return bad("empty --chr list");
+  } else {
+    name_chr.push_back("");
+    f_mut.push_back(options.get("mut"));
+  }
+  const int n_chr = (int)name_chr.size();
+  {
+    std::set<std::string> uniq(name_chr.begin(), name_chr.end());
+    if ((int)uniq.size() != n_chr) return bad("duplicate chromosome names in --chr");
+  }
+  std::vector<TargetLine> tl;
+  if (!read_targets_file(options.get("targets"), name_chr, has_chr, tl)) return 1;
+  std::vector<std::string> masks;   // distinct target_mask prefixes
+  {
+    std::map<std::string, int> mid;
+    for (auto& t : tl) {
+      if (t.mask.empty()) continue;
+      auto it = mid.find(t.mask);
+      if (it == mid.end()) { it = mid.emplace(t.mask, (int)masks.size()).first; masks.push_back(t.mask); }
+      t.mask_id = it->second;
+    }
+  }
+  Phases ph;
+  std::cerr << "---------------------------------------------------------" << std::endl;
+  std::cerr << "Calculating Colate tmp input files for " << tl.size() << " targets.." << std::endl;
+
+  // the .mut text, read once: parsed on the GPU, or by the host reader (zlib) if a file only exists as .gz
+  std::vector<std::vector<char>> texts(n_chr);
+  bool all_plain = !options.count("host_parse");
+  for (int c = 0; c < n_chr && all_plain; c++) {
+    FILE* f = fopen(f_mut[c].c_str(), "rb");
+    if (!f) { all_plain = false; break; }
+    fseek(f, 0, SEEK_END);
+    const long sz = ftell(f);
+    fseek(f, 0, SEEK_SET);
+    texts[c].resize((size_t)std::max(sz, 0L));
+    if (sz > 0 && fread(texts[c].data(), 1, (size_t)sz, f) != (size_t)sz) all_plain = false;
+    fclose(f);
+  }
+  struct { std::vector<int64_t> off; std::vector<int32_t> pos; std::vector<float> ab, ae; std::vector<uint32_t> meta, words; } sh;
+  if (!all_plain) {
+    texts.clear();
+    sh.off.assign(n_chr + 1, 0);
+    for (int c = 0; c < n_chr; c++) {
+      const int64_t n = colate_read_mut(f_mut[c].c_str(), 0, nullptr, nullptr, nullptr, nullptr);
+      if (n < 0) { std::cerr << colate_last_error() << std::endl; return 1; }
+      const size_t o = sh.pos.size();
+      sh.pos.resize(o + n); sh.ab.resize(o + n); sh.ae.resize(o + n); sh.meta.resize(o + n); sh.words.resize(o + n);
+      if (colate_read_mut(f_mut[c].c_str(), n, sh.pos.data() + o, sh.ab.data() + o, sh.ae.data() + o, sh.meta.data() + o) < 0 ||
+          colate_read_mut_words(f_mut[c].c_str(), n, sh.words.data() + o) < 0) {
+        std::cerr << colate_last_error() << std::endl;
+        return 1;
+      }
+      sh.off[c + 1] = (int64_t)sh.pos.size();
+    }
+  }
+  ph.tick("read .mut");
+  RefGenome refg;
+  if (!refg.read(options, name_chr)) return 1;
+  ph.tick("read --ref_genome");
+
+  colate_handle* h = nullptr;
+  if (colate_create(options.count("device") ? atoi(options.get("device").c_str()) : 0, &h)) return die("colate_create");
+  struct Destroy { colate_handle* h; ~Destroy() { colate_destroy(h); } } destroy{h};
+  std::vector<int64_t> site_off(n_chr + 1, 0);
+  std::vector<int32_t> pos;
+  if (all_plain) {
+    int64_t bytes = 0;
+    for (auto& t : texts) bytes += (int64_t)t.size();
+    if (colate_ingest_begin(h, n_chr, bytes / 20 + n_chr)) return die("colate_ingest_begin");
+    for (int c = 0; c < n_chr; c++) {
+      const int64_t n = colate_ingest_mut_text(h, texts[c].data(), (int64_t)texts[c].size(), 0);
+      if (n < 0) return die(f_mut[c]);
+      site_off[c + 1] = site_off[c] + n;
+    }
+    if (colate_ingest_end(h)) return die("colate_ingest_end");
+    texts.clear();
+    pos.resize((size_t)site_off[n_chr]);
+    if (colate_ingest_fetch(h, 0, site_off[n_chr], pos.data(), nullptr, nullptr, nullptr)) return die("colate_ingest_fetch");
+  } else {
+    site_off = sh.off;
+    if (colate_set_sites(h, n_chr, sh.off.data(), sh.pos.data(), sh.ab.data(), sh.ae.data(), sh.meta.data(), 0)) return die("colate_set_sites");
+    if (colate_set_maketmp_words(h, sh.words.data(), 0)) return die("colate_set_maketmp_words");
+    pos = sh.pos;
+  }
+  // the device writer walks the rows as the reference's forward-only record cursor does: positions must ascend per chromosome
+  for (int c = 0; c < n_chr; c++)
+    for (int64_t m = site_off[c] + 1; m < site_off[c + 1]; m++)
+      if (pos[m] < pos[m - 1]) {
+        std::cerr << "Error: " << f_mut[c] << ": positions of a .mut file are not ascending (the reference's sequential reader needs sorted input)" << std::endl;
+        return 1;
+      }
+  ph.tick("parse .mut");
+  if (colate_set_ref_genome(h, n_chr, (const uint8_t* const*)refg.seq.data(), refg.len.data())) return die("colate_set_ref_genome");
+  ph.tick("upload --ref_genome");
+  // every distinct mask once: make_tmp pass bits per row
+  std::vector<std::vector<uint32_t>> mask_bits(masks.size());
+  std::vector<std::string> mask_err(masks.size());
+  for (size_t k = 0; k < masks.size(); k++) {
+    mask_bits[k].assign((size_t)site_off[n_chr] / 32 + 2, 0);
+    for (int c = 0; c < n_chr && mask_err[k].empty(); c++) {
+      const std::string f = has_chr ? masks[k] + "_chr" + name_chr[c] + ".fa" : masks[k];
+      if (colate_maketmp_mask_bits(f.c_str(), site_off[c + 1] - site_off[c], pos.data() + site_off[c], site_off[c], mask_bits[k].data()))
+        mask_err[k] = colate_last_error();
+    }
+  }
+  ph.tick("masks");
+  std::vector<const char*> names;
+  for (auto& s : name_chr) names.push_back(s.c_str());
+  for (auto& t : tl) {
+    const std::string out = t.out + ".colate.in";
+    const uint32_t* mb = t.mask_id >= 0 ? mask_bits[t.mask_id].data() : nullptr;
+    if (t.mask_id >= 0 && !mask_err[t.mask_id].empty()) t.err = mask_err[t.mask_id];
+    else if (t.bam) {
+      if (colate_pileup_bam(h, 0, t.input.c_str(), n_chr, names.data(), nullptr, nullptr, filters[0], filters[1], filters[2], 0, nullptr))
+        t.err = t.input + ": " + colate_last_error();
+      else if ((t.records = colate_maketmp_write_pileup(h, 0, n_chr, names.data(), mb, out.c_str())) < 0)
+        t.err = colate_last_error();
+      if (ph.on && t.err.empty()) {
+        double b[10], w[4];
+        colate_last_bam_timing(h, b);
+        colate_last_maketmp_timing(h, w);
+        fprintf(stderr, "[timing] line %d bam: inflate %.3f s, walk %.3f s, pileup_bam %.3f s; writer kernels %.3f ms, d2h %.3f ms, write %.3f s\n",
+                t.line, b[1], b[2], b[6], w[0], w[1], w[2]);
+      }
+    } else {
+      std::vector<std::string> files;
+      for (auto& nm : name_chr) files.push_back(t.input + "_chr" + nm + ".bcf");
+      std::vector<const char*> fp;
+      for (auto& f : files) fp.push_back(f.c_str());
+      if ((t.records = colate_maketmp_write_bcf(h, n_chr, names.data(), fp.data(), mb, 0, out.c_str())) < 0) t.err = t.input + ": " + colate_last_error();
+      if (ph.on && t.err.empty()) {
+        double b[10], w[4];
+        colate_last_bcf_timing(h, b);
+        colate_last_maketmp_timing(h, w);
+        fprintf(stderr, "[timing] line %d bcf: inflate %.3f s, walk %.3f s, decode+write %.3f s; writer kernels %.3f ms, d2h %.3f ms, write %.3f s\n",
+                t.line, b[1], b[2], b[6], w[0], w[1], w[2]);
+      }
+    }
+    if (!t.err.empty()) remove(out.c_str());   // a failed line leaves no file, not even an older one
+    ph.tick(("target on line " + std::to_string(t.line)).c_str());
+  }
+  if (ph.on) {
+    int64_t cnt[4];
+    colate_upload_counts(h, cnt);
+    fprintf(stderr, "[timing] .mut texts parsed %lld (%lld rows), reference genome uploads %lld (%lld bytes)\n", (long long)cnt[0], (long long)cnt[1],
+            (long long)cnt[2], (long long)cnt[3]);
+  }
+  int n_failed = 0;
+  for (auto& t : tl) {
+    if (t.err.empty()) std::cerr << "target on line " << t.line << " (" << t.out << "): " << t.records << " records written" << std::endl;
+    else { n_failed++; std::cerr << "target on line " << t.line << " (" << t.out << ") FAILED: " << t.err << std::endl; }
+  }
+  if (n_failed) std::cerr << n_failed << " of " << tl.size() << " targets failed" << std::endl;
+  std::cerr << "---------------------------------------------------------" << std::endl << std::endl;
+  return n_failed ? 1 : 0;
+}
+
 // --mode make_tmp with --target_table (make_tmp(), coal.cpp:2923-3069 -> maketmp_table, 2682-2808): host-only
 int run_make_tmp(const Options& options)
 {
+  if (options.count("targets")) return run_make_tmp_batch(options);
   if (!options.count("mut") || !options.count("output")) {
     std::cout << "Not enough arguments supplied." << std::endl;
     std::cout << "Needed: mut, ref_genome, output, either of target_bcf or target_bam. Optional: filters, target_mask, strandfilter, anc_genome." << std::endl;

@@ -54,10 +54,20 @@ struct Pinned {
   ~Pinned() { if (p) cudaFreeHost(p); }
 };
 
+// decoded BCF / VCF record (kernels_bcf.cu).  a0 / a1: first two alleles as colate_maketmp_records codes them (0 empty or absent,
+// the letter, 0xff longer)
+struct BcfCol {
+  int32_t pos;        // 1-based
+  int32_t alt_sum;    // sum of bcf_gt_allele over the n_hap haplotypes
+  uint8_t a0, a1, biallelic, pad;
+};
+static_assert(sizeof(BcfCol) == 12, "BcfCol is 12 bytes");
+
 // one .colate.in file on the device, plus its join onto the site axis
 struct GenomeDev {
   bool set = false, joined = false, has_mask = false;
   bool pileup = false;        // slot filled by colate_set_pileup: `pile` = int32[n_site][4] reads showing A, C, G, T per row
+  bool acgt = false;          // `pile` holds read counts per letter (set_pileup, pileup_*), not the (AAF, DAF) of set_row_counts / rows_from_bcf
   DevBuf pile;
   int64_t n_rec = 0;
   DevBuf bp, aaf, daf, alleles, chr_first, chr_end, mask_bits;
@@ -88,6 +98,8 @@ struct colate_handle {
   int64_t n_site = 0;
   std::vector<int64_t> h_site_off;
   colate::DevBuf site_off, pos, ab, ae, meta, tile_start, tile_rlo;   // tile_*: k_join's tiles of 256 sites
+  colate::DevBuf mkt;           // make_tmp row word per site (maketmp_word.h): colate_ingest_* or colate_set_maketmp_words
+  bool mkt_valid = false;
   std::vector<int32_t> h_tile_start;
   bool tiles_valid = false;
   colate::GenomeDev genomes[COLATE_MAX_GENOMES];
@@ -155,9 +167,20 @@ struct colate_handle {
   bool opt_vcf_paths = false;  // (counted only with the vcf_paths test option: the count is an atomic per line)
   bool opt_bcf_timing = false;
   double bcf_timing[10] = {};
+  // the --ref_genome resident for a job (colate_set_ref_genome): contigs concatenated, upper-cased
+  colate::DevBuf refg;
+  std::vector<int64_t> refg_off;   // n + 1 offsets; empty: none
+  // the device .colate.in writer (kernels_maketmp.cu): per-row (AAF, DAF), emit ballots, per-block counts / offsets, the records
+  colate::DevBuf mk_ad, mk_emit, mk_blk, mk_acc, mk_name, mk_out, mk_mask;
+  colate::Pinned mk_host;
+  double mk_timing[4] = {};
+  // work counters of a job (colate_upload_counts)
+  int64_t mut_texts_parsed = 0, mut_rows_parsed = 0, ref_uploads = 0, ref_h2d_bytes = 0;
 };
 
 namespace colate {
+// kernels_bcf.cu: one BCF or bgzipped text VCF file -> h->bcf_cols (h->bcf_n_rec records of h->bcf_n_hap haplotypes)
+int decode_genotype_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t);
 // kernels_sites.cu
 int run_join(colate_handle* h, int slot);
 int run_flags(colate_handle* h, int tslot, int rslot);

@@ -2,6 +2,7 @@
 // exact bin thresholds, the per-row filter, the chromosome seek emulation, ages / epoch
 // grid, and the readers / writers of the reference's file formats (SURVEY.md App. B).
 #include "internal.h"
+#include "maketmp_word.h"
 #include "exact_sum.cuh"
 
 #include <zlib.h>
@@ -514,6 +515,46 @@ int64_t colate_read_mut(const char* path, int64_t cap, int32_t* pos, float* age_
   return n;
 }
 
+uint32_t colate_maketmp_word(int flipped, int n_branch, const char* mutation_type)
+{
+  char t[16] = {};
+  if (mutation_type) strncpy(t, mutation_type, 15);
+  return colate::maketmp_word(flipped, n_branch, t);
+}
+
+// the make_tmp row words of a .mut[.gz] file: the rows of colate_read_mut, the type as parse_mut_line_fields leaves it
+int64_t colate_read_mut_words(const char* path, int64_t cap, uint32_t* words)
+{
+  std::vector<char> buf;
+  if (!slurp_or_gz(path, buf)) return fail(COLATE_ERR_IO, std::string("Error while reading ") + path + "(.gz).");
+  buf.push_back('\n');
+  buf.push_back('\0');
+  const char* p = buf.data();
+  const char* endp = buf.data() + buf.size() - 1;
+  const char* nl = (const char*)memchr(p, '\n', endp - p);
+  if (!nl) return 0;
+  p = nl + 1;
+  int64_t n = 0;
+  while (p < endp) {
+    nl = (const char*)memchr(p, '\n', endp - p);
+    if (!nl) break;
+    if (nl == p) {
+      if (nl + 1 >= endp) break;
+      return fail(COLATE_ERR_IO, std::string("empty line in ") + path);
+    }
+    if (words) {
+      if (n >= cap) return fail(COLATE_ERR_ARG, "colate_read_mut_words: capacity too small");
+      int32_t ps; float ab, ae; uint32_t meta; int fl, nb; char type[16];
+      if (!parse_mut_line_fields(p, nl, &ps, &ab, &ae, &meta, &fl, &nb, type))
+        return fail(COLATE_ERR_IO, std::string("Error reading following line in mut file: ") + std::string(p, nl));
+      words[n] = colate::maketmp_word(fl, nb, type);
+    }
+    n++;
+    p = nl + 1;
+  }
+  return n;
+}
+
 int64_t colate_read_colate_in(const char* path, int n_chr, const char* const* chr_names, int64_t cap,
                               int32_t* rec_chrom, int32_t* bp, int32_t* aaf, int32_t* daf, uint16_t* alleles)
 {
@@ -667,6 +708,24 @@ extern "C" int64_t colate_read_fasta(const char* path, uint8_t** seq_out)
 }
 
 extern "C" void colate_free(void* p) { free(p); }
+
+// the make_tmp mask rule (maketmp_bam coal.cpp:2589-2595, maketmp_vcf 2381-2395; colate_maketmp_pileup / _records): a row at or
+// beyond the mask's end is DROPPED, bp = 0 is kept, bp >= 1 needs mask[bp - 1] == 'P'
+extern "C" int colate_maketmp_mask_bits(const char* path, int64_t n, const int32_t* pos, int64_t row0, uint32_t* pass_bits)
+{
+  using colate::fail;
+  if (!path || n < 0 || row0 < 0 || (n > 0 && (!pos || !pass_bits))) return fail(COLATE_ERR_ARG, "colate_maketmp_mask_bits: bad arguments");
+  std::vector<char> mask;
+  if (!read_fasta_seq(path, mask)) return fail(COLATE_ERR_IO, std::string("Error while opening file ") + path + ".");
+  for (int64_t k = 0; k < n; k++) {
+    const int32_t b = pos[k];
+    const bool pass = (uint64_t)(int64_t)b < (uint64_t)mask.size() && (b < 1 || mask[b - 1] == 'P');
+    const int64_t m = row0 + k;
+    if (pass) pass_bits[m >> 5] |= (1u << (m & 31));
+    else pass_bits[m >> 5] &= ~(1u << (m & 31));
+  }
+  return 0;
+}
 
 // maketmp_table (coal.cpp:2682-2808): a .colate.in record stream for a haploid target given as a whitespace-separated
 // table of (chromosome, position, allele) triples in --chr order.  For every row of the .mut files that is not

@@ -75,11 +75,15 @@ extern "C" {
 int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_chr, const char* const* chr_names, const uint8_t* const* ref_seqs,
                       const int64_t* ref_lens, int mapq_th, int len_th, int mismatch_th, int64_t chunk_bytes, int32_t* counts_out)
 {
-  if (!h || slot < 0 || slot >= COLATE_MAX_GENOMES || !bam_path || n_chr <= 0 || !chr_names || !ref_seqs || !ref_lens || chunk_bytes < 0)
+  if (!h || slot < 0 || slot >= COLATE_MAX_GENOMES || !bam_path || n_chr <= 0 || !chr_names || (ref_seqs && !ref_lens) || chunk_bytes < 0)
     return fail(COLATE_ERR_ARG, "colate_pileup_bam: bad arguments");
   if (!h->sites_set || n_chr != h->n_chr) return fail(COLATE_ERR_ARG, "colate_pileup_bam: the --chr list must be the site set's chromosomes");
-  for (int c = 0; c < n_chr; c++)
+  const bool resident = ref_seqs == nullptr;   // the genome of colate_set_ref_genome, already on the device
+  if (resident && (int)h->refg_off.size() != n_chr + 1)
+    return fail(COLATE_ERR_STATE, "colate_pileup_bam: ref_seqs = NULL needs colate_set_ref_genome with one contig per chromosome");
+  for (int c = 0; c < n_chr && !resident; c++)
     if (ref_lens[c] < 0 || (ref_lens[c] > 0 && !ref_seqs[c])) return fail(COLATE_ERR_ARG, "colate_pileup_bam: bad reference sequence");
+  auto ref_len_of = [&](int c) { return resident ? h->refg_off[c + 1] - h->refg_off[c] : ref_lens[c]; };
   const auto t_start = std::chrono::steady_clock::now();
   BamReader rd;
   if (int rc = rd.open(bam_path, n_chr, chr_names, bam_threads())) return rc;
@@ -148,17 +152,19 @@ int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_ch
       int64_t r1 = r0 + 1;
       while (r1 < n && w.rec_chr[r1] == c && (size_t)((r1 + 1 < n ? w.rec_off[r1 + 1] : (int64_t)w.n_bytes) - w.rec_off[r0]) <= target) r1++;
       const bool starts = c != cur;
-      if (starts) {
+      if (starts && !resident) {
         // this contig's reference genome, upper-cased on the device
         const int64_t L = ref_lens[c];
         CK(h->bam_ref.ensure((size_t)L + 16));
         if (L) {
           CK(cudaMemcpyAsync(h->bam_ref.p, ref_seqs[c], (size_t)L, cudaMemcpyHostToDevice, s));
+          h->ref_h2d_bytes += L;
           k_upper<<<grid_for(L, 256), 256, 0, s>>>(L, h->bam_ref.as<uint8_t>());
           h->launches += 1;
         }
-        cur = c;
       }
+      cur = c;
+      const uint8_t* d_ref = resident ? h->refg.as<uint8_t>() + h->refg_off[c] : h->bam_ref.as<uint8_t>();
       int32_t* st = h->bam_state.as<int32_t>();
       if (tev[0]) CK(cudaEventRecord(tev[2], s));
       k_bam_decode<<<grid_for(r1 - r0, 256), 256, 0, s>>>(r1 - r0, (const uint8_t*)(d + o_raw), d_rec + r0, d_seqo + r0, d_pos + r0, d_mq + r0,
@@ -181,7 +187,7 @@ int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_ch
         if (w.rec_pos[r1 - 1] < w.rec_pos[r0]) { row_lo = 0; row_hi = -1; }   // refused below; the counts are not used
       }
       if (int rc = run_pileup_reads(h, slot, c, r1 - r0, d_pos + r0, d_mq + r0, d_len + r0, d_seqo + r0, (const uint8_t*)(d + o_seq),
-                                    (const uint8_t*)(d + o_q), h->bam_ref.as<uint8_t>(), ref_lens[c], max_len, mapq_th, len_th, mismatch_th,
+                                    (const uint8_t*)(d + o_q), d_ref, ref_len_of(c), max_len, mapq_th, len_th, mismatch_th,
                                     (uint8_t*)(d + o_pass) + r0, starts, row_lo, row_hi)) {
         cudaStreamSynchronize(s);
         return rc;
@@ -216,6 +222,34 @@ int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_ch
   h->bam_timing[9] = (double)n_records;
   if (flag) return fail(COLATE_ERR_ORDER, "Error: BAM file not sorted by position.");   // htslib.cpp:411-414
   return colate_pileup_end(h, slot, counts_out);
+}
+
+int colate_set_ref_genome(colate_handle* h, int n_chr, const uint8_t* const* ref_seqs, const int64_t* ref_lens)
+{
+  if (!h || n_chr < 0 || (n_chr > 0 && (!ref_seqs || !ref_lens))) return fail(COLATE_ERR_ARG, "colate_set_ref_genome: bad arguments");
+  std::vector<int64_t> off(1, 0);
+  for (int c = 0; c < n_chr; c++) {
+    if (ref_lens[c] < 0 || (ref_lens[c] > 0 && !ref_seqs[c])) return fail(COLATE_ERR_ARG, "colate_set_ref_genome: bad reference sequence");
+    off.push_back(off.back() + ref_lens[c]);
+  }
+  CK(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  CK(cudaStreamSynchronize(s));   // nothing may still read the genome this call replaces
+  h->refg_off.clear();
+  if (n_chr == 0) return 0;
+  CK(h->refg.ensure((size_t)off.back() + 16));
+  for (int c = 0; c < n_chr; c++)
+    if (ref_lens[c]) CK(cudaMemcpyAsync(h->refg.as<uint8_t>() + off[c], ref_seqs[c], (size_t)ref_lens[c], cudaMemcpyHostToDevice, s));
+  if (off.back()) {
+    k_upper<<<grid_for(off.back(), 256), 256, 0, s>>>(off.back(), h->refg.as<uint8_t>());
+    h->launches += 1;
+    CK(cudaGetLastError());
+  }
+  CK(cudaStreamSynchronize(s));   // the caller's sequences are free again
+  h->refg_off = off;
+  h->ref_uploads += 1;
+  h->ref_h2d_bytes += off.back();
+  return 0;
 }
 
 int colate_last_bam_timing(colate_handle* h, double* out)

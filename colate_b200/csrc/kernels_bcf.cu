@@ -18,14 +18,6 @@ using namespace colate;
 
 namespace {
 
-// decoded record.  a0 / a1: first two alleles as colate_maketmp_records codes them (0 empty or absent, the letter, 0xff longer)
-struct BcfCol {
-  int32_t pos;        // 1-based
-  int32_t alt_sum;    // sum of bcf_gt_allele over the n_hap haplotypes
-  uint8_t a0, a1, biallelic, pad;
-};
-static_assert(sizeof(BcfCol) == 12, "BcfCol is 12 bytes");
-
 // first error of a file: (inflated offset of the record << 3) | kind, atomicMin over the records
 enum : unsigned { kErrNoGT = 1, kErrGTValue = 2, kErrGTLength = 3, kErrFields = 4, kErrGTType = 5 };
 
@@ -588,6 +580,10 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
 
 }  // namespace
 
+namespace colate {
+int decode_genotype_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t) { return decode_file(h, path, chunk_bytes, t); }
+}
+
 extern "C" {
 
 int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const char* const* chr_names, const char* const* bcf_paths,
@@ -616,6 +612,7 @@ int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const 
     if (L) {
       CK(h->bcf_ref.ensure((size_t)L + 16));
       CK(cudaMemcpyAsync(h->bcf_ref.p, ref_seqs[c], (size_t)L, cudaMemcpyHostToDevice, s));
+      h->ref_h2d_bytes += L;
     }
     const int64_t r0 = h->h_site_off[c], nr = h->h_site_off[c + 1] - r0;
     if (nr == 0) continue;
@@ -640,6 +637,7 @@ int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const 
   // the slot is a row-count genome, as colate_set_row_counts leaves it
   g.n_rec = 0;
   g.pileup = true;
+  g.acgt = false;
   g.set = true;
   g.joined = false;
   h->flags_done = false;

@@ -23,6 +23,7 @@
 #include <vector>
 
 #include "device.cuh"
+#include "maketmp_word.h"
 
 namespace colate {
 
@@ -174,11 +175,12 @@ __device__ bool dev_strtof(const char* s, const char* e, float& out)
   return true;
 }
 
-// one data line; status[0] = 1 + first bad row (empty line / too few fields), status[1] = rows for the host
+// one data line; status[0] = 1 + first bad row (empty line / too few fields), status[1] = rows for the host.
+// mkt: the make_tmp row word (maketmp_word.h) next to meta
 __global__ void __launch_bounds__(256)
 k_parse_mut(const char* __restrict__ text, int64_t n_bytes, const int64_t* __restrict__ nl_pos, int64_t n_nl, int64_t n_rows,
             int32_t* __restrict__ pos, float* __restrict__ age_begin, float* __restrict__ age_end, uint32_t* __restrict__ meta,
-            unsigned long long* status, int64_t* __restrict__ fb_rows, int64_t fb_cap)
+            uint32_t* __restrict__ mkt, unsigned long long* status, int64_t* __restrict__ fb_rows, int64_t fb_cap)
 {
   const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (row >= n_rows) return;
@@ -232,6 +234,19 @@ k_parse_mut(const char* __restrict__ text, int64_t n_bytes, const int64_t* __res
       if (oka && okd) m = 1u | ((uint32_t)(unsigned char)a << 8) | ((uint32_t)(unsigned char)d << 16);
     }
   }
+  // the make_tmp word reads the first four bytes of type[16] as parse_mut_line_fields fills it: the field's first 15 bytes, "NN"
+  // (no code) for a longer field.  Rows with fewer than 11 fields go to the host (ok is false), which applies its "NA".
+  uint32_t w = 0;
+  if (nf >= 11) {
+    const char* t = f[10];
+    const char* te = t;
+    while (te < nl && *te != ';') te++;
+    const int64_t L = te - t;
+    if (L <= 15) {
+      const char t4[4] = {L > 0 ? t[0] : '\0', L > 1 ? t[1] : '\0', L > 2 ? t[2] : '\0', L > 3 ? t[3] : '\0'};
+      w = maketmp_word(flipped, nb, t4);
+    }
+  }
   if (nf >= 11) {   // upstream; downstream; frequency columns (std::stoi each, mutations.cpp:224-250)
     const char* g = f[10];
     while (g < nl && *g != ';') g++;
@@ -249,7 +264,7 @@ k_parse_mut(const char* __restrict__ text, int64_t n_bytes, const int64_t* __res
       }
     }
   }
-  pos[row] = ps; age_begin[row] = ab; age_end[row] = ae; meta[row] = m;
+  pos[row] = ps; age_begin[row] = ab; age_end[row] = ae; meta[row] = m; mkt[row] = w;
   if (!ok) {
     const unsigned long long k = atomicAdd(status + 1, 1ull);
     if ((int64_t)k < fb_cap) fb_rows[k] = row;
@@ -293,22 +308,20 @@ k_decode_colate_in(const unsigned char* __restrict__ img, const DevRun* __restri
 
 // rows re-parsed on the host (strtof) -> their places in the site arrays
 __global__ void k_patch_rows(int64_t n, const int64_t* __restrict__ idx, const int32_t* __restrict__ ps, const float* __restrict__ a,
-                             const float* __restrict__ e, const uint32_t* __restrict__ m, int32_t* __restrict__ pos,
-                             float* __restrict__ ab, float* __restrict__ ae, uint32_t* __restrict__ meta)
+                             const float* __restrict__ e, const uint32_t* __restrict__ m, const uint32_t* __restrict__ w,
+                             int32_t* __restrict__ pos, float* __restrict__ ab, float* __restrict__ ae, uint32_t* __restrict__ meta,
+                             uint32_t* __restrict__ mkt)
 {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int64_t r = idx[i];
-  pos[r] = ps[i]; ab[r] = a[i]; ae[r] = e[i]; meta[r] = m[i];
+  pos[r] = ps[i]; ab[r] = a[i]; ae[r] = e[i]; meta[r] = m[i]; mkt[r] = w[i];
 }
 
 }  // namespace colate
 
 using namespace colate;
 
-namespace colate {
-bool parse_mut_line_host(const char* p, const char* nl, int32_t* pos, float* ab, float* ae, uint32_t* meta);  // host_misc.cpp
-}
 
 extern "C" {
 
@@ -318,8 +331,9 @@ int colate_ingest_begin(colate_handle* h, int n_chr, int64_t row_capacity)
     return fail(COLATE_ERR_ARG, "colate_ingest_begin: bad arguments");
   CK(cudaSetDevice(h->device));
   CK(h->pos.ensure(row_capacity * 4 + 4)); CK(h->ab.ensure(row_capacity * 4 + 4));
-  CK(h->ae.ensure(row_capacity * 4 + 4)); CK(h->meta.ensure(row_capacity * 4 + 4));
+  CK(h->ae.ensure(row_capacity * 4 + 4)); CK(h->meta.ensure(row_capacity * 4 + 4)); CK(h->mkt.ensure(row_capacity * 4 + 4));
   h->sites_set = false;
+  h->mkt_valid = false;
   h->flags_done = false;
   h->ing_active = true;
   h->ing_cap = row_capacity;
@@ -361,13 +375,14 @@ static int64_t ingest_one(colate_handle* h, const char* d_text, int64_t n_bytes,
     k_parse_mut<<<(unsigned)((n_rows + 255) / 256), 256, 0, s>>>(d_text, n_bytes, h->ing_nl.as<int64_t>(), n_nl, n_rows,
                                                                  h->pos.as<int32_t>() + row0, h->ab.as<float>() + row0,
                                                                  h->ae.as<float>() + row0, h->meta.as<uint32_t>() + row0,
-                                                                 h->ing_status.as<unsigned long long>(), h->ing_fb.as<int64_t>(), fb_cap);
+                                                                 h->mkt.as<uint32_t>() + row0, h->ing_status.as<unsigned long long>(), h->ing_fb.as<int64_t>(), fb_cap);
     CK(cudaEventRecord(h->ev[1], s));
     unsigned long long st[2];
     CK(cudaMemcpyAsync(st, h->ing_status.p, 16, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     CK(cudaGetLastError());
     h->launches += 4;
+    h->mut_texts_parsed += 1;
     float ms = 0;
     cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]);
     h->ing_ms += ms;
@@ -385,33 +400,37 @@ static int64_t ingest_one(colate_handle* h, const char* d_text, int64_t n_bytes,
       CK(cudaMemcpy(nlp.data(), h->ing_nl.p, n_nl * 8, cudaMemcpyDeviceToHost));
       // re-parsed rows are collected and scattered by one small kernel on the handle's stream (ordered against the
       // parse kernel before it and every consumer after it)
-      std::vector<int64_t> pidx; std::vector<int32_t> ppos; std::vector<float> pab, pae; std::vector<uint32_t> pmeta;
+      std::vector<int64_t> pidx; std::vector<int32_t> ppos; std::vector<float> pab, pae; std::vector<uint32_t> pmeta, pw;
       pidx.reserve(rows.size()); ppos.reserve(rows.size()); pab.reserve(rows.size()); pae.reserve(rows.size()); pmeta.reserve(rows.size());
+      pw.reserve(rows.size());
       for (int64_t r : rows) {
         const char* p = ht + nlp[r] + 1;
         const char* nl = ht + (r + 1 < n_nl ? nlp[r + 1] : n_bytes);
         std::string line(p, nl);                                  // NUL-terminated copy: strtof / strtol stop at the field's ';'
         line.push_back('\n');
-        int32_t ps; float a, e; uint32_t m;
-        if (!parse_mut_line_host(line.data(), line.data() + line.size() - 1, &ps, &a, &e, &m))
+        int32_t ps; float a, e; uint32_t m; int fl, nb; char type[16];
+        if (!parse_mut_line_fields(line.data(), line.data() + line.size() - 1, &ps, &a, &e, &m, &fl, &nb, type))
           return fail(COLATE_ERR_IO, "Error reading following line in mut file: " + std::string(p, nl));
-        pidx.push_back(row0 + r); ppos.push_back(ps); pab.push_back(a); pae.push_back(e); pmeta.push_back(m);
+        pidx.push_back(row0 + r); ppos.push_back(ps); pab.push_back(a); pae.push_back(e); pmeta.push_back(m); pw.push_back(maketmp_word(fl, nb, type));
       }
       const size_t np = pidx.size();
-      CK(h->d_tmp.ensure(np * 24 + 64));
+      CK(h->d_tmp.ensure(np * 28 + 64));
       char* base = h->d_tmp.as<char>();
       int64_t* d_idx = (int64_t*)base;
       int32_t* d_pos = (int32_t*)(base + np * 8);
       float* d_ab = (float*)(base + np * 12);
       float* d_ae = (float*)(base + np * 16);
       uint32_t* d_meta = (uint32_t*)(base + np * 20);
+      uint32_t* d_w = (uint32_t*)(base + np * 24);
       CK(cudaMemcpyAsync(d_idx, pidx.data(), np * 8, cudaMemcpyHostToDevice, s));
       CK(cudaMemcpyAsync(d_pos, ppos.data(), np * 4, cudaMemcpyHostToDevice, s));
       CK(cudaMemcpyAsync(d_ab, pab.data(), np * 4, cudaMemcpyHostToDevice, s));
       CK(cudaMemcpyAsync(d_ae, pae.data(), np * 4, cudaMemcpyHostToDevice, s));
       CK(cudaMemcpyAsync(d_meta, pmeta.data(), np * 4, cudaMemcpyHostToDevice, s));
-      k_patch_rows<<<(unsigned)((np + 255) / 256), 256, 0, s>>>((int64_t)np, d_idx, d_pos, d_ab, d_ae, d_meta, h->pos.as<int32_t>(),
-                                                                h->ab.as<float>(), h->ae.as<float>(), h->meta.as<uint32_t>());
+      CK(cudaMemcpyAsync(d_w, pw.data(), np * 4, cudaMemcpyHostToDevice, s));
+      k_patch_rows<<<(unsigned)((np + 255) / 256), 256, 0, s>>>((int64_t)np, d_idx, d_pos, d_ab, d_ae, d_meta, d_w, h->pos.as<int32_t>(),
+                                                                h->ab.as<float>(), h->ae.as<float>(), h->meta.as<uint32_t>(),
+                                                                h->mkt.as<uint32_t>());
       h->launches += 1;
       CK(cudaGetLastError());
       CK(cudaStreamSynchronize(s));   // the host vectors are locals
@@ -531,7 +550,10 @@ int colate_ingest_end(colate_handle* h)
   h->n_site = h->ing_off.back();
   h->h_site_off = h->ing_off;
   h->ing_active = false;
-  return sites_replaced_ext(h);
+  h->mut_rows_parsed += h->n_site;
+  const int rc = sites_replaced_ext(h);
+  h->mkt_valid = rc == 0;
+  return rc;
 }
 
 int colate_ingest_fetch(colate_handle* h, int64_t row0, int64_t n_rows, int32_t* pos, float* age_begin, float* age_end, uint32_t* meta)

@@ -133,6 +133,8 @@ int colate_pileup_end(colate_handle* h, int slot, int32_t* counts_out);
  * Records of unlisted contigs and unmapped records without a contig (refID -1) are skipped.  A missing EOF block is accepted. */
 int colate_pileup_bam(colate_handle* h, int slot, const char* bam_path, int n_chr, const char* const* chr_names, const uint8_t* const* ref_seqs,
                       const int64_t* ref_lens, int mapq_th, int len_th, int mismatch_th, int64_t chunk_bytes, int32_t* counts_out);
+/* ref_seqs = NULL (ref_lens unused): the contigs come from the handle's resident genome (colate_set_ref_genome, one contig per --chr
+ * entry), which stays on the device -- nothing is copied per call (COLATE_ERR_STATE without one). */
 /* Phases of the last colate_pileup_bam: [0] BGZF index s, [1] inflate s (wall, summed over windows), [2] record walk s, [3] host-to-device
  * copies ms, [4] device decode ms, [5] filter + pileup ms ([3]-[5] only with colate_set_option(h, "bam_timing", 1)), [6] whole call s,
  * [7] inflate threads, [8] inflated bytes, [9] records of listed contigs. */
@@ -182,6 +184,47 @@ int colate_bcf_records(colate_handle* h, int64_t r0, int64_t n, int32_t* rec_pos
  * walk s, [3] host-to-device copies ms, [4] k_bcf_decode ms, [5] k_bcf_rows ms ([3]-[5] only with colate_set_option(h, "bcf_timing",
  * 1)), [6] whole call s, [7] inflate threads, [8] inflated bytes, [9] records. */
 int colate_last_bcf_timing(colate_handle* h, double* out10);
+
+/* ---- make_tmp for many targets on one handle (DESIGN.md section 6i) ------------------------------------------------------ */
+/* The --ref_genome of a job, read once (colate_read_fasta per --chr entry) and kept on the device, upper-cased as fasta::Read leaves
+ * it: colate_pileup_bam with ref_seqs = NULL and colate_maketmp_write_bcf read their contigs from it.  n_chr = 0 drops it. */
+int colate_set_ref_genome(colate_handle* h, int n_chr, const uint8_t* const* ref_seqs, const int64_t* ref_lens);
+/* The make_tmp row word: what the row filters of maketmp_bam (coal.cpp:2568, 2584-2587) and maketmp_vcf (2365, 2381-2395) read from
+ * a .mut row, from its mutation type as the .mut reader keeps it (the first 15 characters; a longer type is no code):
+ *   bit 0  COLATE_MKT_VCF  not flipped, one branch, type exactly a/d with a in {A,C,G,T,0} and d in {A,C,G,T,1}
+ *   bit 1  COLATE_MKT_BAM  not flipped, one branch, one-letter a in {A,C,G,T,0}, '/', a non-empty derived string
+ *   bit 2  COLATE_MKT_ONE  the derived string is one letter
+ *   byte 1 the ancestral letter, byte 2 the first derived letter (0 when the row passes neither filter).
+ * colate_ingest_* builds it next to meta on the device; colate_read_mut_words is the host reader's (.mut or .mut.gz), for sites set
+ * with colate_set_sites + colate_set_maketmp_words.  colate_set_sites clears the words. */
+#define COLATE_MKT_VCF 1u
+#define COLATE_MKT_BAM 2u
+#define COLATE_MKT_ONE 4u
+uint32_t colate_maketmp_word(int flipped, int n_branch, const char* mutation_type);
+int64_t colate_read_mut_words(const char* path, int64_t cap, uint32_t* words);
+int colate_set_maketmp_words(colate_handle* h, const uint32_t* words, int location);
+int colate_fetch_maketmp_words(colate_handle* h, int64_t row0, int64_t n_rows, uint32_t* words);
+/* The make_tmp mask rule (NOT the mode-mut rule of colate_mask_bits_from_fasta): a row at or beyond the mask's end is dropped, bp = 0
+ * is kept, bp >= 1 is kept iff mask[bp - 1] == 'P'.  Pass bits of rows [row0, row0 + n), as colate_mask_bits_from_fasta. */
+int colate_maketmp_mask_bits(const char* path, int64_t n, const int32_t* pos, int64_t row0, uint32_t* pass_bits);
+/* The .colate.in of make_tmp written on the device (k_maketmp_rows, a scan, k_maketmp_scatter; one copy of the bytes to pinned host
+ * memory, then the file).  Byte for byte what colate_maketmp_pileup / colate_maketmp_records write from the same arrays, for .mut
+ * positions that ascend within each chromosome (COLATE_ERR_ORDER otherwise, checked before anything is written).  mask_bits: make_tmp
+ * pass bits per row (colate_maketmp_mask_bits) or NULL.  Nothing is written on failure.  Return the records written or < 0.
+ *   _pileup: the A/C/G/T counts of pileup slot `slot` (colate_pileup_bam, colate_pileup_end or colate_set_pileup), maketmp_bam's rules.
+ *   _bcf:    per --chr entry c the BCF or bgzipped VCF bcf_paths[c], decoded as colate_decode_bcf does and written right after its
+ *            decode, maketmp_vcf's rules; rows without a record read the genome of colate_set_ref_genome (none: such rows are
+ *            dropped).  COLATE_ERR_ARG "allele sum above the number of haplotypes" as colate_maketmp_records.  Leaves the last
+ *            file's records decoded (colate_bcf_records) and its phases in colate_last_bcf_timing ([5]: the writer's kernels). */
+int64_t colate_maketmp_write_pileup(colate_handle* h, int slot, int n_chr, const char* const* chr_names, const uint32_t* mask_bits,
+                                    const char* out_file);
+int64_t colate_maketmp_write_bcf(colate_handle* h, int n_chr, const char* const* chr_names, const char* const* bcf_paths, const uint32_t* mask_bits,
+                                 int64_t chunk_bytes, const char* out_file);
+/* The last writer call: [0] writer kernels ms (CUDA events), [1] device-to-host copy ms, [2] file write s, [3] records. */
+int colate_last_maketmp_timing(colate_handle* h, double* out4);
+/* Work done on this handle since creation: [0] .mut texts parsed on the device, [1] .mut rows parsed (colate_ingest_end), [2] calls of
+ * colate_set_ref_genome, [3] reference-genome bytes copied host-to-device (colate_set_ref_genome, colate_pileup_bam, colate_rows_from_bcf). */
+int colate_upload_counts(colate_handle* h, int64_t* out4);
 
 /* P/N mask of genome `slot` evaluated at the site positions (fasta::Read,
  * include/src/data.cpp:213-237; test at coal.cpp:2169-2174): bit m of pass_bits = row m is
