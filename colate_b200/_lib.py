@@ -61,6 +61,8 @@ SIGNATURES = {
     "colate_last_bam_timing": (C.c_int, [VP, f64]),
     "colate_bam_scan": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_char_p), C.c_int64, i64, i32, i32, i32]),
     "colate_rows_from_bcf": (C.c_int, [VP, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), VP, VP, C.c_int64, VP, VP]),
+    "colate_rows_from_bcf_roles": (C.c_int, [VP, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.c_int, C.c_int64]),
+    "colate_copy_genome": (C.c_int, [VP, C.c_int, C.c_int]),
     "colate_decode_bcf": (C.c_int, [VP, C.c_char_p, C.c_int64, VP, VP]),
     "colate_bcf_records": (C.c_int, [VP, C.c_int64, C.c_int64, VP, VP, VP, VP, VP]),
     "colate_last_bcf_timing": (C.c_int, [VP, f64]),

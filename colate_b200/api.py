@@ -369,6 +369,20 @@ class Handle:
                                          ptr(daf) if fetch else None))
         return (aaf, daf) if fetch else None
 
+    def rows_from_bcf_roles(self, target_slot, reference_slot, paths, genome=0, chunk_bytes=0):
+        """Both roles' row counts from one decode of the files (colate_rows_from_bcf_roles): slot target_slot gets what
+        rows_from_bcf(target_slot, paths, "target") gives, reference_slot what rows_from_bcf(reference_slot, paths, "reference")
+        gives; either may be -1 to skip that role.  genome 0: no --ref_genome, 1: the genome of set_ref_genome, read on the device."""
+        n = len(paths)
+        names = (C.c_char_p * n)(*[str(c).encode() for c in range(n)])
+        files = (C.c_char_p * n)(*[str(p).encode() for p in paths])
+        check(lib().colate_rows_from_bcf_roles(self._h, int(target_slot), int(reference_slot), n, names, files, int(genome), chunk_bytes))
+
+    def copy_genome(self, dst, src):
+        """Slot src's per-row counts (a pileup or row-count genome) copied into slot dst on the device, dst's mask and join state
+        cleared (colate_copy_genome): one decoded file under several masks."""
+        check(lib().colate_copy_genome(self._h, int(dst), int(src)))
+
     def decode_bcf(self, path, chunk_bytes=0) -> dict:
         """One BCF or bgzipped text VCF file's records as the device reduces them (colate_decode_bcf + colate_bcf_records): pos (1-based), a0 / a1 (first
         two alleles: 0 empty or absent, the letter, 0xff longer), alt_sum (sum of the GT allele indices), biallelic, and n_hap."""

@@ -376,6 +376,31 @@ int colate_set_mask(colate_handle* h, int slot, const uint32_t* pass_bits, int l
   return 0;
 }
 
+int colate_copy_genome(colate_handle* h, int dst, int src)
+{
+  if (!h || dst < 0 || dst >= COLATE_MAX_GENOMES || src < 0 || src >= COLATE_MAX_GENOMES || dst == src)
+    return fail(COLATE_ERR_ARG, "colate_copy_genome: bad arguments");
+  if (!h->sites_set) return fail(COLATE_ERR_STATE, "colate_copy_genome: call colate_set_sites first");
+  const GenomeDev& s = h->genomes[src];
+  if (!s.set || !s.pileup)
+    return fail(COLATE_ERR_STATE, "colate_copy_genome: the source slot holds no pileup or row counts (.colate.in record slots are not copied)");
+  CK(cudaSetDevice(h->device));
+  GenomeDev& g = h->genomes[dst];
+  const size_t bytes = (size_t)h->n_site * 16;
+  CK(g.pile.ensure(bytes + 16));
+  if (bytes) CK(cudaMemcpyAsync(g.pile.p, s.pile.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+  g.n_rec = 0;
+  g.pileup = true;
+  g.acgt = s.acgt;
+  g.set = true;
+  g.joined = false;
+  g.has_mask = false;
+  h->flags_done = false;
+  CK(cudaMemsetAsync(h->order_flag.as<int>() + 1 + dst, 0, 4, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
 int colate_stage1_flags(colate_handle* h, int target_slot, int reference_slot, int64_t* n_used_chr, int32_t* n_blocks_chr)
 {
   if (!h || target_slot < 0 || target_slot >= COLATE_MAX_GENOMES || reference_slot < 0 || reference_slot >= COLATE_MAX_GENOMES)

@@ -21,6 +21,7 @@
 #include <sstream>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "../../include/colate_b200.h"
@@ -48,11 +49,16 @@ void help()
                "         [--reference_age <years>] [--years_per_gen <float>] [--coal <file>] [--seed <int>]\n"
                "         [--num_bootstraps <int>] [--device <int> | --devices <i,j,...>] [--host_parse] -o <output prefix>\n"
                "  Colate --mode mut --mut <prefix> --pairs <file> --seed <int> (--bins x,y,step | --coal <file>) [--chr <file>]\n"
-               "         [--years_per_gen <float>] [--num_bootstraps <int>] [--devices <i,j,...>] [--host_parse]\n"
+               "         [--ref_genome <prefix>] [--filters mapq,length,mismatches] [--years_per_gen <float>] [--num_bootstraps <int>]\n"
+               "         [--devices <i,j,...>] [--host_parse]\n"
                "    a cohort in one job: every non-blank line of <file> not starting with '#' is one run\n"
                "      <target_tmp> <reference_tmp> <output_prefix> [target_age=<years>] [reference_age=<years>]\n"
                "      [target_mask=<prefix>] [reference_mask=<prefix>]\n"
-               "    with the shared flags; each line's .coal / .bin equal those of the single-pair run with the same flags\n"
+               "      target_bam=<t.bam> reference_bam=<r.bam> <output_prefix> [same keys]     (needs --ref_genome)\n"
+               "      target_bcf=<prefix> reference_bcf=<prefix> <output_prefix> [same keys]   (needs --chr)\n"
+               "    with the shared flags; each line's .coal / .bin (and, for bam and bcf lines, .colate_mat) equal those of the\n"
+               "    single-pair run with the same flags; every BAM file and BCF / VCF prefix is decoded once per device (a failing\n"
+               "    input fails the lines that use it, the others complete, the exit status is 1)\n"
                "  Colate --mode mut --mut <prefix> --target_bam <t.bam> --reference_bam <r.bam> --ref_genome <prefix> (--bins x,y,step | --coal <file>)\n"
                "         [--chr <file>] [--target_mask <prefix>] [--reference_mask <prefix>] [--target_age <years>] [--reference_age <years>]\n"
                "         [--years_per_gen <float>] [--seed <int>] [--num_bootstraps <int>] [--filters mapq,length,mismatches] [--device <int>]\n"
@@ -626,14 +632,19 @@ int run_mut(const Options& options)
 }
 
 // ---- --pairs: a cohort of target / reference runs in one job ------------------------------------------------------------
-// Every line is the run `Colate --mode mut --target_tmp T --reference_tmp R -o OUT [--target_age ..] ...` with the shared
-// flags, and its .coal / .bin are those of that run.  The .mut text is parsed once per device, every genome (a .colate.in
-// file under one mask) is decoded once into a slot of its own, all pairs consume prefixes of the one --seed generator
-// stream (colate_set_stream_cache), and the EM of all pairs' replicates runs on their mixed epoch grids in one launch
+// Every line is the run `Colate --mode mut --target_tmp T --reference_tmp R -o OUT [--target_age ..] ...` (or its --target_bam /
+// --reference_bam or --target_bcf / --reference_bcf form) with the shared flags, and its .coal / .bin (and, for BAM and BCF lines,
+// .colate_mat) are those of that run.  The .mut text is parsed once per device, --ref_genome is read once and uploaded once per
+// device, every genome (an input under one mask, a BCF prefix once per role) fills a slot of its own, every input file is decoded
+// once per device (further slots of it are device copies, colate_copy_genome), all pairs consume prefixes of the one --seed
+// generator stream (colate_set_stream_cache), and the EM of all pairs' replicates runs on their mixed epoch grids in one launch
 // (colate_stage3_em_grids).
+enum InputKind { kTmp = 0, kBam = 1, kBcf = 2 };
+
 struct PairLine {
   int line = 0;
-  std::string tmp[2], out, age[2], mask[2];
+  int kind = kTmp;
+  std::string input[2], out, age[2], mask[2];
   bool has_age[2] = {false, false};
   int genome[2] = {-1, -1};   // index into the job's genome list
   bool cached = false;        // <out>.colate_mat exists: the reference's stale-cache path
@@ -646,10 +657,24 @@ struct PairLine {
   std::vector<int32_t> iters;
 };
 
-struct GenomeKey { std::string tmp, mask; bool operator<(const GenomeKey& o) const { return tmp != o.tmp ? tmp < o.tmp : mask < o.mask; } };
+// one slot's content: an input file (a .colate.in, a BAM, a BCF / VCF prefix) under a mask; a BCF prefix per role (its rows are
+// resolved by role), a BAM or a .colate.in for both roles alike (role 0)
+struct GenomeKey {
+  int kind = kTmp;
+  std::string input;
+  int role = 0;
+  std::string mask;
+  bool operator<(const GenomeKey& o) const { return std::tie(kind, input, role, mask) < std::tie(o.kind, o.input, o.role, o.mask); }
+};
+
+// the shared flags the pairs-file check needs
+struct PairsFlags {
+  bool has_chr = false, ref_genome = false, strandfilter = false;
+  std::vector<std::string> name_chr;
+};
 
 // The pairs file, checked completely before any device is touched.  false: the message (naming the line) is on stderr.
-bool read_pairs_file(const std::string& path, std::vector<PairLine>& pl, std::vector<GenomeKey>& genomes)
+bool read_pairs_file(const std::string& path, const PairsFlags& fl, std::vector<PairLine>& pl, std::vector<GenomeKey>& genomes)
 {
   std::ifstream is(path);
   if (is.fail()) { std::cerr << "Error: cannot open the pairs file " << path << std::endl; return false; }
@@ -658,6 +683,14 @@ bool read_pairs_file(const std::string& path, std::vector<PairLine>& pl, std::ve
   std::string text;
   int ln = 0;
   auto bad = [&](const std::string& what) { std::cerr << "Error in pairs file " << path << ", line " << ln << ": " << what << std::endl; return false; };
+  // an input field: <file.colate.in>, or target_bam= / target_bcf= (field 0), reference_bam= / reference_bcf= (field 1)
+  static const char* kInputKeys[2][2] = {{"target_bam=", "target_bcf="}, {"reference_bam=", "reference_bcf="}};
+  auto input_key = [](const std::string& f, int role, int* kind) {
+    for (int k = 0; k < 2; k++)
+      if (f.rfind(kInputKeys[role][k], 0) == 0) { *kind = k == 0 ? kBam : kBcf; return (int)strlen(kInputKeys[role][k]); }
+    return 0;
+  };
+  static const char* kKindName[3] = {".colate.in", "bam", "bcf"};
   while (std::getline(is, text)) {
     ln++;
     std::stringstream ss(text);
@@ -668,7 +701,22 @@ bool read_pairs_file(const std::string& path, std::vector<PairLine>& pl, std::ve
     if (f.size() < 3) return bad("expected <target_tmp> <reference_tmp> <output_prefix> [key=value ...], found " + std::to_string(f.size()) + " field(s)");
     PairLine p;
     p.line = ln;
-    p.tmp[0] = f[0]; p.tmp[1] = f[1]; p.out = f[2];
+    int kinds[2] = {kTmp, kTmp};
+    for (int g = 0; g < 2; g++) {
+      int k = kTmp;
+      if (input_key(f[g], 1 - g, &k))
+        return bad("'" + f[g].substr(0, f[g].find('=') + 1) + "' in field " + std::to_string(g + 1) + " (the first field is the target, the second the reference)");
+      const int n = input_key(f[g], g, &k);
+      if (n && n == (int)f[g].size()) return bad("'" + f[g] + "' is not of the form key=value");
+      kinds[g] = k;
+      p.input[g] = f[g].substr(n);
+    }
+    if (kinds[0] != kinds[1])
+      return bad(std::string("a ") + kKindName[kinds[0]] + " target with a " + kKindName[kinds[1]] +
+                 " reference (the reference's mixed front-ends are not supported: both inputs are .colate.in files, both target_bam= / "
+                 "reference_bam=, or both target_bcf= / reference_bcf=)");
+    p.kind = kinds[0];
+    p.out = f[2];
     std::set<std::string> seen;
     for (size_t k = 3; k < f.size(); k++) {
       const size_t eq = f[k].find('=');
@@ -679,20 +727,37 @@ bool read_pairs_file(const std::string& path, std::vector<PairLine>& pl, std::ve
       else if (key == "reference_age") { p.age[1] = val; p.has_age[1] = true; }
       else if (key == "target_mask") p.mask[0] = val;
       else if (key == "reference_mask") p.mask[1] = val;
-      else return bad("unknown key '" + key + "' (known: target_age, reference_age, target_mask, reference_mask)");
+      else if (key == "target_bam" || key == "target_bcf" || key == "reference_bam" || key == "reference_bcf")
+        return bad("'" + key + "=' goes in field " + (key[0] == 't' ? "1" : "2") + " of the line");
+      else
+        return bad("unknown key '" + key + "' (known: target_age, reference_age, target_mask, reference_mask; target_bam, target_bcf in field 1, "
+                   "reference_bam, reference_bcf in field 2)");
     }
     auto dup = out_line.find(p.out);
     if (dup != out_line.end()) return bad("output prefix " + p.out + " is already used on line " + std::to_string(dup->second));
     out_line[p.out] = ln;
+    if (p.kind == kBam) {
+      if (fl.strandfilter) return bad("--strandfilter is not supported with BAM inputs (its read filter is not restated)");
+      if (!fl.ref_genome) return bad("BAM inputs need --ref_genome");
+    }
+    if (p.kind == kBcf && !fl.has_chr) return bad("BCF inputs need --chr (one <prefix>_chr<c>.bcf file per chromosome)");
     for (int g = 0; g < 2; g++) {
-      FILE* fp = fopen(p.tmp[g].c_str(), "rb");
-      if (!fp) return bad("cannot read " + p.tmp[g]);
-      fclose(fp);
-      const GenomeKey key{p.tmp[g], p.mask[g]};
+      std::vector<std::string> files{p.input[g]};
+      if (p.kind == kBcf) {
+        files.clear();
+        for (auto& nm : fl.name_chr) files.push_back(p.input[g] + "_chr" + nm + ".bcf");
+      }
+      for (auto& file : files) {
+        FILE* fp = fopen(file.c_str(), "rb");
+        if (!fp) return bad("cannot read " + file);
+        fclose(fp);
+      }
+      const GenomeKey key{p.kind, p.input[g], p.kind == kBcf ? g : 0, p.mask[g]};
       auto it = gidx.find(key);
       if (it == gidx.end()) {
         if ((int)genomes.size() == COLATE_MAX_GENOMES)
-          return bad("more than " + std::to_string(COLATE_MAX_GENOMES) + " distinct genomes ((.colate.in, mask) combinations) in one job");
+          return bad("more than " + std::to_string(COLATE_MAX_GENOMES) +
+                     " distinct genomes ((input, mask) combinations; a BCF prefix once per role) in one job");
         it = gidx.emplace(key, (int)genomes.size()).first;
         genomes.push_back(key);
       }
@@ -718,9 +783,32 @@ int run_cohort(const Options& options)
   if (!options.count("mut")) { std::cerr << "Error: --pairs needs --mut" << std::endl; return 1; }
   if (!options.count("seed")) { std::cerr << "Error: --pairs needs --seed (all pairs share the generator stream of that seed)" << std::endl; return 1; }
   if (!options.count("bins") && !options.count("coal")) { std::cerr << "Error: --bins or --coal is required." << std::endl; return 1; }
+  // file lists, coal.cpp:3290-3316
+  std::vector<std::string> name_chr, f_mut;
+  if (options.count("chr")) {
+    std::ifstream is(options.get("chr"));
+    if (is.fail()) std::cerr << "Error while opening file " << options.get("chr") << std::endl;
+    std::string line;
+    while (std::getline(is, line)) { name_chr.push_back(line); f_mut.push_back(options.get("mut") + "_chr" + line + ".mut"); }
+  } else {
+    name_chr.push_back("");
+    f_mut.push_back(options.get("mut"));
+  }
+  PairsFlags fl;
+  fl.has_chr = options.count("chr");
+  fl.ref_genome = options.count("ref_genome");
+  fl.strandfilter = options.count("strandfilter");
+  fl.name_chr = name_chr;
   std::vector<PairLine> pl;
   std::vector<GenomeKey> genomes;
-  if (!read_pairs_file(pairs_path, pl, genomes)) return 1;
+  if (!read_pairs_file(pairs_path, fl, pl, genomes)) return 1;
+  bool any_bam = false, live_ref = false;   // live_ref: some pair to be computed reads --ref_genome
+  for (auto& p : pl) {
+    any_bam = any_bam || p.kind == kBam;
+    if (!p.cached && (p.kind == kBam || (p.kind == kBcf && fl.ref_genome))) live_ref = true;
+  }
+  int filters[3];
+  if (!parse_filters(options, filters) && any_bam) { std::cerr << "Error: --filters takes three integers: mapq,length,mismatches" << std::endl; return 1; }
 
   const int seed = atoi(options.get("seed").c_str());
   int R = 1;
@@ -739,17 +827,6 @@ int run_cohort(const Options& options)
   const int G = (int)dev_ids.size();
   std::cerr << "Cohort: " << pl.size() << " pairs, " << genomes.size() << " genomes, " << G << " device(s)" << std::endl;
 
-  // file lists, coal.cpp:3290-3316
-  std::vector<std::string> name_chr, f_mut;
-  if (options.count("chr")) {
-    std::ifstream is(options.get("chr"));
-    if (is.fail()) std::cerr << "Error while opening file " << options.get("chr") << std::endl;
-    std::string line;
-    while (std::getline(is, line)) { name_chr.push_back(line); f_mut.push_back(options.get("mut") + "_chr" + line + ".mut"); }
-  } else {
-    name_chr.push_back("");
-    f_mut.push_back(options.get("mut"));
-  }
   const int n_chr = (int)name_chr.size();
   {
     std::set<std::string> uniq(name_chr.begin(), name_chr.end());
@@ -791,6 +868,8 @@ int run_cohort(const Options& options)
       }
     }
   }
+  RefGenome refg;   // --ref_genome, read once for all devices (fasta::Read, data.cpp:213-237)
+  if (live_ref && !refg.read(options, name_chr)) return 1;
   // the epoch grid of an age, coal.cpp:3503-3646
   auto grid_of_age = [&](PairLine& p, double ypg) -> bool {
     p.epochs.assign(4096, 0.0);
@@ -807,7 +886,8 @@ int run_cohort(const Options& options)
   colate_mt_seed((uint32_t)seed, mt0);
   constexpr int C2 = 2 * COLATE_NUM_AGE_BINS;
   constexpr int kEmBatch = 2048;   // replicates per EM launch
-  std::vector<std::string> dev_err(G);
+  std::vector<std::string> dev_err(G), dev_summary(G);
+  std::vector<int64_t> n_bam(G, 0), n_bcf(G, 0);   // per device: BAM files piled, BCF / VCF files decoded
 
   // one host thread per device; pairs are dealt round-robin in file order
   auto work = [&](int g) {
@@ -846,38 +926,76 @@ int run_cohort(const Options& options)
         if (colate_set_sites(h, n_chr, sh.off.data(), sh.pos.data(), sh.ab.data(), sh.ae.data(), sh.meta.data(), 0)) { dev_fail("colate_set_sites"); return; }
         pos = sh.pos;
       }
-      std::map<int, int> slot_of;     // genome -> slot on this device
-      std::map<int, std::string> genome_err;
+      // --ref_genome once per device, where a pair of this device reads it
+      bool dev_ref = false;
+      for (PairLine* p : mine) dev_ref = dev_ref || (!p->cached && (p->kind == kBam || (p->kind == kBcf && fl.ref_genome)));
+      if (dev_ref && colate_set_ref_genome(h, n_chr, (const uint8_t* const*)refg.seq.data(), refg.len.data())) { dev_fail("colate_set_ref_genome"); return; }
+      std::map<int, int> slot_of;     // genome -> slot on this device, in the order the pairs first use them
+      std::vector<int> order;
       for (PairLine* p : mine) {
         if (p->cached) continue;
-        for (int k = 0; k < 2; k++) {
-          const int gi = p->genome[k];
-          if (slot_of.count(gi)) continue;
-          const int slot = (int)slot_of.size();
-          slot_of[gi] = slot;
+        for (int k = 0; k < 2; k++)
+          if (!slot_of.count(p->genome[k])) { slot_of[p->genome[k]] = (int)order.size(); order.push_back(p->genome[k]); }
+      }
+      std::map<int, std::string> genome_err;
+      // BAM and BCF inputs: decoded once per device (both roles of a BCF prefix from one decode); the input's further slots (other
+      // masks) are device copies of its first slot of the same role.  first[(input, role)] = that slot, or its error.
+      std::map<std::pair<std::string, int>, int> first;
+      std::map<std::string, std::string> input_err;
+      for (const int gi : order) {
+        const GenomeKey& gk = genomes[gi];
+        const int slot = slot_of[gi];
+        const std::string ik = std::to_string(gk.kind) + ":" + gk.input;   // the input file(s) of this genome
+        if (gk.kind == kTmp) {
           std::vector<char> image;
-          FILE* f = fopen(genomes[gi].tmp.c_str(), "rb");
-          if (!f) { genome_err[gi] = "cannot read " + genomes[gi].tmp; continue; }
+          FILE* f = fopen(gk.input.c_str(), "rb");
+          if (!f) { genome_err[gi] = "cannot read " + gk.input; continue; }
           fseek(f, 0, SEEK_END);
           const long sz = ftell(f);
           fseek(f, 0, SEEK_SET);
           image.resize((size_t)std::max(sz, 0L));
           const bool short_read = sz > 0 && fread(image.data(), 1, (size_t)sz, f) != (size_t)sz;
           fclose(f);
-          if (short_read) { genome_err[gi] = "short read on " + genomes[gi].tmp; continue; }
+          if (short_read) { genome_err[gi] = "short read on " + gk.input; continue; }
           if (colate_ingest_colate_in(h, slot, image.data(), (int64_t)image.size(), n_chr, names.data(), 0) < 0) {
-            genome_err[gi] = genomes[gi].tmp + ": " + colate_last_error();
+            genome_err[gi] = gk.input + ": " + colate_last_error();
             continue;
           }
-          if (genomes[gi].mask.empty()) continue;
-          std::vector<uint32_t> bits(((size_t)site_off[n_chr] + 31) / 32 + 1, 0);
-          bool ok = true;
-          for (int c = 0; c < n_chr && ok; c++)
-            ok = !colate_mask_bits_from_fasta(mask_file(genomes[gi].mask, c).c_str(), site_off[c + 1] - site_off[c], pos.data() + site_off[c], site_off[c],
-                                              bits.data());
-          if (ok) ok = !colate_set_mask(h, slot, bits.data(), 0);
-          if (!ok) genome_err[gi] = "mask " + genomes[gi].mask + ": " + colate_last_error();
+        } else {
+          if (!first.count({ik, gk.role}) && !input_err.count(ik)) {
+            if (gk.kind == kBam) {
+              n_bam[g]++;
+              if (colate_pileup_bam(h, slot, gk.input.c_str(), n_chr, names.data(), nullptr, nullptr, filters[0], filters[1], filters[2], 0, nullptr))
+                input_err[ik] = gk.input + ": " + colate_last_error();
+              else
+                first[{ik, 0}] = slot;
+            } else {
+              int rs[2] = {-1, -1};   // the first slot of each role of this prefix on this device
+              for (const int gj : order)
+                if (genomes[gj].kind == kBcf && genomes[gj].input == gk.input && rs[genomes[gj].role] < 0) rs[genomes[gj].role] = slot_of[gj];
+              std::vector<std::string> files;
+              for (auto& nm : name_chr) files.push_back(gk.input + "_chr" + nm + ".bcf");
+              std::vector<const char*> fp;
+              for (auto& x : files) fp.push_back(x.c_str());
+              n_bcf[g] += n_chr;
+              if (colate_rows_from_bcf_roles(h, rs[0], rs[1], n_chr, names.data(), fp.data(), fl.ref_genome ? 1 : 0, 0))
+                input_err[ik] = gk.input + ": " + colate_last_error();
+              else
+                for (int r = 0; r < 2; r++) if (rs[r] >= 0) first[{ik, r}] = rs[r];
+            }
+          }
+          if (input_err.count(ik)) { genome_err[gi] = input_err[ik]; continue; }
+          const int src = first[{ik, gk.role}];
+          if (src != slot && colate_copy_genome(h, slot, src)) { genome_err[gi] = gk.input + ": " + colate_last_error(); continue; }
         }
+        if (gk.mask.empty()) continue;
+        std::vector<uint32_t> bits(((size_t)site_off[n_chr] + 31) / 32 + 1, 0);
+        bool ok = true;
+        for (int c = 0; c < n_chr && ok; c++)
+          ok = !colate_mask_bits_from_fasta(mask_file(gk.mask, c).c_str(), site_off[c + 1] - site_off[c], pos.data() + site_off[c], site_off[c],
+                                            bits.data());
+        if (ok) ok = !colate_set_mask(h, slot, bits.data(), 0);
+        if (!ok) genome_err[gi] = "mask " + gk.mask + ": " + colate_last_error();
       }
       // stages i-ii per pair (coal.cpp:3317-3451) and its epoch grid
       if (colate_set_stream_cache(h, 1)) { dev_fail("colate_set_stream_cache"); return; }
@@ -888,6 +1006,8 @@ int run_cohort(const Options& options)
         if (!p->err.empty()) continue;
         double ypg = 28.0;
         p->age_gen = colate_age_generations(p->has_age[0] ? p->age[0].c_str() : nullptr, p->has_age[1] ? p->age[1].c_str() : nullptr, has_ypg, ypg_flag, &ypg);
+        // BAM and BCF lines: raw count weights in stage i, counts / 1e3 from stage ii (as the single-pair run sets it)
+        if (colate_set_option(h, "front_end", p->kind == kTmp ? 0 : 1)) { dev_fail("colate_set_option"); return; }
         uint32_t mt[COLATE_MT_WORDS];
         if (colate_stage1(h, slot_of[p->genome[0]], slot_of[p->genome[1]], mt0, &p->num_blocks, nullptr, nullptr, &p->n_used, mt)) {
           p->err = std::string("stage i: ") + colate_last_error();
@@ -902,9 +1022,11 @@ int run_cohort(const Options& options)
             continue;
           }
         }
+        if (R == 0) p->counts.assign(C2, 0.0);   // the .colate_mat of R = 0 holds the age grid alone
         grid_of_age(*p, ypg);
       }
       colate_set_stream_cache(h, 0);
+      if (colate_set_option(h, "front_end", 0)) { dev_fail("colate_set_option"); return; }
       // stage iii: every replicate of every pair on its own grid, kEmBatch replicates per launch (coal.cpp:3675-3827)
       if (R > 0) {
         std::vector<PairLine*> run;
@@ -971,6 +1093,13 @@ int run_cohort(const Options& options)
         p->err = std::string("EM: ") + colate_last_error();
       if (colate_set_age_bins(h, nullptr)) { dev_fail("colate_set_age_bins"); return; }
     }
+    int64_t cnt[4];
+    colate_upload_counts(h, cnt);
+    char line[256];
+    snprintf(line, sizeof line, "device %d (handle %d of %d): BAM files piled %lld, BCF/VCF files decoded %lld, .mut texts parsed %lld (%lld rows), "
+             "reference genome uploads %lld (%lld bytes)", dev_ids[g], g + 1, G, (long long)n_bam[g], (long long)n_bcf[g], (long long)cnt[0],
+             (long long)cnt[1], (long long)cnt[2], (long long)cnt[3]);
+    dev_summary[g] = line;
   };
   {
     std::vector<std::thread> th;
@@ -979,9 +1108,15 @@ int run_cohort(const Options& options)
     for (auto& t : th) t.join();
   }
   for (auto& e : dev_err) if (!e.empty()) std::cerr << e << std::endl;
-  // outputs in file order; a failed pair writes nothing
+  for (auto& x : dev_summary) if (!x.empty()) std::cerr << x << std::endl;
+  // outputs in file order; a failed pair writes nothing.  BAM and BCF lines keep their bootstrap counts (coal.cpp:3336-3343,
+  // 3453-3465), written first as the single-pair run does; a line from the stale cache leaves its .colate_mat as it is
+  double age_bin[COLATE_NUM_AGE_BINS];
+  colate_age_bins(age_bin);
   int n_failed = 0;
   for (auto& p : pl) {
+    if (p.err.empty() && p.kind != kTmp && !p.cached && colate_write_colate_mat((p.out + ".colate_mat").c_str(), R, age_bin, p.counts.data()))
+      p.err = std::string("writing the output: ") + colate_last_error();
     if (p.err.empty() && (colate_write_coal((p.out + ".coal").c_str(), R, p.E, p.epochs.data(), p.rates.data(), p.age_gen > 0.0, p.ep_null) ||
                           colate_write_bin((p.out + ".bin").c_str(), R, p.E, p.epochs.data(), p.rates.data(), p.iters.data())))
       p.err = std::string("writing the output: ") + colate_last_error();

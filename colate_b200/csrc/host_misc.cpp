@@ -630,7 +630,8 @@ int colate_write_coal(const char* path, int R, int E, const double* epochs, doub
 int colate_write_colate_mat(const char* path, int R, const double* age_bin, const double* counts)
 {
   // coal.cpp:3336-3343 (grid line) and 3453-3465 (two lines per replicate), operator<<(double) with default flags == "%g"
-  if (!path || R <= 0 || !age_bin || !counts) return fail(COLATE_ERR_ARG, "colate_write_colate_mat: bad arguments");
+  // R = 0 (--num_bootstraps 0): the grid line alone, as the reference writes it; counts may then be NULL
+  if (!path || R < 0 || !age_bin || (R > 0 && !counts)) return fail(COLATE_ERR_ARG, "colate_write_colate_mat: bad arguments");
   FILE* f = fopen(path, "w");
   if (!f) return fail(COLATE_ERR_IO, std::string("cannot write ") + path);
   for (int b = 0; b < colate::NBINS; b++) fprintf(f, "%g ", age_bin[b]);

@@ -1,8 +1,8 @@
 // BCF records decoded on the device, then resolved against the .mut rows (the decoder half of parse_vcfvcf, coal.cpp:997-1137).
 // The host (host_bcf.cpp) inflates the BGZF blocks of one window of the file into pinned memory and finds the record boundaries;
 // k_bcf_decode reduces every record to 12 bytes (position, the codes of its first two alleles, the GT allele sum, the biallelic
-// flag), which stay resident for the whole file while the raw bytes stream through; k_bcf_rows<role> gives every .mut row of
-// the chromosome its (AAF, DAF) straight in the slot's row-count columns.  Window n+1 is inflated on the host while window n
+// flag), which stay resident for the whole file while the raw bytes stream through; k_bcf_rows gives every .mut row of the
+// chromosome its (AAF, DAF) straight in the row-count columns of a target slot, a reference slot or both.  Window n+1 is inflated on the host while window n
 // is on the device.  Bgzipped text VCF (host_vcf.cpp) takes the same path with k_vcf_decode in place of k_bcf_decode: the
 // format is detected from the file's first inflated bytes (open_genotypes), as htslib's bcf_open does.
 #include <algorithm>
@@ -411,23 +411,23 @@ __global__ void __launch_bounds__(256) k_vcf_decode(int64_t k0, int64_t k1, int6
 __device__ __forceinline__ bool letter(uint32_t x) { return x != 0u && x != 0xffu; }
 
 // thread = .mut row of the chromosome: the record at the row is the first one at or after its position (both cursors of
-// parse_vcfvcf, coal.cpp:1001-1006 / 1074-1079, reduce to this lower bound: rows and records ascend).  role 1 (reference,
-// coal.cpp:1008-1062): the record's two alleles are the row's in either order (flipped: DAF = N - allele sum) and it is
-// biallelic; no record: DAF = N if --ref_genome shows the derived allele; DAF = 0 drops the row.  role 0 (target, 1081-1131):
-// as the reference, or the record reports one allele (second empty or absent), one of the row's, with allele sum 0 (DAF = N if
-// it is the derived one); no record: --ref_genome gives N for the derived base, 0 for the ancestral one.  Output: the slot's
-// row counts (AAF, DAF) = (N - DAF, DAF), zeros where the row is not usable for this genome (as k_pack_row_counts packs them).
-template <int ROLE>
+// parse_vcfvcf, coal.cpp:1001-1006 / 1074-1079, reduce to this lower bound: rows and records ascend).  Reference rules
+// (coal.cpp:1008-1062): the record's two alleles are the row's in either order (flipped: DAF = N - allele sum) and it is
+// biallelic; no record: DAF = N if --ref_genome shows the derived allele; DAF = 0 drops the row.  Target rules (1081-1131): as
+// the reference, or the record reports one allele (second empty or absent), one of the row's, with allele sum 0 (DAF = N if it
+// is the derived one); no record: --ref_genome gives N for the derived base, 0 for the ancestral one.  One lower bound and one
+// genome read serve both roles: pile_t gets the target's row counts, pile_r the reference's (a null array is skipped), each as
+// (AAF, DAF) = (N - DAF, DAF), zeros where the row is not usable for that role (as k_pack_row_counts packs them).
 __global__ void k_bcf_rows(int64_t row0, int64_t n_rows, const int32_t* __restrict__ site_pos, const uint32_t* __restrict__ meta,
                            const BcfCol* __restrict__ cols, int64_t n_rec, int32_t N, const uint8_t* __restrict__ ref, int64_t ref_len,
-                           int4* __restrict__ pile)
+                           int4* __restrict__ pile_t, int4* __restrict__ pile_r)
 {
   const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (m >= n_rows) return;
   const int64_t row = row0 + m;
   const uint32_t mt = meta[row];
   const uint32_t anc = (mt >> 8) & 0xffu, der = (mt >> 16) & 0xffu;
-  int32_t daf = -1;                                           // -1: not usable
+  int32_t daf_t = -1, daf_r = -1;                             // -1: not usable
   if ((mt & 1u) && anc != der) {                              // coal.cpp:966-995: the lookups only happen for these rows
     const int32_t bp = site_pos[row];
     int64_t lo = 0, hi = n_rec;
@@ -437,19 +437,20 @@ __global__ void k_bcf_rows(int64_t row0, int64_t n_rows, const int32_t* __restri
       const bool two = letter(c.a0) && letter(c.a1);
       const bool same = two && c.a0 == anc && c.a1 == der, flip = two && c.a0 == der && c.a1 == anc;
       if (same || flip) {
-        if (c.biallelic) daf = flip ? N - c.alt_sum : c.alt_sum;
-      } else if (ROLE == 0 && c.a0 != 0 && c.a1 == 0) {
-        if (letter(c.a0) && (c.a0 == anc || c.a0 == der) && c.biallelic && c.alt_sum == 0) daf = c.a0 == der ? N : 0;
+        if (c.biallelic) daf_t = daf_r = flip ? N - c.alt_sum : c.alt_sum;
+      } else if (c.a0 != 0 && c.a1 == 0) {
+        if (letter(c.a0) && (c.a0 == anc || c.a0 == der) && c.biallelic && c.alt_sum == 0) daf_t = c.a0 == der ? N : 0;
       }
     } else if (ref && bp >= 1 && (int64_t)bp - 1 < ref_len) {
       uint32_t b = ref[bp - 1];
       if (b >= 'a' && b <= 'z') b -= 32;                      // fasta::Read upper-cases (data.cpp:213-237)
-      if (b == der) daf = N;
-      else if (ROLE == 0 && b == anc) daf = 0;
+      if (b == der) daf_t = daf_r = N;
+      else if (b == anc) daf_t = 0;
     }
-    if (ROLE == 1 && daf == 0) daf = -1;
+    if (daf_r == 0) daf_r = -1;
   }
-  pile[row] = daf >= 0 ? make_int4(N - daf, daf, 0, -1) : make_int4(0, 0, 0, -1);
+  if (pile_t) pile_t[row] = daf_t >= 0 ? make_int4(N - daf_t, daf_t, 0, -1) : make_int4(0, 0, 0, -1);
+  if (pile_r) pile_r[row] = daf_r >= 0 ? make_int4(N - daf_r, daf_r, 0, -1) : make_int4(0, 0, 0, -1);
 }
 
 inline int grid_for(int64_t n, int threads) { return (int)((n + threads - 1) / threads); }
@@ -578,6 +579,73 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
   return 0;
 }
 
+// the row counts of the target slot t_slot and / or the reference slot r_slot (-1: that role is skipped) from one decode of every
+// chromosome's file.  Genome: host contigs (ref_seqs / ref_lens, uploaded per chromosome), the handle's resident genome
+// (resident), or none.
+int rows_from_bcf(colate_handle* h, int t_slot, int r_slot, int n_chr, const char* const* chr_names, const char* const* bcf_paths,
+                  const uint8_t* const* ref_seqs, const int64_t* ref_lens, bool resident, int64_t chunk_bytes)
+{
+  CK(cudaSetDevice(h->device));
+  const auto t_start = std::chrono::steady_clock::now();
+  double t[10] = {};
+  cudaStream_t s = h->stream;
+  const size_t n_site = (size_t)h->n_site;
+  const int slots[2] = {t_slot, r_slot};
+  for (int sl : slots)
+    if (sl >= 0) CK(h->genomes[sl].pile.ensure(n_site * 16 + 16));
+  int4* pile_t = t_slot >= 0 ? h->genomes[t_slot].pile.as<int4>() : nullptr;
+  int4* pile_r = r_slot >= 0 ? h->genomes[r_slot].pile.as<int4>() : nullptr;
+  cudaEvent_t tev[2] = {};
+  if (h->opt_bcf_timing)
+    for (auto& e : tev) CK(cudaEventCreate(&e));
+  struct TEv { cudaEvent_t* e; ~TEv() { for (int i = 0; i < 2; i++) if (e[i]) cudaEventDestroy(e[i]); } } tev_guard{tev};
+  for (int c = 0; c < n_chr; c++) {
+    if (int rc = decode_file(h, bcf_paths[c], chunk_bytes, t)) return fail(rc, std::string("chromosome ") + chr_names[c] + ": " + colate_last_error());
+    const uint8_t* ref = nullptr;
+    int64_t L = 0;
+    if (resident) {
+      L = h->refg_off[c + 1] - h->refg_off[c];
+      ref = L ? h->refg.as<uint8_t>() + h->refg_off[c] : nullptr;
+    } else if (ref_seqs && ref_seqs[c] && ref_lens[c]) {
+      L = ref_lens[c];
+      CK(h->bcf_ref.ensure((size_t)L + 16));
+      CK(cudaMemcpyAsync(h->bcf_ref.p, ref_seqs[c], (size_t)L, cudaMemcpyHostToDevice, s));
+      h->ref_h2d_bytes += L;
+      ref = h->bcf_ref.as<uint8_t>();
+    }
+    const int64_t r0 = h->h_site_off[c], nr = h->h_site_off[c + 1] - r0;
+    if (nr == 0) continue;
+    if (tev[0]) CK(cudaEventRecord(tev[0], s));
+    k_bcf_rows<<<grid_for(nr, 256), 256, 0, s>>>(r0, nr, h->pos.as<int32_t>(), h->meta.as<uint32_t>(), h->bcf_cols.as<BcfCol>(), h->bcf_n_rec,
+                                                 h->bcf_n_hap, ref, L, pile_t, pile_r);
+    h->launches += 1;
+    CK(cudaGetLastError());
+    if (tev[0]) {
+      CK(cudaEventRecord(tev[1], s));
+      CK(cudaEventSynchronize(tev[1]));
+      float ms = 0;
+      CK(cudaEventElapsedTime(&ms, tev[0], tev[1]));
+      t[5] += ms;
+    }
+  }
+  // the slots are row-count genomes, as colate_set_row_counts leaves them
+  for (int sl : slots) {
+    if (sl < 0) continue;
+    GenomeDev& g = h->genomes[sl];
+    g.n_rec = 0;
+    g.pileup = true;
+    g.acgt = false;
+    g.set = true;
+    g.joined = false;
+    CK(cudaMemsetAsync(h->order_flag.as<int>() + 1 + sl, 0, 4, s));
+  }
+  h->flags_done = false;
+  CK(cudaStreamSynchronize(s));
+  t[6] = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
+  memcpy(h->bcf_timing, t, sizeof t);
+  return 0;
+}
+
 }  // namespace
 
 namespace colate {
@@ -595,66 +663,34 @@ int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const 
   if (!h->sites_set || n_chr != h->n_chr) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf: one file per chromosome of the site set");
   for (int c = 0; c < n_chr; c++)
     if (!bcf_paths[c] || (ref_seqs && (ref_lens[c] < 0 || (ref_lens[c] > 0 && !ref_seqs[c])))) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf: bad arguments");
-  CK(cudaSetDevice(h->device));
-  const auto t_start = std::chrono::steady_clock::now();
-  double t[10] = {};
-  cudaStream_t s = h->stream;
-  GenomeDev& g = h->genomes[slot];
-  const size_t n_site = (size_t)h->n_site;
-  CK(g.pile.ensure(n_site * 16 + 16));
-  cudaEvent_t tev[2] = {};
-  if (h->opt_bcf_timing)
-    for (auto& e : tev) CK(cudaEventCreate(&e));
-  struct TEv { cudaEvent_t* e; ~TEv() { for (int i = 0; i < 2; i++) if (e[i]) cudaEventDestroy(e[i]); } } tev_guard{tev};
-  for (int c = 0; c < n_chr; c++) {
-    if (int rc = decode_file(h, bcf_paths[c], chunk_bytes, t)) return fail(rc, std::string("chromosome ") + chr_names[c] + ": " + colate_last_error());
-    const int64_t L = ref_seqs && ref_seqs[c] ? ref_lens[c] : 0;
-    if (L) {
-      CK(h->bcf_ref.ensure((size_t)L + 16));
-      CK(cudaMemcpyAsync(h->bcf_ref.p, ref_seqs[c], (size_t)L, cudaMemcpyHostToDevice, s));
-      h->ref_h2d_bytes += L;
-    }
-    const int64_t r0 = h->h_site_off[c], nr = h->h_site_off[c + 1] - r0;
-    if (nr == 0) continue;
-    if (tev[0]) CK(cudaEventRecord(tev[0], s));
-    const uint8_t* ref = L ? h->bcf_ref.as<uint8_t>() : nullptr;
-    if (role == 0)
-      k_bcf_rows<0><<<grid_for(nr, 256), 256, 0, s>>>(r0, nr, h->pos.as<int32_t>(), h->meta.as<uint32_t>(), h->bcf_cols.as<BcfCol>(), h->bcf_n_rec,
-                                                      h->bcf_n_hap, ref, L, g.pile.as<int4>());
-    else
-      k_bcf_rows<1><<<grid_for(nr, 256), 256, 0, s>>>(r0, nr, h->pos.as<int32_t>(), h->meta.as<uint32_t>(), h->bcf_cols.as<BcfCol>(), h->bcf_n_rec,
-                                                      h->bcf_n_hap, ref, L, g.pile.as<int4>());
-    h->launches += 1;
-    CK(cudaGetLastError());
-    if (tev[0]) {
-      CK(cudaEventRecord(tev[1], s));
-      CK(cudaEventSynchronize(tev[1]));
-      float ms = 0;
-      CK(cudaEventElapsedTime(&ms, tev[0], tev[1]));
-      t[5] += ms;
-    }
-  }
-  // the slot is a row-count genome, as colate_set_row_counts leaves it
-  g.n_rec = 0;
-  g.pileup = true;
-  g.acgt = false;
-  g.set = true;
-  g.joined = false;
-  h->flags_done = false;
-  CK(cudaMemsetAsync(h->order_flag.as<int>() + 1 + slot, 0, 4, s));
+  if (int rc = rows_from_bcf(h, role == 0 ? slot : -1, role == 1 ? slot : -1, n_chr, chr_names, bcf_paths, ref_seqs, ref_lens, false, chunk_bytes))
+    return rc;
   if (aaf_out || daf_out) {
+    const size_t n_site = (size_t)h->n_site;
     std::vector<int32_t> p4(n_site * 4);
-    if (n_site) CK(cudaMemcpyAsync(p4.data(), g.pile.p, n_site * 16, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if (n_site) CK(cudaMemcpyAsync(p4.data(), h->genomes[slot].pile.p, n_site * 16, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     for (size_t m = 0; m < n_site; m++) {
       if (aaf_out) aaf_out[m] = p4[4 * m];
       if (daf_out) daf_out[m] = p4[4 * m + 1];
     }
   }
-  CK(cudaStreamSynchronize(s));
-  t[6] = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
-  memcpy(h->bcf_timing, t, sizeof t);
   return 0;
+}
+
+int colate_rows_from_bcf_roles(colate_handle* h, int target_slot, int reference_slot, int n_chr, const char* const* chr_names,
+                               const char* const* bcf_paths, int genome, int64_t chunk_bytes)
+{
+  if (!h || target_slot < -1 || target_slot >= COLATE_MAX_GENOMES || reference_slot < -1 || reference_slot >= COLATE_MAX_GENOMES ||
+      (target_slot < 0 && reference_slot < 0) || target_slot == reference_slot || (genome != 0 && genome != 1) || n_chr <= 0 || !chr_names ||
+      !bcf_paths || chunk_bytes < 0)
+    return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_roles: bad arguments");
+  if (!h->sites_set || n_chr != h->n_chr) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_roles: one file per chromosome of the site set");
+  for (int c = 0; c < n_chr; c++)
+    if (!bcf_paths[c]) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_roles: bad arguments");
+  if (genome == 1 && (int)h->refg_off.size() != n_chr + 1)
+    return fail(COLATE_ERR_STATE, "colate_rows_from_bcf_roles: genome = 1 needs colate_set_ref_genome with one contig per chromosome");
+  return rows_from_bcf(h, target_slot, reference_slot, n_chr, chr_names, bcf_paths, nullptr, nullptr, genome == 1, chunk_bytes);
 }
 
 int colate_decode_bcf(colate_handle* h, const char* bcf_path, int64_t chunk_bytes, int64_t* n_records, int32_t* n_hap)

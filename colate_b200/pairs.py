@@ -73,27 +73,37 @@ def all_pairs(handle: api.Handle, n_genomes: int, seed: int, bins: str = "3,7,0.
 
 
 def cohort(handle: api.Handle, pairs, seed: int, bins: str | None = None, coal: str | None = None, num_bootstraps: int = 1,
-           years_per_gen=None, max_iter: int = 100000, em_batch: int = 2048):
+           years_per_gen=None, max_iter: int = 100000, em_batch: int = 2048, front_ends=None):
     """A cohort: pairs = [(target_slot, reference_slot, target_age, reference_age)], ages in years as the CLI takes them (str,
     number or None), genomes (and their masks) already in the handle's slots.  Per pair: stage i from the --seed state (the
     generator stream is shared, colate_set_stream_cache), `num_bootstraps` block weights drawn from the pair's post-stage-i state,
     stage ii at the pair's age and the pair's epoch grid (--bins, or --coal with its initial rates).  Then the EM of all
     P x num_bootstraps replicates on their mixed grids (Handle.stage3_em_grids, em_batch replicates per call).
-    Every pair's result is what `api.mut()` returns for that pair alone.  Returns dict(pairs=[per-pair dict(epochs, ep_null,
+    Every pair's result is what `api.mut()` returns for that pair alone.
+    front_ends: None leaves the handle's "front_end" option as it is.  A list of 0 / 1, one per pair, sets the option to that
+    value before the pair's stage i (1 for BAM / BCF genomes: raw count weights and counts / 1e3, as `api.mut` with front_end = 1
+    gives them; 0 for .colate.in genomes) and sets it back to 0 at the end.  Returns dict(pairs=[per-pair dict(epochs, ep_null,
     is_ancient, rates[R][E], iters[R], ll[R], num_blocks, n_used, counts[R][2][185])], seconds=dict(stage12, em))."""
     if (bins is None) == (coal is None):
         raise ValueError("give exactly one of bins and coal")
     R = int(num_bootstraps)
     if R < 1:
         raise ValueError("num_bootstraps must be >= 1")
+    pairs = list(pairs)
+    if front_ends is not None:
+        front_ends = [int(f) for f in front_ends]
+        if len(front_ends) != len(pairs) or any(f not in (0, 1) for f in front_ends):
+            raise ValueError("front_ends: one 0 / 1 per pair")
     txt = lambda a: None if a is None else str(a)
     t0 = time.perf_counter()
     mt0 = api.mt_seed(seed)
     out, grids, grid_key = [], [], {}
     handle.set_stream_cache(True)       # every pair reseeds with the same --seed: one generator stream serves them all
     try:
-        for t_slot, r_slot, t_age, r_age in pairs:
+        for p, (t_slot, r_slot, t_age, r_age) in enumerate(pairs):
             age, ypg = api.ages(txt(t_age), txt(r_age), years_per_gen)
+            if front_ends is not None:
+                handle.set_option("front_end", front_ends[p])
             s1 = handle.stage1(mt0, target_slot=int(t_slot), reference_slot=int(r_slot), fetch=False)
             w = api.draw_block_weights(s1.mt_state, R, s1.num_blocks)
             counts = handle.stage2_bootstrap_dev(w, None, s1.num_blocks, age, fetch=True)
@@ -111,6 +121,8 @@ def cohort(handle: api.Handle, pairs, seed: int, bins: str | None = None, coal: 
                             counts=counts, grid=grid_key[key]))
     finally:
         handle.set_stream_cache(False)
+        if front_ends is not None:
+            handle.set_option("front_end", 0)
     t1 = time.perf_counter()
     P = len(out)
     grid_of = np.repeat(np.array([p["grid"] for p in out], dtype=np.int32), R)

@@ -174,6 +174,13 @@ int colate_last_bam_timing(colate_handle* h, double* out10);
 #define COLATE_BCF_REFERENCE 1
 int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const char* const* chr_names, const char* const* bcf_paths,
                          const uint8_t* const* ref_seqs, const int64_t* ref_lens, int64_t chunk_bytes, int32_t* aaf_out, int32_t* daf_out);
+/* Both roles from one decode (DESIGN.md section 6j): every chromosome's file is decoded once and k_bcf_rows resolves each row under
+ * the target rules into slot target_slot and under the reference rules into slot reference_slot, each exactly as colate_rows_from_bcf
+ * with that role leaves it.  Either slot may be -1 (that role is skipped), not both; they differ.  genome = 0: no --ref_genome;
+ * genome = 1: the handle's resident genome (colate_set_ref_genome, one contig per chromosome), read in place (COLATE_ERR_STATE
+ * without one). */
+int colate_rows_from_bcf_roles(colate_handle* h, int target_slot, int reference_slot, int n_chr, const char* const* chr_names,
+                               const char* const* bcf_paths, int genome, int64_t chunk_bytes);
 /* Decode only: one BCF or bgzipped text VCF file's records reduced on the device as colate_rows_from_bcf does (same checks), kept on the device;
  * colate_bcf_records copies records [r0, r0 + n) out in the arrays colate_maketmp_records takes (position 1-based, allele codes,
  * allele sum, biallelic flag).  *n_hap = samples x GT length. */
@@ -230,6 +237,11 @@ int colate_upload_counts(colate_handle* h, int64_t* out4);
  * include/src/data.cpp:213-237; test at coal.cpp:2169-2174): bit m of pass_bits = row m is
  * NOT rejected by the mask (positions at or beyond the mask end pass).  NULL clears it. */
 int colate_set_mask(colate_handle* h, int slot, const uint32_t* pass_bits, int location);
+/* Genome `src`'s per-row counts (a pileup or row-count slot: colate_pileup_bam, colate_set_pileup, colate_set_row_counts,
+ * colate_rows_from_bcf[_roles], ...) copied into slot `dst` on the device, so one decoded file can sit under several masks
+ * without being decoded again.  dst's mask and join state are cleared.  COLATE_ERR_STATE for a .colate.in record slot or an
+ * unset one. */
+int colate_copy_genome(colate_handle* h, int dst, int src);
 
 /* ---- stage i: parse_tmptmp, coal.cpp:2071-2321 (called at coal.cpp:3317) ------------- */
 
@@ -444,7 +456,8 @@ int64_t colate_maketmp_records(int n_chr, const char* const* chr_names, const ch
                                const uint8_t* rec_biallelic, const int32_t* n_hap, const char* const* ref_genomes,
                                const char* const* target_masks, const char* out_file);
 /* <out>.colate_mat as mut() writes it for every front-end but tmp/tmp (coal.cpp:3336-3343, 3453-3465): the age grid, then per
- * replicate the shared and the not-shared count vector (already divided by 1e3), default ostream formatting. */
+ * replicate the shared and the not-shared count vector (already divided by 1e3), default ostream formatting.  R = 0 writes the
+ * grid line alone (counts may be NULL). */
 int colate_write_colate_mat(const char* path, int R, const double* age_bin, const double* counts);
 /* <out>.coal (coal.cpp:3660-3672, 3830-3844) and the raw fp64 side output <out>.bin. */
 int colate_write_coal(const char* path, int R, int E, const double* epochs, double* rates, int is_ancient, int ep_null);
