@@ -64,6 +64,9 @@ SIGNATURES = {
     "colate_rows_from_bcf_roles": (C.c_int, [VP, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.c_int, C.c_int64]),
     "colate_copy_genome": (C.c_int, [VP, C.c_int, C.c_int]),
     "colate_decode_bcf": (C.c_int, [VP, C.c_char_p, C.c_int64, VP, VP]),
+    "colate_rows_from_bcf_genome": (C.c_int, [VP, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.c_char_p, C.c_int, C.c_int64]),
+    "colate_decode_bcf_genome": (C.c_int, [VP, C.c_char_p, C.c_int, C.POINTER(C.c_char_p), C.c_int64, VP, VP, VP]),
+    "colate_bcf_genome_scan": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_char_p), C.c_int64, VP, VP, VP, VP]),
     "colate_bcf_records": (C.c_int, [VP, C.c_int64, C.c_int64, VP, VP, VP, VP, VP]),
     "colate_last_bcf_timing": (C.c_int, [VP, f64]),
     "colate_bcf_scan": (C.c_int, [C.c_char_p, C.c_int64, VP, VP, VP, VP, VP, VP]),
@@ -116,6 +119,7 @@ SIGNATURES = {
     "colate_maketmp_mask_bits": (C.c_int, [C.c_char_p, C.c_int64, VP, C.c_int64, VP]),
     "colate_maketmp_write_pileup": (C.c_int64, [VP, C.c_int, C.c_int, C.POINTER(C.c_char_p), VP, C.c_char_p]),
     "colate_maketmp_write_bcf": (C.c_int64, [VP, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), VP, C.c_int64, C.c_char_p]),
+    "colate_maketmp_write_bcf_genome": (C.c_int64, [VP, C.c_int, C.POINTER(C.c_char_p), C.c_char_p, VP, C.c_int64, C.c_char_p]),
     "colate_last_maketmp_timing": (C.c_int, [VP, f64]),
     "colate_upload_counts": (C.c_int, [VP, i64]),
     "colate_write_colate_mat": (C.c_int, [C.c_char_p, C.c_int, f64, f64]),

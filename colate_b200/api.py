@@ -147,6 +147,17 @@ def bcf_scan(path: str, window_bytes: int = 0) -> dict:
     return {k: int(x[0]) for k, x in zip(keys, v)}
 
 
+def bcf_genome_scan(path: str, chr_names, window_bytes: int = 0) -> dict:
+    """Host-only walk of a whole-genome BCF or bgzipped text VCF (no GPU): per --chr entry the records of its contig (<name> or
+    chr<name>) and their first / last POS (0-based), and the header's sample count (colate_bcf_genome_scan).  Raises ColateError for
+    the files colate_rows_from_bcf_genome refuses on the host."""
+    n = len(chr_names)
+    names = (C.c_char_p * n)(*[str(s).encode() for s in chr_names])
+    cnt = np.zeros(n, np.int64); first = np.zeros(n, np.int32); last = np.zeros(n, np.int32); ns = np.zeros(1, np.int32)
+    check(lib().colate_bcf_genome_scan(str(path).encode(), n, names, window_bytes, ptr(cnt), ptr(first), ptr(last), ptr(ns)))
+    return {"n_records": cnt, "first_pos": first, "last_pos": last, "n_sample": int(ns[0])}
+
+
 def vcf_scan(path: str, window_bytes: int = 0) -> dict:
     """Host-only walk of a bgzipped text VCF (no GPU): the record count, the first / last POS (0-based, as htslib's bcf1_t.pos), the
     header's sample count and the records' CHROM (colate_vcf_scan).  Raises ColateError for the files colate_rows_from_bcf refuses
@@ -331,6 +342,14 @@ class Handle:
         mb = None if mask_bits is None else np.ascontiguousarray(mask_bits, dtype=np.uint32)
         return check(lib().colate_maketmp_write_bcf(self._h, n, names, files, ptr(mb), chunk_bytes, str(out_file).encode()))
 
+    def maketmp_write_bcf_genome(self, path, chr_names, out_file, mask_bits=None, chunk_bytes=0) -> int:
+        """maketmp_write_bcf from one whole-genome BCF / VCF file (colate_maketmp_write_bcf_genome): chromosome c reads the contig
+        chr_names[c] or chr<chr_names[c]>."""
+        n = len(chr_names)
+        names = (C.c_char_p * n)(*[str(s).encode() for s in chr_names])
+        mb = None if mask_bits is None else np.ascontiguousarray(mask_bits, dtype=np.uint32)
+        return check(lib().colate_maketmp_write_bcf_genome(self._h, n, names, str(path).encode(), ptr(mb), chunk_bytes, str(out_file).encode()))
+
     def last_maketmp_timing(self) -> dict:
         t = np.zeros(4)
         check(lib().colate_last_maketmp_timing(self._h, t))
@@ -377,6 +396,30 @@ class Handle:
         names = (C.c_char_p * n)(*[str(c).encode() for c in range(n)])
         files = (C.c_char_p * n)(*[str(p).encode() for p in paths])
         check(lib().colate_rows_from_bcf_roles(self._h, int(target_slot), int(reference_slot), n, names, files, int(genome), chunk_bytes))
+
+    def rows_from_bcf_genome(self, target_slot, reference_slot, path, chr_names, genome=0, chunk_bytes=0):
+        """rows_from_bcf_roles from one whole-genome BCF / VCF file (colate_rows_from_bcf_genome): chromosome c of the site set reads
+        the records of the contig chr_names[c] or chr<chr_names[c]>, as its own file would hold them.  The file is decoded once."""
+        n = len(chr_names)
+        names = (C.c_char_p * n)(*[str(s).encode() for s in chr_names])
+        check(lib().colate_rows_from_bcf_genome(self._h, int(target_slot), int(reference_slot), n, names, str(path).encode(), int(genome),
+                                                chunk_bytes))
+
+    def decode_bcf_genome(self, path, chr_names, chunk_bytes=0) -> list:
+        """decode_bcf of a whole-genome file (colate_decode_bcf_genome): per --chr entry the dict decode_bcf gives for its contig."""
+        n = len(chr_names)
+        names = (C.c_char_p * n)(*[str(s).encode() for s in chr_names])
+        first = np.zeros(n, np.int64); cnt = np.zeros(n, np.int64); nh = np.zeros(n, np.int32)
+        check(lib().colate_decode_bcf_genome(self._h, str(path).encode(), n, names, chunk_bytes, ptr(first), ptr(cnt), ptr(nh)))
+        out = []
+        for c in range(n):
+            k = int(cnt[c])
+            d = {"pos": np.zeros(k, np.int32), "a0": np.zeros(k, np.uint8), "a1": np.zeros(k, np.uint8), "alt_sum": np.zeros(k, np.int32),
+                 "biallelic": np.zeros(k, np.uint8)}
+            check(lib().colate_bcf_records(self._h, int(first[c]), k, *[ptr(d[x]) for x in ("pos", "a0", "a1", "alt_sum", "biallelic")]))
+            d["n_hap"] = int(nh[c])
+            out.append(d)
+        return out
 
     def copy_genome(self, dst, src):
         """Slot src's per-row counts (a pileup or row-count genome) copied into slot dst on the device, dst's mask and join state

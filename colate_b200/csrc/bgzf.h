@@ -17,6 +17,9 @@ struct BgzfBlock {
   uint64_t uoff;      // offset of the block's first inflated byte in the inflated stream
 };
 
+// A --chr entry <name> reads the contig <name> or chr<name> (bam_parser, htslib.cpp:388): BAM, and whole-genome BCF / VCF.
+bool contig_matches(const std::string& contig, const std::string& entry);
+
 class BgzfFile {
  public:
   ~BgzfFile();

@@ -68,6 +68,8 @@ void help()
                "         [--reference_age <years>] [--years_per_gen <float>] [--seed <int>] [--num_bootstraps <int>] [--device <int>]\n"
                "         -o <output prefix>     (reads <prefix>_chr<c>.bcf per --chr entry, BCF or bgzipped VCF as for htslib;\n"
                "                                 also writes <output prefix>.colate_mat; one device)\n"
+               "    a BCF / VCF <prefix> without any <prefix>_chr<c>.bcf that is itself a file is read as a whole genome: --chr entry\n"
+               "    c reads its contig c or chr<c> (everywhere target_bcf / reference_bcf are read, --pairs and --targets lines too)\n"
                "  Colate --mode make_tmp --mut <prefix> --chr <file> --target_bcf <prefix> --ref_genome <prefix> [--target_mask <prefix>]\n"
                "         [--device <int>] -o <output prefix>     (writes <output prefix>.colate.in)\n"
                "  Colate --mode make_tmp --mut <prefix> --target_bam <t.bam> --ref_genome <prefix> [--chr <file>] [--target_mask <prefix>]\n"
@@ -249,6 +251,29 @@ bool bcf_args_ok(const Options& o, bool need_both)
   return true;
 }
 
+// A BCF / VCF input X (--target_bcf, --reference_bcf, target_bcf= / reference_bcf= lines): per-chromosome files X_chr<c>.bcf, as
+// the reference opens them, when any of them exists; otherwise X itself when it is a regular file, read as a whole genome (one
+// file, --chr entry c reading the contig c or chr<c>); otherwise the per-chromosome files, whose absence is reported as before.
+struct GenotypeInput {
+  bool whole = false;
+  std::vector<std::string> files;   // the per-chromosome files, or X
+};
+GenotypeInput genotype_input(const std::string& x, const std::vector<std::string>& name_chr)
+{
+  GenotypeInput in;
+  bool any = false;
+  struct stat st;
+  for (auto& nm : name_chr) {
+    in.files.push_back(x + "_chr" + nm + ".bcf");
+    any |= stat(in.files.back().c_str(), &st) == 0;
+  }
+  if (!any && stat(x.c_str(), &st) == 0 && S_ISREG(st.st_mode)) {
+    in.whole = true;
+    in.files.assign(1, x);
+  }
+  return in;
+}
+
 int run_mut(const Options& options)
 {
   if (!options.count("mut") || !options.count("output")) {  // coal.cpp:3077-3086
@@ -377,12 +402,13 @@ int run_mut(const Options& options)
     for (auto& s : name_chr) names.push_back(s.c_str());
     const std::string files[2] = {options.get(bam ? "target_bam" : bcf ? "target_bcf" : "target_tmp"),
                                   options.get(bam ? "reference_bam" : bcf ? "reference_bcf" : "reference_tmp")};
-    std::vector<std::string> bcf_files[2];   // <prefix>_chr<c>.bcf, as the reference opens them
+    GenotypeInput bcf_in[2];   // <prefix>_chr<c>.bcf, as the reference opens them, or one whole-genome file
     std::vector<const char*> bcf_paths[2];
     for (int g = 0; g < 2 && bcf; g++) {
-      for (auto& nm : name_chr) bcf_files[g].push_back(files[g] + "_chr" + nm + ".bcf");
-      for (auto& f : bcf_files[g]) bcf_paths[g].push_back(f.c_str());
+      bcf_in[g] = genotype_input(files[g], name_chr);
+      for (auto& f : bcf_in[g].files) bcf_paths[g].push_back(f.c_str());
     }
+    const bool bcf_whole = bcf_in[0].whole || bcf_in[1].whole;
     struct GenomeHost { int64_t n = 0; std::vector<char> image; std::vector<int32_t> rc, bp, aaf, daf; std::vector<uint16_t> al; std::vector<int64_t> first, end; } gh[2];
     RefGenome refg;
     int filters[3];
@@ -471,8 +497,18 @@ int run_mut(const Options& options)
       // BAM genomes: the pileup of each file at the rows (parse_onebambam's bam_parser, coal.cpp:1799-2069); BCF genomes: the
       // decoder half of parse_vcfvcf (coal.cpp:997-1137) per genome.  Both front-ends: raw count weights and 1e3 normalisation
       if (counts_front_end && colate_set_option(d.h, "front_end", 1)) { d.fail("colate_set_option"); return; }
+      // a whole-genome input reads --ref_genome resident on the device
+      if (bcf_whole && !refg.seq.empty() && colate_set_ref_genome(d.h, n_chr, (const uint8_t* const*)refg.seq.data(), refg.len.data())) {
+        d.fail("colate_set_ref_genome");
+        return;
+      }
       for (int g = 0; g < 2; g++) {
-        if (bcf) {
+        if (bcf && bcf_in[g].whole) {
+          if (colate_rows_from_bcf_genome(d.h, g == 0 ? 0 : -1, g == 1 ? 1 : -1, n_chr, names.data(), files[g].c_str(), refg.seq.empty() ? 0 : 1, 0)) {
+            d.fail(files[g]);
+            return;
+          }
+        } else if (bcf) {
           if (colate_rows_from_bcf(d.h, g, g == 0 ? COLATE_BCF_TARGET : COLATE_BCF_REFERENCE, n_chr, names.data(), bcf_paths[g].data(),
                                    refg.seq.empty() ? nullptr : (const uint8_t* const*)refg.seq.data(), refg.seq.empty() ? nullptr : refg.len.data(), 0,
                                    nullptr, nullptr)) {
@@ -742,11 +778,7 @@ bool read_pairs_file(const std::string& path, const PairsFlags& fl, std::vector<
     }
     if (p.kind == kBcf && !fl.has_chr) return bad("BCF inputs need --chr (one <prefix>_chr<c>.bcf file per chromosome)");
     for (int g = 0; g < 2; g++) {
-      std::vector<std::string> files{p.input[g]};
-      if (p.kind == kBcf) {
-        files.clear();
-        for (auto& nm : fl.name_chr) files.push_back(p.input[g] + "_chr" + nm + ".bcf");
-      }
+      const std::vector<std::string> files = p.kind == kBcf ? genotype_input(p.input[g], fl.name_chr).files : std::vector<std::string>{p.input[g]};
       for (auto& file : files) {
         FILE* fp = fopen(file.c_str(), "rb");
         if (!fp) return bad("cannot read " + file);
@@ -973,12 +1005,12 @@ int run_cohort(const Options& options)
               int rs[2] = {-1, -1};   // the first slot of each role of this prefix on this device
               for (const int gj : order)
                 if (genomes[gj].kind == kBcf && genomes[gj].input == gk.input && rs[genomes[gj].role] < 0) rs[genomes[gj].role] = slot_of[gj];
-              std::vector<std::string> files;
-              for (auto& nm : name_chr) files.push_back(gk.input + "_chr" + nm + ".bcf");
+              const GenotypeInput in = genotype_input(gk.input, name_chr);
               std::vector<const char*> fp;
-              for (auto& x : files) fp.push_back(x.c_str());
-              n_bcf[g] += n_chr;
-              if (colate_rows_from_bcf_roles(h, rs[0], rs[1], n_chr, names.data(), fp.data(), fl.ref_genome ? 1 : 0, 0))
+              for (auto& x : in.files) fp.push_back(x.c_str());
+              n_bcf[g] += (int64_t)in.files.size();
+              if (in.whole ? colate_rows_from_bcf_genome(h, rs[0], rs[1], n_chr, names.data(), fp[0], fl.ref_genome ? 1 : 0, 0)
+                           : colate_rows_from_bcf_roles(h, rs[0], rs[1], n_chr, names.data(), fp.data(), fl.ref_genome ? 1 : 0, 0))
                 input_err[ik] = gk.input + ": " + colate_last_error();
               else
                 for (int r = 0; r < 2; r++) if (rs[r] >= 0) first[{ik, r}] = rs[r];
@@ -1216,7 +1248,7 @@ int run_make_tmp_bcf(const Options& options)
   std::cerr << options.get("target_bcf") << ".." << std::endl;
   if (!bcf_args_ok(options, false)) return 1;
   if (!options.count("ref_genome")) { std::cerr << "Option 'ref_genome' has no value" << std::endl; return 1; }   // cxxopts throws in the reference
-  std::vector<std::string> name_chr, f_mut, f_ref, f_mask, f_bcf;
+  std::vector<std::string> name_chr, f_mut, f_ref, f_mask;
   {
     std::ifstream is(options.get("chr"));
     if (is.fail()) { std::cerr << "Error while opening file " << options.get("chr") << std::endl; return 1; }
@@ -1225,7 +1257,6 @@ int run_make_tmp_bcf(const Options& options)
       name_chr.push_back(line);
       f_mut.push_back(options.get("mut") + "_chr" + line + ".mut");
       f_ref.push_back(options.get("ref_genome") + "_chr" + line + ".fa");
-      f_bcf.push_back(options.get("target_bcf") + "_chr" + line + ".bcf");
       if (options.count("target_mask")) f_mask.push_back(options.get("target_mask") + "_chr" + line + ".fa");
     }
   }
@@ -1235,19 +1266,26 @@ int run_make_tmp_bcf(const Options& options)
     std::set<std::string> uniq(name_chr.begin(), name_chr.end());
     if ((int)uniq.size() != n_chr) { std::cerr << "Duplicate chromosome names in --chr" << std::endl; return 1; }
   }
+  const GenotypeInput in = genotype_input(options.get("target_bcf"), name_chr);
   colate_handle* h = nullptr;
   if (colate_create(options.count("device") ? atoi(options.get("device").c_str()) : 0, &h)) return die("colate_create");
   struct Destroy { colate_handle* h; ~Destroy() { colate_destroy(h); } } destroy{h};
-  std::vector<int64_t> off(n_chr + 1, 0);
+  std::vector<int64_t> off(n_chr + 1, 0), rec_first(n_chr, 0), rec_n(n_chr, 0);
   std::vector<int32_t> pos, alt, n_hap(n_chr);
   std::vector<uint8_t> a0, a1, bi;
+  if (in.whole) {   // one decode of the whole-genome file, every chromosome's records resident
+    std::vector<const char*> nm;
+    for (auto& x : name_chr) nm.push_back(x.c_str());
+    if (colate_decode_bcf_genome(h, in.files[0].c_str(), n_chr, nm.data(), 0, rec_first.data(), rec_n.data(), n_hap.data())) return die(in.files[0]);
+  }
   for (int c = 0; c < n_chr; c++) {
     std::cerr << "parsing CHR: " << c + 1 << " / " << n_chr << std::endl;
-    int64_t n = 0;
-    if (colate_decode_bcf(h, f_bcf[c].c_str(), 0, &n, &n_hap[c])) return die(f_bcf[c]);
+    const std::string& f = in.files[in.whole ? 0 : c];
+    if (!in.whole && colate_decode_bcf(h, f.c_str(), 0, &rec_n[c], &n_hap[c])) return die(f);
+    const int64_t n = rec_n[c];
     const size_t o = pos.size();
     pos.resize(o + n); a0.resize(o + n); a1.resize(o + n); alt.resize(o + n); bi.resize(o + n);
-    if (colate_bcf_records(h, 0, n, pos.data() + o, a0.data() + o, a1.data() + o, alt.data() + o, bi.data() + o)) return die(f_bcf[c]);
+    if (colate_bcf_records(h, rec_first[c], n, pos.data() + o, a0.data() + o, a1.data() + o, alt.data() + o, bi.data() + o)) return die(f);
     off[c + 1] = off[c] + n;
   }
   std::vector<const char*> names, muts, refs, masks;
@@ -1332,8 +1370,7 @@ bool read_targets_file(const std::string& path, const std::vector<std::string>& 
       fclose(fp);
     } else {
       if (!has_chr) return bad("target_bcf needs --chr (one <prefix>_chr<c>.bcf file per chromosome)");
-      for (auto& nm : name_chr) {
-        const std::string fbcf = t.input + "_chr" + nm + ".bcf";
+      for (auto& fbcf : genotype_input(t.input, name_chr).files) {
         FILE* fp = fopen(fbcf.c_str(), "rb");
         if (!fp) return bad("cannot read " + fbcf);
         fclose(fp);
@@ -1491,11 +1528,12 @@ int run_make_tmp_batch(const Options& options)
                 t.line, b[1], b[2], b[6], w[0], w[1], w[2]);
       }
     } else {
-      std::vector<std::string> files;
-      for (auto& nm : name_chr) files.push_back(t.input + "_chr" + nm + ".bcf");
+      const GenotypeInput in = genotype_input(t.input, name_chr);
       std::vector<const char*> fp;
-      for (auto& f : files) fp.push_back(f.c_str());
-      if ((t.records = colate_maketmp_write_bcf(h, n_chr, names.data(), fp.data(), mb, 0, out.c_str())) < 0) t.err = t.input + ": " + colate_last_error();
+      for (auto& f : in.files) fp.push_back(f.c_str());
+      t.records = in.whole ? colate_maketmp_write_bcf_genome(h, n_chr, names.data(), fp[0], mb, 0, out.c_str())
+                           : colate_maketmp_write_bcf(h, n_chr, names.data(), fp.data(), mb, 0, out.c_str());
+      if (t.records < 0) t.err = t.input + ": " + colate_last_error();
       if (ph.on && t.err.empty()) {
         double b[10], w[4];
         colate_last_bcf_timing(h, b);

@@ -159,7 +159,8 @@ struct colate_handle {
   bool opt_bam_timing = false;
   double bam_timing[10] = {};
   // colate_rows_from_bcf / colate_decode_bcf (kernels_bcf.cu): one window's bytes and record offsets, the decoded columns of one
-  // file (12 B per record, resident), the current chromosome's reference genome, the decode state (GT length, first error)
+  // file (12 B per record, resident), the current chromosome's reference genome, the decode state (GT length, first error; per
+  // contig for a whole-genome file)
   colate::DevBuf bcf_buf, bcf_cols, bcf_ref, bcf_state;
   int64_t bcf_n_rec = 0;       // records of the last decoded file in bcf_cols
   int32_t bcf_n_hap = 0;
@@ -181,6 +182,12 @@ struct colate_handle {
 namespace colate {
 // kernels_bcf.cu: one BCF or bgzipped text VCF file -> h->bcf_cols (h->bcf_n_rec records of h->bcf_n_hap haplotypes)
 int decode_genotype_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t);
+// one whole-genome file: --chr entry c's records at h->bcf_cols [first[c], first[c] + n[c]), n_hap[c] haplotypes
+struct GenomeRecs {
+  std::vector<int64_t> first, n;
+  std::vector<int32_t> n_hap;
+};
+int decode_genotype_genome(colate_handle* h, const char* path, int n_chr, const char* const* chr_names, int64_t chunk_bytes, double* t, GenomeRecs* gr);
 // kernels_sites.cu
 int run_join(colate_handle* h, int slot);
 int run_flags(colate_handle* h, int tslot, int rslot);

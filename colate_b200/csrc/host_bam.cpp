@@ -48,7 +48,6 @@ int BamReader::parse_header(int n_chr, const char* const* chr_names)
     o += 4 + l_name + 4;
   }
   drop_header(o);
-  // --chr entry <name> = header contig <name> or chr<name> (bam_parser, htslib.cpp:388)
   listed_of_ref_.assign(n_ref, -1);
   ref_of_listed_.assign(n_chr, -1);
   done_.assign(n_chr, 0);
@@ -56,7 +55,7 @@ int BamReader::parse_header(int n_chr, const char* const* chr_names)
     const std::string a = chr_names[c], b = "chr" + a;
     listed_names_.push_back(a);
     for (int32_t r = 0; r < n_ref; r++) {
-      if (ref_names_[r] != a && ref_names_[r] != b) continue;
+      if (!contig_matches(ref_names_[r], a)) continue;
       if (ref_of_listed_[c] >= 0)
         return fail(COLATE_ERR_IO, path_ + ": contig " + a + " of the --chr list appears in the BAM header as both " + ref_names_[ref_of_listed_[c]] +
                                        " and " + ref_names_[r]);

@@ -31,6 +31,8 @@ BgzfFile::~BgzfFile()
   if (fd_ >= 0) close(fd_);
 }
 
+bool contig_matches(const std::string& contig, const std::string& entry) { return contig == entry || contig == "chr" + entry; }
+
 int BgzfFile::err(const std::string& what, uint64_t off, bool compressed)
 {
   return fail(COLATE_ERR_IO, path_ + ": " + what + " at " + (compressed ? "byte offset " : "inflated byte offset ") + std::to_string(off));

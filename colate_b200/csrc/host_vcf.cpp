@@ -82,8 +82,8 @@ int VcfReader::read_header()
   return 0;
 }
 
-// one record line buf[o, e) (newline excluded): CHROM and POS
-int VcfReader::line(const uint8_t* buf, size_t o, size_t e, BcfWindow& w)
+// one record line buf[o, e) (newline excluded; the next line starts at next): CHROM and POS
+int VcfReader::line(const uint8_t* buf, size_t o, size_t e, size_t next, BcfWindow& w)
 {
   const uint64_t at = w.ustart + o;
   if (e == o) return err("empty VCF line", at, false);
@@ -100,6 +100,14 @@ int VcfReader::line(const uint8_t* buf, size_t o, size_t e, BcfWindow& w)
   }
   if (!ok) return err("VCF POS that is not a plain decimal in [0, 2147483646]", at, false);
   const int32_t pos = (int32_t)(v - 1);
+  if (!listed.empty()) {
+    if (ce - o != chrom.size() || memcmp(buf + o, chrom.data(), ce - o) != 0 || !walking_) {
+      chrom.assign((const char*)buf + o, ce - o);
+      walking_ = true;
+      if (int rc = enter_contig(chrom, at)) return rc;
+    }
+    return cur_ >= 0 ? listed_record(w, o, next, pos, at) : 0;
+  }
   if (n_records == 0) {
     chrom.assign((const char*)buf + o, ce - o);
     first_pos = pos;
@@ -127,6 +135,7 @@ int VcfReader::fill(uint8_t* buf, size_t target, BcfWindow& w)
   w.n_bytes = n;
   w.rec_off.clear();
   w.rec_pos.clear();
+  w.runs.clear();
   const bool last = at_end();
   // newlines: in the carried bytes (a cut line, or after the header what its blocks held past it) found here, in the inflated
   // blocks listed by the inflate threads (BgzfFile::newlines)
@@ -136,12 +145,15 @@ int VcfReader::fill(uint8_t* buf, size_t target, BcfWindow& w)
     const bool found = nl || k < newlines.size();
     if (!found && !last) break;                               // partial line: carried into the next window
     const size_t e = nl ? (size_t)(nl - buf) : found ? (size_t)newlines[k++] : n;   // the last line may lack its newline
-    if (int rc = line(buf, o, e, w)) return rc;
-    o = found ? e + 1 : e;
+    const size_t next = found ? e + 1 : e;
+    if (int rc = line(buf, o, e, next, w)) return rc;
+    o = next;
   }
   w.text_end = (int64_t)o;
+  if (listed.empty() && !w.rec_off.empty()) w.runs.push_back(BcfRun{0, 0, (int64_t)w.rec_off.size(), (int64_t)o});
   carry_tail(buf, o, n, w.ustart);
   walk_s += now_s() - t0;
+  if (at_end() && !listed.empty()) return listed_complete();
   if (at_end() && n_records == 0) return err("VCF file without records (the reference reads a first record unconditionally)", carry_uoff_, false);
   return 0;
 }
@@ -179,5 +191,37 @@ extern "C" int colate_vcf_scan(const char* path, int64_t window_bytes, int64_t* 
     memcpy(chrom, c.data(), k);
     chrom[k] = 0;
   }
+  return 0;
+}
+
+// Host-only scan of a whole-genome BCF or bgzipped text VCF (no GPU; the format detected as open_genotypes does): per --chr entry
+// the records of its contig, their first and last POS (0-based), and the header's sample count, with every host check of
+// colate_rows_from_bcf_genome.
+extern "C" int colate_bcf_genome_scan(const char* path, int n_chr, const char* const* chr_names, int64_t window_bytes, int64_t* n_records,
+                                      int32_t* first_pos, int32_t* last_pos, int32_t* n_sample)
+{
+  using namespace colate;
+  if (!path || n_chr <= 0 || !chr_names) return fail(COLATE_ERR_ARG, "colate_bcf_genome_scan: bad arguments");
+  for (int c = 0; c < n_chr; c++)
+    if (!chr_names[c]) return fail(COLATE_ERR_ARG, "colate_bcf_genome_scan: bad arguments");
+  std::unique_ptr<GenotypeReader> rd;
+  if (int rc = open_genotypes(path, (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency())), &rd)) return rc;
+  rd->set_listed(n_chr, chr_names);
+  const size_t target = window_bytes > 0 ? (size_t)window_bytes : (size_t)64 << 20;
+  std::vector<uint8_t> buf;
+  BcfWindow w;
+  for (;;) {
+    const size_t need = rd->next_window_bytes(target);
+    if (need == 0) break;
+    if (buf.size() < need) buf.resize(need);
+    if (int rc = rd->fill(buf.data(), target, w)) return rc;
+  }
+  if (int rc = rd->listed_complete()) return rc;
+  for (int c = 0; c < n_chr; c++) {
+    if (n_records) n_records[c] = rd->listed_n[c];
+    if (first_pos) first_pos[c] = rd->listed_first[c];
+    if (last_pos) last_pos[c] = rd->listed_last[c];
+  }
+  if (n_sample) *n_sample = rd->n_sample;
   return 0;
 }

@@ -1,7 +1,8 @@
 // BCF records decoded on the device, then resolved against the .mut rows (the decoder half of parse_vcfvcf, coal.cpp:997-1137).
 // The host (host_bcf.cpp) inflates the BGZF blocks of one window of the file into pinned memory and finds the record boundaries;
 // k_bcf_decode reduces every record to 12 bytes (position, the codes of its first two alleles, the GT allele sum, the biallelic
-// flag), which stay resident for the whole file while the raw bytes stream through; k_bcf_rows gives every .mut row of the
+// flag), which stay resident for the whole file while the raw bytes stream through (a whole-genome file: the records of every
+// --chr contig, each contig's kept apart); k_bcf_rows gives every .mut row of the
 // chromosome its (AAF, DAF) straight in the row-count columns of a target slot, a reference slot or both.  Window n+1 is inflated on the host while window n
 // is on the device.  Bgzipped text VCF (host_vcf.cpp) takes the same path with k_vcf_decode in place of k_bcf_decode: the
 // format is detected from the file's first inflated bytes (open_genotypes), as htslib's bcf_open does.
@@ -476,17 +477,25 @@ int ensure_cols(colate_handle* h, int64_t n, int64_t keep)
   return 0;
 }
 
-// one BCF or bgzipped text VCF file -> h->bcf_cols (h->bcf_n_rec records of h->bcf_n_hap haplotypes).  t[]: timing accumulators as colate_last_bcf_timing
-int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t)
+// One BCF or bgzipped text VCF file -> h->bcf_cols.  A per-chromosome file (gr null): h->bcf_n_rec records of h->bcf_n_hap
+// haplotypes.  A whole-genome file (gr: n_chr --chr entries chr_names, GenotypeReader::set_listed): the records of every listed
+// contig in file order, entry c's at [gr->first[c], gr->first[c] + gr->n[c]) with GT length gr->n_hap[c]; contigs outside the
+// list are not copied to the device.  Each contig has its own state (GT length, first error: 16 bytes in h->bcf_state), and its
+// first record is decoded alone: its GT length is the one every later record of the contig must have.  t[]: timing
+// accumulators as colate_last_bcf_timing
+int decode_file(colate_handle* h, const char* path, int n_chr, const char* const* chr_names, int64_t chunk_bytes, double* t, GenomeRecs* gr)
 {
   std::unique_ptr<GenotypeReader> rdp;
   if (int rc = open_genotypes(path, bcf_threads(), &rdp)) return rc;
   GenotypeReader& rd = *rdp;
+  if (gr) rd.set_listed(n_chr, chr_names);
+  const int n_state = gr ? n_chr : 1;
   const int gt_key = rd.text ? -1 : static_cast<BcfReader&>(rd).gt_key;
   cudaStream_t s = h->stream;
-  CK(h->bcf_state.ensure(32));
-  CK(cudaMemsetAsync(h->bcf_state.p, 0xff, 16, s));          // GT length -1, no error (~0)
-  CK(cudaMemsetAsync(h->bcf_state.as<char>() + 16, 0, 16, s));   // text VCF, vcf_paths option: lines on the fast / the general path
+  CK(h->bcf_state.ensure((size_t)n_state * 16 + 16));
+  CK(cudaMemsetAsync(h->bcf_state.p, 0xff, (size_t)n_state * 16, s));               // per contig: GT length -1, no error (~0)
+  char* const paths = h->bcf_state.as<char>() + (size_t)n_state * 16;               // text VCF, vcf_paths option: lines on the fast / the general path
+  CK(cudaMemsetAsync(paths, 0, 16, s));
   const size_t target = chunk_bytes > 0 ? (size_t)chunk_bytes : (size_t)64 << 20;
   Pinned raw[2], offs[2];
   cudaEvent_t done[2];
@@ -500,6 +509,7 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     for (auto& e : tev) CK(cudaEventCreate(&e));
   struct TEv { cudaEvent_t* e; ~TEv() { for (int i = 0; i < 3; i++) if (e[i]) cudaEventDestroy(e[i]); } } tev_guard{tev};
   int64_t n_rec = 0, n_inflated = 0;
+  std::vector<int64_t> first(n_state, -1), seen(n_state, 0);
   BcfWindow w;
   auto drain = [&]() { cudaStreamSynchronize(s); };
   for (int wi = 0;; wi++) {
@@ -518,25 +528,35 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     const size_t o_off = up(w.n_bytes), total = o_off + (size_t)n * 8;
     CK(h->bcf_buf.ensure(total + 16));   // (a reallocation waits for the device: cudaFree synchronises; k_vcf_decode reads past the end)
     char* d = h->bcf_buf.as<char>();
+    const int64_t* d_off = (const int64_t*)(d + o_off);
     if (tev[0]) CK(cudaEventRecord(tev[0], s));
-    CK(cudaMemcpyAsync(d, raw[b].p, w.n_bytes, cudaMemcpyHostToDevice, s));
+    // the bytes of the runs only, each at its window offset
+    for (const BcfRun& r : w.runs) {
+      const int64_t b0 = w.rec_off[r.first];
+      CK(cudaMemcpyAsync(d + b0, (const char*)raw[b].p + b0, (size_t)(r.end - b0), cudaMemcpyHostToDevice, s));
+    }
     CK(cudaMemcpyAsync(d + o_off, offs[b].p, (size_t)n * 8, cudaMemcpyHostToDevice, s));
     if (tev[0]) CK(cudaEventRecord(tev[1], s));
-    // the file's first record alone first: its GT length is the one every later record must have
-    for (int64_t k0 = 0; k0 < n;) {
-      const int64_t k1 = n_rec == 0 && k0 == 0 ? 1 : n;
-      if (rd.text)
-        k_vcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k0, k1, n, (const uint8_t*)d, (const int64_t*)(d + o_off), w.text_end, w.ustart,
-                                                                   rd.n_sample, h->bcf_cols.as<BcfCol>() + n_rec + k0, h->bcf_state.as<int32_t>(),
-                                                                   (unsigned long long*)(h->bcf_state.as<char>() + 8),
-                                                                   h->opt_vcf_paths ? (unsigned long long*)(h->bcf_state.as<char>() + 16) : nullptr);
-      else
-        k_bcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k1 - k0, (const uint8_t*)d, (const int64_t*)(d + o_off) + k0, w.ustart, gt_key,
-                                                                   h->bcf_cols.as<BcfCol>() + n_rec + k0, h->bcf_state.as<int32_t>(),
-                                                                   (unsigned long long*)(h->bcf_state.as<char>() + 8));
-      h->launches += 1;
-      CK(cudaGetLastError());
-      k0 = k1;
+    for (const BcfRun& r : w.runs) {
+      const int si = gr ? r.c : 0;
+      int32_t* nhap_state = (int32_t*)(h->bcf_state.as<char>() + (size_t)si * 16);
+      unsigned long long* err = (unsigned long long*)(h->bcf_state.as<char>() + (size_t)si * 16 + 8);
+      BcfCol* cols = h->bcf_cols.as<BcfCol>() + n_rec + r.first;
+      if (seen[si] == 0) first[si] = n_rec + r.first;
+      for (int64_t k0 = 0; k0 < r.n;) {
+        const int64_t k1 = seen[si] == 0 && k0 == 0 ? 1 : r.n;
+        if (rd.text)
+          k_vcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k0, k1, r.n, (const uint8_t*)d, d_off + r.first, r.end, w.ustart, rd.n_sample,
+                                                                     cols + k0, nhap_state, err,
+                                                                     h->opt_vcf_paths ? (unsigned long long*)paths : nullptr);
+        else
+          k_bcf_decode<<<grid_for((k1 - k0) * 32, 256), 256, 0, s>>>(k1 - k0, (const uint8_t*)d, d_off + r.first + k0, w.ustart, gt_key, cols + k0,
+                                                                     nhap_state, err);
+        h->launches += 1;
+        CK(cudaGetLastError());
+        k0 = k1;
+      }
+      seen[si] += r.n;
     }
     if (tev[0]) {
       CK(cudaEventRecord(tev[2], s));
@@ -552,38 +572,52 @@ int decode_file(colate_handle* h, const char* path, int64_t chunk_bytes, double*
     pending[b] = true;
   }
   CK(cudaStreamSynchronize(s));
-  if (n_rec == 0) return rd.err(std::string(rd.text ? "VCF" : "BCF") + " file without records (the reference reads a first record unconditionally)", 0, false);
-  struct { int32_t nhap, pad; unsigned long long err, paths[2]; } st;
-  CK(cudaMemcpy(&st, h->bcf_state.p, 32, cudaMemcpyDeviceToHost));
-  h->vcf_paths[0] = rd.text ? (int64_t)st.paths[0] : 0;
-  h->vcf_paths[1] = rd.text ? (int64_t)st.paths[1] : 0;
+  if (gr) {
+    if (int rc = rd.listed_complete()) return rc;
+  } else if (n_rec == 0) {
+    return rd.err(std::string(rd.text ? "VCF" : "BCF") + " file without records (the reference reads a first record unconditionally)", 0, false);
+  }
+  struct St { int32_t nhap, pad; unsigned long long err; };
+  std::vector<St> st((size_t)n_state + 1);
+  CK(cudaMemcpy(st.data(), h->bcf_state.p, (size_t)n_state * 16 + 16, cudaMemcpyDeviceToHost));
+  const unsigned long long* np = (const unsigned long long*)&st[n_state];
+  h->vcf_paths[0] = rd.text ? (int64_t)np[0] : 0;
+  h->vcf_paths[1] = rd.text ? (int64_t)np[1] : 0;
   t[0] += rd.index_s;
   t[1] += rd.inflate_s;
   t[2] += rd.walk_s;
   t[7] = rd.n_threads;
   t[8] += (double)n_inflated;
   t[9] += (double)n_rec;
-  if (st.err != ~0ull) {
-    static const char* what[] = {"", "BCF record without a GT field", "BCF record with a missing or vector-end genotype (or an allele index below 0)",
-                                 "BCF record whose GT length differs from the file's first record's", "BCF record whose typed fields run past its l_shared / l_indiv",
-                                 "BCF record whose GT is not an integer vector"};
-    static const char* what_vcf[] = {"", "VCF line without a GT value (no FORMAT column, no GT key in FORMAT, or a sample column that stops before GT)",
-                                     "VCF line with a missing allele ('.') in a GT", "VCF line whose samples x ploidy differs from the file's first line's",
-                                     "VCF line with fewer than 8 fixed fields", "VCF line with a GT that is not allele([/|]allele)* (allele: digits up to 2^29)",
-                                     "VCF line whose sample-column count differs from the header's",
-                                     "VCF line whose samples have different ploidies"};
-    return rd.err((rd.text ? what_vcf : what)[st.err & 7], st.err >> 3, false);
+  static const char* what[] = {"", "BCF record without a GT field", "BCF record with a missing or vector-end genotype (or an allele index below 0)",
+                               "BCF record whose GT length differs from the file's first record's", "BCF record whose typed fields run past its l_shared / l_indiv",
+                               "BCF record whose GT is not an integer vector"};
+  static const char* what_vcf[] = {"", "VCF line without a GT value (no FORMAT column, no GT key in FORMAT, or a sample column that stops before GT)",
+                                   "VCF line with a missing allele ('.') in a GT", "VCF line whose samples x ploidy differs from the file's first line's",
+                                   "VCF line with fewer than 8 fixed fields", "VCF line with a GT that is not allele([/|]allele)* (allele: digits up to 2^29)",
+                                   "VCF line whose sample-column count differs from the header's",
+                                   "VCF line whose samples have different ploidies"};
+  for (int si = 0; si < n_state; si++) {
+    if (st[si].err == ~0ull) continue;
+    const int rc = rd.err((rd.text ? what_vcf : what)[st[si].err & 7], st[si].err >> 3, false);
+    return gr ? fail(rc, std::string("chromosome ") + chr_names[si] + ": " + colate_last_error()) : rc;
   }
   h->bcf_n_rec = n_rec;
-  h->bcf_n_hap = st.nhap;
+  h->bcf_n_hap = st[0].nhap;
+  if (gr) {
+    gr->first = first;
+    gr->n = seen;
+    gr->n_hap.resize(n_chr);
+    for (int c = 0; c < n_chr; c++) gr->n_hap[c] = st[c].nhap;
+  }
   return 0;
 }
 
 // the row counts of the target slot t_slot and / or the reference slot r_slot (-1: that role is skipped) from one decode of every
-// chromosome's file.  Genome: host contigs (ref_seqs / ref_lens, uploaded per chromosome), the handle's resident genome
-// (resident), or none.
+// chromosome's file (bcf_paths), or of one whole-genome file (genome_path).  Genome: host contigs (ref_seqs / ref_lens, uploaded
+// per chromosome), the handle's resident genome (resident), or none.
 int rows_from_bcf(colate_handle* h, int t_slot, int r_slot, int n_chr, const char* const* chr_names, const char* const* bcf_paths,
-                  const uint8_t* const* ref_seqs, const int64_t* ref_lens, bool resident, int64_t chunk_bytes)
+                  const char* genome_path, const uint8_t* const* ref_seqs, const int64_t* ref_lens, bool resident, int64_t chunk_bytes)
 {
   CK(cudaSetDevice(h->device));
   const auto t_start = std::chrono::steady_clock::now();
@@ -599,8 +633,13 @@ int rows_from_bcf(colate_handle* h, int t_slot, int r_slot, int n_chr, const cha
   if (h->opt_bcf_timing)
     for (auto& e : tev) CK(cudaEventCreate(&e));
   struct TEv { cudaEvent_t* e; ~TEv() { for (int i = 0; i < 2; i++) if (e[i]) cudaEventDestroy(e[i]); } } tev_guard{tev};
+  GenomeRecs gr;
+  if (genome_path)
+    if (int rc = decode_file(h, genome_path, n_chr, chr_names, chunk_bytes, t, &gr)) return rc;
   for (int c = 0; c < n_chr; c++) {
-    if (int rc = decode_file(h, bcf_paths[c], chunk_bytes, t)) return fail(rc, std::string("chromosome ") + chr_names[c] + ": " + colate_last_error());
+    if (!genome_path)
+      if (int rc = decode_file(h, bcf_paths[c], 0, nullptr, chunk_bytes, t, nullptr))
+        return fail(rc, std::string("chromosome ") + chr_names[c] + ": " + colate_last_error());
     const uint8_t* ref = nullptr;
     int64_t L = 0;
     if (resident) {
@@ -615,9 +654,12 @@ int rows_from_bcf(colate_handle* h, int t_slot, int r_slot, int n_chr, const cha
     }
     const int64_t r0 = h->h_site_off[c], nr = h->h_site_off[c + 1] - r0;
     if (nr == 0) continue;
+    // a whole-genome file: chromosome c's records alone, so the lower bound stays inside them as in its own file
+    const BcfCol* cols = h->bcf_cols.as<BcfCol>() + (genome_path ? gr.first[c] : 0);
+    const int64_t n_c = genome_path ? gr.n[c] : h->bcf_n_rec;
+    const int32_t N = genome_path ? gr.n_hap[c] : h->bcf_n_hap;
     if (tev[0]) CK(cudaEventRecord(tev[0], s));
-    k_bcf_rows<<<grid_for(nr, 256), 256, 0, s>>>(r0, nr, h->pos.as<int32_t>(), h->meta.as<uint32_t>(), h->bcf_cols.as<BcfCol>(), h->bcf_n_rec,
-                                                 h->bcf_n_hap, ref, L, pile_t, pile_r);
+    k_bcf_rows<<<grid_for(nr, 256), 256, 0, s>>>(r0, nr, h->pos.as<int32_t>(), h->meta.as<uint32_t>(), cols, n_c, N, ref, L, pile_t, pile_r);
     h->launches += 1;
     CK(cudaGetLastError());
     if (tev[0]) {
@@ -649,7 +691,11 @@ int rows_from_bcf(colate_handle* h, int t_slot, int r_slot, int n_chr, const cha
 }  // namespace
 
 namespace colate {
-int decode_genotype_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t) { return decode_file(h, path, chunk_bytes, t); }
+int decode_genotype_file(colate_handle* h, const char* path, int64_t chunk_bytes, double* t) { return decode_file(h, path, 0, nullptr, chunk_bytes, t, nullptr); }
+int decode_genotype_genome(colate_handle* h, const char* path, int n_chr, const char* const* chr_names, int64_t chunk_bytes, double* t, GenomeRecs* gr)
+{
+  return decode_file(h, path, n_chr, chr_names, chunk_bytes, t, gr);
+}
 }
 
 extern "C" {
@@ -663,7 +709,7 @@ int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const 
   if (!h->sites_set || n_chr != h->n_chr) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf: one file per chromosome of the site set");
   for (int c = 0; c < n_chr; c++)
     if (!bcf_paths[c] || (ref_seqs && (ref_lens[c] < 0 || (ref_lens[c] > 0 && !ref_seqs[c])))) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf: bad arguments");
-  if (int rc = rows_from_bcf(h, role == 0 ? slot : -1, role == 1 ? slot : -1, n_chr, chr_names, bcf_paths, ref_seqs, ref_lens, false, chunk_bytes))
+  if (int rc = rows_from_bcf(h, role == 0 ? slot : -1, role == 1 ? slot : -1, n_chr, chr_names, bcf_paths, nullptr, ref_seqs, ref_lens, false, chunk_bytes))
     return rc;
   if (aaf_out || daf_out) {
     const size_t n_site = (size_t)h->n_site;
@@ -690,7 +736,44 @@ int colate_rows_from_bcf_roles(colate_handle* h, int target_slot, int reference_
     if (!bcf_paths[c]) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_roles: bad arguments");
   if (genome == 1 && (int)h->refg_off.size() != n_chr + 1)
     return fail(COLATE_ERR_STATE, "colate_rows_from_bcf_roles: genome = 1 needs colate_set_ref_genome with one contig per chromosome");
-  return rows_from_bcf(h, target_slot, reference_slot, n_chr, chr_names, bcf_paths, nullptr, nullptr, genome == 1, chunk_bytes);
+  return rows_from_bcf(h, target_slot, reference_slot, n_chr, chr_names, bcf_paths, nullptr, nullptr, nullptr, genome == 1, chunk_bytes);
+}
+
+int colate_rows_from_bcf_genome(colate_handle* h, int target_slot, int reference_slot, int n_chr, const char* const* chr_names, const char* path,
+                                int genome, int64_t chunk_bytes)
+{
+  if (!h || target_slot < -1 || target_slot >= COLATE_MAX_GENOMES || reference_slot < -1 || reference_slot >= COLATE_MAX_GENOMES ||
+      (target_slot < 0 && reference_slot < 0) || target_slot == reference_slot || (genome != 0 && genome != 1) || n_chr <= 0 || !chr_names ||
+      !path || chunk_bytes < 0)
+    return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_genome: bad arguments");
+  if (!h->sites_set || n_chr != h->n_chr) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_genome: one --chr entry per chromosome of the site set");
+  for (int c = 0; c < n_chr; c++)
+    if (!chr_names[c]) return fail(COLATE_ERR_ARG, "colate_rows_from_bcf_genome: bad arguments");
+  if (genome == 1 && (int)h->refg_off.size() != n_chr + 1)
+    return fail(COLATE_ERR_STATE, "colate_rows_from_bcf_genome: genome = 1 needs colate_set_ref_genome with one contig per chromosome");
+  return rows_from_bcf(h, target_slot, reference_slot, n_chr, chr_names, nullptr, path, nullptr, nullptr, genome == 1, chunk_bytes);
+}
+
+int colate_decode_bcf_genome(colate_handle* h, const char* path, int n_chr, const char* const* chr_names, int64_t chunk_bytes, int64_t* rec_first,
+                             int64_t* n_records, int32_t* n_hap)
+{
+  if (!h || !path || n_chr <= 0 || !chr_names || chunk_bytes < 0) return fail(COLATE_ERR_ARG, "colate_decode_bcf_genome: bad arguments");
+  for (int c = 0; c < n_chr; c++)
+    if (!chr_names[c]) return fail(COLATE_ERR_ARG, "colate_decode_bcf_genome: bad arguments");
+  CK(cudaSetDevice(h->device));
+  const auto t_start = std::chrono::steady_clock::now();
+  double t[10] = {};
+  h->bcf_n_rec = 0;
+  GenomeRecs gr;
+  if (int rc = decode_file(h, path, n_chr, chr_names, chunk_bytes, t, &gr)) return rc;
+  t[6] = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
+  memcpy(h->bcf_timing, t, sizeof t);
+  for (int c = 0; c < n_chr; c++) {
+    if (rec_first) rec_first[c] = gr.first[c];
+    if (n_records) n_records[c] = gr.n[c];
+    if (n_hap) n_hap[c] = gr.n_hap[c];
+  }
+  return 0;
 }
 
 int colate_decode_bcf(colate_handle* h, const char* bcf_path, int64_t chunk_bytes, int64_t* n_records, int32_t* n_hap)
@@ -700,7 +783,7 @@ int colate_decode_bcf(colate_handle* h, const char* bcf_path, int64_t chunk_byte
   const auto t_start = std::chrono::steady_clock::now();
   double t[10] = {};
   h->bcf_n_rec = 0;
-  if (int rc = decode_file(h, bcf_path, chunk_bytes, t)) return rc;
+  if (int rc = decode_file(h, bcf_path, 0, nullptr, chunk_bytes, t, nullptr)) return rc;
   t[6] = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
   memcpy(h->bcf_timing, t, sizeof t);
   if (n_records) *n_records = h->bcf_n_rec;

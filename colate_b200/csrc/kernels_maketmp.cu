@@ -300,6 +300,37 @@ struct Writer {
   }
 };
 
+// colate_maketmp_write_bcf (bcf_paths, one file per chromosome) and colate_maketmp_write_bcf_genome (genome_path, one file)
+int64_t write_bcf(colate_handle* h, const char* fn, int n_chr, const char* const* chr_names, const char* const* bcf_paths, const char* genome_path,
+                  const uint32_t* mask_bits, int64_t chunk_bytes, const char* out_file)
+{
+  const bool has_refg = !h->refg_off.empty();
+  if (has_refg && (int)h->refg_off.size() != n_chr + 1)
+    return fail(COLATE_ERR_STATE, std::string(fn) + ": the genome of colate_set_ref_genome has another number of chromosomes");
+  const auto t_start = std::chrono::steady_clock::now();
+  Writer w{h, fn};
+  if (int rc = w.begin(n_chr, chr_names, mask_bits)) return rc;
+  double t[10] = {};
+  GenomeRecs gr;
+  // a whole-genome file: every chromosome's records resident from one decode
+  if (genome_path)
+    if (int rc = decode_genotype_genome(h, genome_path, n_chr, chr_names, chunk_bytes, t, &gr)) return rc;
+  for (int c = 0; c < n_chr; c++) {
+    // per-chromosome files: decoded records are resident for one file at a time, each chromosome's written right after its decode
+    if (!genome_path)
+      if (int rc = decode_genotype_file(h, bcf_paths[c], chunk_bytes, t)) return fail(rc, "chromosome " + w.names[c] + ": " + colate_last_error());
+    const uint8_t* ref = has_refg ? h->refg.as<uint8_t>() + h->refg_off[c] : nullptr;
+    const int64_t ref_len = has_refg ? h->refg_off[c + 1] - h->refg_off[c] : 0;
+    const BcfCol* cols = h->bcf_cols.as<BcfCol>() + (genome_path ? gr.first[c] : 0);
+    if (int rc = w.chromosome<kRecords>(c, nullptr, cols, genome_path ? gr.n[c] : h->bcf_n_rec, genome_path ? gr.n_hap[c] : h->bcf_n_hap, ref, ref_len))
+      return rc;
+  }
+  t[5] = w.kernel_ms;
+  t[6] = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
+  memcpy(h->bcf_timing, t, sizeof t);
+  return w.finish(out_file, "allele sum above the number of haplotypes (the reference asserts, coal.cpp:2511)");
+}
+
 }  // namespace
 
 extern "C" {
@@ -348,24 +379,16 @@ int64_t colate_maketmp_write_bcf(colate_handle* h, int n_chr, const char* const*
   if (!h || !bcf_paths || chunk_bytes < 0 || !out_file) return fail(COLATE_ERR_ARG, "colate_maketmp_write_bcf: bad arguments");
   for (int c = 0; c < n_chr; c++)
     if (!bcf_paths[c]) return fail(COLATE_ERR_ARG, "colate_maketmp_write_bcf: bad arguments");
-  const bool has_refg = !h->refg_off.empty();
-  if (has_refg && (int)h->refg_off.size() != n_chr + 1)
-    return fail(COLATE_ERR_STATE, "colate_maketmp_write_bcf: the genome of colate_set_ref_genome has another number of chromosomes");
-  const auto t_start = std::chrono::steady_clock::now();
-  Writer w{h, "colate_maketmp_write_bcf"};
-  if (int rc = w.begin(n_chr, chr_names, mask_bits)) return rc;
-  double t[10] = {};
-  for (int c = 0; c < n_chr; c++) {
-    // decoded records are resident for one file at a time: each chromosome's records are written right after its decode
-    if (int rc = decode_genotype_file(h, bcf_paths[c], chunk_bytes, t)) return fail(rc, "chromosome " + w.names[c] + ": " + colate_last_error());
-    const uint8_t* ref = has_refg ? h->refg.as<uint8_t>() + h->refg_off[c] : nullptr;
-    const int64_t ref_len = has_refg ? h->refg_off[c + 1] - h->refg_off[c] : 0;
-    if (int rc = w.chromosome<kRecords>(c, nullptr, h->bcf_cols.as<BcfCol>(), h->bcf_n_rec, h->bcf_n_hap, ref, ref_len)) return rc;
-  }
-  t[5] = w.kernel_ms;
-  t[6] = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
-  memcpy(h->bcf_timing, t, sizeof t);
-  return w.finish(out_file, "allele sum above the number of haplotypes (the reference asserts, coal.cpp:2511)");
+  return write_bcf(h, "colate_maketmp_write_bcf", n_chr, chr_names, bcf_paths, nullptr, mask_bits, chunk_bytes, out_file);
+}
+
+int64_t colate_maketmp_write_bcf_genome(colate_handle* h, int n_chr, const char* const* chr_names, const char* path, const uint32_t* mask_bits,
+                                        int64_t chunk_bytes, const char* out_file)
+{
+  if (!h || !path || n_chr <= 0 || !chr_names || chunk_bytes < 0 || !out_file) return fail(COLATE_ERR_ARG, "colate_maketmp_write_bcf_genome: bad arguments");
+  for (int c = 0; c < n_chr; c++)
+    if (!chr_names[c]) return fail(COLATE_ERR_ARG, "colate_maketmp_write_bcf_genome: bad arguments");
+  return write_bcf(h, "colate_maketmp_write_bcf_genome", n_chr, chr_names, nullptr, path, mask_bits, chunk_bytes, out_file);
 }
 
 int colate_last_maketmp_timing(colate_handle* h, double* out4)

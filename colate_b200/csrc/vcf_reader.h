@@ -1,7 +1,7 @@
 // Bgzipped text VCF input on the host (VCF specification v4.3, section 1): the header (the ## lines and the #CHROM line) and
 // the walk over the record lines, which reads CHROM and POS only.  The device parses the rest of every line (k_vcf_decode,
 // kernels_bcf.cu).  htslib's bcf_open reads such a file wherever the reference opens <prefix>_chr<c>.bcf, so the same
-// per-chromosome rules as BCF apply: one contig per file, positions ascending.
+// rules as BCF apply: one contig per per-chromosome file, positions ascending; whole-genome files as GenotypeReader::set_listed.
 #pragma once
 #include <string>
 
@@ -20,10 +20,11 @@ class VcfReader : public GenotypeReader {
   // window's end starts the next window; the file's last line may lack its newline.
   int fill(uint8_t* buf, size_t target, BcfWindow& w) override;
   int gt_key = -1;       // dictionary index of GT, as BcfReader (only its presence matters here)
-  std::string chrom;     // CHROM of the records
+  std::string chrom;     // CHROM of the records (a whole-genome file: of the previous record)
 
  private:
-  int line(const uint8_t* buf, size_t o, size_t e, BcfWindow& w);
+  int line(const uint8_t* buf, size_t o, size_t e, size_t next, BcfWindow& w);
+  bool walking_ = false;
 };
 
 }  // namespace colate

@@ -486,9 +486,10 @@ def bcf_typed_str(s) -> bytes:
 BCF_FLAG = b"\x00"      # an INFO flag: type 0, size 0
 
 
-def bcf_header(n_sample, ids=(("FORMAT", "GT"),), idx=None, contigs=("1",), minor=2, extra=b"") -> bytes:
+def bcf_header(n_sample, ids=(("FORMAT", "GT"),), idx=None, contigs=("1",), minor=2, extra=b"", contig_idx=None) -> bytes:
     """Magic, l_text and header text.  ids: (kind, ID) pairs (FILTER / INFO / FORMAT) in order of appearance; PASS is implicit.
-    idx: None (no IDX=, as a hand-written header) or {ID: number} (IDX= on every line, as bcftools writes; PASS gets 0)."""
+    idx: None (no IDX=, as a hand-written header) or {ID: number} (IDX= on every line, as bcftools writes; PASS gets 0).
+    contig_idx: None or {contig: number}, the IDX= of the ##contig lines (which then need not follow their order)."""
     import struct
     lines = [b"##fileformat=VCFv4.3"]
     ix = (lambda i: b",IDX=%d" % idx[i]) if idx is not None else (lambda i: b"")
@@ -497,7 +498,8 @@ def bcf_header(n_sample, ids=(("FORMAT", "GT"),), idx=None, contigs=("1",), mino
         typ = b"String" if i == "GT" else b"Integer"
         lines.append(b'##%s=<ID=%s,Number=1,Type=%s,Description="a \\"quoted\\", IDX=99 text"%s>' % (kind.encode(), i.encode(), typ, ix(i)))
     for k, c in enumerate(contigs):
-        lines.append(b"##contig=<ID=%s,length=1000000000%s>" % (c.encode(), b",IDX=%d" % k if idx is not None else b""))
+        k = contig_idx[c] if contig_idx is not None else k
+        lines.append(b"##contig=<ID=%s,length=1000000000%s>" % (c.encode(), b",IDX=%d" % k if idx is not None or contig_idx is not None else b""))
     lines.append(bytes(extra) if extra else b"##source=colate_b200.synth")
     cols = b"#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO"
     if n_sample:

@@ -181,13 +181,27 @@ int colate_rows_from_bcf(colate_handle* h, int slot, int role, int n_chr, const 
  * without one). */
 int colate_rows_from_bcf_roles(colate_handle* h, int target_slot, int reference_slot, int n_chr, const char* const* chr_names,
                                const char* const* bcf_paths, int genome, int64_t chunk_bytes);
+/* A whole-genome BCF or bgzipped text VCF file (DESIGN.md section 6k): --chr entry c (chr_names[c], one per chromosome of the site
+ * set) reads the records of the contig named c or chr<c> (BCF: CHROM indexes the header's ##contig lines, IDX= honoured; VCF: the
+ * CHROM text), which are exactly the records of that chromosome's own file.  The file is decoded once; the listed contigs' records
+ * stay resident, each contig with its own GT length, and every chromosome's rows are resolved against its contig's records alone.
+ * The result is colate_rows_from_bcf_roles' on the per-chromosome files, bit for bit; roles, slots and genome as there.  Refused as
+ * there, errors on the device prefixed "chromosome <c>: ", and on the host: a listed contig whose records are not one contiguous run
+ * (COLATE_ERR_ORDER), a listed contig without records, a contig matching two entries, an entry matched by two contigs with records,
+ * a BCF record whose CHROM no ##contig line defines.  Records of other contigs are inflated and walked past unchecked. */
+int colate_rows_from_bcf_genome(colate_handle* h, int target_slot, int reference_slot, int n_chr, const char* const* chr_names, const char* path,
+                                int genome, int64_t chunk_bytes);
 /* Decode only: one BCF or bgzipped text VCF file's records reduced on the device as colate_rows_from_bcf does (same checks), kept on the device;
  * colate_bcf_records copies records [r0, r0 + n) out in the arrays colate_maketmp_records takes (position 1-based, allele codes,
  * allele sum, biallelic flag).  *n_hap = samples x GT length. */
 int colate_decode_bcf(colate_handle* h, const char* bcf_path, int64_t chunk_bytes, int64_t* n_records, int32_t* n_hap);
 int colate_bcf_records(colate_handle* h, int64_t r0, int64_t n, int32_t* rec_pos, uint8_t* rec_a0, uint8_t* rec_a1, int32_t* rec_alt_sum,
                        uint8_t* rec_biallelic);
-/* Phases of the last colate_rows_from_bcf / colate_decode_bcf, summed over its files: [0] BGZF index s, [1] inflate s, [2] record
+/* Decode only, a whole-genome file (as colate_rows_from_bcf_genome): --chr entry c's records are colate_bcf_records [rec_first[c],
+ * rec_first[c] + n_records[c]), of n_hap[c] haplotypes. */
+int colate_decode_bcf_genome(colate_handle* h, const char* path, int n_chr, const char* const* chr_names, int64_t chunk_bytes, int64_t* rec_first,
+                             int64_t* n_records, int32_t* n_hap);
+/* Phases of the last colate_rows_from_bcf / colate_decode_bcf (and their whole-genome twins), summed over its files: [0] BGZF index s, [1] inflate s, [2] record
  * walk s, [3] host-to-device copies ms, [4] k_bcf_decode ms, [5] k_bcf_rows ms ([3]-[5] only with colate_set_option(h, "bcf_timing",
  * 1)), [6] whole call s, [7] inflate threads, [8] inflated bytes, [9] records. */
 int colate_last_bcf_timing(colate_handle* h, double* out10);
@@ -227,6 +241,9 @@ int64_t colate_maketmp_write_pileup(colate_handle* h, int slot, int n_chr, const
                                     const char* out_file);
 int64_t colate_maketmp_write_bcf(colate_handle* h, int n_chr, const char* const* chr_names, const char* const* bcf_paths, const uint32_t* mask_bits,
                                  int64_t chunk_bytes, const char* out_file);
+/*   _bcf_genome: one whole-genome BCF or bgzipped VCF (as colate_rows_from_bcf_genome), decoded once, then written as _bcf. */
+int64_t colate_maketmp_write_bcf_genome(colate_handle* h, int n_chr, const char* const* chr_names, const char* path, const uint32_t* mask_bits,
+                                        int64_t chunk_bytes, const char* out_file);
 /* The last writer call: [0] writer kernels ms (CUDA events), [1] device-to-host copy ms, [2] file write s, [3] records. */
 int colate_last_maketmp_timing(colate_handle* h, double* out4);
 /* Work done on this handle since creation: [0] .mut texts parsed on the device, [1] .mut rows parsed (colate_ingest_end), [2] calls of
@@ -430,6 +447,10 @@ int colate_bcf_scan(const char* path, int64_t window_bytes, int64_t* n_records, 
  * on such a file.  A BCF file is refused (colate_bcf_scan reads it).  0 or a negative status. */
 int colate_vcf_scan(const char* path, int64_t window_bytes, int64_t* n_records, int32_t* first_pos, int32_t* last_pos, int32_t* n_sample,
                     char* chrom, int64_t chrom_cap);
+/* Whole-genome BCF or bgzipped text VCF file, host only (no GPU): per --chr entry the records of its contig, their first and last POS
+ * (0-based), and the header's sample count, with every host check of colate_rows_from_bcf_genome.  0 or a negative status. */
+int colate_bcf_genome_scan(const char* path, int n_chr, const char* const* chr_names, int64_t window_bytes, int64_t* n_records, int32_t* first_pos,
+                           int32_t* last_pos, int32_t* n_sample);
 /* fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz.  *seq_out: malloc'd,
  * release with colate_free.  Returns the length or < 0. */
 int64_t colate_read_fasta(const char* path, uint8_t** seq_out);
