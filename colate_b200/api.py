@@ -15,6 +15,8 @@ import numpy as np
 from . import _lib
 from ._lib import MAX_BLOCKS, MT_WORDS, NBINS, check, lib, ptr
 
+SAMPLE_TILE_WORDS = 32 * 200    # generator words of one tile of 32 used rows (internal.h)
+
 
 def libm_exact() -> bool:
     """True if the host libm matches the device exp/log/log1p bit for bit (glibc 2.39, FMA variants)."""
@@ -707,6 +709,30 @@ class Handle:
         check(lib().colate_test_mt_stream(self._h, np.ascontiguousarray(mt_state, dtype=np.uint32), word0, n_words,
                                           log2_chunk_sites, out))
         return out[:n_words], out[n_words:]
+
+    def mt_stream_tiled(self, mt_state, word0, n_words, log2_chunk_sites, p0=0, n_phys=None):
+        """Test hook: engine words [word0, word0+n) in k_sample's tile order, as stage i lays them out -> (physical words
+        [p0, p0 + n_phys) of the stream buffer, window after).  Word 0 of the buffer is the first word of the chunk that holds
+        word0 and tiling starts at off = word0 % (200 << log2_chunk_sites) (colate_test_stream_phys).  n_phys=None: up to one
+        tile past the stream's end.  Without the stream cache, words no kernel wrote read 0xA5A5A5A5."""
+        S = 200 << log2_chunk_sites
+        if n_phys is None:
+            n_phys = max(word0 + n_words - word0 // S * S, 4) + SAMPLE_TILE_WORDS - p0
+        out = np.zeros(n_phys, dtype=np.uint32)
+        after = np.zeros(MT_WORDS, dtype=np.uint32)
+        check(lib().colate_test_mt_stream_tiled(self._h, np.ascontiguousarray(mt_state, dtype=np.uint32), word0, n_words,
+                                                log2_chunk_sites, p0, n_phys, ptr(out), ptr(after)))
+        return out, after
+
+    GEN_KERNELS = ("linear", "tiled_w32", "tiled_w64", "pre_w32", "pre_w64", "tma")
+
+    def last_gen(self):
+        """Test hook: the generator kernel of the last stream generation (internal.h: GEN_*): "linear" (k_gen<false>),
+        "tiled_w32" / "tiled_w64" (k_gen<true, false, W32>), "pre_w32" / "pre_w64" (k_gen<true, true, W32>), "tma"
+        (k_gen_tma), or None."""
+        k = C.c_int(0)
+        check(lib().colate_test_last_gen(self._h, C.byref(k)))
+        return self.GEN_KERNELS[k.value] if k.value >= 0 else None
 
     # ---- convenience: load a synth.Sites / synth.Genome pair
     def load(self, sites, target, reference, tmask=None, rmask=None):

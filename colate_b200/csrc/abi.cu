@@ -584,6 +584,15 @@ int colate_set_option(colate_handle* h, const char* key, int64_t value)
   if (!strcmp(key, "bcf_timing")) { h->opt_bcf_timing = value != 0; return 0; }
   // vcf_paths = 1 (test hook): k_vcf_decode counts the lines it decodes on its fast and general paths (colate_test_last_vcf_paths)
   if (!strcmp(key, "vcf_paths")) { h->opt_vcf_paths = value != 0; return 0; }
+  // gen_path: the tile-ordered generator kernel.  0 = k_gen_tma where it applies unless COLATE_GEN_NO_TMA is set, 1 = k_gen
+  // always, 2 = k_gen_tma where it applies (chunks of >= 4 rows, stream starting on a chunk boundary) whatever the variable says
+  if (!strcmp(key, "gen_path")) {
+    if (value < 0 || value > 2) return fail(COLATE_ERR_ARG, "gen_path: 0 (auto), 1 (k_gen) or 2 (TMA where it applies)");
+    h->opt_gen_path = (int)value;
+    return 0;
+  }
+  // gen_w64 = 1 (test hook): k_gen addresses the stream with 64-bit offsets at any size, not only past 2^31 words
+  if (!strcmp(key, "gen_w64")) { h->opt_gen_w64 = value != 0; return 0; }
   // front_end: which of mut()'s input branches the handle reproduces (coal.cpp:3175-3319).  0 = tmp/tmp (parse_tmptmp: pseudo-
   // genotype weights, no normalisation).  1 = the bcf / bam front-ends fed from pre-decoded per-row counts (SURVEY.md 8f N3):
   // raw count weights (coal.cpp:2005-2039, 1164-1197) and both count vectors of stage ii divided by 1e3 (coal.cpp:3453-3463).
@@ -906,6 +915,42 @@ int colate_test_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t wo
   if (rc) return rc;
   if (n_words > 0) CK(cudaMemcpyAsync(out, p, (size_t)n_words * 4, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+// test hook: engine words [word0, word0+n) laid out in k_sample's tile order as stage i lays them out; physical words
+// [p0, p0 + n_phys) of the stream buffer (word 0 = the first word of the chunk that holds word0; internal.h: stream_phys with
+// off = word0 mod 200 * 2^k) to out_phys, the state window after the last word to out_after (may be NULL).  Without the stream
+// cache the buffer is first filled with the canary word 0xA5A5A5A5 up to one tile past the stream's end, so that stray stores
+// show; with it the buffer holds the cached stream and is left alone.
+int colate_test_mt_stream_tiled(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words, int log2_chunk_sites,
+                                int64_t p0, int64_t n_phys, uint32_t* out_phys, uint32_t* out_after)
+{
+  if (!h || !mt_state || word0 < 0 || n_words < 0 || log2_chunk_sites < 0 || log2_chunk_sites > 40 || p0 < 0 || n_phys < 0 ||
+      (n_phys > 0 && !out_phys))
+    return fail(COLATE_ERR_ARG, "colate_test_mt_stream_tiled: bad arguments");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  if (!h->stream_cache_on) {
+    const int64_t S = (int64_t)200 << log2_chunk_sites, total_local = word0 + n_words - word0 / S * S;
+    const size_t words = (size_t)std::max<int64_t>(total_local, 4) + SAMPLE_TILE_WORDS;   // run_mt_stream's tiled buffer
+    CK(h->rng_stream.ensure(words * 4 + 64));
+    CK(cudaMemsetAsync(h->rng_stream.p, 0xA5, words * 4, s));
+  }
+  uint32_t* p = nullptr;
+  int rc = run_mt_stream(h, mt_state, word0, n_words, log2_chunk_sites, &p, out_after, true);
+  if (rc) return rc;
+  if (p0 + n_phys > (int64_t)(h->rng_stream.cap / 4)) return fail(COLATE_ERR_ARG, "colate_test_mt_stream_tiled: range past the stream buffer");
+  if (n_phys > 0) CK(cudaMemcpyAsync(out_phys, h->rng_stream.as<uint32_t>() + p0, (size_t)n_phys * 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// test hook: the generator kernel of the handle's last run_mt_stream launch (internal.h: GEN_*; -1 none yet)
+int colate_test_last_gen(colate_handle* h, int* kernel)
+{
+  if (!h || !kernel) return fail(COLATE_ERR_ARG, "colate_test_last_gen: bad arguments");
+  *kernel = h->gen_kernel;
   return 0;
 }
 

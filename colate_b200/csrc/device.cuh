@@ -121,6 +121,10 @@ struct colate_handle {
   int64_t n_used = 0;
   int n_blocks_local = 0;
   int64_t mt_total_local = 0;
+  // generator kernel choice (colate_set_option gen_path / gen_w64) and the last one launched (colate_test_last_gen)
+  int opt_gen_path = 0;
+  bool opt_gen_w64 = false;
+  int gen_kernel = -1;
   // generator-stream cache (colate_set_stream_cache): state, offset and length of the tile-ordered stream in rng_stream
   bool stream_cache_on = false, sc_valid = false, mt_tail_gather = false;
   uint32_t sc_state[624] = {};

@@ -49,6 +49,8 @@ inline int64_t stream_phys(int64_t o, int64_t off)
   const uint32_t w = (uint32_t)(q - row * 200u), c = w / SAMPLE_CHUNK_WORDS, ww = w - c * SAMPLE_CHUNK_WORDS;
   return off + (int64_t)((((row >> 5) * (200 / SAMPLE_CHUNK_WORDS) + c) * 32 + (row & 31)) * SAMPLE_CHUNK_WORDS + ww);
 }
+// the generator kernels (kernels_mt.cu), as colate_test_last_gen reports the last one launched: k_gen<TILED, PRE, W32>, k_gen_tma
+constexpr int GEN_LINEAR = 0, GEN_TILED_W32 = 1, GEN_TILED_W64 = 2, GEN_PRE_W32 = 3, GEN_PRE_W64 = 4, GEN_TMA = 5;
 
 // error plumbing (thread-local message behind colate_last_error())
 void set_error(const std::string& msg);
@@ -106,4 +108,7 @@ int colate_test_bin_fast(colate_handle* h, int n, const double* ages, int32_t* f
 int colate_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, uint64_t* out3);
 int colate_test_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words,
                           int log2_chunk_sites, uint32_t* out);
+int colate_test_mt_stream_tiled(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words, int log2_chunk_sites,
+                                int64_t p0, int64_t n_phys, uint32_t* out_phys, uint32_t* out_after);
+int colate_test_last_gen(colate_handle* h, int* kernel);
 }

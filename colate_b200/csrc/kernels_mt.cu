@@ -259,7 +259,7 @@ k_gen(const uint32_t* __restrict__ windows, int64_t chunk_words, int64_t total_w
 // finished group of 4 rows (cp.async.bulk.tensor.4d shared -> global, under the next round's recurrence); the ring holds 5
 // groups and the copy warp lets only the two latest rounds' stores be in flight before it joins the next barrier.
 // (Measured before this: one plain bulk copy per 80-byte piece, 33 per round -- 2.0 ms, the copy engine pays per operation.)
-// Chunks are whole multiples of 4 rows (2^k rows, k >= 3); the very last group of the stream may carry up to 3 rows of
+// Chunks are whole multiples of 4 rows (2^k rows, k >= 2); the very last group of the stream may carry up to 3 rows of
 // whatever the ring held beyond the last word: they land inside the last tile, which the buffer always holds whole and
 // whose rows past n_used k_sample does not count.
 constexpr int GEN_GROUP_WORDS = 800;                 // 4 rows
@@ -484,20 +484,25 @@ int run_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t word0, int
   }
   if (total_local > 0) {
     if (tiled && off % 200 != 0) return fail(COLATE_ERR_ARG, "tiled generator stream must start at a row boundary");
-    const bool w32 = total_local + SAMPLE_TILE_WORDS < ((int64_t)1 << 31);
+    // gen_w64 / gen_path (colate_set_option): 64-bit addressing at any size; k_gen only, or TMA wherever it applies
+    // whatever COLATE_GEN_NO_TMA says (the variable is read once per process, the options per handle)
+    const bool w32 = !h->opt_gen_w64 && total_local + SAMPLE_TILE_WORDS < ((int64_t)1 << 31);
     uint32_t* win = h->windows.as<uint32_t>();
     uint32_t* st = h->rng_stream.as<uint32_t>();
     uint32_t* tl = h->mt_tail.as<uint32_t>();
-    if (!tiled) k_gen<false, false, false><<<M, 256, 0, s>>>(win, S, total_local, st, 0, tl);
+    if (!tiled) { k_gen<false, false, false><<<M, 256, 0, s>>>(win, S, total_local, st, 0, tl); h->gen_kernel = GEN_LINEAR; }
     else if (off == 0) {
       CUtensorMap tm;
-      static const bool no_tma = getenv("COLATE_GEN_NO_TMA") != nullptr;
-      if (k >= 2 && !no_tma && encode_stream_map(st, total_local, &tm)) k_gen_tma<<<M, 288, 0, s>>>(win, S, total_local, tm, tl);
-      else if (w32) k_gen<true, false, true><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl);
-      else k_gen<true, false, false><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl);
+      static const bool no_tma_env = getenv("COLATE_GEN_NO_TMA") != nullptr;
+      const bool no_tma = h->opt_gen_path == 1 || (h->opt_gen_path == 0 && no_tma_env);
+      if (k >= 2 && !no_tma && encode_stream_map(st, total_local, &tm)) {
+        k_gen_tma<<<M, 288, 0, s>>>(win, S, total_local, tm, tl);
+        h->gen_kernel = GEN_TMA;
+      } else if (w32) { k_gen<true, false, true><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl); h->gen_kernel = GEN_TILED_W32; }
+      else { k_gen<true, false, false><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl); h->gen_kernel = GEN_TILED_W64; }
     }
-    else if (w32) k_gen<true, true, true><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl);
-    else k_gen<true, true, false><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl);
+    else if (w32) { k_gen<true, true, true><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl); h->gen_kernel = GEN_PRE_W32; }
+    else { k_gen<true, true, false><<<M, 256, 0, s>>>(win, S, total_local, st, off, tl); h->gen_kernel = GEN_PRE_W64; }
     h->launches += 1;
     CK(cudaGetLastError());
   }
