@@ -141,6 +141,8 @@ TEST_HOOKS = {
     "colate_test_last_vcf_paths": (C.c_int, [VP, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "colate_test_bin_fast": (C.c_int, [VP, C.c_int, f64, i32, i32]),
     "colate_test_bin_sweep": (C.c_int, [VP, C.c_uint32, C.c_uint32, _p(dtype=np.uint64, flags="C_CONTIGUOUS")]),
+    "colate_test_replay": (C.c_int, [VP, C.c_int, i64, C.c_int64, VP, VP, VP, VP, VP, VP, VP, f64, i64, C.POINTER(C.c_int)]),
+    "colate_test_replay_row": (C.c_int, [VP, C.c_int, C.c_int, f64, f64, i32, f64]),
     "colate_test_mt_stream": (C.c_int, [VP, u32, C.c_int64, C.c_int64, C.c_int, u32]),
     "colate_test_mt_stream_tiled": (C.c_int, [VP, u32, C.c_int64, C.c_int64, C.c_int, C.c_int64, C.c_int64, VP, VP]),
     "colate_test_last_gen": (C.c_int, [VP, C.POINTER(C.c_int)]),

@@ -703,6 +703,34 @@ class Handle:
         check(lib().colate_test_bin_sweep(self._h, lo_bits, hi_bits, out))
         return int(out[0]), int(out[1]), int(out[2]) * 1e-9
 
+    def test_replay(self, blk_rank_start, counts, age_begin, w_shared, w_notshared, emp_bin, emp_ws, emp_wn):
+        """Test hook: k_emp and k_replay, launched as stage i launches them, on rows given directly -> (out_f [nb][4][185],
+        out_n [nb][3][185], out_of_range).  counts[n_rows][192] uint8 per count slot; age_begin <= 0: the row adds nothing to
+        shared; emp_bin 255: no emp contribution; block b holds rows [blk_rank_start[b], blk_rank_start[b + 1])."""
+        brs = np.ascontiguousarray(blk_rank_start, dtype=np.int64)
+        nb = brs.shape[0] - 1
+        cnt = np.ascontiguousarray(counts, dtype=np.uint8)
+        n = cnt.shape[0]
+        assert cnt.shape == (n, 192)
+        f = [np.ascontiguousarray(x, dtype=np.float64) for x in (age_begin, w_shared, w_notshared, emp_ws, emp_wn)]
+        eb = np.ascontiguousarray(emp_bin, dtype=np.uint8)
+        assert all(x.shape == (n,) for x in f + [eb])
+        out_f = np.zeros((max(nb, 0), 4, NBINS)); out_n = np.zeros((max(nb, 0), 3, NBINS), dtype=np.int64)
+        oor = C.c_int(0)
+        check(lib().colate_test_replay(self._h, nb, brs, n, ptr(cnt), ptr(f[0]), ptr(f[1]), ptr(f[2]), ptr(eb), ptr(f[3]), ptr(f[4]),
+                                       out_f, out_n, C.byref(oor)))
+        return out_f, out_n, bool(oor.value)
+
+    def test_replay_row(self, which: str, acc, w, c):
+        """Test hook: the device's replay_row ("replay_row") or exsum::add_repeated ("add_repeated") element by element."""
+        a = np.ascontiguousarray(acc, dtype=np.float64)
+        ww = np.ascontiguousarray(w, dtype=np.float64)
+        cc = np.ascontiguousarray(c, dtype=np.int32)
+        assert a.shape == ww.shape == cc.shape
+        out = np.zeros_like(a)
+        check(lib().colate_test_replay_row(self._h, ("replay_row", "add_repeated").index(which), a.shape[0], a, ww, cc, out))
+        return out
+
     def mt_stream(self, mt_state, word0, n_words, log2_chunk_sites=3):
         """Test hook: engine words [word0, word0+n) generated by the device path (+ window after)."""
         out = np.zeros(n_words + MT_WORDS, dtype=np.uint32)

@@ -904,6 +904,33 @@ int colate_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, 
   return run_test_bin_sweep(h, lo_bits, hi_bits, out3);
 }
 
+// test hooks of the exact replay: k_emp and k_replay (the launches of stage i) on rows given as counts[n_rows][192], age_begin
+// (<= 0: the row adds nothing to shared), the two weights and the emp contribution (bin 255: none), blocks
+// [blk_rank_start[b], blk_rank_start[b + 1]) -> out_f[n_blocks][4][185], out_n[n_blocks][3][185] and the bin-185 flag; and the
+// device's replay_row (which = 0) / exsum::add_repeated (which = 1) element by element
+int colate_test_replay(colate_handle* h, int n_blocks, const int64_t* blk_rank_start, int64_t n_rows, const uint8_t* counts,
+                       const double* age_begin, const double* w_shared, const double* w_notshared, const uint8_t* emp_bin,
+                       const double* emp_ws, const double* emp_wn, double* out_f, int64_t* out_n, int* out_of_range)
+{
+  if (!h || n_blocks < 0 || n_blocks > MAX_BLOCKS || n_rows < 0 || !blk_rank_start || !out_f || !out_n || !out_of_range ||
+      (n_rows > 0 && (!counts || !age_begin || !w_shared || !w_notshared || !emp_bin || !emp_ws || !emp_wn)))
+    return fail(COLATE_ERR_ARG, "colate_test_replay: bad arguments");
+  for (int b = 0; b < n_blocks; b++)
+    if (blk_rank_start[b] < 0 || blk_rank_start[b] > blk_rank_start[b + 1] || blk_rank_start[b + 1] > n_rows)
+      return fail(COLATE_ERR_ARG, "colate_test_replay: block ranges must ascend inside [0, n_rows]");
+  CK(cudaSetDevice(h->device));
+  return run_test_replay(h, n_blocks, blk_rank_start, n_rows, counts, age_begin, w_shared, w_notshared, emp_bin, emp_ws, emp_wn, out_f,
+                         out_n, out_of_range);
+}
+int colate_test_replay_row(colate_handle* h, int which, int n, const double* acc, const double* w, const int32_t* c, double* out)
+{
+  if (!h || which < 0 || which > 1 || n <= 0 || !acc || !w || !c || !out) return fail(COLATE_ERR_ARG, "colate_test_replay_row: bad arguments");
+  for (int i = 0; i < n; i++)
+    if (c[i] < 0) return fail(COLATE_ERR_ARG, "colate_test_replay_row: negative count");
+  CK(cudaSetDevice(h->device));
+  return run_test_replay_row(h, which, n, acc, w, c, out);
+}
+
 // test hook: raw engine words [word0, word0+n) of the stream behind `mt_state`, via the device path
 int colate_test_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words, int log2_chunk_sites,
                           uint32_t* out)

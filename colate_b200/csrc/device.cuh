@@ -210,6 +210,10 @@ int run_pileup_reads(colate_handle* h, int slot, int chr, int64_t n_reads, const
                      int mapq_th, int len_th, int mismatch_th, uint8_t* pass_scratch, bool starts_contig, int64_t row_lo, int64_t row_hi);
 int run_test_bin_fast(colate_handle* h, int n, const double* a_host, int32_t* fast_host, int32_t* exact_host);
 int run_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, uint64_t* out3_host);
+int run_test_replay(colate_handle* h, int n_blocks, const int64_t* blk_rank_start, int64_t n_rows, const uint8_t* counts,
+                    const double* age_begin, const double* w_shared, const double* w_notshared, const uint8_t* emp_bin,
+                    const double* emp_ws, const double* emp_wn, double* out_f, int64_t* out_n, int* out_of_range);
+int run_test_replay_row(colate_handle* h, int which, int n, const double* acc, const double* w, const int32_t* c, double* out);
 // kernels_mt.cu
 int run_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words, int log2_chunk_sites,
                   uint32_t** stream_at_word0, uint32_t* window_after /* host, may be null */,

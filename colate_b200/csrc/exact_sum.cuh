@@ -9,7 +9,8 @@
 // (so that d and the rounding error are exact) and the sum is not a tie.  The steps that fit
 // below the next power of two are taken at once, the step across it is a single rounded
 // addition, and the rest continues in the new binade.  Validated against the plain loop by
-// tests/test_host.py (host, colate_test_add_repeated) and the stage-i parity tests (device).
+// tests/test_host.py (host, colate_test_add_repeated) and tests/test_gpu_replay.py (device,
+// colate_test_replay_row).
 #pragma once
 #include <cstdint>
 #include <cstring>

@@ -106,6 +106,10 @@ int colate_test_em_prims(colate_handle* h, int which, int n, const double* a, co
 int colate_test_last_em(colate_handle* h, int* kernel, int* csize);
 int colate_test_bin_fast(colate_handle* h, int n, const double* ages, int32_t* fast, int32_t* exact);
 int colate_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, uint64_t* out3);
+int colate_test_replay(colate_handle* h, int n_blocks, const int64_t* blk_rank_start, int64_t n_rows, const uint8_t* counts,
+                       const double* age_begin, const double* w_shared, const double* w_notshared, const uint8_t* emp_bin,
+                       const double* emp_ws, const double* emp_wn, double* out_f, int64_t* out_n, int* out_of_range);
+int colate_test_replay_row(colate_handle* h, int which, int n, const double* acc, const double* w, const int32_t* c, double* out);
 int colate_test_mt_stream(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words,
                           int log2_chunk_sites, uint32_t* out);
 int colate_test_mt_stream_tiled(colate_handle* h, const uint32_t* mt_state, int64_t word0, int64_t n_words, int log2_chunk_sites,

@@ -467,7 +467,8 @@ __global__ void k_chr(int n_chr, const int64_t* __restrict__ site_off, const int
 }
 
 // used rows -> dense records in rank order:
-//   hdr[r]  = {(age_end - age_begin) * 2^-64, age_begin, weight into shared (-0.0: none), weight into notshared} (fp64 x4)
+//   hdr[r]  = {(age_end - age_begin) * 2^-64, age_begin, weight into shared, weight into notshared} (fp64 x4); rows with
+//             age_begin <= 0 add nothing to shared (k_replay tests .y, not the weight: raw count weights may be negative)
 //   e_b2/e_ws/e_wn[r] = bin and weights of the row's single "emp" contribution (255 = none)
 //   u_blk[r] = genomic block (index local to this handle)
 __global__ void k_compact(int64_t n_site, int n_chr, const int64_t* __restrict__ site_off, const int32_t* __restrict__ pos,
@@ -501,15 +502,16 @@ __global__ void k_compact(int64_t n_site, int n_chr, const int64_t* __restrict__
   const double abd = (double)b;
   // float * int -> float, then / double (coal.cpp:2255-2256, 2269, 2291-2292)
   // raw_weights (the bcf / bam front-ends, SURVEY.md 8f N3): the counts themselves, int * int -> double
-  // (coal.cpp:2005-2006, 2019, 2038-2039; 1164-1165, 1179, 1196-1197 with AAF_target = N_target - DAF_target)
-  const double num_s = raw_weights ? (double)(dt * dafr) : (double)__fmul_rn(fd, __int2float_rn(dafr));
-  const double num_n = raw_weights ? (double)(at * dafr) : (double)__fmul_rn(fa, __int2float_rn(dafr));
+  // (coal.cpp:2005-2006, 2019, 2038-2039; 1164-1165, 1179, 1196-1197 with AAF_target = N_target - DAF_target).  The
+  // reference multiplies in int: a product past 2^31 (depths above ~46 k on both sides) wraps to a negative weight, and the
+  // reference adds that.  The wrap is spelled out in unsigned arithmetic here (signed overflow is undefined in C++).
+  const double num_s = raw_weights ? (double)(int32_t)((uint32_t)dt * (uint32_t)dafr) : (double)__fmul_rn(fd, __int2float_rn(dafr));
+  const double num_n = raw_weights ? (double)(int32_t)((uint32_t)at * (uint32_t)dafr) : (double)__fmul_rn(fa, __int2float_rn(dafr));
   const double den = __dmul_rn((double)nr, 100.0);
   // .x = (age_end - age_begin) * 2^-64: the sampling kernel multiplies it with the 64-bit integer
   // x2:x1 converted once (exact power-of-two scaling, same rounding as U * (age_end - age_begin))
-  // .z is -0.0 for rows with age_begin <= 0: they add nothing to the shared histogram (coal.cpp:2259)
-  hdr[r] = make_double4(__dmul_rn(__dsub_rn((double)e, abd), 0x1p-64), abd, abd > 0.0 ? __ddiv_rn(num_s, den) : -0.0,
-                        __ddiv_rn(num_n, den));
+  // .y = age_begin: rows with .y <= 0 add nothing to the shared histogram (coal.cpp:2259)
+  hdr[r] = make_double4(__dmul_rn(__dsub_rn((double)e, abd), 0x1p-64), abd, __ddiv_rn(num_s, den), __ddiv_rn(num_n, den));
   uint8_t b2 = 255;
   double ws = 0.0, wn = 0.0;
   if (abd <= 0.0) {  // coal.cpp:2247-2256 with age == 0
@@ -892,7 +894,8 @@ struct __align__(16) ReplayStage {
   double4 hdr[RP_SITES];
 };
 
-// one collapsed step of the slow path: acc + c * d(w) when that is what c rounded additions give
+// one collapsed step of the slow path: acc + c * d(w) when that is what c rounded additions give.  A negative w (a wrapped
+// raw-count product) compares as a huge unsigned high word and takes the plain additions of add_repeated.
 __device__ __forceinline__ double replay_row(double acc, double w, int c)
 {
   const int E = __double2hiint(acc) >> 20;
@@ -901,7 +904,7 @@ __device__ __forceinline__ double replay_row(double acc, double w, int c)
   const double err = __dsub_rn(w, d);
   const double t = __fma_rn((double)c, d, acc);
   const bool ok = (E > 54) & (E < 0x7fe) & (fabs(err) != __hiloint2double((E - 53) << 20, 0)) &
-                  (__double2hiint(w) < ((E - 1) << 20)) & ((__double2hiint(t) >> 20) == E);
+                  ((uint32_t)__double2hiint(w) < (uint32_t)((E - 1) << 20)) & ((__double2hiint(t) >> 20) == E);
   return ok ? t : exsum::add_repeated(acc, w, c);
 }
 
@@ -927,8 +930,10 @@ __device__ __forceinline__ uint32_t rp_byte_mask(uint32_t m) { return (((m & 0xf
 // 3 bin-warps (48 bins, four CTAs per block and histogram) beat 6 / 12 bin-warps (0.54 / 0.61): the warps of a
 // CTA share the count-tile ring and move at the pace of the slowest.  A run that
 // leaves the binade, meets a rounding tie or a weight too large for the shortcut is redone row by
-// row (replay_row / exact_sum.cuh) by all RP_Q lanes of the bin alike, over the rows with a count.
-// blockIdx.y: 2 * group + (0 shared, 1 not shared).  hdr.z carries -0.0 for rows that add nothing to shared.
+// row (replay_row / exact_sum.cuh) by all RP_Q lanes of the bin alike, over the rows with a count.  The collapse assumes
+// moves that never go down; a negative weight (the raw count weights of the bcf / bam front-ends wrap past 2^31 in the
+// reference's int product) counts as too large, and its run is redone row by row.
+// blockIdx.y: 2 * group + (0 shared, 1 not shared).  Rows with hdr.y = age_begin <= 0 add nothing to shared.
 template <int WHICH>
 __device__ __forceinline__ void replay_body(int group, ReplayStage* st, uint64_t* full, uint64_t* empty,
                                             const int64_t* __restrict__ blk_rank_start, const uint8_t* __restrict__ cnt,
@@ -986,8 +991,8 @@ __device__ __forceinline__ void replay_body(int group, ReplayStage* st, uint64_t
     uint32_t live = (hi >= 32 ? 0xffffffffu : (1u << hi) - 1u) & ~((1u << lo) - 1u);
     const uint32_t* cwp = (const uint32_t*)&st[slot].cnt[cslot][0];   // this bin's counts in the tile's 32 rows, 4 rows per word
     const double* hp = (const double*)&st[slot].hdr[0] + 2 + WHICH;
-    // ... and add to this histogram (-0.0 weight: nothing to add), one bit per row
-    if (WHICH == 0) live &= __ballot_sync(0xffffffffu, ((const int*)(hp + 4 * lane))[1] >= 0);
+    // ... and add to this histogram (shared: rows with age_begin > 0), one bit per row
+    if (WHICH == 0) live &= __ballot_sync(0xffffffffu, st[slot].hdr[lane].y > 0.0);
 #pragma unroll
     for (int run = 0; run < RP_SITES / RP_ROWS; run++) {
       const int g0 = run * RP_ROWS;
@@ -1011,10 +1016,10 @@ __device__ __forceinline__ void replay_body(int group, ReplayStage* st, uint64_t
       if (anyb == 0) continue;
 #endif
       const bool any = ((anyb >> gsh) & GMASK) != 0;                   // some row of the run counts for this bin
-      const int E = __double2hiint(acc) >> 20;                         // biased exponent (acc >= 0)
+      const int E = __double2hiint(acc) >> 20;                         // biased exponent (acc < 0: E < 0, row by row)
       const double M = __hiloint2double((E << 20) | 0x80000, 0);       // 1.5 * 2^E: ulp(M) == ulp(acc)
       const int hu_hi = (E - 53) << 20;                                // high word of ulp(acc) / 2 (the low word is 0)
-      const int wmax_hi = (E - 1) << 20;                               // w must stay below 2^(E-1)
+      const uint32_t wmax_hi = (uint32_t)((E - 1) << 20);              // w must stay below 2^(E-1) and not be negative
       bool badl = (E <= 54) | (E >= 0x7fe);
       constexpr int NTS = RP_RPL >= 8 ? 4 : 2;
       double ts[4] = {0.0, 0.0, 0.0, 0.0};                             // exact sums: any order
@@ -1028,12 +1033,12 @@ __device__ __forceinline__ void replay_body(int group, ReplayStage* st, uint64_t
         const double d = __dsub_rn(__dadd_rn(w, M), M);
         const double err = __dsub_rn(w, d);
         // |err| <= ulp / 2, and ulp / 2 itself is the only such value with its exponent field: a tie shows in the exponent alone
-        badl |= (c != 0) & ((((__double2hiint(err) ^ hu_hi) & 0x7ff00000) == 0) | (__double2hiint(w) >= wmax_hi));
+        badl |= (c != 0) & ((((__double2hiint(err) ^ hu_hi) & 0x7ff00000) == 0) | ((uint32_t)__double2hiint(w) >= wmax_hi));
         // (double)c without the quarter-rate I2F.F64: 2^52 + c is a register pair, one DADD takes the 2^52 off
         ts[i & (NTS - 1)] = __fma_rn(__dsub_rn(__hiloint2double(0x43300000, c), 0x1p52), d, ts[i & (NTS - 1)]);
 #ifdef REPLAY_PROF
         pf_c_tie |= (c != 0) & (((__double2hiint(err) ^ hu_hi) & 0x7ff00000) == 0);
-        pf_c_big |= (c != 0) & (__double2hiint(w) >= wmax_hi);
+        pf_c_big |= (c != 0) & ((uint32_t)__double2hiint(w) >= wmax_hi);
 #endif
       }
       double t = NTS == 4 ? __dadd_rn(__dadd_rn(ts[0], ts[1]), __dadd_rn(ts[2], ts[3])) : __dadd_rn(ts[0], ts[1]);
@@ -1084,7 +1089,7 @@ __device__ __forceinline__ void replay_body(int group, ReplayStage* st, uint64_t
             nzr &= nzr - 1;
             const double w = hp[4 * r];
             const int c = st[slot].cnt[cslot][r];
-            if ((__double_as_longlong(w) << 1) != 0 && __double2hiint(w) >= 0) {   // x + 0.0 == x
+            if ((__double_as_longlong(w) << 1) != 0) {   // x + (+-0.0) == x (acc is never -0.0)
               // a handful of samples (the usual case: 100 samples of a row spread over its bins): the reference's own additions
               if (c <= 4) { for (int j = 0; j < c; j++) acc = __dadd_rn(acc, w); }
               else acc = replay_row(acc, w, c);
@@ -1181,6 +1186,21 @@ k_emp(const int64_t* __restrict__ blk_rank_start, const uint8_t* __restrict__ e_
 
 // ------------------------------------------------------------------------------------------
 static inline int grid_for(int64_t n, int threads) { return (int)((n + threads - 1) / threads); }
+
+// The two launches of the exact histograms, shared by stage i (run_compact / run_replay) and the test hook
+// colate_test_replay: n_blocks genomic blocks, rows [blk_rank_start[b], blk_rank_start[b + 1]) of block b.
+// k_replay: count tiles [tile][slot][row % 32] and double4 headers of whole tiles -> out_f[b][0..1], out_n[b][0..1], misc[3]
+static void launch_replay(cudaStream_t s, int n_blocks, const int64_t* blk_rank_start, const uint8_t* cnt_tiles, const double4* hdr,
+                          double* out_f, int64_t* out_n, int64_t* misc)
+{
+  k_replay<<<dim3(n_blocks, 2 * RP_GROUPS), RP_THREADS, 0, s>>>(blk_rank_start, cnt_tiles, hdr, out_f, out_n, misc);
+}
+// k_emp: the rows' single emp contributions (bin 255: none) -> out_f[b][2..3], out_n[b][2]
+static void launch_emp(cudaStream_t s, int n_blocks, const int64_t* blk_rank_start, const uint8_t* e_b2, const double* e_ws,
+                       const double* e_wn, double* out_f, int64_t* out_n)
+{
+  k_emp<<<n_blocks, 32, 0, s>>>(blk_rank_start, e_b2, e_ws, e_wn, out_f, out_n);
+}
 
 int run_join(colate_handle* h, int slot)
 {
@@ -1320,8 +1340,8 @@ int run_compact(colate_handle* h)
   if (h->n_blocks_local > 0) {
     // the emp histograms need nothing but the compacted rows: on the side stream, under the sampler; run_replay joins it
     CK(cudaStreamWaitEvent(h->side_stream, h->ev[3], 0));
-    k_emp<<<h->n_blocks_local, 32, 0, h->side_stream>>>(h->blk_rank_start.as<int64_t>(), h->u_eb2.as<uint8_t>(), h->u_ews.as<double>(),
-                                                        h->u_ewn.as<double>(), h->out_f.as<double>(), h->out_n.as<int64_t>());
+    launch_emp(h->side_stream, h->n_blocks_local, h->blk_rank_start.as<int64_t>(), h->u_eb2.as<uint8_t>(), h->u_ews.as<double>(),
+               h->u_ewn.as<double>(), h->out_f.as<double>(), h->out_n.as<int64_t>());
     h->launches += 1;
     CK(cudaEventRecord(h->side_done, h->side_stream));
   }
@@ -1383,8 +1403,8 @@ int run_replay(colate_handle* h)
   const int nb = h->n_blocks_local;
   CK(cudaEventRecord(h->ev[4], s));
   if (nb > 0) {
-    k_replay<<<dim3(nb, 2 * RP_GROUPS), RP_THREADS, 0, s>>>(h->blk_rank_start.as<int64_t>(), h->u_cnt.as<uint8_t>(), h->u_hdr.as<double4>(),
-                                                h->out_f.as<double>(), h->out_n.as<int64_t>(), h->misc.as<int64_t>());
+    launch_replay(s, nb, h->blk_rank_start.as<int64_t>(), h->u_cnt.as<uint8_t>(), h->u_hdr.as<double4>(), h->out_f.as<double>(),
+                  h->out_n.as<int64_t>(), h->misc.as<int64_t>());
     h->launches += 1;
     CK(cudaStreamWaitEvent(s, h->side_done, 0));   // k_emp's slices of out_f / out_n (run_compact launched it on the side stream)
   }
@@ -1451,6 +1471,81 @@ int run_test_bin_sweep(colate_handle* h, uint32_t lo_bits, uint32_t hi_bits, uin
   CK(cudaMemcpyAsync(out3_host, h->d_scratch.p, 24, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
   CK(cudaGetLastError());
+  return 0;
+}
+
+// test hooks of the exact replay: k_replay and k_emp on given rows through the launches stage i uses, and the device's
+// replay_row / exsum::add_repeated element by element
+__global__ void k_test_replay_row(int which, int n, const double* __restrict__ acc, const double* __restrict__ w, const int32_t* __restrict__ c,
+                                  double* __restrict__ out)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = which == 0 ? replay_row(acc[i], w[i], c[i]) : exsum::add_repeated(acc[i], w[i], c[i]);
+}
+
+int run_test_replay_row(colate_handle* h, int which, int n, const double* acc, const double* w, const int32_t* c, double* out)
+{
+  cudaStream_t s = h->stream;
+  CK(h->d_scratch.ensure((size_t)n * 28 + 64));
+  double* d_acc = h->d_scratch.as<double>();
+  double* d_w = d_acc + n;
+  double* d_out = d_w + n;
+  int32_t* d_c = (int32_t*)(d_out + n);
+  CK(cudaMemcpyAsync(d_acc, acc, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(d_w, w, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(d_c, c, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+  k_test_replay_row<<<grid_for(n, 256), 256, 0, s>>>(which, n, d_acc, d_w, d_c, d_out);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out, d_out, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// The rows are laid out as k_compact and k_sample leave them: count tiles [tile][slot][row % 32], double4 headers
+// {0, age_begin, w_shared, w_notshared}, the rows of the last tile past n_rows zeroed.
+int run_test_replay(colate_handle* h, int n_blocks, const int64_t* blk_rank_start, int64_t n_rows, const uint8_t* counts,
+                    const double* age_begin, const double* w_shared, const double* w_notshared, const uint8_t* emp_bin,
+                    const double* emp_ws, const double* emp_wn, double* out_f, int64_t* out_n, int* out_of_range)
+{
+  cudaStream_t s = h->stream;
+  const int64_t n_tiles = std::max<int64_t>((n_rows + TS_ROWS - 1) / TS_ROWS, 1), n32 = n_tiles * TS_ROWS;
+  std::vector<uint8_t> tiles((size_t)n_tiles * TILE_BYTES, 0);
+  std::vector<double4> hdr((size_t)n32, make_double4(0.0, 0.0, 0.0, 0.0));
+  for (int64_t r = 0; r < n_rows; r++) {
+    for (int slot = 0; slot < ROW_BYTES; slot++)
+      tiles[(size_t)(r / TS_ROWS) * TILE_BYTES + slot * TS_ROWS + r % TS_ROWS] = counts[(size_t)r * ROW_BYTES + slot];
+    hdr[(size_t)r] = make_double4(0.0, age_begin[r], w_shared[r], w_notshared[r]);
+  }
+  const size_t off_cnt = 0, off_hdr = off_cnt + tiles.size(), off_brs = off_hdr + hdr.size() * sizeof(double4),
+               off_eb = off_brs + (size_t)(n_blocks + 1) * 8, off_ews = (off_eb + (size_t)n32 + 7) / 8 * 8, off_ewn = off_ews + (size_t)n32 * 8,
+               off_f = off_ewn + (size_t)n32 * 8, off_n = off_f + (size_t)n_blocks * 4 * NBINS * 8, off_misc = off_n + (size_t)n_blocks * 3 * NBINS * 8,
+               total = off_misc + 64;
+  CK(h->d_tmp.ensure(total));
+  char* d = h->d_tmp.as<char>();
+  CK(cudaMemsetAsync(d, 0, total, s));
+  CK(cudaMemcpyAsync(d + off_cnt, tiles.data(), tiles.size(), cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(d + off_hdr, hdr.data(), hdr.size() * sizeof(double4), cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(d + off_brs, blk_rank_start, (size_t)(n_blocks + 1) * 8, cudaMemcpyHostToDevice, s));
+  if (n_rows > 0) {
+    CK(cudaMemcpyAsync(d + off_eb, emp_bin, (size_t)n_rows, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + off_ews, emp_ws, (size_t)n_rows * 8, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(d + off_ewn, emp_wn, (size_t)n_rows * 8, cudaMemcpyHostToDevice, s));
+  }
+  const int64_t* brs = (const int64_t*)(d + off_brs);
+  double* f = (double*)(d + off_f);
+  int64_t* nn = (int64_t*)(d + off_n);
+  int64_t* misc = (int64_t*)(d + off_misc);
+  if (n_blocks > 0) {
+    launch_emp(s, n_blocks, brs, (const uint8_t*)(d + off_eb), (const double*)(d + off_ews), (const double*)(d + off_ewn), f, nn);
+    launch_replay(s, n_blocks, brs, (const uint8_t*)(d + off_cnt), (const double4*)(d + off_hdr), f, nn, misc);
+    CK(cudaGetLastError());
+  }
+  int64_t m[8];
+  CK(cudaMemcpyAsync(out_f, f, (size_t)n_blocks * 4 * NBINS * 8, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(out_n, nn, (size_t)n_blocks * 3 * NBINS * 8, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(m, misc, 64, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  *out_of_range = m[3] != 0;
   return 0;
 }
 
