@@ -122,6 +122,11 @@ SIGNATURES = {
     "colate_maketmp_write_bcf_genome": (C.c_int64, [VP, C.c_int, C.POINTER(C.c_char_p), C.c_char_p, VP, C.c_int64, C.c_char_p]),
     "colate_last_maketmp_timing": (C.c_int, [VP, f64]),
     "colate_upload_counts": (C.c_int, [VP, i64]),
+    "colate_geno_scan": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.POINTER(C.c_char_p), VP, VP, VP, VP]),
+    "colate_maketmp_write_geno": (C.c_int64, [VP, C.c_char_p, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.c_int, C.POINTER(C.c_char_p),
+                                              C.POINTER(C.c_char_p), VP, VP, VP, VP, VP]),
+    "colate_last_geno_timing": (C.c_int, [VP, f64]),
+    "colate_geno_upload_counts": (C.c_int, [VP, i64]),
     "colate_write_colate_mat": (C.c_int, [C.c_char_p, C.c_int, f64, f64]),
     "colate_write_coal": (C.c_int, [C.c_char_p, C.c_int, C.c_int, f64, f64, C.c_int, C.c_int]),
     "colate_write_bin": (C.c_int, [C.c_char_p, C.c_int, C.c_int, f64, f64, i32]),

@@ -172,6 +172,24 @@ def vcf_scan(path: str, window_bytes: int = 0) -> dict:
     return out
 
 
+_GENO_FORMATS = {"eigenstrat": 0, "plink": 1}
+_GENO_KINDS = ("packed", "text", "bed")
+
+
+def _cstrs(xs):
+    return (C.c_char_p * len(xs))(*[str(x).encode() for x in xs])
+
+
+def geno_scan(prefix: str, fmt: str, chr_names) -> dict:
+    """Host-only scan of a genotype matrix (no GPU, colate_geno_scan): fmt "eigenstrat" (<prefix>.geno / .snp / .ind) or "plink"
+    (<prefix>.bed / .bim / .fam); the SNP and individual counts, the SNPs of each --chr entry (contig c, chr<c>, 23 for X, 24 for
+    Y) and the matrix kind ("packed", "text" or "bed").  Raises ColateError for every file colate_maketmp_write_geno refuses."""
+    n = len(chr_names)
+    ns = np.zeros(1, np.int64); ni = np.zeros(1, np.int64); per = np.zeros(n, np.int64); kind = np.zeros(1, np.int32)
+    check(lib().colate_geno_scan(str(prefix).encode(), _GENO_FORMATS[fmt], n, _cstrs(chr_names), ptr(ns), ptr(ni), ptr(per), ptr(kind)))
+    return {"n_snp": int(ns[0]), "n_ind": int(ni[0]), "entry_snps": per, "kind": _GENO_KINDS[int(kind[0])]}
+
+
 def read_fasta(path: str) -> np.ndarray:
     """fasta::Read (data.cpp:213-237): header line dropped, upper-cased, concatenated; <path> or <path>.gz."""
     p = C.POINTER(C.c_uint8)()
@@ -361,6 +379,30 @@ class Handle:
         c = np.zeros(4, np.int64)
         check(lib().colate_upload_counts(self._h, c))
         return dict(zip(("mut_texts_parsed", "mut_rows_parsed", "ref_uploads", "ref_h2d_bytes"), c.tolist()))
+
+    def maketmp_write_geno(self, prefix, fmt, ind_ids, chr_names, out_files, mask_ids=None, mask_bits=None) -> dict:
+        """The .colate.in of many individuals of one genotype matrix written on the device (colate_maketmp_write_geno): fmt "eigenstrat"
+        (<prefix>.geno / .snp / .ind) or "plink" (<prefix>.bed / .bim / .fam); mask_ids[i] = -1 or a row of mask_bits
+        ([n_mask, (n_site + 31) / 32] make_tmp pass bits).  Returns per individual the records written (-1: its file could not be
+        written), the heterozygous calls skipped and the cut-off entry, and the number of failed files."""
+        n = len(ind_ids)
+        rec = np.zeros(n, np.int64); het = np.zeros(n, np.int64); cut = np.zeros(n, np.int32)
+        mid = None if mask_ids is None else np.ascontiguousarray(mask_ids, dtype=np.int32)
+        mb = None if mask_bits is None else np.ascontiguousarray(mask_bits, dtype=np.uint32)
+        failed = check(lib().colate_maketmp_write_geno(self._h, str(prefix).encode(), _GENO_FORMATS[fmt], n, _cstrs(ind_ids), len(chr_names),
+                                                       _cstrs(chr_names), _cstrs(out_files), ptr(mid), ptr(mb), ptr(rec), ptr(het), ptr(cut)))
+        return {"records": rec, "het_skipped": het, "cutoff": cut, "failed": int(failed)}
+
+    def last_geno_timing(self) -> dict:
+        t = np.zeros(10)
+        check(lib().colate_last_geno_timing(self._h, t))
+        keys = ("scan_s", "upload_s", "join_ms", "called_ms", "rows_ms", "scatter_ms", "d2h_s", "write_s", "total_s", "bytes")
+        return dict(zip(keys, t.tolist()))
+
+    def geno_upload_counts(self) -> dict:
+        c = np.zeros(2, np.int64)
+        check(lib().colate_geno_upload_counts(self._h, c))
+        return {"matrix_uploads": int(c[0]), "matrix_h2d_bytes": int(c[1])}
 
     def last_bam_timing(self) -> dict:
         """Phases of the last pileup_from_bam (colate_last_bam_timing; copy / decode / pileup need set_option("bam_timing", 1))."""

@@ -153,7 +153,9 @@ void colate_destroy(colate_handle* h)
                     &h->windows, &h->rng_stream, &h->mt_tail, &h->poly, &h->thr10, &h->d_counts, &h->d_blockstats, &h->d_weights, &h->d_epochs,
                     &h->d_rates, &h->d_iters, &h->d_ll, &h->d_agebin, &h->d_tmp, &h->d_em_scratch, &h->d_gr_tab, &h->d_gr_rates, &h->order_flag, &h->ing_raw, &h->deep_rows, &h->tile_start, &h->tile_rlo, &h->bam_buf, &h->bam_ref, &h->bam_state,
                     &h->bcf_buf, &h->bcf_cols, &h->bcf_ref, &h->bcf_state, &h->mkt, &h->refg, &h->mk_ad, &h->mk_emit, &h->mk_blk, &h->mk_acc,
-                    &h->mk_name, &h->mk_out, &h->mk_mask};
+                    &h->mk_name, &h->mk_out, &h->mk_mask, &h->gn_mat, &h->gn_snp_pos, &h->gn_allele, &h->gn_entry_off, &h->gn_site_off,
+                    &h->gn_join, &h->gn_called, &h->gn_col, &h->gn_cut, &h->gn_mask_of, &h->gn_masks, &h->gn_name, &h->gn_ad, &h->gn_emit,
+                    &h->gn_blk, &h->gn_blk_off, &h->gn_acc, &h->gn_out};
   for (DevBuf* b : bufs) b->release();
   for (auto& g : h->genomes) {
     DevBuf* gb[] = {&g.bp, &g.aaf, &g.daf, &g.alleles, &g.chr_first, &g.chr_end, &g.mask_bits, &g.j_aaf, &g.j_daf, &g.j_prevbp, &g.j_flag, &g.pile};

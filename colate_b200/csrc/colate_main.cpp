@@ -40,7 +40,7 @@ const char* kValueOpts[] = {"mode", "anc", "mut", "target_bcf", "reference_bcf",
                             "anc_genome", "mask", "mask_cutoff", "chr", "bins", "lineage_bin", "outgroup_tmrca", "years_per_gen",
                             "coal", "seed", "num_bootstraps", "filters", "groups", "poplabels", "map", "input", "output",
                             // additions of this build
-                            "num_bootstrap", "device", "devices", "pairs", "targets"};
+                            "num_bootstrap", "device", "devices", "pairs", "targets", "target_geno", "target_bed", "individuals"};
 
 void help()
 {
@@ -81,6 +81,15 @@ void help()
                "      (target_bam=<t.bam> | target_bcf=<prefix>) <output_prefix> [target_mask=<prefix>]\n"
                "    with the shared flags; each line's <output_prefix>.colate.in equals that of the single-target run (target_bcf needs --chr;\n"
                "    a failing line writes no file, the others complete, the exit status is 1)\n"
+               "  Colate --mode make_tmp --mut <prefix> --ref_genome <prefix> --chr <file> (--target_geno <prefix> | --target_bed <prefix>)\n"
+               "         --individuals <file> [--device <int>]\n"
+               "    many individuals of one genotype matrix in one job: EIGENSTRAT <prefix>.geno (packed or text) / .snp / .ind, or SNP-major\n"
+               "    PLINK <prefix>.bed / .bim / .fam; --chr entry c reads the SNPs of contig c or chr<c> (23 for X, 24 for Y).  Every non-blank\n"
+               "    line of <file> not starting with '#' is <ID> <output_prefix> [target_mask=<prefix>] (ID: .ind column 1 or .fam IID).\n"
+               "    Each <output_prefix>.colate.in equals the --target_table run on the table of that individual's homozygous calls; heterozygous\n"
+               "    calls are skipped and counted (a haploid table cannot hold them: give diploid individuals as BCF / VCF).  An individual\n"
+               "    without a homozygous call on some --chr entry writes nothing on that entry and every later one, as the table run does\n"
+               "    (a warning names them).  A failing line writes no file, the others complete, the exit status is 1.\n"
             << std::endl;
 }
 
@@ -1561,9 +1570,240 @@ int run_make_tmp_batch(const Options& options)
   return n_failed ? 1 : 0;
 }
 
+// ---- --target_geno / --target_bed: make_tmp for many individuals of one genotype matrix ----------------------------------------
+// Every line is the run `Colate --mode make_tmp --target_table T [--target_mask M] -o OUT` with the shared flags, where T lists the
+// individual's homozygous calls per --chr entry; its OUT.colate.in is that run's, byte for byte (DESIGN.md section 6l).  The .mut text
+// is parsed once, the matrix uploaded once, every distinct mask becomes per-row bits once; colate_maketmp_write_geno writes the files.
+struct IndLine {
+  int line = 0;
+  std::string id, out, mask;
+  int mask_id = -1;
+};
+
+// The individuals file, checked completely before any device is touched.  false: the message (naming the line) is on stderr.
+bool read_individuals_file(const std::string& path, const std::string& f_ind, const std::vector<std::string>& ids, const std::vector<std::string>& name_chr,
+                           std::vector<IndLine>& il)
+{
+  std::ifstream is(path);
+  if (is.fail()) { std::cerr << "Error: cannot open the individuals file " << path << std::endl; return false; }
+  std::map<std::string, int> n_id, out_line;
+  for (auto& x : ids) n_id[x]++;
+  std::string text;
+  int ln = 0;
+  auto bad = [&](const std::string& what) { std::cerr << "Error in individuals file " << path << ", line " << ln << ": " << what << std::endl; return false; };
+  while (std::getline(is, text)) {
+    ln++;
+    std::stringstream ss(text);
+    std::vector<std::string> f;
+    std::string tok;
+    while (ss >> tok) f.push_back(tok);
+    if (f.empty() || f[0][0] == '#') continue;
+    if (f.size() < 2 || f.size() > 3) return bad("expected <ID> <output_prefix> [target_mask=<prefix>], found " + std::to_string(f.size()) + " field(s)");
+    IndLine t;
+    t.line = ln;
+    t.id = f[0];
+    t.out = f[1];
+    if (t.id.find('=') != std::string::npos || t.out.find('=') != std::string::npos) return bad("expected <ID> <output_prefix> before any key=value");
+    if (f.size() == 3) {
+      const size_t eq = f[2].find('=');
+      if (eq == std::string::npos || eq == 0 || eq + 1 == f[2].size()) return bad("'" + f[2] + "' is not of the form key=value");
+      const std::string key = f[2].substr(0, eq);
+      if (key != "target_mask") return bad("unknown key '" + key + "' (known: target_mask)");
+      t.mask = f[2].substr(eq + 1);
+      for (auto& nm : name_chr) {
+        const std::string fm = t.mask + "_chr" + nm + ".fa";
+        if (!file_exists(fm) && !file_exists(fm + ".gz")) return bad("cannot read the mask " + fm);
+      }
+    }
+    auto k = n_id.find(t.id);
+    if (k == n_id.end()) return bad("individual " + t.id + " is not in " + f_ind);
+    if (k->second > 1) return bad("individual " + t.id + " occurs " + std::to_string(k->second) + " times in " + f_ind);
+    auto dup = out_line.find(t.out);
+    if (dup != out_line.end()) return bad("output prefix " + t.out + " is already used on line " + std::to_string(dup->second));
+    out_line[t.out] = ln;
+    il.push_back(t);
+  }
+  if (il.empty()) { std::cerr << "Error: the individuals file " << path << " lists no individual" << std::endl; return false; }
+  return true;
+}
+
+int run_make_tmp_geno(const Options& options)
+{
+  auto bad = [](const std::string& what) { std::cerr << "Error: " << what << std::endl; return 1; };
+  if (options.count("target_geno") && options.count("target_bed")) return bad("give one of --target_geno and --target_bed");
+  const bool eig = options.count("target_geno");
+  const std::string flag = eig ? "--target_geno" : "--target_bed";
+  if (!eig && !options.count("target_bed")) return bad("--individuals needs --target_geno or --target_bed");
+  for (const char* k : {"targets", "target_bam", "target_bcf", "target_table", "target_tmp", "target_mask", "output"})
+    if (options.count(k))
+      return bad(std::string("--") + (strcmp(k, "output") ? k : "output/-o") + " cannot be combined with " + flag + " (outputs and masks go per line of --individuals)");
+  if (options.count("strandfilter")) return bad("--strandfilter does not apply to genotype matrices");
+  if (options.count("filters")) return bad("--filters does not apply to genotype matrices");
+  const std::string dev = options.count("devices") ? options.get("devices") : "";
+  if (dev.find(',') != std::string::npos) return bad(flag + " runs on one device (--device <i>)");
+  if (!options.count("individuals")) return bad(flag + " needs --individuals");
+  if (!options.count("mut")) return bad(flag + " needs --mut");
+  if (!options.count("ref_genome")) return bad(flag + " needs --ref_genome");
+  if (!options.count("chr")) return bad(flag + " needs --chr (the contigs of the matrix to write)");
+  std::vector<std::string> name_chr, f_mut;
+  {
+    std::ifstream is(options.get("chr"));
+    if (is.fail()) return bad("cannot open " + options.get("chr"));
+    std::string line;
+    while (std::getline(is, line)) { name_chr.push_back(line); f_mut.push_back(options.get("mut") + "_chr" + line + ".mut"); }
+    if (name_chr.empty()) return bad("empty --chr list");
+    if ((int)std::set<std::string>(name_chr.begin(), name_chr.end()).size() != (int)name_chr.size()) return bad("duplicate chromosome names in --chr");
+  }
+  const int n_chr = (int)name_chr.size();
+  for (auto& nm : name_chr) {   // as the --target_table run: only the presence of the genome files matters
+    const std::string f = options.get("ref_genome") + "_chr" + nm + ".fa";
+    if (!file_exists(f) && !file_exists(f + ".gz")) return bad("cannot read " + f);
+  }
+  std::vector<const char*> names;
+  for (auto& s : name_chr) names.push_back(s.c_str());
+  const std::string prefix = options.get(eig ? "target_geno" : "target_bed");
+  const int format = eig ? COLATE_GENO_EIGENSTRAT : COLATE_GENO_PLINK;
+  int64_t n_snp = 0, n_ind = 0;
+  std::vector<int64_t> entry_snps(n_chr);
+  int32_t kind = 0;
+  if (colate_geno_scan(prefix.c_str(), format, n_chr, names.data(), &n_snp, &n_ind, entry_snps.data(), &kind)) return bad(colate_last_error());
+  // the IDs (colate_geno_scan has checked every line's field count)
+  const std::string f_ind = prefix + (eig ? ".ind" : ".fam");
+  std::vector<std::string> ids;
+  {
+    std::ifstream is(f_ind);
+    std::string line;
+    while (std::getline(is, line)) {
+      std::stringstream ss(line);
+      std::string a, b;
+      if (!(ss >> a)) continue;
+      ids.push_back(eig ? a : (ss >> b, b));
+    }
+  }
+  std::vector<IndLine> il;
+  if (!read_individuals_file(options.get("individuals"), f_ind, ids, name_chr, il)) return 1;
+  std::vector<std::string> masks;   // distinct target_mask prefixes
+  {
+    std::map<std::string, int> mid;
+    for (auto& t : il) {
+      if (t.mask.empty()) continue;
+      auto it = mid.find(t.mask);
+      if (it == mid.end()) { it = mid.emplace(t.mask, (int)masks.size()).first; masks.push_back(t.mask); }
+      t.mask_id = it->second;
+    }
+  }
+  Phases ph;
+  std::cerr << "---------------------------------------------------------" << std::endl;
+  std::cerr << "Calculating Colate tmp input files for " << il.size() << " individuals of " << prefix << " (" << n_snp << " SNPs, "
+            << n_ind << " individuals).." << std::endl;
+
+  // the .mut text, read once: parsed on the GPU, or by the host reader (zlib) if a file only exists as .gz
+  std::vector<std::vector<char>> texts(n_chr);
+  bool all_plain = !options.count("host_parse");
+  for (int c = 0; c < n_chr && all_plain; c++) {
+    std::ifstream f(f_mut[c], std::ios::binary);
+    if (!f) { all_plain = false; break; }
+    texts[c].assign(std::istreambuf_iterator<char>(f), std::istreambuf_iterator<char>());
+  }
+  colate_handle* h = nullptr;
+  if (colate_create(options.count("device") ? atoi(options.get("device").c_str()) : 0, &h)) return die("colate_create");
+  struct Destroy { colate_handle* h; ~Destroy() { colate_destroy(h); } } destroy{h};
+  std::vector<int64_t> site_off(n_chr + 1, 0);
+  std::vector<int32_t> pos;
+  if (all_plain) {
+    int64_t bytes = 0;
+    for (auto& t : texts) bytes += (int64_t)t.size();
+    if (colate_ingest_begin(h, n_chr, bytes / 20 + n_chr)) return die("colate_ingest_begin");
+    for (int c = 0; c < n_chr; c++) {
+      const int64_t n = colate_ingest_mut_text(h, texts[c].data(), (int64_t)texts[c].size(), 0);
+      if (n < 0) return die(f_mut[c]);
+      site_off[c + 1] = site_off[c] + n;
+    }
+    if (colate_ingest_end(h)) return die("colate_ingest_end");
+    texts.clear();
+    pos.resize((size_t)site_off[n_chr]);
+    if (colate_ingest_fetch(h, 0, site_off[n_chr], pos.data(), nullptr, nullptr, nullptr)) return die("colate_ingest_fetch");
+  } else {
+    std::vector<float> ab, ae;
+    std::vector<uint32_t> meta, words;
+    for (int c = 0; c < n_chr; c++) {
+      const int64_t n = colate_read_mut(f_mut[c].c_str(), 0, nullptr, nullptr, nullptr, nullptr);
+      if (n < 0) { std::cerr << colate_last_error() << std::endl; return 1; }
+      const size_t o = pos.size();
+      pos.resize(o + n); ab.resize(o + n); ae.resize(o + n); meta.resize(o + n); words.resize(o + n);
+      if (colate_read_mut(f_mut[c].c_str(), n, pos.data() + o, ab.data() + o, ae.data() + o, meta.data() + o) < 0 ||
+          colate_read_mut_words(f_mut[c].c_str(), n, words.data() + o) < 0) {
+        std::cerr << colate_last_error() << std::endl;
+        return 1;
+      }
+      site_off[c + 1] = (int64_t)pos.size();
+    }
+    if (colate_set_sites(h, n_chr, site_off.data(), pos.data(), ab.data(), ae.data(), meta.data(), 0)) return die("colate_set_sites");
+    if (colate_set_maketmp_words(h, words.data(), 0)) return die("colate_set_maketmp_words");
+  }
+  for (int c = 0; c < n_chr; c++)   // the table cursor walks forward only: positions must ascend per chromosome
+    for (int64_t m = site_off[c] + 1; m < site_off[c + 1]; m++)
+      if (pos[m] < pos[m - 1]) {
+        std::cerr << "Error: " << f_mut[c] << ": positions of a .mut file are not ascending (the reference's sequential reader needs sorted input)" << std::endl;
+        return 1;
+      }
+  ph.tick("parse .mut");
+  const size_t mask_words = (size_t)(site_off[n_chr] + 31) / 32;
+  std::vector<uint32_t> mask_bits(masks.size() * mask_words + 1, 0);
+  for (size_t k = 0; k < masks.size(); k++)
+    for (int c = 0; c < n_chr; c++) {
+      const std::string f = masks[k] + "_chr" + name_chr[c] + ".fa";
+      if (colate_maketmp_mask_bits(f.c_str(), site_off[c + 1] - site_off[c], pos.data() + site_off[c], site_off[c], mask_bits.data() + k * mask_words)) {
+        std::cerr << "Error: " << colate_last_error() << std::endl;
+        return 1;
+      }
+    }
+  ph.tick("masks");
+  const int n = (int)il.size();
+  std::vector<std::string> outs;
+  std::vector<const char*> id_p, out_p;
+  std::vector<int32_t> mask_ids;
+  for (auto& t : il) outs.push_back(t.out + ".colate.in");
+  for (int i = 0; i < n; i++) { id_p.push_back(il[i].id.c_str()); out_p.push_back(outs[i].c_str()); mask_ids.push_back(il[i].mask_id); }
+  std::vector<int64_t> records(n, -1), het(n, 0);
+  std::vector<int32_t> cut(n, n_chr);
+  const int64_t n_failed = colate_maketmp_write_geno(h, prefix.c_str(), format, n, id_p.data(), n_chr, names.data(), out_p.data(), mask_ids.data(),
+                                                     mask_bits.data(), records.data(), het.data(), cut.data());
+  if (n_failed < 0) return die("colate_maketmp_write_geno");
+  ph.tick("write the individuals");
+  if (ph.on) {
+    double t[10];
+    int64_t cnt[4], up[2];
+    colate_last_geno_timing(h, t);
+    colate_upload_counts(h, cnt);
+    colate_geno_upload_counts(h, up);
+    fprintf(stderr, "[timing] geno: scan %.3f s, upload %.3f s, join %.3f ms, called %.3f ms, rows %.3f ms, scatter %.3f ms, d2h %.3f s, write %.3f s, total %.3f s, %.0f bytes\n",
+            t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], t[8], t[9]);
+    fprintf(stderr, "[timing] .mut texts parsed %lld (%lld rows), matrix uploads %lld (%lld bytes)\n", (long long)cnt[0], (long long)cnt[1],
+            (long long)up[0], (long long)up[1]);
+  }
+  for (int i = 0; i < n; i++) {
+    const IndLine& t = il[i];
+    if (cut[i] < n_chr)
+      std::cerr << "Warning: individual " << t.id << " (line " << t.line << ") has no homozygous call on --chr entry " << name_chr[cut[i]]
+                << ": as in the --target_table run, that entry and every later one write nothing" << std::endl;
+    if (records[i] >= 0)
+      std::cerr << "individual on line " << t.line << " (" << t.id << " -> " << t.out << "): " << records[i] << " records written, " << het[i]
+                << " heterozygous calls skipped" << std::endl;
+    else {
+      remove(outs[i].c_str());
+      std::cerr << "individual on line " << t.line << " (" << t.id << " -> " << t.out << ") FAILED: cannot write " << outs[i] << std::endl;
+    }
+  }
+  if (n_failed) std::cerr << n_failed << " of " << n << " individuals failed" << std::endl;
+  std::cerr << "---------------------------------------------------------" << std::endl << std::endl;
+  return n_failed ? 1 : 0;
+}
+
 // --mode make_tmp with --target_table (make_tmp(), coal.cpp:2923-3069 -> maketmp_table, 2682-2808): host-only
 int run_make_tmp(const Options& options)
 {
+  if (options.count("target_geno") || options.count("target_bed") || options.count("individuals")) return run_make_tmp_geno(options);
   if (options.count("targets")) return run_make_tmp_batch(options);
   if (!options.count("mut") || !options.count("output")) {
     std::cout << "Not enough arguments supplied." << std::endl;

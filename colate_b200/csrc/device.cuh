@@ -181,6 +181,13 @@ struct colate_handle {
   double mk_timing[4] = {};
   // work counters of a job (colate_upload_counts)
   int64_t mut_texts_parsed = 0, mut_rows_parsed = 0, ref_uploads = 0, ref_h2d_bytes = 0;
+  // make_tmp from a genotype matrix (kernels_geno.cu): the listed SNPs' matrix rows, their positions / alleles / entry offsets, the
+  // per-row SNP ranges, per-individual columns / cut-offs / masks, the batch's per-row and record buffers, two pinned upload windows
+  colate::DevBuf gn_mat, gn_snp_pos, gn_allele, gn_entry_off, gn_site_off, gn_join, gn_called, gn_col, gn_cut, gn_mask_of, gn_masks, gn_name;
+  colate::DevBuf gn_ad, gn_emit, gn_blk, gn_blk_off, gn_acc, gn_out;
+  colate::Pinned gn_win[2];
+  double gn_timing[10] = {};
+  int64_t geno_uploads = 0, geno_h2d_bytes = 0;   // colate_geno_upload_counts
 };
 
 namespace colate {
@@ -192,6 +199,11 @@ struct GenomeRecs {
   std::vector<int32_t> n_hap;
 };
 int decode_genotype_genome(colate_handle* h, const char* path, int n_chr, const char* const* chr_names, int64_t chunk_bytes, double* t, GenomeRecs* gr);
+// kernels_maketmp.cu: k_maketmp_scan and k_maketmp_scatter of one chromosome's rows [row0, row0 + n_rows) on h->stream, after a rows
+// kernel of 256 threads per CTA left their (AAF, DAF), emit ballots and CTA counts; acc[0..2] carry the file's totals (DESIGN.md 6i).
+// The make_tmp row words name the records' letters.  Records of 18 + L bytes go to out.
+int maketmp_scan_scatter(colate_handle* h, int64_t row0, int64_t n_rows, const int32_t* blk_cnt, int64_t* blk_off, long long* acc, const int2* ad,
+                         const uint32_t* emit, const uint8_t* name, int L, uint8_t* out);
 // kernels_sites.cu
 int run_join(colate_handle* h, int slot);
 int run_flags(colate_handle* h, int tslot, int rslot);

@@ -176,6 +176,25 @@ k_maketmp_scatter(int64_t row0, int64_t n_rows, const int32_t* __restrict__ pos,
 
 inline int64_t blocks_for(int64_t n) { return (n + MK_THREADS - 1) / MK_THREADS; }
 
+}  // namespace
+
+// the scan and the scatter of one chromosome, after a rows kernel left ad / emit / blk_cnt for its rows [row0, row0 + n_rows)
+int colate::maketmp_scan_scatter(colate_handle* h, int64_t row0, int64_t n_rows, const int32_t* blk_cnt, int64_t* blk_off, long long* acc,
+                                 const int2* ad, const uint32_t* emit, const uint8_t* name, int L, uint8_t* out)
+{
+  const int64_t nb = blocks_for(n_rows);
+  const size_t smem = (size_t)MK_THREADS * (18 + L);
+  if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_maketmp_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_maketmp_scan<<<1, 1024, 0, h->stream>>>(blk_cnt, nb, blk_off, acc, 18 + L);
+  k_maketmp_scatter<<<(unsigned)nb, MK_THREADS, smem, h->stream>>>(row0, n_rows, h->pos.as<int32_t>(), h->mkt.as<uint32_t>(), ad, emit, blk_off, acc,
+                                                                    name, L, out);
+  h->launches += 2;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+namespace {
+
 // One writer call: the state every chromosome of it shares.
 struct Writer {
   colate_handle* h;
@@ -249,19 +268,15 @@ struct Writer {
     int32_t* blk_cnt = h->mk_blk.as<int32_t>();
     int64_t* blk_off = (int64_t*)(h->mk_blk.as<char>() + (((size_t)nb * 4 + 15) & ~(size_t)15));
     long long* acc = h->mk_acc.as<long long>();
-    const size_t smem = (size_t)MK_THREADS * (18 + L);
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_maketmp_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaEventRecord(ev[0], s));
     k_maketmp_rows<KIND><<<(unsigned)nb, MK_THREADS, 0, s>>>(r0, nr, h->pos.as<int32_t>(), h->mkt.as<uint32_t>(), d_mask, pile, cols, n_rec, N, ref,
                                                               ref_len, h->mk_ad.as<int2>(), h->mk_emit.as<uint32_t>(), blk_cnt,
                                                               (unsigned long long*)(acc + 3));
-    k_maketmp_scan<<<1, 1024, 0, s>>>(blk_cnt, nb, blk_off, acc, 18 + L);
-    k_maketmp_scatter<<<(unsigned)nb, MK_THREADS, smem, s>>>(r0, nr, h->pos.as<int32_t>(), h->mkt.as<uint32_t>(), h->mk_ad.as<int2>(),
-                                                              h->mk_emit.as<uint32_t>(), blk_off, acc, h->mk_name.as<uint8_t>() + name_off[c], L,
-                                                              h->mk_out.as<uint8_t>());
+    h->launches++;
+    if (int rc = maketmp_scan_scatter(h, r0, nr, blk_cnt, blk_off, acc, h->mk_ad.as<int2>(), h->mk_emit.as<uint32_t>(),
+                                      h->mk_name.as<uint8_t>() + name_off[c], L, h->mk_out.as<uint8_t>()))
+      return rc;
     CK(cudaEventRecord(ev[1], s));
-    h->launches += 3;
-    CK(cudaGetLastError());
     CK(cudaEventSynchronize(ev[1]));
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, ev[0], ev[1]));

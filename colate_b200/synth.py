@@ -668,3 +668,53 @@ def vcf_lines_np(pos0, a0, a1, alleles, phased=None, chrom=b"1") -> np.ndarray:
     keep = np.ones((n, cols), bool)
     keep[:, head.size:head.size + W] = buf[:, head.size:head.size + W] != 0
     return buf[keep]
+
+
+# ---- genotype matrices (DESIGN.md section 6l) ------------------------------------------------------------------------------------
+# calls[s, k] of SNP s and individual k: 0 homozygous for the SNP's first allele (.snp column 5, .bim A1), 1 homozygous for its second
+# (.snp column 6, .bim A2), 2 heterozygous, 3 missing.  snps: (id, chromosome, position, first allele, second allele) per SNP.
+def _pack2(codes: np.ndarray, shift_of_k) -> np.ndarray:
+    """[n_snp, n_ind] 2-bit values -> [n_snp, ceil(n_ind / 4)] bytes, individual k at bit shift_of_k(k % 4) of byte k // 4."""
+    n_snp, n_ind = codes.shape
+    pad = np.zeros((n_snp, (-n_ind) % 4), np.uint8)
+    v = np.concatenate([codes.astype(np.uint8), pad], axis=1).reshape(n_snp, -1, 4)
+    out = np.zeros(v.shape[:2], np.uint8)
+    for j in range(4):
+        out |= v[:, :, j] << shift_of_k(j)
+    return out
+
+
+def write_eigenstrat(prefix: str, snps, ids, calls: np.ndarray, packed: bool = True, pops=None):
+    """<prefix>.geno / .snp / .ind.  packed: EIGENSOFT's packedancestrymap (a "GENO nind nsnp hash hash" record, then one record of
+    max(48, ceil(nind / 4)) bytes per SNP, individual k in bits 7-2(k%4) .. 6-2(k%4) of byte k / 4, value = copies of column 5,
+    3 missing); otherwise text, one line of nind digits per SNP (9 missing).  The header hashes are written as 0."""
+    calls = np.asarray(calls, np.uint8)
+    n_snp, n_ind = calls.shape
+    copies = np.array([2, 0, 1, 3], np.uint8)[calls]
+    with open(prefix + ".snp", "w") as f:
+        f.write("".join(f"{i}\t{c}\t0.0\t{p}\t{a}\t{b}\n" for i, c, p, a, b in snps))
+    with open(prefix + ".ind", "w") as f:
+        f.write("".join(f"{x}\tU\t{pops[k] if pops else 'pop'}\n" for k, x in enumerate(ids)))
+    with open(prefix + ".geno", "wb") as f:
+        if packed:
+            rlen = max(48, (n_ind + 3) // 4)
+            f.write(f"GENO {n_ind} {n_snp} 0 0".encode().ljust(rlen, b"\0"))
+            rows = np.zeros((n_snp, rlen), np.uint8)
+            rows[:, :(n_ind + 3) // 4] = _pack2(copies, lambda j: 6 - 2 * j)
+            f.write(rows.tobytes())
+        else:
+            digits = np.where(copies == 3, ord("9"), ord("0") + copies).astype(np.uint8)
+            f.write(np.concatenate([digits, np.full((n_snp, 1), ord("\n"), np.uint8)], axis=1).tobytes())
+
+
+def write_plink(prefix: str, snps, ids, calls: np.ndarray):
+    """<prefix>.bed (SNP-major PLINK 1: magic 6c 1b 01, ceil(nind / 4) bytes per SNP, individual k in bits 2(k%4) .. 2(k%4)+1:
+    00 homozygous A1, 01 missing, 10 heterozygous, 11 homozygous A2), .bim and .fam."""
+    calls = np.asarray(calls, np.uint8)
+    with open(prefix + ".bim", "w") as f:
+        f.write("".join(f"{c}\t{i}\t0\t{p}\t{a}\t{b}\n" for i, c, p, a, b in snps))
+    with open(prefix + ".fam", "w") as f:
+        f.write("".join(f"fam{k}\t{x}\t0\t0\t0\t-9\n" for k, x in enumerate(ids)))
+    with open(prefix + ".bed", "wb") as f:
+        f.write(b"\x6c\x1b\x01")
+        f.write(_pack2(np.array([0, 3, 2, 1], np.uint8)[calls], lambda j: 2 * j).tobytes())

@@ -250,6 +250,37 @@ int colate_last_maketmp_timing(colate_handle* h, double* out4);
  * colate_set_ref_genome, [3] reference-genome bytes copied host-to-device (colate_set_ref_genome, colate_pileup_bam, colate_rows_from_bcf). */
 int colate_upload_counts(colate_handle* h, int64_t* out4);
 
+/* ---- make_tmp from a genotype matrix (DESIGN.md section 6l) ------------------------------------------------------------ */
+/* format: COLATE_GENO_EIGENSTRAT reads <prefix>.geno (packed "GENO" or text), .snp and .ind; COLATE_GENO_PLINK reads the SNP-major
+ * <prefix>.bed, .bim and .fam.  --chr entry c holds the SNPs whose contig is c or chr<c> (23 for X, 24 for Y), in file order. */
+#define COLATE_GENO_EIGENSTRAT 0
+#define COLATE_GENO_PLINK 1
+/* Host only (no GPU): the SNP and individual counts, the SNPs per --chr entry and the matrix kind (0 packed EIGENSTRAT, 1 text
+ * EIGENSTRAT, 2 PLINK .bed), with every host refusal of colate_maketmp_write_geno: COLATE_ERR_IO for an unreadable file, a line
+ * with too few fields, alleles missing from .snp / .bim, a position that is not an integer in [0, 2^31), a bad .bed magic, an
+ * individual-major .bed, a TGENO file, GENO header counts or a file size that disagree with the .snp / .ind (.bim / .fam) lines,
+ * a text call other than 0 1 2 9; COLATE_ERR_ORDER for SNP positions that descend within an entry.  Messages name file and line. */
+int colate_geno_scan(const char* prefix, int format, int n_chr, const char* const* chr_names, int64_t* n_snp, int64_t* n_ind,
+                     int64_t* entry_snps, int32_t* kind);
+/* The .colate.in of n_ind individuals (ind_ids: .ind column 1 / .fam IID, each present exactly once) written on the device into
+ * out_files[i], each byte for byte what colate_maketmp_table(chr_names, the .mut files, T_i, masks_i, has_ref_genome = 1, ...) writes
+ * for the table T_i of "c position allele" lines of the individual's homozygous calls, per --chr entry c in order (heterozygous and
+ * missing calls write no line).  The handle holds the ingested .mut rows of the same --chr list (ascending positions per chromosome,
+ * COLATE_ERR_ORDER otherwise).  mask_ids[i]: -1 or the index of the individual's make_tmp pass bits (colate_maketmp_mask_bits) in
+ * mask_bits, (n_site + 31) / 32 words per mask; mask_ids may be NULL.  The matrix is uploaded once per call.
+ * Optional outputs per individual: records_out (-1: its file could not be written, and is removed), het_skipped_out (heterozygous
+ * calls on the listed entries), cutoff_out (the first entry without a homozygous call: the table cursor then consumes the rest of
+ * the table, so that entry and every later one write nothing; n_chr if none).  Returns the number of files that could not be
+ * written (the others are complete), or < 0 for a failure of the whole call, which writes nothing. */
+int64_t colate_maketmp_write_geno(colate_handle* h, const char* prefix, int format, int n_ind, const char* const* ind_ids, int n_chr,
+                                  const char* const* chr_names, const char* const* out_files, const int32_t* mask_ids, const uint32_t* mask_bits,
+                                  int64_t* records_out, int64_t* het_skipped_out, int32_t* cutoff_out);
+/* The last colate_maketmp_write_geno: [0] host scan s, [1] matrix upload s, [2] k_geno_join ms, [3] k_geno_called ms, [4] k_geno_rows
+ * ms, [5] scans and scatters ms, [6] device-to-host copies s, [7] file writes s, [8] whole call s, [9] bytes written. */
+int colate_last_geno_timing(colate_handle* h, double* out10);
+/* Matrix uploads on this handle since creation: [0] uploads, [1] bytes copied host-to-device. */
+int colate_geno_upload_counts(colate_handle* h, int64_t* out2);
+
 /* P/N mask of genome `slot` evaluated at the site positions (fasta::Read,
  * include/src/data.cpp:213-237; test at coal.cpp:2169-2174): bit m of pass_bits = row m is
  * NOT rejected by the mask (positions at or beyond the mask end pass).  NULL clears it. */
